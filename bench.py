@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun)
     python bench.py --impl reference ...                     (the reference's torch-CPU path)
+    python bench.py ... --dump-outputs DIR                   (also save the last timed step's top-k lists)
 
 Headline workload (config.workload = "C4", BASELINE.json configs[3], the shape `metric` is quoted on):
 a 100 000 000 x 768 bf16 unit-norm synthetic gallery (153.6 GB -- fits ONE B200), 16 queries per step,
@@ -68,7 +69,37 @@ def parse():
     ap.add_argument("--no-fused", action="store_true", help="N > 1: NCCL all-gather variant instead of the fused NVLink gather")
     ap.add_argument("--c3-rows", type=int, default=C3_ROWS)
     ap.add_argument("--c5-queries", type=int, default=C5_QUERIES)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the top-k lists of the last timed step to DIR/*.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the timed search of --impl ours")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, values, indices):
+    """What the timed search returned in its last step, for comparing two builds output for output:
+    DIR/topk_values.npy (float32 [Q, k]) and DIR/topk_indices.npy (float64 [Q, k], global row ids, exact
+    below 2**53).  When the lists would exceed 64 MB, a fixed, seeded sample of query rows is written
+    instead, and DIR/query_rows.npy (float64) names the rows kept."""
+    import numpy as np
+    v = values.cpu().numpy().astype(np.float32)
+    i = indices.cpu().numpy().astype(np.float64)
+    arrays = {"topk_values": v, "topk_indices": i}
+    per_row = v.shape[1] * (v.itemsize + i.itemsize) + 8
+    if v.shape[0] * per_row > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 4096) // per_row          # 4096: room for the three .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(v.shape[0], size=keep, replace=False))
+        arrays = {"topk_values": v[rows], "topk_indices": i[rows], "query_rows": rows.astype(np.float64)}
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
 
 
 def measured_peaks():
@@ -666,6 +697,8 @@ def main():
     t_setup = time.perf_counter() - b.t_start
 
     head = b.measure(gal, sg, q_host, args.k, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:          # every rank holds the merged lists
+        dump_outputs(args.dump_outputs, *head["out"])
     gather_desc = None if sg is None else ("fused into the select kernels over NVLink peer memory" if sg.fused_active
                                            else "NCCL all_gather_into_tensor of packed keys + merge kernel")
     extra = {}

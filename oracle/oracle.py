@@ -217,7 +217,7 @@ def lab_process_images(image_features: torch.Tensor, text_features: dict, classe
     the image tower: per batch of `batch` images (lab3.py:73) normalise the rows
     (`feats / feats.norm(dim=1, keepdim=True)`), then class by class `feats @ text_features[cls].t()`;
     items whose label is "error" are skipped.  Same batching as the reference, so the fp32 CPU
-    results are bit-identical to the recorded golden."""
+    results are bit-identical to the recorded golden on the CPU it was recorded on."""
     out = {cls: [] for cls in classes}
     for lo in range(0, image_features.shape[0], batch):
         feats = image_features[lo:lo + batch].float()

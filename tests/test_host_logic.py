@@ -380,6 +380,40 @@ def test_bench_reference_arm_contract():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_rejects_zero_steps_and_dumps_of_the_reference_arm():
+    import sys
+    root = Path(__file__).resolve().parent.parent
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, str(root / "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=120, cwd=root)
+        assert out.returncode == 2 and out.stdout == "", out.stderr[-2000:]
+
+
+def test_bench_dump_outputs_full_and_sampled(tmp_path, monkeypatch):
+    """dump_outputs keeps the lists whole below the size limit and a fixed, seeded row sample above it."""
+    import bench
+    gen = torch.Generator().manual_seed(0)
+    v = torch.randn(300, 20, generator=gen)
+    i = torch.randint(0, 1 << 40, (300, 20), generator=gen)
+    bench.dump_outputs(tmp_path / "full", v, i)
+    assert sorted(p.name for p in (tmp_path / "full").iterdir()) == ["topk_indices.npy", "topk_values.npy"]
+    got_v, got_i = np.load(tmp_path / "full" / "topk_values.npy"), np.load(tmp_path / "full" / "topk_indices.npy")
+    assert got_v.dtype == np.float32 and got_i.dtype == np.float64
+    np.testing.assert_array_equal(got_v, v.numpy())
+    np.testing.assert_array_equal(got_i.astype(np.int64), i.numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4096 + 100 * (20 * 12 + 8))
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, v, i)
+        assert sum(p.stat().st_size for p in (tmp_path / d).iterdir()) <= bench.DUMP_LIMIT_BYTES
+    rows = np.load(tmp_path / "a" / "query_rows.npy")
+    assert rows.shape == (100,) and np.all(np.diff(rows) > 0)
+    for name in ("query_rows", "topk_values", "topk_indices"):
+        np.testing.assert_array_equal(np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy"))
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "topk_values.npy"), v.numpy()[rows.astype(np.int64)])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "topk_indices.npy").astype(np.int64),
+                                  i.numpy()[rows.astype(np.int64)])
+
+
 def test_bench_traffic_table_is_keyed_by_shape():
     import json
     root = Path(__file__).resolve().parent.parent
