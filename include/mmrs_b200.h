@@ -242,6 +242,66 @@ int mmrs_search_topk_fused_gather_async(
     int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status, void* stream);
 int mmrs_gather_status(const int32_t* h_status, int32_t world);
 
+/* ---- row-filtered search ---------------------------------------------------------------- */
+
+/*
+ * A row filter is an allow-list bitmap over the rows of one gallery (shard): uint32 words, bit
+ * (r & 31) of word (r >> 5) set when local row r may be returned.  PADDING CONTRACT: the array holds
+ * at least 4 * ceil(n_rows / 128) words (whole 128-row tiles); bits at or past n_rows are ignored, but
+ * those words must be readable.  A shard of a global filter whose first row is a multiple of 128 is the
+ * pointer d_words + first_row / 32 (its tail bits belong to the next shard and are ignored).
+ *
+ * mmrs_pack_row_filter builds one from a device byte mask d_allowed [n_rows] (non-zero = allowed):
+ * n_words >= 4 * ceil(n_rows / 128), words past the last row are zeroed; *d_count (device int64)
+ * receives the number of allowed rows.  Asynchronous on `stream`.
+ */
+int mmrs_pack_row_filter(const uint8_t* d_allowed, int64_t n_rows, uint32_t* d_words, int64_t n_words,
+                         int64_t* d_count, void* stream);
+
+/*
+ * The _filtered forms of the searches above: the same arguments plus d_row_filter (before `stream`),
+ * and the same top-k as an unfiltered search over the allowed rows only, indices still those of the
+ * full gallery (+ index_offset).  NULL = every row (exactly the unfiltered call).  k may exceed the
+ * number of allowed rows: the missing positions get value -inf, index -1 (key 0 in the key outputs,
+ * which every merge ignores), so a shard with few or no allowed rows still contributes k entries.
+ * A captured graph is keyed on the filter pointer; the words are read when the search runs.
+ */
+int mmrs_search_topk_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                    int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                    int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                    int64_t index_offset, int32_t path, float* d_out_values,
+                                    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+                                    int32_t* h_status, const uint32_t* d_row_filter, void* stream);
+int mmrs_search_topk_host_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim,
+                                         int64_t ld_gallery, int32_t gallery_dtype, const float* h_queries,
+                                         int32_t n_queries, int64_t ld_queries, int32_t k,
+                                         int32_t normalize_queries, float scale, int64_t index_offset,
+                                         int32_t path, float* h_out_values, int64_t* h_out_indices,
+                                         void* d_workspace, size_t workspace_bytes, int32_t* h_status,
+                                         const uint32_t* d_row_filter, void* stream);
+int mmrs_search_topk_exhaustive_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                         int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
+                                         void* d_workspace, size_t workspace_bytes,
+                                         const uint32_t* d_row_filter, void* stream);
+int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim,
+                                         int64_t ld_gallery, int32_t gallery_dtype, const float* d_queries,
+                                         int32_t n_queries, int64_t ld_queries, int32_t k,
+                                         int32_t normalize_queries, float scale, int64_t index_offset,
+                                         int32_t path, uint64_t* d_out_keys, void* d_workspace,
+                                         size_t workspace_bytes, int32_t* h_status,
+                                         const uint32_t* d_row_filter, void* stream);
+/* k_out must not exceed the allowed rows over all ranks (the merge pads with -inf / -1 otherwise). */
+int mmrs_search_topk_fused_gather_async_filtered(
+    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
+    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
+    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path,
+    uint64_t* const* d_peer_bufs, uint32_t* const* d_peer_flags, uint64_t* d_local_buf,
+    uint32_t* d_local_flags, int32_t rank, int32_t world, int64_t list_stride, float* d_out_values,
+    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status,
+    const uint32_t* d_row_filter, void* stream);
+
 /* ---- multi-GPU merge -------------------------------------------------------------------- */
 
 size_t mmrs_topk_merge_workspace_bytes(int32_t n_lists, int32_t n_queries, int32_t k_in);

@@ -87,6 +87,19 @@ SIGNATURES = {
     "mmrs_profile_read": (C.c_int, [_vp, _vp, _vp, _vp, _i32]),
     "mmrs_threshold_sweep_labeled": (C.c_int, [_vp, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "mmrs_threshold_sweep": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _sz, _vp]),
+    # row-filtered search: the unfiltered signature + the bitmap pointer before the stream
+    "mmrs_pack_row_filter": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp]),
+    "mmrs_search_topk_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
+                                                  _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "mmrs_search_topk_host_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
+                                                       _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "mmrs_search_topk_exhaustive_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
+                                                       _i64, _vp, _vp, _vp, _sz, _vp, _vp]),
+    "mmrs_search_topk_keys_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
+                                                       _i64, _i32, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "mmrs_search_topk_fused_gather_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
+                                                               _i32, _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32,
+                                                               _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
 }
 for _name, (_res, _args) in SIGNATURES.items():
     _fn = getattr(lib, _name)

@@ -334,6 +334,7 @@ struct SearchArgs {
   int64_t g_list_stride = 0;
   int32_t g_k_out = 0;
   uint64_t g_timeout_ns = 0;
+  const uint32_t* row_filter = nullptr;   // allow-list bitmap over the local rows (mmrs_pack_row_filter); nullptr = all
 };
 
 static uint64_t gather_timeout_ns() {
@@ -376,6 +377,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
   base.gallery = a.gallery; base.n_rows = a.n_rows; base.ld = a.ld; base.dim = a.dim;
   base.queries = w.q_f32; base.ldq = ldq; base.scale = a.scale;
   base.cap = pl.cap;
+  base.row_filter = a.row_filter;
 
   for (int32_t s0 = 0; s0 < a.n_queries; s0 += kSuperChunk) {
     const int32_t s1 = (a.n_queries - s0) < kSuperChunk ? a.n_queries : s0 + kSuperChunk;
@@ -402,6 +404,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
       }
       sp.index_offset = a.index_offset;
       sp.flags = w.flags;
+      sp.pad_short = a.row_filter != nullptr;
       if (fused && sp.final_pass) {
         sp.g_role = 1; sp.g_world = a.g_world; sp.g_rank = a.g_rank;
         sp.g_peer_bufs = a.g_peer_bufs; sp.g_peer_flags = a.g_peer_flags;
@@ -428,6 +431,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
     sp.g_role = 2; sp.g_world = a.g_world; sp.g_rank = a.g_rank; sp.g_peer_bufs = a.g_peer_bufs; sp.g_peer_flags = a.g_peer_flags;
     sp.g_list_stride = a.g_list_stride; sp.g_status_index = a.n_queries * a.k;
     sp.g_epoch = w.gscratch; sp.g_counter = w.gscratch + 2; sp.g_status_out = w.gscratch + kGStatus;
+    sp.pad_short = a.row_filter != nullptr;
     rc = profiled_launch(3, 0, 0, stream, [&]() { return launch_select(sp, a.n_queries, stream); });
     if (rc != MMRS_OK) return rc;
   }
@@ -446,6 +450,7 @@ static int enqueue_exhaustive(const SearchArgs& a, const DeviceInfo& dev, const 
   base.queries = w.q_f32; base.ldq = ldq; base.scale = a.scale;
   base.cap = all_rows;
   base.sched = TileSchedule{pl.n_tiles, 1, 0, pl.n_tiles};
+  base.row_filter = a.row_filter;
   MMRS_CUDA(cudaMemsetAsync(w.flags, 0, 8 * sizeof(int32_t), stream));
   {
     int rc = enqueue_prep(a, w, stream);
@@ -466,6 +471,7 @@ static int enqueue_exhaustive(const SearchArgs& a, const DeviceInfo& dev, const 
     sp.out_values = a.d_values + static_cast<int64_t>(q) * a.k;
     sp.out_indices = a.d_indices + static_cast<int64_t>(q) * a.k;
     sp.index_offset = a.index_offset; sp.flags = w.flags;
+    sp.pad_short = a.row_filter != nullptr;
     MMRS_LAUNCH(launch_select(sp, 1, stream));
   }
   return MMRS_OK;
@@ -491,8 +497,9 @@ struct GraphKey {
   int32_t g_world, g_rank; const void* g_bufs; const void* g_flags; const void* g_local_buf; const void* g_local_flags;
   int64_t g_stride; int32_t g_k_out; uint64_t g_timeout_ns;
   uint64_t knobs;   // the kernel-shape environment knobs the captured launches were configured with
+  const void* row_filter;   // the captured scans read the bitmap through this pointer
   bool operator==(const GraphKey& o) const {
-    return knobs == o.knobs && g_world == o.g_world && g_rank == o.g_rank && g_bufs == o.g_bufs && g_flags == o.g_flags &&
+    return knobs == o.knobs && row_filter == o.row_filter && g_world == o.g_world && g_rank == o.g_rank && g_bufs == o.g_bufs && g_flags == o.g_flags &&
            g_local_buf == o.g_local_buf && g_local_flags == o.g_local_flags && g_stride == o.g_stride && g_k_out == o.g_k_out &&
            g_timeout_ns == o.g_timeout_ns && has_values == o.has_values && has_indices == o.has_indices &&
            has_keys == o.has_keys && gallery == o.gallery && n_rows == o.n_rows && dim == o.dim && ld == o.ld &&
@@ -601,7 +608,7 @@ static int launch_search_graph(const SearchArgs& a, const DeviceInfo& dev, const
                dev.device, env_int("MMRS_RATIO_LOG2", -1), env_int("MMRS_DENSE_TILES", -1),
                a.d_values != nullptr, a.d_indices != nullptr, a.d_keys != nullptr,
                a.g_world, a.g_rank, a.g_peer_bufs, a.g_peer_flags, a.g_local_buf, a.g_local_flags, a.g_list_stride,
-               a.g_k_out, a.g_timeout_ns, knob_hash()};
+               a.g_k_out, a.g_timeout_ns, knob_hash(), a.row_filter};
   // the lock is held across patch + launch: an executable graph must not be updated or launched from
   // two threads at once (two threads sharing one workspace would be a caller bug anyway)
   std::lock_guard<std::mutex> lk(g_graph_mu);
@@ -668,6 +675,12 @@ static int flags_to_status(int32_t f) {
   if (f & kFlagWatchdog) return fail(MMRS_ERR_INTERNAL, "K2 pipeline watchdog fired (mbarrier wait timed out)");
   if (f & kFlagShort) return fail(MMRS_ERR_INTERNAL, "select saw fewer than k unique candidates");
   if (f & kFlagOverflow) return fail(MMRS_ERR_INTERNAL, "candidate list overflow");
+  return MMRS_OK;
+}
+
+static int check_row_filter(const uint32_t* f) {
+  if (reinterpret_cast<uintptr_t>(f) % sizeof(uint32_t) != 0)
+    return fail(MMRS_ERR_ARG, "row filter pointer must be 4-byte aligned");
   return MMRS_OK;
 }
 
@@ -850,7 +863,18 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
                                 int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
                                 int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                                 int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                void* d_workspace, size_t workspace_bytes, void* stream_) {
+                                void* d_workspace, size_t workspace_bytes, void* stream) {
+  return mmrs_search_topk_exhaustive_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
+                                              ld_queries, k, normalize_queries, scale, index_offset, d_out_values,
+                                              d_out_indices, d_workspace, workspace_bytes, nullptr, stream);
+}
+
+int mmrs_search_topk_exhaustive_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                         int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
+                                         void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
+                                         void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceInfo dev;
   int rc = current_device(&dev);
@@ -867,6 +891,9 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
   const Workspace w = carve(d_workspace, n_rows, dim, n_queries, 1, true, true);
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, MMRS_PATH_AUTO, d_out_values, d_out_indices};
+  a.row_filter = d_row_filter;
+  rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
   rc = enqueue_exhaustive(a, dev, w, stream);
   if (rc != MMRS_OK) return rc;
   int32_t* h = pinned_status();
@@ -911,8 +938,22 @@ int mmrs_search_topk_async(const void* d_gallery, int64_t n_rows, int32_t dim, i
                            int64_t index_offset, int32_t path, float* d_out_values,
                            int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
                            int32_t* h_status, void* stream) {
+  return mmrs_search_topk_async_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
+                                         ld_queries, k, normalize_queries, scale, index_offset, path, d_out_values,
+                                         d_out_indices, d_workspace, workspace_bytes, h_status, nullptr, stream);
+}
+
+int mmrs_search_topk_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                    int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                    int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                    int64_t index_offset, int32_t path, float* d_out_values,
+                                    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+                                    int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, d_out_values, d_out_indices};
+  a.row_filter = d_row_filter;
+  const int rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
   return search_enqueue(a, nullptr, nullptr, nullptr, d_workspace, workspace_bytes, h_status,
                         static_cast<cudaStream_t>(stream), nullptr, nullptr);
 }
@@ -923,9 +964,23 @@ int mmrs_search_topk_host_async(const void* d_gallery, int64_t n_rows, int32_t d
                                 int64_t index_offset, int32_t path, float* h_out_values,
                                 int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
                                 int32_t* h_status, void* stream) {
+  return mmrs_search_topk_host_async_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, h_queries, n_queries,
+                                              ld_queries, k, normalize_queries, scale, index_offset, path, h_out_values,
+                                              h_out_indices, d_workspace, workspace_bytes, h_status, nullptr, stream);
+}
+
+int mmrs_search_topk_host_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                         int32_t gallery_dtype, const float* h_queries, int32_t n_queries,
+                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                         int64_t index_offset, int32_t path, float* h_out_values,
+                                         int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
+                                         int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
   if (n_queries > 0 && !h_queries) return fail(MMRS_ERR_ARG, "null host query pointer");
+  const int rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, nullptr, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, nullptr, nullptr};
+  a.row_filter = d_row_filter;
   static const float dummy = 0.f;
   if (n_queries == 0) h_queries = &dummy;
   return search_enqueue(a, h_queries, h_out_values, h_out_indices, d_workspace, workspace_bytes,
@@ -938,11 +993,27 @@ int mmrs_search_topk_keys_async(const void* d_gallery, int64_t n_rows, int32_t d
                                 int64_t index_offset, int32_t path, uint64_t* d_out_keys,
                                 void* d_workspace, size_t workspace_bytes, int32_t* h_status,
                                 void* stream) {
+  return mmrs_search_topk_keys_async_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
+                                              ld_queries, k, normalize_queries, scale, index_offset, path, d_out_keys,
+                                              d_workspace, workspace_bytes, h_status, nullptr, stream);
+}
+
+int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                         int64_t index_offset, int32_t path, uint64_t* d_out_keys,
+                                         void* d_workspace, size_t workspace_bytes, int32_t* h_status,
+                                         const uint32_t* d_row_filter, void* stream) {
+  {
+    const int rc = check_row_filter(d_row_filter);
+    if (rc != MMRS_OK) return rc;
+  }
   if (index_offset < 0 || index_offset + n_rows > 0x100000000ll)
     return fail(MMRS_ERR_ARG, "global row ids must fit 32 bits");
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, nullptr, nullptr};
   a.d_keys = d_out_keys;
+  a.row_filter = d_row_filter;
   if (!d_out_keys) return fail(MMRS_ERR_ARG, "null key output pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   uint64_t* tail = d_out_keys + static_cast<int64_t>(n_queries < 0 ? 0 : n_queries) * k;
@@ -990,8 +1061,25 @@ int mmrs_search_topk_fused_gather_async(const void* d_gallery, int64_t n_rows, i
                                         uint64_t* const* d_peer_bufs, uint32_t* const* d_peer_flags,
                                         uint64_t* d_local_buf, uint32_t* d_local_flags, int32_t rank, int32_t world,
                                         int64_t list_stride, float* d_out_values, int64_t* d_out_indices,
-                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status, void* stream_) {
+                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status, void* stream) {
+  return mmrs_search_topk_fused_gather_async_filtered(
+      d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries, k_local, k_out,
+      normalize_queries, scale, index_offset, path, d_peer_bufs, d_peer_flags, d_local_buf, d_local_flags, rank, world,
+      list_stride, d_out_values, d_out_indices, d_workspace, workspace_bytes, h_status, nullptr, stream);
+}
+
+int mmrs_search_topk_fused_gather_async_filtered(
+    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
+    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
+    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path, uint64_t* const* d_peer_bufs,
+    uint32_t* const* d_peer_flags, uint64_t* d_local_buf, uint32_t* d_local_flags, int32_t rank, int32_t world,
+    int64_t list_stride, float* d_out_values, int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+    int32_t* h_status, const uint32_t* d_row_filter, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  {
+    const int rc = check_row_filter(d_row_filter);
+    if (rc != MMRS_OK) return rc;
+  }
   if (world < 1 || world > kMaxWorld || rank < 0 || rank >= world || !d_peer_bufs || !d_peer_flags || !d_local_buf ||
       !d_local_flags)
     return fail(MMRS_ERR_ARG, "bad rank / world / peer pointers");
@@ -1009,6 +1097,7 @@ int mmrs_search_topk_fused_gather_async(const void* d_gallery, int64_t n_rows, i
   a.g_world = world; a.g_rank = rank; a.g_peer_bufs = d_peer_bufs; a.g_peer_flags = d_peer_flags;
   a.g_local_buf = d_local_buf; a.g_local_flags = d_local_flags;
   a.g_list_stride = list_stride; a.g_k_out = k_out; a.g_timeout_ns = gather_timeout_ns();
+  a.row_filter = d_row_filter;
   for (int r = 0; r <= world + 1; ++r) h_status[r] = 0;
   Workspace w{};
   // ONE graph: prep (epoch bump + ack wait) -> scans / selects -> producer select -> wait -> merge select
@@ -1112,6 +1201,24 @@ int mmrs_selfjoin_pairs(const void* d_emb, int64_t n_rows, int32_t dim, int64_t 
   MMRS_CUDA(cudaStreamSynchronize(stream));
   if (h64[0] > capacity)
     return fail(MMRS_ERR_CAPACITY, "%lld pairs found, capacity %lld", (long long)h64[0], (long long)capacity);
+  return MMRS_OK;
+}
+
+int mmrs_pack_row_filter(const uint8_t* d_allowed, int64_t n_rows, uint32_t* d_words, int64_t n_words,
+                         int64_t* d_count, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_rows < 1 || !d_allowed || !d_words || !d_count) return fail(MMRS_ERR_ARG, "bad arguments");
+  const int64_t need = (n_rows + kTileRows - 1) / kTileRows * (kTileRows / 32);
+  if (n_words < need)
+    return fail(MMRS_ERR_ARG, "%lld words, need %lld (whole %d-row tiles)", (long long)n_words, (long long)need, kTileRows);
+  rc = check_row_filter(d_words);
+  if (rc != MMRS_OK) return rc;
+  MMRS_CUDA(cudaMemsetAsync(d_count, 0, sizeof(int64_t), stream));
+  MMRS_LAUNCH(launch_pack_row_filter(d_allowed, n_rows, d_words, n_words, reinterpret_cast<unsigned long long*>(d_count),
+                                     dev.sm_count, stream));
   return MMRS_OK;
 }
 

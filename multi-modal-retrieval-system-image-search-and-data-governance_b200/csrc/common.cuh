@@ -169,7 +169,13 @@ struct ScanParams {
   uint32_t* cnt;          // [n_queries]
   const float* thr;       // [n_queries] current lower bound on the k-th best score
   int32_t cap;
+  // kModeDense / kModeFilter, optional: allow-list bitmap over the rows (bit r & 31 of word r >> 5),
+  // zero-padded to whole tiles; an excluded row is key 0 in dense mode and never appended.
+  // nullptr = every row.  kModeScores ignores it.
+  const uint32_t* row_filter;
 };
+
+__device__ __forceinline__ bool row_allowed(uint32_t word, int64_t row) { return (word >> (row & 31)) & 1u; }
 
 struct SelectParams {
   uint64_t* cand;         // [n_queries, cap]
@@ -198,6 +204,10 @@ struct SelectParams {
   const uint32_t* g_epoch;         // device: sequence number of this call on this slot (starts at 1)
   uint32_t* g_counter;             // device: CTAs done (returns to 0)
   uint32_t* g_status_out;          // consumer: [g_world] private snapshot of the ranks' status words
+  // row-filtered search: fewer than k non-zero keys is legitimate (few allowed rows seen so far, or a
+  // shard with fewer than k allowed rows).  Non-final pass: thr = -inf, so the next phase appends every
+  // allowed row; final pass: positions n_win .. k-1 get value -inf, index -1, key 0.
+  int32_t pad_short;
 };
 
 // launchers (defined in the .cu files, called from api.cu)
@@ -224,6 +234,8 @@ cudaError_t launch_scan_gemv(const ScanParams& p, int32_t dtype, int mode, int s
                              cudaStream_t stream);
 cudaError_t launch_select(const SelectParams& p, int32_t n_queries, cudaStream_t stream);
 cudaError_t launch_fill_u32(uint32_t* p, uint32_t v, int64_t n, cudaStream_t stream);
+cudaError_t launch_pack_row_filter(const uint8_t* allowed, int64_t n_rows, uint32_t* words, int64_t n_words,
+                                   unsigned long long* count, int sm_count, cudaStream_t stream);
 cudaError_t launch_pack_keys(const float* values, const int64_t* indices, int32_t n_lists,
                              int32_t n_queries, int32_t k_in, uint64_t* cand, int32_t cap,
                              cudaStream_t stream);

@@ -156,14 +156,19 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
         const int64_t row = row0 + my_r;
         const float s = v[0] * p.scale;
         const int q = p.q0 + my_q;
+        // the bitmap covers whole tiles, so the word of a tail row past last_row is readable (and zero)
+        bool row_ok = row <= last_row;
+        if constexpr (MODE != kModeScores) {
+          if (p.row_filter != nullptr) row_ok = row_ok && row_allowed(__ldg(p.row_filter + (row >> 5)), row);
+        }
         if constexpr (MODE == kModeScores) {
-          if (row <= last_row) p.out_scores[static_cast<int64_t>(q) * p.ld_out + row] = s;
+          if (row_ok) p.out_scores[static_cast<int64_t>(q) * p.ld_out + row] = s;
         } else if constexpr (MODE == kModeDense) {
           const int64_t slot = static_cast<int64_t>(j) * kTileRows + (row - tile_row0);
           p.cand[static_cast<int64_t>(q) * p.cap + slot] =
-              row <= last_row ? make_key(s, static_cast<uint32_t>(row)) : 0ull;
+              row_ok ? make_key(s, static_cast<uint32_t>(row)) : 0ull;
         } else {
-          if (row <= last_row && !(s < my_thr)) {
+          if (row_ok && !(s < my_thr)) {
             const uint32_t pos = atomicAdd(p.cnt + q, 1u);
             if (pos < static_cast<uint32_t>(p.cap))
               p.cand[static_cast<int64_t>(q) * p.cap + pos] = make_key(s, static_cast<uint32_t>(row));
@@ -316,6 +321,31 @@ __global__ void fill_kernel(X* p, X v, int64_t n) {
 cudaError_t launch_fill_u32(uint32_t* p, uint32_t v, int64_t n, cudaStream_t stream) {
   if (n <= 0) return cudaSuccess;
   fill_kernel<uint32_t><<<static_cast<int>((n + 255) / 256), 256, 0, stream>>>(p, v, n);
+  return cudaGetLastError();
+}
+
+// ---- row filter: bool mask -> allow-list bitmap ------------------------------------------------
+// One warp per 32-row word: a ballot over the mask bytes is the word; words past the last row are
+// written as 0 (the padding the scan kernels rely on).  *count (zeroed by the caller) += popcount.
+__global__ void __launch_bounds__(256) pack_row_filter_kernel(const uint8_t* __restrict__ allowed, int64_t n_rows,
+                                                              uint32_t* __restrict__ words, int64_t n_words,
+                                                              unsigned long long* count) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+  uint32_t n = 0;
+  for (int64_t w = (blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5; w < n_words; w += n_warps) {
+    const int64_t r = w * 32 + lane;
+    const uint32_t b = __ballot_sync(0xffffffffu, r < n_rows && allowed[r] != 0);
+    if (lane == 0) { words[w] = b; n += __popc(b); }
+  }
+  if (lane == 0 && n) atomicAdd(count, static_cast<unsigned long long>(n));
+}
+cudaError_t launch_pack_row_filter(const uint8_t* allowed, int64_t n_rows, uint32_t* words, int64_t n_words,
+                                   unsigned long long* count, int sm_count, cudaStream_t stream) {
+  if (n_words <= 0) return cudaSuccess;
+  int64_t grid = (n_words * 32 + 255) / 256;
+  if (grid > static_cast<int64_t>(sm_count) * 8) grid = static_cast<int64_t>(sm_count) * 8;
+  pack_row_filter_kernel<<<static_cast<int>(grid), 256, 0, stream>>>(allowed, n_rows, words, n_words, count);
   return cudaGetLastError();
 }
 

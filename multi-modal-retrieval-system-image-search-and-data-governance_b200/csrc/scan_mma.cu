@@ -353,10 +353,16 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
       const float* thr_s = sh->thr + (PAIR ? un.chunk * kMaxQ : 0);
       const float* thr_raw_s = sh->thr_raw + (PAIR ? un.chunk * kMaxQ : 0);
       const uint32_t as = it & 1, aphase = (it >> 1) & 1;
+      const int64_t row = static_cast<int64_t>(t) * kBlockM + r_in_tile;
+      // row filter: the warp's 32 rows are one bitmap word (padded to whole tiles, so always readable);
+      // loaded before the accumulator wait so that its latency hides behind the MMAs
+      uint32_t filter_word = ~0u;
+      if constexpr (MODE != kModeScores) {
+        if (p.row_filter != nullptr) filter_word = __ldg(p.row_filter + (row >> 5));
+      }
       if (!mbar_wait(&sh->tmem_full[as], aphase, &sh->abort, flags)) break;
       tcgen05_fence_after();
-      const int64_t row = static_cast<int64_t>(t) * kBlockM + r_in_tile;
-      const bool row_ok = row <= last_row;
+      const bool row_ok = row <= last_row && row_allowed(filter_word, row);
       const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
                               as * static_cast<uint32_t>(cfg.acc_stride);
       bool released = false;

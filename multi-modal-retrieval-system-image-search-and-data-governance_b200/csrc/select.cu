@@ -234,10 +234,11 @@ __device__ __forceinline__ void select_body(const SelectParams& p, SelShared& sh
   });
   __syncthreads();
   const uint32_t n_win = sh.n_out;
-  if (n_win < k || n_win > limit) {  // uniqueness violated (bug guard)
+  if ((n_win < k && !p.pad_short) || n_win > limit) {  // uniqueness violated (bug guard)
     if (tid == 0) atomicOr(p.flags, kFlagShort);
     if (n_win > limit) return;
   }
+  const bool short_list = p.pad_short && n_win < k;   // fewer than k allowed rows so far
 
   if (p.final_pass) {
     // rank by counting: position = number of winners with a larger key
@@ -256,12 +257,26 @@ __device__ __forceinline__ void select_body(const SelectParams& p, SelShared& sh
         for (int r = 0; r < p.g_world; ++r) p.g_peer_bufs[r][off] = gkey;
       }
     }
+    if (short_list) {
+      // every position still gets written (a shard's list keeps exactly k entries; key 0 merges as nothing)
+      for (uint32_t i = n_win + tid; i < k; i += kSelThreads) {
+        const int64_t o = static_cast<int64_t>(q) * k + i;
+        if (p.out_values) p.out_values[o] = __int_as_float(0xff800000);
+        if (p.out_indices) p.out_indices[o] = -1;
+        if (p.out_keys) p.out_keys[o] = 0ull;
+        if (p.g_role == 1) {
+          const int64_t off = static_cast<int64_t>(p.g_rank) * p.g_list_stride + o;
+          for (int r = 0; r < p.g_world; ++r) p.g_peer_bufs[r][off] = 0ull;
+        }
+      }
+    }
   } else {
-    // next list = the winners (unsorted); bound = score part of the pivot (<= every winner's score)
+    // next list = the winners (unsorted); bound = score part of the pivot (<= every winner's score).
+    // Fewer than k winners: no bound yet, the next phase appends every (allowed) row.
     for (uint32_t i = tid; i < n_win; i += kSelThreads) list[i] = sh.winners[i];
     if (tid == 0) {
       p.cnt[q] = n_win;
-      p.thr[q] = key_score(thr_key);
+      p.thr[q] = short_list ? __int_as_float(0xff800000) : key_score(thr_key);
     }
   }
 }
@@ -344,7 +359,7 @@ __device__ __forceinline__ void select_dispatch_impl(const SelectParams& p, SelS
       n = p.cap;
     }
   }
-  if (n < static_cast<uint32_t>(p.k)) {  // cannot happen on a correct schedule; never read past the list
+  if (n < static_cast<uint32_t>(p.k) && !p.pad_short) {  // cannot happen on a correct unfiltered schedule
     if (tid == 0) atomicOr(p.flags, kFlagShort);
     return;
   }

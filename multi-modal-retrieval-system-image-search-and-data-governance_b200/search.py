@@ -16,6 +16,7 @@ import torch
 
 from . import _cabi
 from .gallery import DeviceGallery, _pad_dim
+from .row_filter import RowFilter, filter_words, pack_mask
 
 # module-level configuration with the reference's names (code/search_image.py:14-38); scripts
 # that `from search_image import *` and set these keep working
@@ -95,9 +96,10 @@ class PendingSearch:
 
 
 def _search_exhaustive(gal: DeviceGallery, q: torch.Tensor, k: int, normalize_queries: bool, scale: float,
-                       path: str, values: torch.Tensor, indices: torch.Tensor) -> None:
+                       path: str, values: torch.Tensor, indices: torch.Tensor, row_filter_ptr: int = 0) -> None:
     """The exact fallback for a batch whose candidate lists overflowed (MMRS_ERR_RETRY): every row a
-    key, one query at a time.  Its 8-bytes-per-row workspace lives only for this call."""
+    key, one query at a time.  Its 8-bytes-per-row workspace lives only for this call.
+    `row_filter_ptr`: device bitmap of the allowed rows (0 = all)."""
     lib = _cabi.lib
     dev = gal.device
     nq = int(q.shape[0])
@@ -108,19 +110,41 @@ def _search_exhaustive(gal: DeviceGallery, q: torch.Tensor, k: int, normalize_qu
         g_ptr, g_ld, g_dtype = _operand(gal, nq, path)
         ws_bytes = lib.mmrs_search_exhaustive_workspace_bytes(gal.n_rows, gal.padded_dim, nq)
         ws = torch.empty(int(ws_bytes) + 256, dtype=torch.uint8, device=dev)
-        _cabi.check(lib.mmrs_search_topk_exhaustive(
-            g_ptr, gal.n_rows, gal.padded_dim, g_ld, g_dtype, qd.data_ptr(), nq, qd.stride(0), k,
-            int(bool(normalize_queries)), float(scale), gal.row_offset, dv.data_ptr(), di.data_ptr(),
-            DeviceGallery.aligned_ptr(ws), ws_bytes, _stream_handle(dev)))
+        args = (g_ptr, gal.n_rows, gal.padded_dim, g_ld, g_dtype, qd.data_ptr(), nq, qd.stride(0), k,
+                int(bool(normalize_queries)), float(scale), gal.row_offset, dv.data_ptr(), di.data_ptr(),
+                DeviceGallery.aligned_ptr(ws), ws_bytes)
+        if row_filter_ptr:
+            _cabi.check(lib.mmrs_search_topk_exhaustive_filtered(*args, row_filter_ptr, _stream_handle(dev)))
+        else:
+            _cabi.check(lib.mmrs_search_topk_exhaustive(*args, _stream_handle(dev)))
         if dv is not values:
             values.copy_(dv)
             indices.copy_(di)
         del ws
 
 
+def _filter_arg(row_filter, gal: DeviceGallery):
+    """`row_filter` checked against the gallery: None, a RowFilter, or a 1-D bool mask tensor."""
+    if row_filter is None:
+        return None
+    if isinstance(row_filter, RowFilter):
+        n, dev = row_filter.n_rows, row_filter.device
+    else:
+        row_filter = row_filter if isinstance(row_filter, torch.Tensor) else torch.from_numpy(np.asarray(row_filter))
+        if row_filter.dim() != 1 or row_filter.dtype != torch.bool:
+            raise ValueError(f"row_filter must be a RowFilter or a 1-D bool mask, got {row_filter.dtype} "
+                             f"{tuple(row_filter.shape)}")
+        n, dev = int(row_filter.numel()), (row_filter.device if row_filter.is_cuda else None)
+    if n != gal.n_rows:
+        raise ValueError(f"row_filter covers {n} rows, the gallery has {gal.n_rows}")
+    if dev is not None and dev != gal.device:
+        raise ValueError(f"row_filter is on {dev}, the gallery on {gal.device}")
+    return row_filter
+
+
 def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: bool = True,
                 scale: float = 1.0, mode: Optional[str] = None, path: str = "auto", sync: bool = True,
-                out=None):
+                out=None, row_filter=None):
     """Per-query top-k of `scale * q @ G.T` without materialising the score matrix.
 
     Returns `(values [Q, k] fp32 descending, indices [Q, k] int64)` exactly like
@@ -132,6 +156,10 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
     batches can be in flight.  `out=(values, indices)` writes into caller-owned tensors (pinned host
     tensors for host queries) instead of allocating; either way the library replays ONE captured
     graph per (shape, stream) slot and only re-points its query / result nodes.
+    `row_filter` (a RowFilter or a bool mask [N]) restricts the search to the allowed rows: the result
+    is the top-k of `gallery[mask]` with indices of the full gallery; `k` may not exceed the allowed
+    rows.  A RowFilter costs one graph capture per slot; a mask is packed into a buffer of the slot on
+    every call (and its allowed count read back: one host sync).
     """
     gal = _as_gallery(gallery, mode)
     q, on_host = _prep_queries(queries, gal)
@@ -141,6 +169,9 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
         raise ValueError("k must be >= 1")
     if k > gal.n_rows:
         raise RuntimeError("selected index k out of range")  # torch.topk's message
+    filt = _filter_arg(row_filter, gal)
+    if isinstance(filt, RowFilter) and k > filt.n_allowed:
+        raise RuntimeError("selected index k out of range")
     lib = _cabi.lib
     dev = gal.device
     if torch.cuda.current_device() != dev.index:
@@ -160,18 +191,49 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
         values = torch.empty((nq, k), dtype=torch.float32, device=dev)
         indices = torch.empty((nq, k), dtype=torch.int64, device=dev)
     if nq == 0:
+        if filt is not None and not isinstance(filt, RowFilter) and k > int(filt.sum()):
+            raise RuntimeError("selected index k out of range")
         return (values, indices) if sync else PendingSearch(values, indices, None, None, None, None, None)
     if on_host and not q.is_pinned():
         q = q.pin_memory()
     slot = gal.search_slot(nq, k, on_host, stream.cuda_stream)
+    filt_ptr = 0
+    if isinstance(filt, RowFilter):
+        filt_ptr = filt.words.data_ptr()
+    elif filt is not None:
+        # a per-call mask goes into the slot's own bitmap: a stable pointer, so the slot keeps replaying
+        # one graph; calls on the slot run in stream order, so the next pack cannot overtake this search
+        words = slot.extra.get("row_filter")
+        if words is None:
+            words = slot.extra["row_filter"] = torch.empty(filter_words(gal.n_rows), dtype=torch.int32, device=dev)
+        filt = filt.to(dev)
+        if k > int(pack_mask(filt, words).item()):
+            raise RuntimeError("selected index k out of range")
+        filt_ptr = words.data_ptr()
     g_ptr, g_ld, g_dtype = _operand(gal, nq, path)
     args = (g_ptr, gal.n_rows, gal.padded_dim, g_ld, g_dtype,
             q.data_ptr(), nq, q.stride(0), k, int(bool(normalize_queries)), float(scale),
             gal.row_offset, _cabi.PATHS[path], values.data_ptr(), indices.data_ptr(), slot.ptr, slot.nbytes)
 
     def redo(v, i):
-        _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i)
+        if filt is None:
+            _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i)
+        else:
+            # by now the slot's bitmap may hold a later call's mask: repack this call's own
+            f = filt if isinstance(filt, RowFilter) else RowFilter(filt)
+            _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i, f.words.data_ptr())
 
+    if filt is not None:
+        ticket, status, event = slot.acquire()
+        fn = lib.mmrs_search_topk_host_async_filtered if on_host else lib.mmrs_search_topk_async_filtered
+        st = fn(*args, status.data_ptr(), filt_ptr, stream.cuda_stream)
+        if st != _cabi.OK:
+            slot.release(ticket)
+            _cabi.check(st)
+        event.record(stream)
+        pend = PendingSearch(values, indices, slot, ticket, status, event, redo)
+        pend._keepalive = (q, filt)
+        return pend.wait() if sync else pend
     if sync:
         fn = lib.mmrs_search_topk_host if on_host else lib.mmrs_search_topk
         st = fn(*args, stream.cuda_stream)

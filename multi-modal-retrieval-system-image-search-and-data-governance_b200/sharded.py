@@ -20,6 +20,7 @@ import torch.distributed as dist
 
 from . import _cabi
 from .gallery import DeviceGallery
+from .row_filter import RowFilter
 
 
 def shard_bounds(n_rows: int, world: int, align: int = 128) -> list[tuple[int, int]]:
@@ -177,10 +178,12 @@ class ShardedGallery:
         return (torch.empty((nq, k), dtype=torch.float32, device=dev),
                 torch.empty((nq, k), dtype=torch.int64, device=dev), None, None)
 
-    def _search_topk_keys(self, queries, k: int, normalize_queries: bool, scale: float, path: str, out=None):
+    def _search_topk_keys(self, queries, k: int, normalize_queries: bool, scale: float, path: str, out=None,
+                          local_filter: Optional[RowFilter] = None):
         """CUDA fast path: local top-k as packed 64-bit keys -> ONE all-gather (Q*k*8 bytes per rank)
         -> merge kernel reading the gathered buffer in place.  Nothing synchronises with the host
-        until the final status check.  Shards shorter than k pad their lists with key 0."""
+        until the final status check.  Shards shorter than k pad their lists with key 0, and so does a
+        shard with fewer than k allowed rows (the library pads them)."""
         gal = self.local
         dev = gal.device
         lib = _cabi.lib
@@ -205,11 +208,13 @@ class ShardedGallery:
         shard_status = None
         if nq:
             dst = buf if short is None else short
-            st = lib.mmrs_search_topk_keys_async(
-                gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
-                q.data_ptr(), nq, q.stride(0), k_local, int(bool(normalize_queries)), float(scale),
-                gal.row_offset, _cabi.PATHS[path], dst.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr(),
-                stream.cuda_stream)
+            args = (gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
+                    q.data_ptr(), nq, q.stride(0), k_local, int(bool(normalize_queries)), float(scale),
+                    gal.row_offset, _cabi.PATHS[path], dst.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr())
+            if local_filter is None:
+                st = lib.mmrs_search_topk_keys_async(*args, stream.cuda_stream)
+            else:
+                st = lib.mmrs_search_topk_keys_async_filtered(*args, local_filter.words.data_ptr(), stream.cuda_stream)
             if st != _cabi.OK:
                 slot.release(ticket)
                 _cabi.check(st)
@@ -250,7 +255,7 @@ class ShardedGallery:
             _cabi.check(merge_rc)
             return res
 
-        finish._keepalive = (q, keep)
+        finish._keepalive = (q, keep, local_filter)
         return finish
 
     # ---- search fused with its all-gather over NVLink peer memory -----------------------------------
@@ -277,7 +282,8 @@ class ShardedGallery:
             slot.extra["fused"] = st
         return st
 
-    def _search_topk_fused(self, queries, k: int, normalize_queries: bool, scale: float, path: str, out=None):
+    def _search_topk_fused(self, queries, k: int, normalize_queries: bool, scale: float, path: str, out=None,
+                           local_filter: Optional[RowFilter] = None):
         """Local scan -> last select stores its keys into EVERY rank's buffer over NVLink and raises
         a ready flag -> a one-warp kernel waits for all flags -> merge select.  One library call, one
         graph replay, no NCCL, no host sync until the final status check; every buffer the call
@@ -295,12 +301,15 @@ class ShardedGallery:
         q, on_host, keep = self._stage_queries(slot, queries)
         dv, di, hv, hi = self._results(slot, nq, k, dev, on_host, out)
         ticket, status, event = slot.acquire()
-        rc = lib.mmrs_search_topk_fused_gather_async(
-            gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
-            q.data_ptr(), nq, q.stride(0), k_local, k, int(bool(normalize_queries)), float(scale),
-            gal.row_offset, _cabi.PATHS[path], st["bufs"].data_ptr(), st["flags"].data_ptr(),
-            st["t"].data_ptr(), st["local_flags"], self.rank, self.world, st["stride"],
-            dv.data_ptr(), di.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr(), stream.cuda_stream)
+        args = (gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
+                q.data_ptr(), nq, q.stride(0), k_local, k, int(bool(normalize_queries)), float(scale),
+                gal.row_offset, _cabi.PATHS[path], st["bufs"].data_ptr(), st["flags"].data_ptr(),
+                st["t"].data_ptr(), st["local_flags"], self.rank, self.world, st["stride"],
+                dv.data_ptr(), di.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr())
+        if local_filter is None:
+            rc = lib.mmrs_search_topk_fused_gather_async(*args, stream.cuda_stream)
+        else:   # a shard with fewer than k allowed rows still stores k keys (padded with key 0)
+            rc = lib.mmrs_search_topk_fused_gather_async_filtered(*args, local_filter.words.data_ptr(), stream.cuda_stream)
         if rc != _cabi.OK:
             slot.release(ticket)
             _cabi.check(rc)
@@ -321,17 +330,34 @@ class ShardedGallery:
             _cabi.check(rc)
             return (hv, hi) if on_host else (dv, di)
 
-        finish._keepalive = (q, keep)
+        finish._keepalive = (q, keep, local_filter)
         return finish
 
+    def _local_filter(self, row_filter):
+        """(filter over the GLOBAL rows as a RowFilter -- a bool mask is packed here --, this rank's slice of it)."""
+        dev = getattr(self.local, "device", None)
+        f = row_filter if isinstance(row_filter, RowFilter) else RowFilter(row_filter, device=dev)
+        if f.n_rows != self.n_rows_global:
+            raise ValueError(f"row_filter covers {f.n_rows} rows, the sharded gallery has {self.n_rows_global}")
+        if dev is not None and f.device != dev:
+            raise ValueError(f"row_filter is on {f.device}, this rank's shard on {dev}")
+        lo = self.local.row_offset
+        return f, f.shard(lo, lo + len(self.local))
+
     def search_topk(self, queries: torch.Tensor, k: int, *, normalize_queries: bool = True,
-                    scale: float = 1.0, path: str = "auto", sync: bool = True, out=None):
+                    scale: float = 1.0, path: str = "auto", sync: bool = True, out=None, row_filter=None):
         """Global top-k, identical on every rank.  `queries` must be the same on all ranks.
         `sync=False` returns an object whose `.wait()` yields `(values, indices)`, so that several
         batches (and their all-gathers) can be in flight.  `out=(values, indices)`: caller-owned result
-        tensors (pinned host tensors for host queries)."""
+        tensors (pinned host tensors for host queries).  `row_filter`: a RowFilter (or bool mask) over the
+        GLOBAL rows, the same on every rank like the queries; each rank searches its slice of it."""
         if k > self.n_rows_global:
             raise RuntimeError("selected index k out of range")
+        local_filter = None
+        if row_filter is not None:
+            row_filter, local_filter = self._local_filter(row_filter)
+            if k > row_filter.n_allowed:      # every rank decides alike from the same filter: no collective
+                raise RuntimeError("selected index k out of range")
         if self._fast and self.world > 1:
             if isinstance(queries, np.ndarray):
                 queries = torch.from_numpy(queries)
@@ -339,40 +365,58 @@ class ShardedGallery:
                 queries = queries.unsqueeze(0)
             nq = int(queries.shape[0])
             if nq == 0:
-                out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path)
+                out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path,
+                                                 row_filter=row_filter)
                 return out_t if sync else _PendingSharded(lambda: out_t, None)
             # fused NVLink gather: every rank contributes its full top-k (needs >= k rows in every shard)
             fused = self._fused_ok and 1 <= nq <= 1024 and self.min_shard_rows >= k
             finish = None
             if fused:
                 try:
-                    finish = self._search_topk_fused(queries, k, normalize_queries, scale, path, out)
+                    finish = self._search_topk_fused(queries, k, normalize_queries, scale, path, out, local_filter)
                 except (ImportError, AttributeError, RuntimeError) as e:   # no symmetric memory here
                     if isinstance(e, _cabi.MmrsError):
                         raise
                     self._fused_ok = False
             if finish is None:
-                finish = self._search_topk_keys(queries, k, normalize_queries, scale, path, out)
+                finish = self._search_topk_keys(queries, k, normalize_queries, scale, path, out, local_filter)
             general = lambda: self.search_topk_general(queries, k, normalize_queries=normalize_queries,
-                                                       scale=scale, path=path)
+                                                       scale=scale, path=path, row_filter=row_filter)
             pend = _PendingSharded(finish, general)
             return pend.wait() if sync else pend
-        out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path)
+        out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path,
+                                         row_filter=row_filter)
         return out_t if sync else _PendingSharded(lambda: out_t, None)
 
     def search_topk_general(self, queries: torch.Tensor, k: int, *, normalize_queries: bool = True,
-                            scale: float = 1.0, path: str = "auto"):
+                            scale: float = 1.0, path: str = "auto", row_filter=None):
         """(values, indices) lists, two all-gathers, merge -- also the path every rank takes together
         when some rank's candidate list overflowed (None from the fast path on EVERY rank alike: the
-        shard statuses were gathered with the keys)."""
+        shard statuses were gathered with the keys).  With a `row_filter` a rank searches for
+        min(k, its allowed rows) and one without allowed rows skips its local search."""
         n_local = len(self.local)
         k_local = min(k, n_local)
+        local_filter = None
+        if row_filter is not None:
+            row_filter, local_filter = self._local_filter(row_filter)
+            if k > row_filter.n_allowed:
+                raise RuntimeError("selected index k out of range")
+            k_local = min(k, local_filter.n_allowed)
         on_host = False
         if self._fast and self.world > 1 and not (isinstance(queries, torch.Tensor) and queries.is_cuda):
             on_host = True                    # NCCL gathers device tensors: search on the device, copy back
             queries = torch.as_tensor(queries).to(self.local.device)
-        v, i = self._search(queries, self.local, k_local, normalize_queries=normalize_queries,
-                            scale=scale, path=path)
+        if local_filter is None:
+            v, i = self._search(queries, self.local, k_local, normalize_queries=normalize_queries,
+                                scale=scale, path=path)
+        elif k_local > 0:
+            v, i = self._search(queries, self.local, k_local, normalize_queries=normalize_queries,
+                                scale=scale, path=path, row_filter=local_filter)
+        else:                                 # no allowed row here: contribute padding only
+            nq = 1 if len(queries.shape) == 1 else int(queries.shape[0])
+            dev = getattr(self.local, "device", torch.device("cpu"))
+            v = torch.empty((nq, 0), dtype=torch.float32, device=dev)
+            i = torch.empty((nq, 0), dtype=torch.int64, device=dev)
         if self.world == 1:
             return v, i
         if k_local < k:
