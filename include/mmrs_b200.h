@@ -302,6 +302,80 @@ int mmrs_search_topk_fused_gather_async_filtered(
     int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status,
     const uint32_t* d_row_filter, void* stream);
 
+/* ---- label-conditioned search ----------------------------------------------------------- */
+
+/* label_match of the _labeled searches */
+#define MMRS_LABEL_SAME 0    /* only rows whose label equals the query's label             */
+#define MMRS_LABEL_OTHER 1   /* only rows whose label differs from it (hard negatives)      */
+
+/*
+ * Row labels are one int32 class id per row of the gallery (shard), each in [0, 2^31 - 1).
+ * PADDING CONTRACT (the bitmap's): the array holds at least 128 * ceil(n_rows / 128) elements (whole
+ * 128-row tiles); labels at or past n_rows are never compared, but must be readable.  A shard of a
+ * global label array whose first row is a multiple of 128 is the pointer d_row_labels + first_row.
+ *
+ * The _labeled forms of the five _filtered searches take the _filtered arguments plus d_row_labels,
+ * d_query_labels and label_match (before `stream`).  d_query_labels is a DEVICE int32 [n_queries] in
+ * every form, the host-I/O one included.  For query q with c = d_query_labels[q]:
+ *   c < 0               no label restriction: exactly the unlabeled search of that query;
+ *   MMRS_LABEL_SAME     only rows r with d_row_labels[r] == c;
+ *   MMRS_LABEL_OTHER    only rows r with d_row_labels[r] != c;
+ * and with d_row_filter as well, a row must pass both.  Values, order and tie rule are those of the
+ * unlabeled search over the eligible rows.  A query with fewer than k eligible rows (a small class, a
+ * label absent from the gallery) is NOT an error: positions n_eligible .. k-1 get value -inf, index -1
+ * (key 0 in the key outputs).  d_row_labels == NULL is exactly the _filtered call.  A captured graph is
+ * keyed on both label pointers and label_match; the labels are read when the search runs, so a caller
+ * that rewrites the query labels in place between calls keeps replaying one graph.
+ */
+int mmrs_search_topk_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                   int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                   int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                   int64_t index_offset, int32_t path, float* d_out_values,
+                                   int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+                                   int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                   const int32_t* d_query_labels, int32_t label_match, void* stream);
+int mmrs_search_topk_host_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim,
+                                        int64_t ld_gallery, int32_t gallery_dtype, const float* h_queries,
+                                        int32_t n_queries, int64_t ld_queries, int32_t k,
+                                        int32_t normalize_queries, float scale, int64_t index_offset,
+                                        int32_t path, float* h_out_values, int64_t* h_out_indices,
+                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status,
+                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                        const int32_t* d_query_labels, int32_t label_match, void* stream);
+int mmrs_search_topk_exhaustive_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                        int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
+                                        void* d_workspace, size_t workspace_bytes,
+                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                        const int32_t* d_query_labels, int32_t label_match, void* stream);
+int mmrs_search_topk_keys_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim,
+                                        int64_t ld_gallery, int32_t gallery_dtype, const float* d_queries,
+                                        int32_t n_queries, int64_t ld_queries, int32_t k,
+                                        int32_t normalize_queries, float scale, int64_t index_offset,
+                                        int32_t path, uint64_t* d_out_keys, void* d_workspace,
+                                        size_t workspace_bytes, int32_t* h_status,
+                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                        const int32_t* d_query_labels, int32_t label_match, void* stream);
+/* The merge select pads: fewer than k_out eligible rows over all ranks give -inf / -1. */
+int mmrs_search_topk_fused_gather_async_labeled(
+    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
+    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
+    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path,
+    uint64_t* const* d_peer_bufs, uint32_t* const* d_peer_flags, uint64_t* d_local_buf,
+    uint32_t* d_local_flags, int32_t rank, int32_t world, int64_t list_stride, float* d_out_values,
+    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status,
+    const uint32_t* d_row_filter, const int32_t* d_row_labels, const int32_t* d_query_labels,
+    int32_t label_match, void* stream);
+/*
+ * mmrs_topk_merge_keys_async for lists that may hold fewer than k_out non-zero keys per query over all
+ * lists (the gathered keys of a labeled search): the missing positions get value -inf, index -1.
+ */
+int mmrs_topk_merge_keys_padded_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries,
+                                      int32_t k_in, int64_t list_stride, int32_t k_out,
+                                      float* d_out_values, int64_t* d_out_indices, int32_t* d_status,
+                                      int32_t* h_status, void* stream);
+
 /* ---- multi-GPU merge -------------------------------------------------------------------- */
 
 size_t mmrs_topk_merge_workspace_bytes(int32_t n_lists, int32_t n_queries, int32_t k_in);

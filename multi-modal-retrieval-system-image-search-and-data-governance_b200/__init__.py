@@ -20,12 +20,14 @@ functions for this path (same names, positional order and return tuples):
     code/main_custom.py    find_thresholds(..., grid="overlap") (:46-91), get_similarity_from_matrix (:93-105)
 
 plus the tensor-level entry points they sit on: search_topk, full_scores, find_duplicate_pairs,
-DeviceGallery, ShardedGallery, and RowFilter (row-filtered search_topk: leave rows out per call).  Everything computes through the C-ABI CUDA library
+DeviceGallery, ShardedGallery, RowFilter (row-filtered search_topk: leave rows out per call) and
+RowLabels (label-conditioned search_topk: each query searches the rows of its own class, or of every other).  Everything computes through the C-ABI CUDA library
 (include/mmrs_b200.h); there is no CPU path -- without a B200 the calls raise.
 """
 from . import _cabi  # noqa: F401  (fails loudly when the CUDA library is missing)
 from .gallery import DeviceGallery, load_feature_cache
 from .row_filter import RowFilter
+from .row_labels import RowLabels
 from .search import (best_threshold_on_device, calc_combined_metrics, cls_acc, cluster_prototype, construct_dataset,
                      cosine_similarity_scores, eval_threshold, evaluate_thresholds, find_thresholds, full_scores,
                      get_cluster_features, get_image_text_features, get_similarity, get_similarity_from_matrix,
@@ -36,7 +38,7 @@ from .dedup import (calculate_image_hash, detect_and_remove_cross_set_duplicates
 from .sharded import ShardedGallery, shard_bounds
 
 __all__ = [
-    "DeviceGallery", "RowFilter", "ShardedGallery", "best_threshold_on_device", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
+    "DeviceGallery", "RowFilter", "RowLabels", "ShardedGallery", "best_threshold_on_device", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
     "cluster_prototype", "construct_dataset", "cosine_similarity_scores", "get_cluster_features", "get_image_text_features",
     "image_text_prototypes", "topk_of_scores",
     "detect_and_remove_cross_set_duplicates", "evaluate_thresholds", "eval_threshold", "find_thresholds",

@@ -14,6 +14,8 @@ ABI_VERSION = 2
 DTYPE_F32, DTYPE_BF16, DTYPE_BF16X3 = 0, 1, 2
 PATH_AUTO, PATH_GEMV, PATH_MMA = 0, 1, 2
 PATHS = {"auto": PATH_AUTO, "gemv": PATH_GEMV, "mma": PATH_MMA}
+LABEL_SAME, LABEL_OTHER = 0, 1
+LABEL_MATCH = {"same": LABEL_SAME, "other": LABEL_OTHER}
 
 
 class MmrsError(RuntimeError):
@@ -100,6 +102,21 @@ SIGNATURES = {
     "mmrs_search_topk_fused_gather_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
                                                                _i32, _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32,
                                                                _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
+    # label-conditioned search: the _filtered signature + row labels, query labels, label_match before the stream
+    "mmrs_search_topk_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
+                                                 _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "mmrs_search_topk_host_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
+                                                      _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32,
+                                                      _vp]),
+    "mmrs_search_topk_exhaustive_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
+                                                      _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _i32, _vp]),
+    "mmrs_search_topk_keys_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
+                                                      _i64, _i32, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "mmrs_search_topk_fused_gather_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
+                                                              _i32, _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32,
+                                                              _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _i32,
+                                                              _vp]),
+    "mmrs_topk_merge_keys_padded_async": (C.c_int, [_vp, _i32, _i32, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
 }
 for _name, (_res, _args) in SIGNATURES.items():
     _fn = getattr(lib, _name)

@@ -335,7 +335,20 @@ struct SearchArgs {
   int32_t g_k_out = 0;
   uint64_t g_timeout_ns = 0;
   const uint32_t* row_filter = nullptr;   // allow-list bitmap over the local rows (mmrs_pack_row_filter); nullptr = all
+  // label-conditioned search (ScanParams): row labels over the local rows (nullptr = unlabeled), device
+  // query labels [n_queries], MMRS_LABEL_SAME / MMRS_LABEL_OTHER
+  const int32_t* row_labels = nullptr;
+  const int32_t* query_labels = nullptr;
+  int32_t label_match = 0;
+  // a query may legitimately see fewer than k eligible rows: the selects pad instead of flagging
+  bool pad_short() const { return row_filter != nullptr || row_labels != nullptr; }
 };
+
+static void set_labels(ScanParams& p, const SearchArgs& a) {
+  p.row_labels = a.row_labels;
+  p.query_labels = a.row_labels ? a.query_labels : nullptr;
+  p.label_match = a.row_labels ? a.label_match : 0;
+}
 
 static uint64_t gather_timeout_ns() {
   const int ms = env_int("MMRS_GATHER_TIMEOUT_MS", 20000);
@@ -378,6 +391,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
   base.queries = w.q_f32; base.ldq = ldq; base.scale = a.scale;
   base.cap = pl.cap;
   base.row_filter = a.row_filter;
+  set_labels(base, a);
 
   for (int32_t s0 = 0; s0 < a.n_queries; s0 += kSuperChunk) {
     const int32_t s1 = (a.n_queries - s0) < kSuperChunk ? a.n_queries : s0 + kSuperChunk;
@@ -404,7 +418,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
       }
       sp.index_offset = a.index_offset;
       sp.flags = w.flags;
-      sp.pad_short = a.row_filter != nullptr;
+      sp.pad_short = a.pad_short();
       if (fused && sp.final_pass) {
         sp.g_role = 1; sp.g_world = a.g_world; sp.g_rank = a.g_rank;
         sp.g_peer_bufs = a.g_peer_bufs; sp.g_peer_flags = a.g_peer_flags;
@@ -431,7 +445,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
     sp.g_role = 2; sp.g_world = a.g_world; sp.g_rank = a.g_rank; sp.g_peer_bufs = a.g_peer_bufs; sp.g_peer_flags = a.g_peer_flags;
     sp.g_list_stride = a.g_list_stride; sp.g_status_index = a.n_queries * a.k;
     sp.g_epoch = w.gscratch; sp.g_counter = w.gscratch + 2; sp.g_status_out = w.gscratch + kGStatus;
-    sp.pad_short = a.row_filter != nullptr;
+    sp.pad_short = a.pad_short();
     rc = profiled_launch(3, 0, 0, stream, [&]() { return launch_select(sp, a.n_queries, stream); });
     if (rc != MMRS_OK) return rc;
   }
@@ -451,6 +465,7 @@ static int enqueue_exhaustive(const SearchArgs& a, const DeviceInfo& dev, const 
   base.cap = all_rows;
   base.sched = TileSchedule{pl.n_tiles, 1, 0, pl.n_tiles};
   base.row_filter = a.row_filter;
+  set_labels(base, a);   // one query per pass below, with that query's own label (query_labels[q0])
   MMRS_CUDA(cudaMemsetAsync(w.flags, 0, 8 * sizeof(int32_t), stream));
   {
     int rc = enqueue_prep(a, w, stream);
@@ -471,7 +486,7 @@ static int enqueue_exhaustive(const SearchArgs& a, const DeviceInfo& dev, const 
     sp.out_values = a.d_values + static_cast<int64_t>(q) * a.k;
     sp.out_indices = a.d_indices + static_cast<int64_t>(q) * a.k;
     sp.index_offset = a.index_offset; sp.flags = w.flags;
-    sp.pad_short = a.row_filter != nullptr;
+    sp.pad_short = a.pad_short();
     MMRS_LAUNCH(launch_select(sp, 1, stream));
   }
   return MMRS_OK;
@@ -498,8 +513,10 @@ struct GraphKey {
   int64_t g_stride; int32_t g_k_out; uint64_t g_timeout_ns;
   uint64_t knobs;   // the kernel-shape environment knobs the captured launches were configured with
   const void* row_filter;   // the captured scans read the bitmap through this pointer
+  const void* row_labels; const void* query_labels; int32_t label_match;   // and the labels through these
   bool operator==(const GraphKey& o) const {
-    return knobs == o.knobs && row_filter == o.row_filter && g_world == o.g_world && g_rank == o.g_rank && g_bufs == o.g_bufs && g_flags == o.g_flags &&
+    return knobs == o.knobs && row_filter == o.row_filter && row_labels == o.row_labels &&
+           query_labels == o.query_labels && label_match == o.label_match && g_world == o.g_world && g_rank == o.g_rank && g_bufs == o.g_bufs && g_flags == o.g_flags &&
            g_local_buf == o.g_local_buf && g_local_flags == o.g_local_flags && g_stride == o.g_stride && g_k_out == o.g_k_out &&
            g_timeout_ns == o.g_timeout_ns && has_values == o.has_values && has_indices == o.has_indices &&
            has_keys == o.has_keys && gallery == o.gallery && n_rows == o.n_rows && dim == o.dim && ld == o.ld &&
@@ -608,7 +625,8 @@ static int launch_search_graph(const SearchArgs& a, const DeviceInfo& dev, const
                dev.device, env_int("MMRS_RATIO_LOG2", -1), env_int("MMRS_DENSE_TILES", -1),
                a.d_values != nullptr, a.d_indices != nullptr, a.d_keys != nullptr,
                a.g_world, a.g_rank, a.g_peer_bufs, a.g_peer_flags, a.g_local_buf, a.g_local_flags, a.g_list_stride,
-               a.g_k_out, a.g_timeout_ns, knob_hash(), a.row_filter};
+               a.g_k_out, a.g_timeout_ns, knob_hash(), a.row_filter,
+               a.row_labels, a.row_labels ? a.query_labels : nullptr, a.row_labels ? a.label_match : 0};
   // the lock is held across patch + launch: an executable graph must not be updated or launched from
   // two threads at once (two threads sharing one workspace would be a caller bug anyway)
   std::lock_guard<std::mutex> lk(g_graph_mu);
@@ -684,6 +702,18 @@ static int check_row_filter(const uint32_t* f) {
   return MMRS_OK;
 }
 
+// d_row_labels == NULL: unlabeled (the other two are ignored)
+static int check_labels(const int32_t* row_labels, const int32_t* query_labels, int32_t label_match) {
+  if (!row_labels) return MMRS_OK;
+  if (!query_labels) return fail(MMRS_ERR_ARG, "row labels given without query labels");
+  if (reinterpret_cast<uintptr_t>(row_labels) % sizeof(int32_t) != 0 ||
+      reinterpret_cast<uintptr_t>(query_labels) % sizeof(int32_t) != 0)
+    return fail(MMRS_ERR_ARG, "label pointers must be 4-byte aligned");
+  if (label_match != MMRS_LABEL_SAME && label_match != MMRS_LABEL_OTHER)
+    return fail(MMRS_ERR_ARG, "label_match %d must be MMRS_LABEL_SAME or MMRS_LABEL_OTHER", label_match);
+  return MMRS_OK;
+}
+
 static int validate_search(const SearchArgs& a, const void* ws, size_t ws_bytes, size_t extra) {
   int rc = check_matrix(a.gallery, a.n_rows, a.dim, a.ld, a.dtype, "gallery");
   if (rc != MMRS_OK) return rc;
@@ -704,6 +734,11 @@ static int validate_search(const SearchArgs& a, const void* ws, size_t ws_bytes,
 }  // namespace mmrs
 
 using namespace mmrs;
+
+// the key merge of mmrs_topk_merge_keys_async / _padded_async (defined below)
+static int merge_keys(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
+                      int64_t list_stride, int32_t k_out, float* d_out_values, int64_t* d_out_indices,
+                      int32_t* d_status, int32_t* h_status, bool pad_short, void* stream_);
 
 extern "C" {
 
@@ -874,7 +909,20 @@ int mmrs_search_topk_exhaustive_filtered(const void* d_gallery, int64_t n_rows, 
                                          int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                                          int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
                                          void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
-                                         void* stream_) {
+                                         void* stream) {
+  return mmrs_search_topk_exhaustive_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
+                                             ld_queries, k, normalize_queries, scale, index_offset, d_out_values,
+                                             d_out_indices, d_workspace, workspace_bytes, d_row_filter, nullptr,
+                                             nullptr, 0, stream);
+}
+
+int mmrs_search_topk_exhaustive_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                        int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
+                                        void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
+                                        const int32_t* d_row_labels, const int32_t* d_query_labels,
+                                        int32_t label_match, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceInfo dev;
   int rc = current_device(&dev);
@@ -892,7 +940,10 @@ int mmrs_search_topk_exhaustive_filtered(const void* d_gallery, int64_t n_rows, 
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, MMRS_PATH_AUTO, d_out_values, d_out_indices};
   a.row_filter = d_row_filter;
+  a.row_labels = d_row_labels; a.query_labels = d_query_labels; a.label_match = label_match;
   rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
+  rc = check_labels(d_row_labels, d_query_labels, label_match);
   if (rc != MMRS_OK) return rc;
   rc = enqueue_exhaustive(a, dev, w, stream);
   if (rc != MMRS_OK) return rc;
@@ -949,10 +1000,26 @@ int mmrs_search_topk_async_filtered(const void* d_gallery, int64_t n_rows, int32
                                     int64_t index_offset, int32_t path, float* d_out_values,
                                     int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
                                     int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
+  return mmrs_search_topk_async_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
+                                        ld_queries, k, normalize_queries, scale, index_offset, path, d_out_values,
+                                        d_out_indices, d_workspace, workspace_bytes, h_status, d_row_filter, nullptr,
+                                        nullptr, 0, stream);
+}
+
+int mmrs_search_topk_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                   int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                   int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                   int64_t index_offset, int32_t path, float* d_out_values,
+                                   int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+                                   int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                   const int32_t* d_query_labels, int32_t label_match, void* stream) {
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, d_out_values, d_out_indices};
   a.row_filter = d_row_filter;
-  const int rc = check_row_filter(d_row_filter);
+  a.row_labels = d_row_labels; a.query_labels = d_query_labels; a.label_match = label_match;
+  int rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
+  rc = check_labels(d_row_labels, d_query_labels, label_match);
   if (rc != MMRS_OK) return rc;
   return search_enqueue(a, nullptr, nullptr, nullptr, d_workspace, workspace_bytes, h_status,
                         static_cast<cudaStream_t>(stream), nullptr, nullptr);
@@ -975,12 +1042,28 @@ int mmrs_search_topk_host_async_filtered(const void* d_gallery, int64_t n_rows, 
                                          int64_t index_offset, int32_t path, float* h_out_values,
                                          int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
                                          int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
+  return mmrs_search_topk_host_async_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, h_queries, n_queries,
+                                             ld_queries, k, normalize_queries, scale, index_offset, path, h_out_values,
+                                             h_out_indices, d_workspace, workspace_bytes, h_status, d_row_filter,
+                                             nullptr, nullptr, 0, stream);
+}
+
+int mmrs_search_topk_host_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                        int32_t gallery_dtype, const float* h_queries, int32_t n_queries,
+                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                        int64_t index_offset, int32_t path, float* h_out_values,
+                                        int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
+                                        int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                        const int32_t* d_query_labels, int32_t label_match, void* stream) {
   if (n_queries > 0 && !h_queries) return fail(MMRS_ERR_ARG, "null host query pointer");
-  const int rc = check_row_filter(d_row_filter);
+  int rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
+  rc = check_labels(d_row_labels, d_query_labels, label_match);
   if (rc != MMRS_OK) return rc;
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, nullptr, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, nullptr, nullptr};
   a.row_filter = d_row_filter;
+  a.row_labels = d_row_labels; a.query_labels = d_query_labels; a.label_match = label_match;
   static const float dummy = 0.f;
   if (n_queries == 0) h_queries = &dummy;
   return search_enqueue(a, h_queries, h_out_values, h_out_indices, d_workspace, workspace_bytes,
@@ -1004,8 +1087,23 @@ int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, 
                                          int64_t index_offset, int32_t path, uint64_t* d_out_keys,
                                          void* d_workspace, size_t workspace_bytes, int32_t* h_status,
                                          const uint32_t* d_row_filter, void* stream) {
+  return mmrs_search_topk_keys_async_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
+                                             ld_queries, k, normalize_queries, scale, index_offset, path, d_out_keys,
+                                             d_workspace, workspace_bytes, h_status, d_row_filter, nullptr, nullptr, 0,
+                                             stream);
+}
+
+int mmrs_search_topk_keys_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
+                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
+                                        int64_t index_offset, int32_t path, uint64_t* d_out_keys,
+                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status,
+                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                        const int32_t* d_query_labels, int32_t label_match, void* stream) {
   {
-    const int rc = check_row_filter(d_row_filter);
+    int rc = check_row_filter(d_row_filter);
+    if (rc != MMRS_OK) return rc;
+    rc = check_labels(d_row_labels, d_query_labels, label_match);
     if (rc != MMRS_OK) return rc;
   }
   if (index_offset < 0 || index_offset + n_rows > 0x100000000ll)
@@ -1014,6 +1112,7 @@ int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, 
                k, normalize_queries, scale, index_offset, path, nullptr, nullptr};
   a.d_keys = d_out_keys;
   a.row_filter = d_row_filter;
+  a.row_labels = d_row_labels; a.query_labels = d_query_labels; a.label_match = label_match;
   if (!d_out_keys) return fail(MMRS_ERR_ARG, "null key output pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   uint64_t* tail = d_out_keys + static_cast<int64_t>(n_queries < 0 ? 0 : n_queries) * k;
@@ -1030,7 +1129,24 @@ int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, 
 int mmrs_topk_merge_keys_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
                                int64_t list_stride, int32_t k_out, float* d_out_values,
                                int64_t* d_out_indices, int32_t* d_status, int32_t* h_status,
-                               void* stream_) {
+                               void* stream) {
+  return merge_keys(d_keys_in, n_lists, n_queries, k_in, list_stride, k_out, d_out_values, d_out_indices, d_status,
+                    h_status, false, stream);
+}
+
+int mmrs_topk_merge_keys_padded_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
+                                      int64_t list_stride, int32_t k_out, float* d_out_values,
+                                      int64_t* d_out_indices, int32_t* d_status, int32_t* h_status,
+                                      void* stream) {
+  return merge_keys(d_keys_in, n_lists, n_queries, k_in, list_stride, k_out, d_out_values, d_out_indices, d_status,
+                    h_status, true, stream);
+}
+
+}  // extern "C"
+
+static int merge_keys(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
+                      int64_t list_stride, int32_t k_out, float* d_out_values, int64_t* d_out_indices,
+                      int32_t* d_status, int32_t* h_status, bool pad_short, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceInfo dev;
   int rc = current_device(&dev);
@@ -1049,10 +1165,13 @@ int mmrs_topk_merge_keys_async(const uint64_t* d_keys_in, int32_t n_lists, int32
   sp.out_values = d_out_values; sp.out_indices = d_out_indices; sp.index_offset = 0; sp.flags = d_status;
   if (list_stride < static_cast<int64_t>(n_queries) * k_in) return fail(MMRS_ERR_ARG, "list_stride too small");
   sp.seg_len = k_in; sp.seg_stride = list_stride;
+  sp.pad_short = pad_short;
   MMRS_LAUNCH(launch_select(sp, n_queries, stream));
   MMRS_CUDA(cudaMemcpyAsync(h_status, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
   return MMRS_OK;
 }
+
+extern "C" {
 
 int mmrs_search_topk_fused_gather_async(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
@@ -1074,10 +1193,27 @@ int mmrs_search_topk_fused_gather_async_filtered(
     int32_t normalize_queries, float scale, int64_t index_offset, int32_t path, uint64_t* const* d_peer_bufs,
     uint32_t* const* d_peer_flags, uint64_t* d_local_buf, uint32_t* d_local_flags, int32_t rank, int32_t world,
     int64_t list_stride, float* d_out_values, int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-    int32_t* h_status, const uint32_t* d_row_filter, void* stream_) {
+    int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
+  return mmrs_search_topk_fused_gather_async_labeled(
+      d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries, k_local, k_out,
+      normalize_queries, scale, index_offset, path, d_peer_bufs, d_peer_flags, d_local_buf, d_local_flags, rank, world,
+      list_stride, d_out_values, d_out_indices, d_workspace, workspace_bytes, h_status, d_row_filter, nullptr, nullptr,
+      0, stream);
+}
+
+int mmrs_search_topk_fused_gather_async_labeled(
+    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
+    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
+    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path, uint64_t* const* d_peer_bufs,
+    uint32_t* const* d_peer_flags, uint64_t* d_local_buf, uint32_t* d_local_flags, int32_t rank, int32_t world,
+    int64_t list_stride, float* d_out_values, int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+    int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels, const int32_t* d_query_labels,
+    int32_t label_match, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   {
-    const int rc = check_row_filter(d_row_filter);
+    int rc = check_row_filter(d_row_filter);
+    if (rc != MMRS_OK) return rc;
+    rc = check_labels(d_row_labels, d_query_labels, label_match);
     if (rc != MMRS_OK) return rc;
   }
   if (world < 1 || world > kMaxWorld || rank < 0 || rank >= world || !d_peer_bufs || !d_peer_flags || !d_local_buf ||
@@ -1098,6 +1234,7 @@ int mmrs_search_topk_fused_gather_async_filtered(
   a.g_local_buf = d_local_buf; a.g_local_flags = d_local_flags;
   a.g_list_stride = list_stride; a.g_k_out = k_out; a.g_timeout_ns = gather_timeout_ns();
   a.row_filter = d_row_filter;
+  a.row_labels = d_row_labels; a.query_labels = d_query_labels; a.label_match = label_match;
   for (int r = 0; r <= world + 1; ++r) h_status[r] = 0;
   Workspace w{};
   // ONE graph: prep (epoch bump + ack wait) -> scans / selects -> producer select -> wait -> merge select

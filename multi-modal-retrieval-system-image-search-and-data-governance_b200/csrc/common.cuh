@@ -155,15 +155,22 @@ struct ScanParams {
   int64_t n_rows;
   int64_t ld;             // elements
   int32_t dim;
+  int32_t label_match;    // label-conditioned search: MMRS_LABEL_SAME / MMRS_LABEL_OTHER (see row_labels)
   const float* queries;   // prepared fp32 queries [*, ldq] (normalised, bf16-rounded in bf16 mode)
   int32_t ldq;
   int32_t q0;             // first query of this pass
   int32_t nq;             // queries in this pass (<= template QN)
   float scale;
   TileSchedule sched;
-  // kModeScores
-  float* out_scores;
-  int64_t ld_out;
+  // kModeScores.  The label pointers of a label-conditioned dense / filter launch share their storage:
+  // ScanParams keeps the 128-byte layout of the unlabeled search (growing it changed ptxas's register
+  // allocation of unlabeled kernels, DESIGN.md section 4).
+  //   row_labels: one label per local row, padded to whole tiles (nullptr = unlabeled)
+  //   query_labels: indexed by absolute query id
+  // A pair (row, query) is eligible iff label_ok (below).  Only the kernels' LABELED instantiations
+  // read them; the launchers pick those when row_labels != nullptr in kModeDense / kModeFilter.
+  union { float* out_scores; const int32_t* row_labels; };
+  union { int64_t ld_out; const int32_t* query_labels; };
   // kModeDense / kModeFilter
   uint64_t* cand;         // [n_queries, cap] keys
   uint32_t* cnt;          // [n_queries]
@@ -174,8 +181,13 @@ struct ScanParams {
   // nullptr = every row.  kModeScores ignores it.
   const uint32_t* row_filter;
 };
+static_assert(sizeof(ScanParams) == 128, "the unlabeled kernels were tuned with this parameter layout");
 
 __device__ __forceinline__ bool row_allowed(uint32_t word, int64_t row) { return (word >> (row & 31)) & 1u; }
+// query label < 0: every row; otherwise same: row label == query label, other: !=
+__device__ __forceinline__ bool label_ok(int32_t row_label, int32_t query_label, int32_t match_other) {
+  return query_label < 0 || ((row_label == query_label) != (match_other != 0));
+}
 
 struct SelectParams {
   uint64_t* cand;         // [n_queries, cap]

@@ -58,7 +58,9 @@ struct TransposeReduce {
 constexpr int kGemvThreads = 256;
 constexpr int kGemvWarps = kGemvThreads / 32;
 
-template <typename T, int QN, int R, int MODE>
+// LABELED: label-conditioned search (p.row_labels != nullptr, dense / filter modes only).  A separate
+// instantiation, so that the unlabeled kernels keep their code and registers.
+template <typename T, int QN, int R, int MODE, bool LABELED = false>
 __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanParams p) {
   constexpr int CH = Chunk<T>::CH;
   constexpr int H = CH / 4;  // float4 pieces of a query chunk
@@ -93,6 +95,10 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
   float my_thr = 0.f;
   if constexpr (MODE == kModeFilter) {
     if (owner) my_thr = p.thr[p.q0 + my_q];
+  }
+  int32_t my_label = -1;   // label-conditioned search: the owned query's label (< 0: no restriction)
+  if constexpr (LABELED) {
+    if (owner) my_label = __ldg(p.query_labels + p.q0 + my_q);
   }
 
   const T* __restrict__ gal = static_cast<const T*>(p.gallery);
@@ -160,6 +166,10 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
         bool row_ok = row <= last_row;
         if constexpr (MODE != kModeScores) {
           if (p.row_filter != nullptr) row_ok = row_ok && row_allowed(__ldg(p.row_filter + (row >> 5)), row);
+          // the labels cover whole tiles too
+          if constexpr (LABELED) {
+            if (my_label >= 0) row_ok = row_ok && label_ok(__ldg(p.row_labels + row), my_label, p.label_match);
+          }
         }
         if constexpr (MODE == kModeScores) {
           if (row_ok) p.out_scores[static_cast<int64_t>(q) * p.ld_out + row] = s;
@@ -199,10 +209,13 @@ static cudaError_t launch_gemv_mode(const ScanParams& p, int mode, int sm_count,
     if (grid < 1) grid = 1;
     return launch_pdl(kernel, dim3(grid), dim3(kGemvThreads), smem, stream, p);
   };
+  const bool labeled = p.row_labels != nullptr;
   switch (mode) {
     case kModeScores: return go(scan_gemv_kernel<T, QN, R, kModeScores>);
-    case kModeDense: return go(scan_gemv_kernel<T, QN, R, kModeDense>);
-    default: return go(scan_gemv_kernel<T, QN, R, kModeFilter>);
+    case kModeDense:
+      return labeled ? go(scan_gemv_kernel<T, QN, R, kModeDense, true>) : go(scan_gemv_kernel<T, QN, R, kModeDense>);
+    default:
+      return labeled ? go(scan_gemv_kernel<T, QN, R, kModeFilter, true>) : go(scan_gemv_kernel<T, QN, R, kModeFilter>);
   }
 }
 

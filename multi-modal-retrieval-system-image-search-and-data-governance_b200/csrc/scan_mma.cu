@@ -61,6 +61,13 @@ struct MmaSharedT {
   alignas(16) uint2 stash[EPI][kStash * 32];  // per epilogue thread: parked (column, score) pairs
 };
 
+// Label-conditioned launches keep their query labels in a tail behind the shared struct, laid out like
+// thr (column c of chunk ch at ch * kMaxQ + c); only they size it in, so an unlabeled launch keeps its
+// shared-memory footprint and its ring stages.  Slots of the tail:
+__host__ __device__ __forceinline__ int label_tail_slots(bool pair, int n_qchunks, int n_umma) {
+  return pair && n_qchunks > 1 ? n_qchunks * kMaxQ : n_umma;
+}
+
 struct MmaCfg {
   int32_t n_umma;        // UMMA N: queries of this pass rounded up to 16
   int32_t k_blocks;      // ceil(dim / 64)
@@ -81,7 +88,9 @@ struct MmaCfg {
 // SPLIT is a template parameter on purpose: with the operand-plane count a run-time value the single lane that
 // issues tcgen05.mma carried both code paths and the C5-shaped scan fell from 4.11 back to 4.67 ms per launch
 // (profiles/r02_prefetch_ab.log against r02_sticky_ab.log) -- that loop is issue-bound, every instruction counts.
-template <int MODE, int EPI_WARPS, bool PAIR, int SPLIT>
+// LABELED: label-conditioned search (p.row_labels != nullptr, dense / filter modes only), a separate
+// instantiation so that the unlabeled kernels keep their code and registers.
+template <int MODE, int EPI_WARPS, bool PAIR, int SPLIT, bool LABELED = false>
 __global__ void __launch_bounds__((kCtrlWarps + EPI_WARPS) * 32, EPI_WARPS == 8 ? 2 : 1)
 scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant__ CUtensorMap map_q,
                 const ScanParams p, const MmaCfg cfg, int32_t* flags) {
@@ -175,6 +184,8 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
   // exact test `scale * acc >= thr` before parking a candidate.  Non-positive scales keep the
   // multiply (raw_ok = false).
   const bool raw_ok = p.scale > 0.f;
+  constexpr bool labeled = LABELED && MODE != kModeScores;
+  int32_t* lab_s = reinterpret_cast<int32_t*>(sh + 1);                   // the label tail (labeled launches only)
   {
     const int first_q = PAIR ? p.q0 : p.q0 + static_cast<int>(blockIdx.y) * kMaxQ;
     const int n_q = PAIR ? p.nq : min(p.nq - static_cast<int>(blockIdx.y) * kMaxQ, kMaxQ);
@@ -188,6 +199,11 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
         tr = tr - fabsf(tr) * 4.8e-7f - 1e-37f;
       }
       sh->thr_raw[c] = tr;
+    }
+    if constexpr (labeled) {
+      const int n_lab = label_tail_slots(PAIR, cfg.n_qchunks, cfg.n_umma);
+      for (int c = threadIdx.x; c < n_lab; c += (kCtrlWarps + EPI_WARPS) * 32)
+        lab_s[c] = c < n_q ? __ldg(p.query_labels + first_q + c) : -1;   // padded columns never pass anyway
     }
   }
   tcgen05_fence_before();
@@ -360,6 +376,11 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
       if constexpr (MODE != kModeScores) {
         if (p.row_filter != nullptr) filter_word = __ldg(p.row_filter + (row >> 5));
       }
+      // label-conditioned: this thread's row label (whole tiles are readable), loaded here for the same
+      // reason -- one coalesced 128-byte load per warp
+      int32_t row_label = 0;
+      if constexpr (labeled) row_label = __ldg(p.row_labels + row);
+      const int32_t* lab_u = lab_s + (PAIR ? un.chunk * kMaxQ : 0);
       if (!mbar_wait(&sh->tmem_full[as], aphase, &sh->abort, flags)) break;
       tcgen05_fence_after();
       const bool row_ok = row <= last_row && row_allowed(filter_word, row);
@@ -403,7 +424,7 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
           }
           n_st = 0;
         };
-        auto process16 = [&](const uint32_t (&acc)[16], int c0) {
+        auto process16 = [&](const uint32_t (&acc)[16], int c0, uint32_t eligible) {
           // branch-free pass mask for the 16 columns (every taken branch would expose its full
           // latency), then a short loop over the set bits
           const float4* thr4 = reinterpret_cast<const float4*>((raw_ok ? thr_raw_s : thr_s) + c0);
@@ -420,6 +441,7 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
             }
           }
           if (!row_ok) bits = 0;
+          if constexpr (labeled) bits &= eligible;
           while (bits) {
             const int c = __ffs(bits) - 1;
             bits &= bits - 1;
@@ -433,15 +455,37 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
             ++n_st;
           }
         };
-        for (int c0 = c_begin; c0 < c_end; c0 += 32) {
+        // label-conditioned: which of 16 columns this thread's row may be returned for -- four broadcast
+        // 16-byte shared loads, like the thresholds; computed BEFORE the accumulator loads, while no
+        // accumulator register is live (the 8-warp variants have 80 registers)
+        auto label_mask16 = [&](int c0) -> uint32_t {
+          uint32_t m = 0;
+#pragma unroll
+          for (int c4 = 0; c4 < 4; ++c4) {
+            const int4 lq = reinterpret_cast<const int4*>(lab_u + c0)[c4];
+            const int32_t lv[4] = {lq.x, lq.y, lq.z, lq.w};
+#pragma unroll
+            for (int u4 = 0; u4 < 4; ++u4) m |= label_ok(row_label, lv[u4], p.label_match) ? (1u << (c4 * 4 + u4)) : 0u;
+          }
+          return m;
+        };
+        // the labeled small-pair variant (off by default) reads one 16-column load at a time: with two in
+        // flight it spilled
+        constexpr int kColStep = (labeled && EPI_WARPS == 8 && PAIR) ? 16 : 32;
+        for (int c0 = c_begin; c0 < c_end; c0 += kColStep) {
           uint32_t acc0[16], acc1[16];
-          const bool two = c0 + 16 < c_end;     // warp-uniform
+          const bool two = kColStep == 32 && c0 + 16 < c_end;     // warp-uniform
+          uint32_t elig0 = ~0u, elig1 = ~0u;
+          if constexpr (labeled) {
+            elig0 = label_mask16(c0);
+            if (two) elig1 = label_mask16(c0 + 16);
+          }
           __syncwarp();
           tmem_ld16(taddr0 + static_cast<uint32_t>(c0), acc0);
           if (two) tmem_ld16(taddr0 + static_cast<uint32_t>(c0 + 16), acc1);   // both loads in flight
           tmem_ld_wait();
-          process16(acc0, c0);
-          if (two) process16(acc1, c0 + 16);
+          process16(acc0, c0, elig0);
+          if (two) process16(acc1, c0 + 16, elig1);
         }
         // the accumulator is read out: hand it back to the MMA warp BEFORE waiting for the slot
         // atomics of the parked candidates (an L2 round trip that used to sit on the critical path
@@ -462,8 +506,9 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
           for (int c = 0; c < 16; ++c) {
             if (c0 + c < nq) {
               const float s = __uint_as_float(acc[c]) * p.scale;
+              const bool ok = row_ok && (!labeled || label_ok(row_label, lab_u[c0 + c], p.label_match));
               p.cand[static_cast<int64_t>(q0 + c0 + c) * p.cap + slot] =
-                  row_ok ? make_key(s, static_cast<uint32_t>(row)) : 0ull;
+                  ok ? make_key(s, static_cast<uint32_t>(row)) : 0ull;
             }
           }
         } else {
@@ -571,12 +616,17 @@ cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, in
   const size_t stage_bytes = split * (static_cast<size_t>(kABytes) + static_cast<size_t>(b_rows) * kBlockK * 2);
   const bool half_sm = small || small_pair;   // footprint of half an SM: two CTAs (of two searches) per SM
   const size_t shared_struct = half_sm ? sizeof(MmaSharedT<1, 8>) : (pair ? sizeof(MmaSharedT<kMaxQChunks>) : sizeof(MmaSharedT<1>));
-  const size_t budget = (half_sm ? 113 * 1024 : 227 * 1024) - shared_struct - 1024 - (half_sm ? 1024 : 0);
+  // label-conditioned launches add the label tail (the kernel's lab_s); unlabeled ones are sized as before
+  const bool labeled = mode != kModeScores && p.row_labels != nullptr;
+  const size_t label_tail =
+      labeled ? (static_cast<size_t>(label_tail_slots(pair, n_qchunks, cfg.n_umma)) * sizeof(int32_t) + 15) / 16 * 16 : 0;
+  const size_t budget =
+      (half_sm ? 113 * 1024 : 227 * 1024) - shared_struct - label_tail - 1024 - (half_sm ? 1024 : 0);
   int stages = static_cast<int>(budget / stage_bytes);
   if (stages > kMaxStages) stages = kMaxStages;
   if (stages < 2) return cudaErrorInvalidValue;
   cfg.stages = stages;
-  const size_t smem = 1024 + stage_bytes * stages + shared_struct;
+  const size_t smem = 1024 + stage_bytes * stages + shared_struct + label_tail;
 
   CUtensorMap map_g, map_q;
   if (static_cast<int64_t>(split) * p.n_rows > 0x7fffffffll - kBlockM) return cudaErrorInvalidValue;
@@ -626,42 +676,42 @@ cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, in
   if (small) {
     switch (mode) {
       case kModeScores: return go(scan_mma_kernel<kModeScores, 8, false, 1>);
-      case kModeDense: return go(scan_mma_kernel<kModeDense, 8, false, 1>);
-      default: return go(scan_mma_kernel<kModeFilter, 8, false, 1>);
+      case kModeDense: return labeled ? go(scan_mma_kernel<kModeDense, 8, false, 1, true>) : go(scan_mma_kernel<kModeDense, 8, false, 1>);
+      default: return labeled ? go(scan_mma_kernel<kModeFilter, 8, false, 1, true>) : go(scan_mma_kernel<kModeFilter, 8, false, 1>);
     }
   }
   if (small_pair) {
     switch (mode) {   // 65..128 queries: CTA pairs with the footprint of half an SM
       case kModeScores: return go(scan_mma_kernel<kModeScores, 8, true, 1>);
-      case kModeDense: return go(scan_mma_kernel<kModeDense, 8, true, 1>);
-      default: return go(scan_mma_kernel<kModeFilter, 8, true, 1>);
+      case kModeDense: return labeled ? go(scan_mma_kernel<kModeDense, 8, true, 1, true>) : go(scan_mma_kernel<kModeDense, 8, true, 1>);
+      default: return labeled ? go(scan_mma_kernel<kModeFilter, 8, true, 1, true>) : go(scan_mma_kernel<kModeFilter, 8, true, 1>);
     }
   }
   if (pair && split == 1) {
     switch (mode) {   // > 128 queries: one CTA per SM, CTA pairs, 16 epilogue warps each
       case kModeScores: return go(scan_mma_kernel<kModeScores, 16, true, 1>);
-      case kModeDense: return go(scan_mma_kernel<kModeDense, 16, true, 1>);
-      default: return go(scan_mma_kernel<kModeFilter, 16, true, 1>);
+      case kModeDense: return labeled ? go(scan_mma_kernel<kModeDense, 16, true, 1, true>) : go(scan_mma_kernel<kModeDense, 16, true, 1>);
+      default: return labeled ? go(scan_mma_kernel<kModeFilter, 16, true, 1, true>) : go(scan_mma_kernel<kModeFilter, 16, true, 1>);
     }
   }
   if (pair) {
     switch (mode) {   // fp32 emulation, 49..128 queries: CTA pairs, three planes per operand
       case kModeScores: return go(scan_mma_kernel<kModeScores, 16, true, 3>);
-      case kModeDense: return go(scan_mma_kernel<kModeDense, 16, true, 3>);
-      default: return go(scan_mma_kernel<kModeFilter, 16, true, 3>);
+      case kModeDense: return labeled ? go(scan_mma_kernel<kModeDense, 16, true, 3, true>) : go(scan_mma_kernel<kModeDense, 16, true, 3>);
+      default: return labeled ? go(scan_mma_kernel<kModeFilter, 16, true, 3, true>) : go(scan_mma_kernel<kModeFilter, 16, true, 3>);
     }
   }
   if (split == 3) {
     switch (mode) {   // fp32 emulation, up to 48 queries
       case kModeScores: return go(scan_mma_kernel<kModeScores, 16, false, 3>);
-      case kModeDense: return go(scan_mma_kernel<kModeDense, 16, false, 3>);
-      default: return go(scan_mma_kernel<kModeFilter, 16, false, 3>);
+      case kModeDense: return labeled ? go(scan_mma_kernel<kModeDense, 16, false, 3, true>) : go(scan_mma_kernel<kModeDense, 16, false, 3>);
+      default: return labeled ? go(scan_mma_kernel<kModeFilter, 16, false, 3, true>) : go(scan_mma_kernel<kModeFilter, 16, false, 3>);
     }
   }
   switch (mode) {   // MMRS_K2_NO_PAIR / MMRS_K2_BIG_SMEM
     case kModeScores: return go(scan_mma_kernel<kModeScores, 16, false, 1>);
-    case kModeDense: return go(scan_mma_kernel<kModeDense, 16, false, 1>);
-    default: return go(scan_mma_kernel<kModeFilter, 16, false, 1>);
+    case kModeDense: return labeled ? go(scan_mma_kernel<kModeDense, 16, false, 1, true>) : go(scan_mma_kernel<kModeDense, 16, false, 1>);
+    default: return labeled ? go(scan_mma_kernel<kModeFilter, 16, false, 1, true>) : go(scan_mma_kernel<kModeFilter, 16, false, 1>);
   }
 }
 

@@ -17,6 +17,7 @@ import torch
 from . import _cabi
 from .gallery import DeviceGallery, _pad_dim
 from .row_filter import RowFilter, filter_words, pack_mask
+from .row_labels import RowLabels, label_match_arg, query_labels_arg
 
 # module-level configuration with the reference's names (code/search_image.py:14-38); scripts
 # that `from search_image import *` and set these keep working
@@ -96,10 +97,12 @@ class PendingSearch:
 
 
 def _search_exhaustive(gal: DeviceGallery, q: torch.Tensor, k: int, normalize_queries: bool, scale: float,
-                       path: str, values: torch.Tensor, indices: torch.Tensor, row_filter_ptr: int = 0) -> None:
+                       path: str, values: torch.Tensor, indices: torch.Tensor, row_filter_ptr: int = 0,
+                       labels=None) -> None:
     """The exact fallback for a batch whose candidate lists overflowed (MMRS_ERR_RETRY): every row a
     key, one query at a time.  Its 8-bytes-per-row workspace lives only for this call.
-    `row_filter_ptr`: device bitmap of the allowed rows (0 = all)."""
+    `row_filter_ptr`: device bitmap of the allowed rows (0 = all).  `labels`: None, or (RowLabels,
+    device int32 query labels [Q], label_match code) -- each query is re-run with its own label."""
     lib = _cabi.lib
     dev = gal.device
     nq = int(q.shape[0])
@@ -113,7 +116,11 @@ def _search_exhaustive(gal: DeviceGallery, q: torch.Tensor, k: int, normalize_qu
         args = (g_ptr, gal.n_rows, gal.padded_dim, g_ld, g_dtype, qd.data_ptr(), nq, qd.stride(0), k,
                 int(bool(normalize_queries)), float(scale), gal.row_offset, dv.data_ptr(), di.data_ptr(),
                 DeviceGallery.aligned_ptr(ws), ws_bytes)
-        if row_filter_ptr:
+        if labels is not None:
+            row_labels, ql, match = labels
+            _cabi.check(lib.mmrs_search_topk_exhaustive_labeled(*args, row_filter_ptr, row_labels.labels.data_ptr(),
+                                                                ql.data_ptr(), match, _stream_handle(dev)))
+        elif row_filter_ptr:
             _cabi.check(lib.mmrs_search_topk_exhaustive_filtered(*args, row_filter_ptr, _stream_handle(dev)))
         else:
             _cabi.check(lib.mmrs_search_topk_exhaustive(*args, _stream_handle(dev)))
@@ -142,9 +149,42 @@ def _filter_arg(row_filter, gal: DeviceGallery):
     return row_filter
 
 
+def _labels_arg(row_labels, query_labels, label_match, gal: DeviceGallery, nq: int):
+    """(RowLabels, query labels tensor as given, label_match code) checked against the gallery, or None."""
+    if row_labels is None and query_labels is None:
+        if label_match != "same":
+            label_match_arg(label_match)         # a typo still raises
+        return None
+    if row_labels is None or query_labels is None:
+        raise ValueError("row_labels and query_labels come together")
+    match = label_match_arg(label_match)
+    if not isinstance(row_labels, RowLabels):
+        raise ValueError(f"row_labels must be a RowLabels, got {type(row_labels).__name__}")
+    if row_labels.n_rows != gal.n_rows:
+        raise ValueError(f"row_labels covers {row_labels.n_rows} rows, the gallery has {gal.n_rows}")
+    if row_labels.device != gal.device:
+        raise ValueError(f"row_labels is on {row_labels.device}, the gallery on {gal.device}")
+    return row_labels, query_labels_arg(query_labels, nq, gal.device), match
+
+
+def _stage_query_labels(slot, ql: torch.Tensor, dev: torch.device):
+    """Copy this call's query labels into the slot's own device int32 buffer on the current stream (a
+    stable pointer: the slot keeps replaying one graph while the labels change per call).  Host labels
+    go through pinned memory with a plain asynchronous copy.  -> (slot buffer, copy source to keep alive)."""
+    n = int(ql.numel())
+    buf = slot.extra.get("query_labels")
+    if buf is None or buf.numel() != n:
+        buf = slot.extra["query_labels"] = torch.empty(n, dtype=torch.int32, device=dev)
+    src = ql.to(torch.int32)
+    if not src.is_cuda:
+        src = src.contiguous().pin_memory()
+    buf.copy_(src, non_blocking=True)
+    return buf, src
+
+
 def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: bool = True,
                 scale: float = 1.0, mode: Optional[str] = None, path: str = "auto", sync: bool = True,
-                out=None, row_filter=None):
+                out=None, row_filter=None, row_labels=None, query_labels=None, label_match: str = "same"):
     """Per-query top-k of `scale * q @ G.T` without materialising the score matrix.
 
     Returns `(values [Q, k] fp32 descending, indices [Q, k] int64)` exactly like
@@ -160,6 +200,13 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
     is the top-k of `gallery[mask]` with indices of the full gallery; `k` may not exceed the allowed
     rows.  A RowFilter costs one graph capture per slot; a mask is packed into a buffer of the slot on
     every call (and its allowed count read back: one host sync).
+    `row_labels` (a RowLabels over the gallery's rows) with `query_labels` (an integer tensor [Q], host or
+    device) makes the search label-conditioned: query q with c = query_labels[q] >= 0 sees only the rows
+    whose label equals c (`label_match="same"`) or differs from c (`"other"`: hard negatives); c < 0 is
+    the unlabeled search of that query, bit for bit.  With a `row_filter` too, a row must pass both.
+    Unlike `row_filter`'s `k > allowed` error, a query with fewer than k eligible rows (a small class, a
+    label absent from the gallery) is padded: positions n_eligible .. k-1 hold value -inf, index -1.
+    The labels are copied into a buffer of the slot on every call (no host sync, one graph per slot).
     """
     gal = _as_gallery(gallery, mode)
     q, on_host = _prep_queries(queries, gal)
@@ -170,6 +217,7 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
     if k > gal.n_rows:
         raise RuntimeError("selected index k out of range")  # torch.topk's message
     filt = _filter_arg(row_filter, gal)
+    labels = _labels_arg(row_labels, query_labels, label_match, gal, nq)
     if isinstance(filt, RowFilter) and k > filt.n_allowed:
         raise RuntimeError("selected index k out of range")
     lib = _cabi.lib
@@ -210,29 +258,42 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
         if k > int(pack_mask(filt, words).item()):
             raise RuntimeError("selected index k out of range")
         filt_ptr = words.data_ptr()
+    if labels is not None:
+        # by the time a retry runs the slot buffer may hold a later call's labels: redo keeps its own copy
+        staged, src = _stage_query_labels(slot, labels[1], dev)
+        labels = (labels[0], staged, labels[2], labels[1], src)
     g_ptr, g_ld, g_dtype = _operand(gal, nq, path)
     args = (g_ptr, gal.n_rows, gal.padded_dim, g_ld, g_dtype,
             q.data_ptr(), nq, q.stride(0), k, int(bool(normalize_queries)), float(scale),
             gal.row_offset, _cabi.PATHS[path], values.data_ptr(), indices.data_ptr(), slot.ptr, slot.nbytes)
 
     def redo(v, i):
+        lab = None
+        if labels is not None:
+            # this call's own labels (the slot buffer may hold a later call's by now)
+            lab = (labels[0], labels[3].to(device=dev, dtype=torch.int32).contiguous(), labels[2])
         if filt is None:
-            _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i)
+            _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i, 0, lab)
         else:
             # by now the slot's bitmap may hold a later call's mask: repack this call's own
             f = filt if isinstance(filt, RowFilter) else RowFilter(filt)
-            _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i, f.words.data_ptr())
+            _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i, f.words.data_ptr(), lab)
 
-    if filt is not None:
+    if filt is not None or labels is not None:
         ticket, status, event = slot.acquire()
-        fn = lib.mmrs_search_topk_host_async_filtered if on_host else lib.mmrs_search_topk_async_filtered
-        st = fn(*args, status.data_ptr(), filt_ptr, stream.cuda_stream)
+        if labels is None:
+            fn = lib.mmrs_search_topk_host_async_filtered if on_host else lib.mmrs_search_topk_async_filtered
+            st = fn(*args, status.data_ptr(), filt_ptr, stream.cuda_stream)
+        else:
+            fn = lib.mmrs_search_topk_host_async_labeled if on_host else lib.mmrs_search_topk_async_labeled
+            st = fn(*args, status.data_ptr(), filt_ptr, labels[0].labels.data_ptr(), labels[1].data_ptr(), labels[2],
+                    stream.cuda_stream)
         if st != _cabi.OK:
             slot.release(ticket)
             _cabi.check(st)
         event.record(stream)
         pend = PendingSearch(values, indices, slot, ticket, status, event, redo)
-        pend._keepalive = (q, filt)
+        pend._keepalive = (q, filt, labels)
         return pend.wait() if sync else pend
     if sync:
         fn = lib.mmrs_search_topk_host if on_host else lib.mmrs_search_topk

@@ -21,6 +21,7 @@ import torch.distributed as dist
 from . import _cabi
 from .gallery import DeviceGallery
 from .row_filter import RowFilter
+from .row_labels import RowLabels, label_match_arg, query_labels_arg
 
 
 def shard_bounds(n_rows: int, world: int, align: int = 128) -> list[tuple[int, int]]:
@@ -179,7 +180,7 @@ class ShardedGallery:
                 torch.empty((nq, k), dtype=torch.int64, device=dev), None, None)
 
     def _search_topk_keys(self, queries, k: int, normalize_queries: bool, scale: float, path: str, out=None,
-                          local_filter: Optional[RowFilter] = None):
+                          local_filter: Optional[RowFilter] = None, labels=None):
         """CUDA fast path: local top-k as packed 64-bit keys -> ONE all-gather (Q*k*8 bytes per rank)
         -> merge kernel reading the gathered buffer in place.  Nothing synchronises with the host
         until the final status check.  Shards shorter than k pad their lists with key 0, and so does a
@@ -206,12 +207,20 @@ class ShardedGallery:
         dv, di, hv, hi = self._results(slot, nq, k, dev, on_host, out)
         ticket, status, event = slot.acquire()
         shard_status = None
+        staged = None
+        if labels is not None:
+            from .search import _stage_query_labels
+            staged = _stage_query_labels(slot, labels[1], dev)
         if nq:
             dst = buf if short is None else short
             args = (gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
                     q.data_ptr(), nq, q.stride(0), k_local, int(bool(normalize_queries)), float(scale),
                     gal.row_offset, _cabi.PATHS[path], dst.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr())
-            if local_filter is None:
+            filt_ptr = local_filter.words.data_ptr() if local_filter is not None else 0
+            if labels is not None:   # a query with fewer than k eligible rows here: its list is padded with key 0
+                st = lib.mmrs_search_topk_keys_async_labeled(*args, filt_ptr, labels[0].labels.data_ptr(),
+                                                             staged[0].data_ptr(), labels[2], stream.cuda_stream)
+            elif local_filter is None:
                 st = lib.mmrs_search_topk_keys_async(*args, stream.cuda_stream)
             else:
                 st = lib.mmrs_search_topk_keys_async_filtered(*args, local_filter.words.data_ptr(), stream.cuda_stream)
@@ -223,9 +232,10 @@ class ShardedGallery:
                 buf[-1] = short[-1]
         dist.all_gather_into_tensor(gathered.view(-1), buf, group=self.group)      # [world, nq*k + 1]
         if nq:
-            _cabi.check(lib.mmrs_topk_merge_keys_async(gathered.data_ptr(), self.world, nq, k, n_keys + 1, k,
-                                                       dv.data_ptr(), di.data_ptr(), d_status.data_ptr(),
-                                                       status[1:].data_ptr(), stream.cuda_stream))
+            # labeled: fewer than k eligible rows over all ranks is legitimate -> -inf / -1
+            merge = lib.mmrs_topk_merge_keys_padded_async if labels is not None else lib.mmrs_topk_merge_keys_async
+            _cabi.check(merge(gathered.data_ptr(), self.world, nq, k, n_keys + 1, k, dv.data_ptr(), di.data_ptr(),
+                              d_status.data_ptr(), status[1:].data_ptr(), stream.cuda_stream))
             table = slot.extra.get("shard_status")          # one pinned row per status ticket of the slot
             if table is None or table.shape[0] <= ticket:
                 table = slot.extra["shard_status"] = torch.zeros((max(ticket + 1, slot.N_STATUS), self.world),
@@ -255,7 +265,7 @@ class ShardedGallery:
             _cabi.check(merge_rc)
             return res
 
-        finish._keepalive = (q, keep, local_filter)
+        finish._keepalive = (q, keep, local_filter, labels, staged)
         return finish
 
     # ---- search fused with its all-gather over NVLink peer memory -----------------------------------
@@ -283,7 +293,7 @@ class ShardedGallery:
         return st
 
     def _search_topk_fused(self, queries, k: int, normalize_queries: bool, scale: float, path: str, out=None,
-                           local_filter: Optional[RowFilter] = None):
+                           local_filter: Optional[RowFilter] = None, labels=None):
         """Local scan -> last select stores its keys into EVERY rank's buffer over NVLink and raises
         a ready flag -> a one-warp kernel waits for all flags -> merge select.  One library call, one
         graph replay, no NCCL, no host sync until the final status check; every buffer the call
@@ -300,13 +310,21 @@ class ShardedGallery:
         st = self._fused_state(slot, nq, k_local)         # collective on first use of the slot
         q, on_host, keep = self._stage_queries(slot, queries)
         dv, di, hv, hi = self._results(slot, nq, k, dev, on_host, out)
+        staged = None
+        if labels is not None:
+            from .search import _stage_query_labels
+            staged = _stage_query_labels(slot, labels[1], dev)
         ticket, status, event = slot.acquire()
         args = (gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
                 q.data_ptr(), nq, q.stride(0), k_local, k, int(bool(normalize_queries)), float(scale),
                 gal.row_offset, _cabi.PATHS[path], st["bufs"].data_ptr(), st["flags"].data_ptr(),
                 st["t"].data_ptr(), st["local_flags"], self.rank, self.world, st["stride"],
                 dv.data_ptr(), di.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr())
-        if local_filter is None:
+        if labels is not None:   # the merge select pads queries with fewer than k eligible rows with -inf / -1
+            rc = lib.mmrs_search_topk_fused_gather_async_labeled(
+                *args, local_filter.words.data_ptr() if local_filter is not None else 0, labels[0].labels.data_ptr(),
+                staged[0].data_ptr(), labels[2], stream.cuda_stream)
+        elif local_filter is None:
             rc = lib.mmrs_search_topk_fused_gather_async(*args, stream.cuda_stream)
         else:   # a shard with fewer than k allowed rows still stores k keys (padded with key 0)
             rc = lib.mmrs_search_topk_fused_gather_async_filtered(*args, local_filter.words.data_ptr(), stream.cuda_stream)
@@ -330,7 +348,7 @@ class ShardedGallery:
             _cabi.check(rc)
             return (hv, hi) if on_host else (dv, di)
 
-        finish._keepalive = (q, keep, local_filter)
+        finish._keepalive = (q, keep, local_filter, labels, staged)
         return finish
 
     def _local_filter(self, row_filter):
@@ -344,15 +362,44 @@ class ShardedGallery:
         lo = self.local.row_offset
         return f, f.shard(lo, lo + len(self.local))
 
+    def _local_labels(self, row_labels, query_labels, label_match, queries):
+        """(RowLabels over this rank's rows -- a view of the global one --, query labels as given, label_match
+        code), or None when unlabeled.  Checked alike on every rank, before any collective."""
+        if row_labels is None and query_labels is None:
+            label_match_arg(label_match)
+            return None
+        if row_labels is None or query_labels is None:
+            raise ValueError("row_labels and query_labels come together")
+        match = label_match_arg(label_match)
+        if not isinstance(row_labels, RowLabels):
+            raise ValueError(f"row_labels must be a RowLabels, got {type(row_labels).__name__}")
+        if row_labels.n_rows != self.n_rows_global:
+            raise ValueError(f"row_labels covers {row_labels.n_rows} rows, the sharded gallery has {self.n_rows_global}")
+        dev = getattr(self.local, "device", None)
+        if dev is not None and row_labels.device != dev:
+            raise ValueError(f"row_labels is on {row_labels.device}, this rank's shard on {dev}")
+        nq = 1 if len(queries.shape) == 1 else int(queries.shape[0])
+        ql = query_labels_arg(query_labels, nq, dev)
+        lo = self.local.row_offset
+        return row_labels.shard(lo, lo + len(self.local)), ql, match
+
     def search_topk(self, queries: torch.Tensor, k: int, *, normalize_queries: bool = True,
-                    scale: float = 1.0, path: str = "auto", sync: bool = True, out=None, row_filter=None):
+                    scale: float = 1.0, path: str = "auto", sync: bool = True, out=None, row_filter=None,
+                    row_labels=None, query_labels=None, label_match: str = "same"):
         """Global top-k, identical on every rank.  `queries` must be the same on all ranks.
         `sync=False` returns an object whose `.wait()` yields `(values, indices)`, so that several
         batches (and their all-gathers) can be in flight.  `out=(values, indices)`: caller-owned result
         tensors (pinned host tensors for host queries).  `row_filter`: a RowFilter (or bool mask) over the
-        GLOBAL rows, the same on every rank like the queries; each rank searches its slice of it."""
+        GLOBAL rows, the same on every rank like the queries; each rank searches its slice of it.
+        `row_labels` (a RowLabels over the GLOBAL rows) / `query_labels` / `label_match`: label-conditioned
+        search as in `search_topk`, the same on every rank (query labels replicated like the queries); a
+        query with fewer than k eligible rows over all shards is padded with -inf / -1."""
         if k > self.n_rows_global:
             raise RuntimeError("selected index k out of range")
+        if isinstance(queries, np.ndarray):
+            queries = torch.from_numpy(queries)
+        labels = self._local_labels(row_labels, query_labels, label_match, queries)
+        lab_kw = dict(row_labels=row_labels, query_labels=query_labels, label_match=label_match)
         local_filter = None
         if row_filter is not None:
             row_filter, local_filter = self._local_filter(row_filter)
@@ -366,34 +413,39 @@ class ShardedGallery:
             nq = int(queries.shape[0])
             if nq == 0:
                 out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path,
-                                                 row_filter=row_filter)
+                                                 row_filter=row_filter, **lab_kw)
                 return out_t if sync else _PendingSharded(lambda: out_t, None)
             # fused NVLink gather: every rank contributes its full top-k (needs >= k rows in every shard)
             fused = self._fused_ok and 1 <= nq <= 1024 and self.min_shard_rows >= k
             finish = None
             if fused:
                 try:
-                    finish = self._search_topk_fused(queries, k, normalize_queries, scale, path, out, local_filter)
+                    finish = self._search_topk_fused(queries, k, normalize_queries, scale, path, out, local_filter, labels)
                 except (ImportError, AttributeError, RuntimeError) as e:   # no symmetric memory here
                     if isinstance(e, _cabi.MmrsError):
                         raise
                     self._fused_ok = False
             if finish is None:
-                finish = self._search_topk_keys(queries, k, normalize_queries, scale, path, out, local_filter)
+                finish = self._search_topk_keys(queries, k, normalize_queries, scale, path, out, local_filter, labels)
             general = lambda: self.search_topk_general(queries, k, normalize_queries=normalize_queries,
-                                                       scale=scale, path=path, row_filter=row_filter)
+                                                       scale=scale, path=path, row_filter=row_filter, **lab_kw)
             pend = _PendingSharded(finish, general)
             return pend.wait() if sync else pend
         out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path,
-                                         row_filter=row_filter)
+                                         row_filter=row_filter, **lab_kw)
         return out_t if sync else _PendingSharded(lambda: out_t, None)
 
     def search_topk_general(self, queries: torch.Tensor, k: int, *, normalize_queries: bool = True,
-                            scale: float = 1.0, path: str = "auto", row_filter=None):
+                            scale: float = 1.0, path: str = "auto", row_filter=None, row_labels=None,
+                            query_labels=None, label_match: str = "same"):
         """(values, indices) lists, two all-gathers, merge -- also the path every rank takes together
         when some rank's candidate list overflowed (None from the fast path on EVERY rank alike: the
         shard statuses were gathered with the keys).  With a `row_filter` a rank searches for
-        min(k, its allowed rows) and one without allowed rows skips its local search."""
+        min(k, its allowed rows) and one without allowed rows skips its local search.  Labeled: positions
+        that no rank could fill hold -inf / -1, as on one GPU."""
+        if isinstance(queries, np.ndarray):
+            queries = torch.from_numpy(queries)
+        labels = self._local_labels(row_labels, query_labels, label_match, queries)
         n_local = len(self.local)
         k_local = min(k, n_local)
         local_filter = None
@@ -406,12 +458,12 @@ class ShardedGallery:
         if self._fast and self.world > 1 and not (isinstance(queries, torch.Tensor) and queries.is_cuda):
             on_host = True                    # NCCL gathers device tensors: search on the device, copy back
             queries = torch.as_tensor(queries).to(self.local.device)
-        if local_filter is None:
+        kw = {} if local_filter is None else {"row_filter": local_filter}
+        if labels is not None:
+            kw.update(row_labels=labels[0], query_labels=labels[1], label_match=label_match)
+        if local_filter is None or k_local > 0:
             v, i = self._search(queries, self.local, k_local, normalize_queries=normalize_queries,
-                                scale=scale, path=path)
-        elif k_local > 0:
-            v, i = self._search(queries, self.local, k_local, normalize_queries=normalize_queries,
-                                scale=scale, path=path, row_filter=local_filter)
+                                scale=scale, path=path, **kw)
         else:                                 # no allowed row here: contribute padding only
             nq = 1 if len(queries.shape) == 1 else int(queries.shape[0])
             dev = getattr(self.local, "device", torch.device("cpu"))
@@ -424,9 +476,19 @@ class ShardedGallery:
             pad = k - k_local
             v = torch.cat([v, torch.full((v.shape[0], pad), float("-inf"), dtype=v.dtype, device=v.device)], 1)
             i = torch.cat([i, torch.full((i.shape[0], pad), 2 ** 32 - 1, dtype=i.dtype, device=i.device)], 1)
+        if labels is not None:
+            # labeled, a query may have fewer than k eligible rows over ALL ranks, so padding can reach the
+            # merged result: every padded position (the local search's -1, the sentinel above) gets its own
+            # sentinel 2^32 - 1 - (rank * k + position), so that the merge sees unique keys, and the merged
+            # -inf positions become the public -1
+            pad = (i < 0) | (i == 2 ** 32 - 1)
+            sentinel = 2 ** 32 - 1 - (self.rank * k + torch.arange(k, dtype=i.dtype, device=i.device))
+            i = torch.where(pad, sentinel.expand_as(i), i)
         gv = _all_gather(v, self.world, self.group)
         gi = _all_gather(i, self.world, self.group)
         mv, mi = self._merge(gv, gi, k)
+        if labels is not None:
+            mi = torch.where(mv == float("-inf"), torch.full_like(mi, -1), mi)
         return (mv.cpu(), mi.cpu()) if on_host else (mv, mi)
 
     def find_duplicate_pairs(self, emb_full: torch.Tensor, threshold: float, raw_join: Optional[Callable] = None):
