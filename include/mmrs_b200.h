@@ -19,6 +19,9 @@
  *                         tool/delete repeated.py:127-135 (pairwise join loop), with the
  *                         predicate cos(e_i, e_j) >= tau named by BASELINE.json
  *   mmrs_threshold_sweep  code/search_image.py:39-79 (eval_threshold / find_thresholds)
+ *   mmrs_score_range_batched + mmrs_threshold_sweep_batched
+ *                         code/search_image.py:382-389 (the per-class loop of get_similarity :105-117 +
+ *                         find_thresholds :58-79) for every class prototype of a batch at once
  *
  * Conventions
  *   - every function returns an int status: 0 = ok, negative = error (table below);
@@ -480,6 +483,39 @@ int mmrs_threshold_sweep_labeled(const float* d_scores, const int64_t* d_targets
                                  double* d_out_thresholds,
                                  int64_t* d_out_counts, void* d_workspace, size_t workspace_bytes,
                                  void* stream);
+
+/*
+ * Per-class threshold tuning for a batch of class prototypes (code/search_image.py:382-389: for each
+ * class c, get_similarity :105-117 splits the scores by targets == c, find_thresholds :58-79 sweeps a
+ * 200-point np.linspace(min, max) grid) with the scores of the whole batch on the device: d_scores is
+ * [n_queries, ld_scores] fp32 (e.g. mmrs_full_scores of the prototypes), d_row_filter (nullable) the
+ * row-filter bitmap of the gallery (bit r & 31 of word r >> 5 set = row r allowed); a filtered-out row is
+ * neither in the range nor counted.
+ *
+ * mmrs_score_range_batched: each query's order-preserving (min, max) over the allowed rows, -0.0 counted
+ * as +0.0 (the key of x is x's bits with the sign bit flipped for x >= 0 and all bits flipped for x < 0).
+ * d_range [n_queries, 2] uint32 is ACCUMULATED with min / max, so initialise it to {0xffffffff, 0}; ranges
+ * of several row shards combine with a MIN / MAX reduction.  Replaces min(pos_res, neg_res) / max (:59-60).
+ *
+ * mmrs_threshold_sweep_batched: per query q, the grid np.linspace(min_q, max_q, n_thresholds) of d_range
+ * built as mmrs_threshold_sweep_labeled builds it (grid_f32 as there) into d_out_thresholds [n_queries,
+ * n_thresholds] fp64, and d_out_counts [n_queries, n_thresholds, 2] int64 = (#pos >= t, #neg >= t) where
+ * the positives of q are the allowed rows r with d_row_labels[r] == d_query_labels[q] (int32 each) and
+ * the negatives every other allowed row (get_similarity's pos_res / neg_res, :111-116); d_out_n_pos
+ * [n_queries] int64 = the positives of q.  Counts and n_pos of several row shards add up when every
+ * shard sweeps the same grid (the reduced range).  Workspace:
+ * mmrs_threshold_sweep_batched_workspace_bytes(n_queries, n_thresholds).  Both calls are asynchronous on
+ * `stream`.
+ */
+size_t mmrs_threshold_sweep_batched_workspace_bytes(int32_t n_queries, int32_t n_thresholds);
+int mmrs_score_range_batched(const float* d_scores, int64_t ld_scores, int32_t n_queries, int64_t n_rows,
+                             const uint32_t* d_row_filter, uint32_t* d_range, void* stream);
+int mmrs_threshold_sweep_batched(const float* d_scores, int64_t ld_scores, int32_t n_queries, int64_t n_rows,
+                                 const int32_t* d_row_labels, const int32_t* d_query_labels,
+                                 const uint32_t* d_row_filter, const uint32_t* d_range,
+                                 int32_t n_thresholds, int32_t grid_f32, double* d_out_thresholds,
+                                 int64_t* d_out_counts, int64_t* d_out_n_pos, void* d_workspace,
+                                 size_t workspace_bytes, void* stream);
 
 /* ---- measurement hooks (bench.py; not needed by a product caller) --------------------------- */
 

@@ -21,7 +21,8 @@ functions for this path (same names, positional order and return tuples):
 
 plus the tensor-level entry points they sit on: search_topk, full_scores, find_duplicate_pairs,
 DeviceGallery, ShardedGallery, RowFilter (row-filtered search_topk: leave rows out per call) and
-RowLabels (label-conditioned search_topk: each query searches the rows of its own class, or of every other).  Everything computes through the C-ABI CUDA library
+RowLabels (label-conditioned search_topk: each query searches the rows of its own class, or of every other)
+and best_thresholds (the best-F1 threshold of every class prototype of a batch, find_thresholds per class).  Everything computes through the C-ABI CUDA library
 (include/mmrs_b200.h); there is no CPU path -- without a B200 the calls raise.
 """
 from . import _cabi  # noqa: F401  (fails loudly when the CUDA library is missing)
@@ -36,9 +37,10 @@ from .search import (best_threshold_on_device, calc_combined_metrics, cls_acc, c
 from .dedup import (calculate_image_hash, detect_and_remove_cross_set_duplicates, find_and_remove_duplicate_images,
                     find_duplicate_pairs, find_and_remove_near_duplicate_images, get_all_images, greedy_first_keeper)
 from .sharded import ShardedGallery, shard_bounds
+from .thresholds import best_thresholds
 
 __all__ = [
-    "DeviceGallery", "RowFilter", "RowLabels", "ShardedGallery", "best_threshold_on_device", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
+    "DeviceGallery", "RowFilter", "RowLabels", "ShardedGallery", "best_threshold_on_device", "best_thresholds", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
     "cluster_prototype", "construct_dataset", "cosine_similarity_scores", "get_cluster_features", "get_image_text_features",
     "image_text_prototypes", "topk_of_scores",
     "detect_and_remove_cross_set_duplicates", "evaluate_thresholds", "eval_threshold", "find_thresholds",

@@ -117,6 +117,11 @@ SIGNATURES = {
                                                               _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _i32,
                                                               _vp]),
     "mmrs_topk_merge_keys_padded_async": (C.c_int, [_vp, _i32, _i32, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
+    # per-class threshold tuning of a batch of prototypes (best_thresholds)
+    "mmrs_threshold_sweep_batched_workspace_bytes": (_sz, [_i32, _i32]),
+    "mmrs_score_range_batched": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp]),
+    "mmrs_threshold_sweep_batched": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp,
+                                               _vp, _sz, _vp]),
 }
 for _name, (_res, _args) in SIGNATURES.items():
     _fn = getattr(lib, _name)

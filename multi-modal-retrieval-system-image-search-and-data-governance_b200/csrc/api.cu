@@ -32,6 +32,13 @@ cudaError_t launch_threshold_sweep_labeled(const float* scores, const int64_t* t
                                            int32_t n_thr, int32_t grid_f32, double* thr_out, int64_t* out_counts,
                                            unsigned long long* hist_ws, uint32_t* mm_ws, int sm_count,
                                            cudaStream_t stream);
+cudaError_t launch_score_range_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n, const uint32_t* filt,
+                                       uint32_t* range, int sm_count, cudaStream_t stream);
+cudaError_t launch_threshold_sweep_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n,
+                                           const int32_t* row_labels, const int32_t* query_labels, const uint32_t* filt,
+                                           const uint32_t* range, int32_t n_thr, int32_t grid_f32, double* thr_out,
+                                           int64_t* out_counts, int64_t* out_n_pos, unsigned long long* hist_ws,
+                                           int sm_count, cudaStream_t stream);
 // K5 on tensor cores (selfjoin_mma.cu)
 bool sjm_pair_mode(int64_t n_rows, int32_t dim, int32_t world);
 int64_t sjm_plan(int64_t n_rows, int32_t rank, int32_t world, bool pair, int64_t* h_panel_start, int32_t max_panels,
@@ -1547,6 +1554,48 @@ int mmrs_threshold_sweep_labeled(const float* d_scores, const int64_t* d_targets
   MMRS_LAUNCH(launch_threshold_sweep_labeled(d_scores, d_targets, label, n, n_thresholds, grid_f32, d_out_thresholds,
                                              d_out_counts, reinterpret_cast<unsigned long long*>(b + 256),
                                              reinterpret_cast<uint32_t*>(b), dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+size_t mmrs_threshold_sweep_batched_workspace_bytes(int32_t n_queries, int32_t n_thresholds) {
+  if (n_queries < 1) n_queries = 1;
+  if (n_thresholds < 1) n_thresholds = 1;
+  return align_up(sizeof(unsigned long long) * 2 * (static_cast<size_t>(n_thresholds) + 1) * n_queries, 256);
+}
+
+int mmrs_score_range_batched(const float* d_scores, int64_t ld_scores, int32_t n_queries, int64_t n_rows,
+                             const uint32_t* d_row_filter, uint32_t* d_range, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_queries == 0 || n_rows == 0) return MMRS_OK;
+  if (n_queries < 0 || n_rows < 0 || ld_scores < n_rows || !d_scores || !d_range) return fail(MMRS_ERR_ARG, "bad arguments");
+  MMRS_LAUNCH(launch_score_range_batched(d_scores, ld_scores, n_queries, n_rows, d_row_filter, d_range, dev.sm_count,
+                                         stream));
+  return MMRS_OK;
+}
+
+int mmrs_threshold_sweep_batched(const float* d_scores, int64_t ld_scores, int32_t n_queries, int64_t n_rows,
+                                 const int32_t* d_row_labels, const int32_t* d_query_labels,
+                                 const uint32_t* d_row_filter, const uint32_t* d_range, int32_t n_thresholds,
+                                 int32_t grid_f32, double* d_out_thresholds, int64_t* d_out_counts,
+                                 int64_t* d_out_n_pos, void* d_workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_thresholds < 1 || n_thresholds > 4096) return fail(MMRS_ERR_ARG, "n_thresholds must be in [1, 4096]");
+  if (n_queries == 0) return MMRS_OK;
+  if (n_queries < 0 || n_rows < 1 || ld_scores < n_rows || !d_scores || !d_row_labels || !d_query_labels || !d_range ||
+      !d_out_thresholds || !d_out_counts || !d_out_n_pos)
+    return fail(MMRS_ERR_ARG, "bad arguments");
+  if (!d_workspace || workspace_bytes < mmrs_threshold_sweep_batched_workspace_bytes(n_queries, n_thresholds))
+    return fail(MMRS_ERR_WORKSPACE, "workspace too small (need mmrs_threshold_sweep_batched_workspace_bytes)");
+  MMRS_LAUNCH(launch_threshold_sweep_batched(d_scores, ld_scores, n_queries, n_rows, d_row_labels, d_query_labels,
+                                             d_row_filter, d_range, n_thresholds, grid_f32, d_out_thresholds,
+                                             d_out_counts, d_out_n_pos, static_cast<unsigned long long*>(d_workspace),
+                                             dev.sm_count, stream));
   return MMRS_OK;
 }
 

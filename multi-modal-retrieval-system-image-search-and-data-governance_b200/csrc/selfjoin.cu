@@ -9,6 +9,8 @@
 // Exact mode: fp32 FFMA, k ascending, one accumulator per pair -- the pair set does not depend
 // on tile shape or launch geometry.  selfjoin_mma.cu is the tensor-core prefilter whose survivors are
 // re-scored with exactly this arithmetic; this kernel serves small inputs and as its cross-check.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace mmrs {
@@ -163,10 +165,12 @@ __global__ void __launch_bounds__(256) sweep_hist_kernel(const S* __restrict__ p
     if (s_hist[i]) atomicAdd(&hist[i], static_cast<unsigned long long>(s_hist[i]));
 }
 
-// ---- fully device-resident variant: scores [n] + integer targets [n], positives = (target == label) ----
-// min / max of the scores -> np.linspace(min, max, T) in fp64 exactly as numpy builds it
-// (y = arange(T) * step + start with a separately rounded multiply and add, last point = stop) ->
-// the same histogram.  Nothing of size N leaves the GPU (code/search_image.py:109 copies all N scores).
+// ---- fully device-resident variant: scores [Q, ld] + row labels, positives = (label == the query's label) ----
+// Per query: min / max of the scores over the allowed rows -> np.linspace(min, max, T) in fp64 exactly as numpy
+// builds it (y = arange(T) * step + start with a separately rounded multiply and add, last point = stop) -> the
+// same histogram.  Nothing of size N leaves the GPU (code/search_image.py:109 copies all N scores).  One query
+// over int64 targets is mmrs_threshold_sweep_labeled; a batch of queries over int32 RowLabels, optionally
+// restricted by a row-filter bitmap, is mmrs_threshold_sweep_batched (best_thresholds).
 __device__ __forceinline__ uint32_t f2ord(float f) {
   const uint32_t u = __float_as_uint(f);
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -174,76 +178,186 @@ __device__ __forceinline__ uint32_t f2ord(float f) {
 __device__ __forceinline__ float ord2f(uint32_t o) {
   return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
 }
-__global__ void __launch_bounds__(256) minmax_kernel(const float* __restrict__ x, int64_t n, uint32_t* mm /*[2] ordered*/) {
-  uint32_t lo = 0xffffffffu, hi = 0u;
-  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const uint32_t o = f2ord(x[i] + 0.0f);
-    lo = o < lo ? o : lo;
-    hi = o > hi ? o : hi;
-  }
-  lo = __reduce_min_sync(0xffffffffu, lo);
-  hi = __reduce_max_sync(0xffffffffu, hi);
-  if ((threadIdx.x & 31) == 0) { atomicMin(mm, lo); atomicMax(mm + 1, hi); }
+__device__ __forceinline__ bool row_allowed(const uint32_t* __restrict__ filt, int64_t i) {
+  return filt == nullptr || ((__ldg(filt + (i >> 5)) >> (i & 31)) & 1u);
 }
+
+// Order-preserving (min, max) of each query's scores, -0.0 canonicalised to +0.0 (x + 0.0f), ACCUMULATED into
+// range [n_q, 2] with atomicMin / atomicMax (a rank's shard combines with the others' the same way).  A CTA
+// covers up to kRangeQG queries of one row range, so a filter word is read once per group of queries.
+constexpr int kRangeQG = 8;
+__global__ void __launch_bounds__(256) score_range_kernel(const float* __restrict__ scores, int64_t ld, int32_t n_q,
+                                                         int64_t n, const uint32_t* __restrict__ filt,
+                                                         uint32_t* __restrict__ range) {
+  const int n_groups = (n_q + kRangeQG - 1) / kRangeQG;
+  for (int g = blockIdx.y; g < n_groups; g += gridDim.y) {
+    const int q0 = g * kRangeQG, nqg = min(kRangeQG, n_q - q0);
+    uint32_t lo[kRangeQG], hi[kRangeQG];
+#pragma unroll
+    for (int j = 0; j < kRangeQG; ++j) { lo[j] = 0xffffffffu; hi[j] = 0u; }
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+      if (!row_allowed(filt, i)) continue;
+#pragma unroll
+      for (int j = 0; j < kRangeQG; ++j) {
+        if (j < nqg) {
+          const uint32_t o = f2ord(scores[(q0 + j) * ld + i] + 0.0f);
+          lo[j] = o < lo[j] ? o : lo[j];
+          hi[j] = o > hi[j] ? o : hi[j];
+        }
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < kRangeQG; ++j) {
+      if (j < nqg) {
+        const uint32_t l = __reduce_min_sync(0xffffffffu, lo[j]);
+        const uint32_t h = __reduce_max_sync(0xffffffffu, hi[j]);
+        if ((threadIdx.x & 31) == 0 && l <= h) { atomicMin(range + 2 * (q0 + j), l); atomicMax(range + 2 * (q0 + j) + 1, h); }
+      }
+    }
+  }
+}
+
 // grid_f32 != 0: NumPy >= 2 semantics (NEP 50): np.linspace of two float32 scalars is computed and
 // returned in float32 (delta, step, t * step and + start each rounded to fp32); grid_f32 == 0: NumPy 1.x
 // semantics, everything in fp64.  Either way multiply and add are rounded separately (no FMA).
-__global__ void linspace_kernel(const uint32_t* __restrict__ mm, int32_t n_thr, int32_t grid_f32,
+// thr [n_q, n_thr]: row q is the grid of range[q].
+__global__ void linspace_kernel(const uint32_t* __restrict__ range, int32_t n_q, int32_t n_thr, int32_t grid_f32,
                                 double* __restrict__ thr) {
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n_thr) return;
-  const float start32 = ord2f(mm[0]), stop32 = ord2f(mm[1]);
-  double v = static_cast<double>(start32);
-  if (n_thr > 1) {
-    if (t == n_thr - 1) {
-      v = static_cast<double>(stop32);
-    } else if (grid_f32) {
-      const float step = __fdiv_rn(__fsub_rn(stop32, start32), static_cast<float>(n_thr - 1));
-      v = static_cast<double>(__fadd_rn(__fmul_rn(static_cast<float>(t), step), start32));
-    } else {
-      const double start = static_cast<double>(start32), stop = static_cast<double>(stop32);
-      const double step = __ddiv_rn(__dsub_rn(stop, start), static_cast<double>(n_thr - 1));
-      v = __dadd_rn(__dmul_rn(static_cast<double>(t), step), start);
+  const int64_t total = static_cast<int64_t>(n_q) * n_thr;
+  for (int64_t idx = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t q = idx / n_thr;
+    const int t = static_cast<int>(idx - q * n_thr);
+    const float start32 = ord2f(range[2 * q]), stop32 = ord2f(range[2 * q + 1]);
+    double v = static_cast<double>(start32);
+    if (n_thr > 1) {
+      if (t == n_thr - 1) {
+        v = static_cast<double>(stop32);
+      } else if (grid_f32) {
+        const float step = __fdiv_rn(__fsub_rn(stop32, start32), static_cast<float>(n_thr - 1));
+        v = static_cast<double>(__fadd_rn(__fmul_rn(static_cast<float>(t), step), start32));
+      } else {
+        const double start = static_cast<double>(start32), stop = static_cast<double>(stop32);
+        const double step = __ddiv_rn(__dsub_rn(stop, start), static_cast<double>(n_thr - 1));
+        v = __dadd_rn(__dmul_rn(static_cast<double>(t), step), start);
+      }
     }
+    thr[idx] = v;
   }
-  thr[t] = v;
-}
-__global__ void __launch_bounds__(256) sweep_hist_labeled_kernel(const float* __restrict__ scores,
-                                                                 const int64_t* __restrict__ targets, int64_t label,
-                                                                 int64_t n, const double* __restrict__ thr,
-                                                                 int32_t n_thr, unsigned long long* __restrict__ hist) {
-  extern __shared__ double s_thr[];
-  uint32_t* s_hist = reinterpret_cast<uint32_t*>(s_thr + n_thr);
-  for (int i = threadIdx.x; i < n_thr; i += blockDim.x) s_thr[i] = thr[i];
-  for (int i = threadIdx.x; i < 2 * (n_thr + 1); i += blockDim.x) s_hist[i] = 0;
-  __syncthreads();
-  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const bool is_neg = targets[i] != label;
-    const double x = static_cast<double>(scores[i]);
-    int lo = 0, hi = n_thr;
-    while (lo < hi) {
-      const int mid = (lo + hi) >> 1;
-      if (x >= s_thr[mid]) lo = mid + 1; else hi = mid;
-    }
-    atomicAdd(&s_hist[(is_neg ? n_thr + 1 : 0) + lo], 1u);
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < 2 * (n_thr + 1); i += blockDim.x)
-    if (s_hist[i]) atomicAdd(&hist[i], static_cast<unsigned long long>(s_hist[i]));
 }
 
-__global__ void sweep_suffix_kernel(const unsigned long long* __restrict__ hist, int32_t n_thr,
-                                    int64_t* __restrict__ out) {
-  // one thread per class (pos / neg): counts[t] = sum_{b > t} hist[b]
+// Label sources of the histogram: which rows are positives of query q.
+struct TargetsLabel {          // int64 targets, one label for every query (mmrs_threshold_sweep_labeled)
+  const int64_t* __restrict__ targets;
+  int64_t label;
+  __device__ __forceinline__ int64_t row(int64_t i) const { return targets[i]; }
+  __device__ __forceinline__ bool positive(int64_t v, int32_t) const { return v == label; }
+};
+struct RowLabelsSource {       // int32 RowLabels, one label per query (mmrs_threshold_sweep_batched)
+  const int32_t* __restrict__ row_labels;
+  const int32_t* __restrict__ query_labels;
+  __device__ __forceinline__ int32_t row(int64_t i) const { return row_labels[i]; }
+  __device__ __forceinline__ bool positive(int32_t v, int32_t query_label) const { return v == query_label; }
+};
+
+// Bin of score x in a grid: the number of thresholds t with x >= thr[t], compared in fp64 as numpy does.
+// kBinWalk: the grid is non-decreasing with distinct ends -- guess the bin from the linear model of the
+// grid and walk to the exact bin against the stored points (the same count as a binary search of a sorted
+// grid, in ~2 shared loads instead of log2(T)); kBinFlat: every point equal (min == max, or T == 1);
+// kBinSearch: anything else (NaN in the grid) -- the binary search of mmrs_threshold_sweep.
+enum : int32_t { kBinSearch = 0, kBinWalk = 1, kBinFlat = 2 };
+__device__ __forceinline__ int grid_bin(double x, const double* __restrict__ thr, int32_t n_thr, int32_t mode,
+                                        double inv_step) {
+  if (mode == kBinFlat) return x >= thr[0] ? n_thr : 0;
+  int lo;
+  if (mode == kBinWalk) {
+    const double d = (x - thr[0]) * inv_step;
+    lo = !(d >= 0.0) ? 0 : (d >= static_cast<double>(n_thr) ? n_thr : static_cast<int>(d) + 1);
+    if (lo > n_thr) lo = n_thr;
+    while (lo > 0 && !(x >= thr[lo - 1])) --lo;
+    while (lo < n_thr && x >= thr[lo]) ++lo;
+    return lo;
+  }
+  int hi = n_thr;
+  lo = 0;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (x >= thr[mid]) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// hist [n_q, 2, n_thr + 1] (pos bins, then neg bins), ACCUMULATED.  A CTA owns a row range and a group of
+// up to `qg` queries whose grids and histograms sit in shared memory, so each row's label and filter word
+// are read once per group.  Filtered-out rows are skipped.
+template <typename L>
+__global__ void __launch_bounds__(512) sweep_hist_labeled_kernel(const float* __restrict__ scores, int64_t ld, int32_t n_q,
+                                                                 int64_t n, L src, const uint32_t* __restrict__ filt,
+                                                                 const double* __restrict__ thr, int32_t n_thr, int32_t qg,
+                                                                 unsigned long long* __restrict__ hist) {
+  extern __shared__ double s_thr[];                                    // [qg][n_thr]
+  double* s_inv = s_thr + static_cast<size_t>(qg) * n_thr;             // [qg]
+  uint32_t* s_hist = reinterpret_cast<uint32_t*>(s_inv + qg);          // [qg][2][n_thr + 1]
+  int32_t* s_qlab = reinterpret_cast<int32_t*>(s_hist + static_cast<size_t>(qg) * 2 * (n_thr + 1));   // [qg]
+  int32_t* s_mode = s_qlab + qg;                                       // [qg]
+  const int hb = 2 * (n_thr + 1);
+  const int n_groups = (n_q + qg - 1) / qg;
+  for (int g = blockIdx.y; g < n_groups; g += gridDim.y) {
+    const int q0 = g * qg, nqg = min(qg, n_q - q0);
+    for (int i = threadIdx.x; i < nqg * n_thr; i += blockDim.x) s_thr[i] = thr[static_cast<int64_t>(q0) * n_thr + i];
+    for (int i = threadIdx.x; i < nqg * hb; i += blockDim.x) s_hist[i] = 0;
+    for (int j = threadIdx.x; j < nqg; j += blockDim.x) {
+      s_mode[j] = kBinWalk;
+      if constexpr (std::is_same<L, RowLabelsSource>::value) s_qlab[j] = src.query_labels[q0 + j];
+      else s_qlab[j] = 0;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nqg * (n_thr - 1); i += blockDim.x) {
+      const int j = i / (n_thr - 1), t = i - j * (n_thr - 1);
+      if (!(s_thr[j * n_thr + t] <= s_thr[j * n_thr + t + 1])) s_mode[j] = kBinSearch;
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < nqg; j += blockDim.x) {
+      const double first = s_thr[j * n_thr], last = s_thr[j * n_thr + n_thr - 1];
+      if (s_mode[j] == kBinWalk && first == last) s_mode[j] = kBinFlat;   // non-decreasing with equal ends
+      s_inv[j] = s_mode[j] == kBinWalk ? static_cast<double>(n_thr - 1) / (last - first) : 0.0;
+    }
+    __syncthreads();
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+      if (!row_allowed(filt, i)) continue;
+      const auto lab = src.row(i);
+#pragma unroll 4
+      for (int j = 0; j < nqg; ++j) {
+        const double x = static_cast<double>(scores[(q0 + j) * ld + i]);
+        const int b = grid_bin(x, s_thr + j * n_thr, n_thr, s_mode[j], s_inv[j]);
+        atomicAdd(&s_hist[j * hb + (src.positive(lab, s_qlab[j]) ? 0 : n_thr + 1) + b], 1u);
+      }
+    }
+    __syncthreads();
+    unsigned long long* h = hist + static_cast<int64_t>(q0) * hb;
+    for (int i = threadIdx.x; i < nqg * hb; i += blockDim.x)
+      if (s_hist[i]) atomicAdd(&h[i], static_cast<unsigned long long>(s_hist[i]));
+    __syncthreads();
+  }
+}
+
+// One CTA per query, one thread per class (pos / neg): counts[q][t] = sum_{b > t} hist[q][b]; n_pos[q] (when
+// non-null) = every positive of the histogram, i.e. the allowed rows of the query's class.
+__global__ void sweep_suffix_kernel(const unsigned long long* __restrict__ hist, int32_t n_q, int32_t n_thr,
+                                    int64_t* __restrict__ out, int64_t* __restrict__ n_pos) {
   const int c = threadIdx.x;
   if (c >= 2) return;
-  const unsigned long long* h = hist + c * (n_thr + 1);
-  unsigned long long run = 0;
-  for (int t = n_thr - 1; t >= 0; --t) {
-    run += h[t + 1];
-    out[2 * t + c] = static_cast<int64_t>(run);
+  for (int64_t q = blockIdx.x; q < n_q; q += gridDim.x) {
+    const unsigned long long* h = hist + (q * 2 + c) * (n_thr + 1);
+    int64_t* o = out + q * 2 * n_thr;
+    unsigned long long run = 0;
+    for (int t = n_thr - 1; t >= 0; --t) {
+      run += h[t + 1];
+      o[2 * t + c] = static_cast<int64_t>(run);
+    }
+    if (c == 0 && n_pos) n_pos[q] = static_cast<int64_t>(run + h[0]);
   }
 }
 
@@ -265,7 +379,7 @@ static cudaError_t launch_threshold_sweep_t(const S* pos, int64_t n_pos, const S
   sweep_hist_kernel<S><<<static_cast<int>(grid), 256, smem, stream>>>(pos, n_pos, neg, n_neg, thr, n_thr, hist_ws);
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  sweep_suffix_kernel<<<1, 32, 0, stream>>>(hist_ws, n_thr, out_counts);
+  sweep_suffix_kernel<<<1, 32, 0, stream>>>(hist_ws, 1, n_thr, out_counts, nullptr);
   return cudaGetLastError();
 }
 cudaError_t launch_threshold_sweep(const float* pos, int64_t n_pos, const float* neg, int64_t n_neg,
@@ -279,30 +393,81 @@ cudaError_t launch_threshold_sweep_f64(const double* pos, int64_t n_pos, const d
   return launch_threshold_sweep_t<double>(pos, n_pos, neg, n_neg, thr, n_thr, out_counts, hist_ws, sm_count, stream);
 }
 
+// Shared memory of the labeled histogram: per query its grid, 1 / step, two histograms, its label and bin mode.
+static size_t sweep_hist_query_bytes(int32_t n_thr) {
+  return sizeof(double) * (n_thr + 1) + sizeof(uint32_t) * 2 * (n_thr + 1) + 2 * sizeof(int32_t);
+}
+constexpr size_t kSweepHistBudget = 48 << 10;   // four 512-thread CTAs per SM at T <= ~1500 (one query: up to 64 KB)
+
+static cudaError_t launch_score_range(const float* scores, int64_t ld, int32_t n_q, int64_t n, const uint32_t* filt,
+                                      uint32_t* range, int sm_count, cudaStream_t stream) {
+  const int n_groups = (n_q + kRangeQG - 1) / kRangeQG;
+  int64_t gx = (n + 256 * 8 - 1) / (256 * 8);
+  const int64_t cap = (static_cast<int64_t>(sm_count) * 4 + n_groups - 1) / n_groups;
+  if (gx > cap) gx = cap;
+  if (gx < 1) gx = 1;
+  score_range_kernel<<<dim3(static_cast<unsigned>(gx), static_cast<unsigned>(n_groups < 65535 ? n_groups : 65535)), 256, 0,
+                       stream>>>(scores, ld, n_q, n, filt, range);
+  return cudaGetLastError();
+}
+
+template <typename L>
+static cudaError_t launch_sweep_labeled(const float* scores, int64_t ld, int32_t n_q, int64_t n, L src,
+                                        const uint32_t* filt, const uint32_t* range, int32_t n_thr, int32_t grid_f32,
+                                        double* thr_out, int64_t* out_counts, int64_t* out_n_pos,
+                                        unsigned long long* hist_ws, int sm_count, cudaStream_t stream) {
+  cudaError_t e = cudaMemsetAsync(hist_ws, 0, sizeof(unsigned long long) * 2 * (n_thr + 1) * static_cast<size_t>(n_q), stream);
+  if (e != cudaSuccess) return e;
+  const int64_t total = static_cast<int64_t>(n_q) * n_thr;
+  const int64_t lgrid = (total + 255) / 256;
+  linspace_kernel<<<static_cast<int>(lgrid < 65535 ? lgrid : 65535), 256, 0, stream>>>(range, n_q, n_thr, grid_f32, thr_out);
+  const size_t per_q = sweep_hist_query_bytes(n_thr);
+  int32_t qg = static_cast<int32_t>(kSweepHistBudget / per_q);
+  if (qg < 1) qg = 1;
+  if (qg > n_q) qg = n_q;
+  const int n_groups = (n_q + qg - 1) / qg;
+  int64_t gx = (n + 512 * 8 - 1) / (512 * 8);
+  const int64_t cap = (static_cast<int64_t>(sm_count) * 4 + n_groups - 1) / n_groups;
+  if (gx > cap) gx = cap;
+  if (gx < 1) gx = 1;
+  e = cudaFuncSetAttribute(sweep_hist_labeled_kernel<L>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                           static_cast<int>(sweep_hist_query_bytes(kSweepMaxT) > kSweepHistBudget
+                                                ? sweep_hist_query_bytes(kSweepMaxT) : kSweepHistBudget));
+  if (e != cudaSuccess) return e;
+  sweep_hist_labeled_kernel<L><<<dim3(static_cast<unsigned>(gx), static_cast<unsigned>(n_groups < 65535 ? n_groups : 65535)),
+                                 512, per_q * qg, stream>>>(scores, ld, n_q, n, src, filt, thr_out, n_thr, qg, hist_ws);
+  sweep_suffix_kernel<<<n_q < 65535 ? n_q : 65535, 32, 0, stream>>>(hist_ws, n_q, n_thr, out_counts, out_n_pos);
+  return cudaGetLastError();
+}
+
 cudaError_t launch_threshold_sweep_labeled(const float* scores, const int64_t* targets, int64_t label, int64_t n,
                                            int32_t n_thr, int32_t grid_f32, double* thr_out, int64_t* out_counts,
                                            unsigned long long* hist_ws, uint32_t* mm_ws, int sm_count,
                                            cudaStream_t stream) {
   if (n_thr < 1 || n_thr > kSweepMaxT || n < 1) return cudaErrorInvalidValue;
-  cudaError_t e = cudaMemsetAsync(hist_ws, 0, sizeof(unsigned long long) * 2 * (n_thr + 1), stream);
+  cudaError_t e = cudaMemsetAsync(mm_ws, 0xff, sizeof(uint32_t), stream);           // min <- 0xffffffff
   if (e != cudaSuccess) return e;
-  e = cudaMemsetAsync(mm_ws, 0xff, sizeof(uint32_t), stream);           // min <- 0xffffffff
+  e = cudaMemsetAsync(mm_ws + 1, 0, sizeof(uint32_t), stream);                      // max <- 0
   if (e != cudaSuccess) return e;
-  e = cudaMemsetAsync(mm_ws + 1, 0, sizeof(uint32_t), stream);          // max <- 0
+  e = launch_score_range(scores, n, 1, n, nullptr, mm_ws, sm_count, stream);
   if (e != cudaSuccess) return e;
-  int64_t grid = (n + 256 * 8 - 1) / (256 * 8);
-  if (grid > sm_count * 4) grid = sm_count * 4;
-  if (grid < 1) grid = 1;
-  minmax_kernel<<<static_cast<int>(grid), 256, 0, stream>>>(scores, n, mm_ws);
-  linspace_kernel<<<(n_thr + 255) / 256, 256, 0, stream>>>(mm_ws, n_thr, grid_f32, thr_out);
-  const size_t smem = sizeof(double) * n_thr + sizeof(uint32_t) * 2 * (n_thr + 1);
-  e = cudaFuncSetAttribute(sweep_hist_labeled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           static_cast<int>(sizeof(double) * kSweepMaxT + sizeof(uint32_t) * 2 * (kSweepMaxT + 1)));
-  if (e != cudaSuccess) return e;
-  sweep_hist_labeled_kernel<<<static_cast<int>(grid), 256, smem, stream>>>(scores, targets, label, n, thr_out, n_thr,
-                                                                            hist_ws);
-  sweep_suffix_kernel<<<1, 32, 0, stream>>>(hist_ws, n_thr, out_counts);
-  return cudaGetLastError();
+  return launch_sweep_labeled(scores, n, 1, n, TargetsLabel{targets, label}, nullptr, mm_ws, n_thr, grid_f32, thr_out,
+                              out_counts, nullptr, hist_ws, sm_count, stream);
+}
+
+cudaError_t launch_score_range_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n, const uint32_t* filt,
+                                       uint32_t* range, int sm_count, cudaStream_t stream) {
+  return launch_score_range(scores, ld, n_q, n, filt, range, sm_count, stream);
+}
+
+cudaError_t launch_threshold_sweep_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n,
+                                           const int32_t* row_labels, const int32_t* query_labels, const uint32_t* filt,
+                                           const uint32_t* range, int32_t n_thr, int32_t grid_f32, double* thr_out,
+                                           int64_t* out_counts, int64_t* out_n_pos, unsigned long long* hist_ws,
+                                           int sm_count, cudaStream_t stream) {
+  if (n_thr < 1 || n_thr > kSweepMaxT || n < 1 || n_q < 1) return cudaErrorInvalidValue;
+  return launch_sweep_labeled(scores, ld, n_q, n, RowLabelsSource{row_labels, query_labels}, filt, range, n_thr, grid_f32,
+                              thr_out, out_counts, out_n_pos, hist_ws, sm_count, stream);
 }
 
 // ---- lexicographic sort of the emitted pairs ----------------------------------------------------------------

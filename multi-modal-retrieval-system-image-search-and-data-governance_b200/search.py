@@ -322,22 +322,31 @@ def full_scores(queries, gallery: GalleryLike, *, normalize_queries: bool = True
     gal = _as_gallery(gallery, mode)
     q, on_host = _prep_queries(queries, gal)
     nq = int(q.shape[0])
-    lib = _cabi.lib
     with torch.cuda.device(gal.device):
         if on_host:
             q = q.to(gal.device)
         out = torch.empty((nq, gal.n_rows), dtype=torch.float32, device=gal.device)
-        if nq > 0:
-            ws_bytes = lib.mmrs_full_scores_workspace_bytes(gal.n_rows, gal.padded_dim, gal.dtype_code, nq)
-            ws = gal.workspace(("scores", nq), ws_bytes)
-            g_ptr, g_ld, g_dtype = _operand(gal, nq, path)
-            _cabi.check(lib.mmrs_full_scores(g_ptr, gal.n_rows, gal.padded_dim,
-                                             g_ld, g_dtype, q.data_ptr(), nq,
-                                             q.stride(0), int(bool(normalize_queries)), float(scale),
-                                             _cabi.PATHS[path], out.data_ptr(), out.stride(0),
-                                             DeviceGallery.aligned_ptr(ws), ws_bytes,
-                                             _stream_handle(gal.device)))
+        _scores_into(gal, q, out, normalize_queries, scale, path)
     return out.cpu() if on_host else out
+
+
+def _scores_into(gal: DeviceGallery, q: torch.Tensor, out: torch.Tensor, normalize_queries: bool, scale: float,
+                 path: str) -> None:
+    """mmrs_full_scores of prepared device queries `q` [nq, padded_dim] into `out` [>= nq, N] (row stride
+    out.stride(0)); the kernel is chosen for nq queries."""
+    nq = int(q.shape[0])
+    if nq == 0:
+        return
+    lib = _cabi.lib
+    ws_bytes = lib.mmrs_full_scores_workspace_bytes(gal.n_rows, gal.padded_dim, gal.dtype_code, nq)
+    ws = gal.workspace(("scores", nq), ws_bytes)
+    g_ptr, g_ld, g_dtype = _operand(gal, nq, path)
+    _cabi.check(lib.mmrs_full_scores(g_ptr, gal.n_rows, gal.padded_dim,
+                                     g_ld, g_dtype, q.data_ptr(), nq,
+                                     q.stride(0), int(bool(normalize_queries)), float(scale),
+                                     _cabi.PATHS[path], out.data_ptr(), out.stride(0),
+                                     DeviceGallery.aligned_ptr(ws), ws_bytes,
+                                     _stream_handle(gal.device)))
 
 
 # one-entry upload cache: the reference re-uploads `features` on every call (:107); a script that
@@ -619,6 +628,23 @@ def _f1_from_counts(tp, fp, n_pos):
     return f1, precision, recall
 
 
+def grid_f32() -> int:
+    """1 when np.linspace of two float32 scalars is float32 (NEP 50, NumPy >= 2), 0 when float64 (NumPy 1.x):
+    the device grid follows the installed numpy."""
+    return int(np.linspace(np.float32(0), np.float32(1), 3).dtype == np.float32)
+
+
+def best_from_counts(thresholds, counts, n_pos: int):
+    """find_thresholds' tail (code/search_image.py:62-79) on the sweep's (tp, fp) counts [T, 2]:
+    -> (best_f1, best_threshold, best_precision, best_recall, f1_scores); the first strict maximum wins."""
+    f1s, ps, rs = _f1_from_counts(counts[:, 0], counts[:, 1], n_pos)
+    best = (0., 0., 0., 0.)
+    for th, f1, p, r in zip(thresholds, f1s, ps, rs):
+        if f1 > best[0]:                      # first strict maximum wins (:74)
+            best = (f1, th, p, r)
+    return best[0], best[1], best[2], best[3], f1s
+
+
 def best_threshold_on_device(scores: torch.Tensor, targets, label, n_points: int = 200):
     """find_thresholds (code/search_image.py:58-79) for scores that never leave the GPU: `scores` is a
     CUDA fp32 vector (e.g. one row of full_scores), `targets` the class ids.  Returns
@@ -637,20 +663,14 @@ def best_threshold_on_device(scores: torch.Tensor, targets, label, n_points: int
         out = torch.empty((n_points, 2), dtype=torch.int64, device=dev)
         ws_bytes = lib.mmrs_threshold_sweep_workspace_bytes(n_points) + 256
         ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
-        # the grid follows the installed numpy: float32 under NEP 50 (NumPy >= 2), float64 before
-        grid_f32 = int(np.linspace(np.float32(0), np.float32(1), 3).dtype == np.float32)
         _cabi.check(lib.mmrs_threshold_sweep_labeled(s.data_ptr(), t.data_ptr(), int(label), s.numel(), n_points,
-                                                     grid_f32, thr.data_ptr(), out.data_ptr(), DeviceGallery.aligned_ptr(ws),
-                                                     ws_bytes, _stream_handle(dev)))
+                                                     grid_f32(), thr.data_ptr(), out.data_ptr(),
+                                                     DeviceGallery.aligned_ptr(ws), ws_bytes, _stream_handle(dev)))
         n_pos = int((t == int(label)).sum().item())
         counts = out.cpu().numpy()
         thresholds = thr.cpu().numpy()
-    f1s, ps, rs = _f1_from_counts(counts[:, 0], counts[:, 1], n_pos)
-    best = (0., 0., 0., 0.)
-    for th, f1, p, r in zip(thresholds, f1s, ps, rs):
-        if f1 > best[0]:                      # first strict maximum wins (:74)
-            best = (f1, th, p, r)
-    return best[0], best[1], best[2], best[3], thresholds, f1s
+    best_f1, best_thr, best_p, best_r, f1s = best_from_counts(thresholds, counts, n_pos)
+    return best_f1, best_thr, best_p, best_r, thresholds, f1s
 
 
 def evaluate_thresholds(similarities, thresholds, positive_class, negative_class):

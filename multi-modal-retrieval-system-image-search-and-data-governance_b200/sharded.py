@@ -97,12 +97,21 @@ class ShardedGallery:
     `local` is the rank's DeviceGallery with `row_offset` = first global row.  `local_search` and
     `merge` exist so the host-side protocol (gather layout, index offsets, tie rule) can be
     exercised on CPU with the gloo backend in tests; the product defaults are the CUDA kernels.
+    `local_range` / `local_counts` do the same for `best_thresholds`' two local steps:
+    `local_range(queries, shard, *, normalize_queries, scale, path, row_filter)` -> int64 [nq, 2] (min, max)
+    score keys, and `local_counts(queries, shard, range, *, row_labels, query_labels, n_points, row_filter,
+    normalize_queries, scale, path, grid_f32)` -> (thresholds [nq, T] float64, counts [nq, T, 2] int64, n_pos
+    [nq] int64) of the shard; the product default is `thresholds.DeviceSweep`.
     `fused=False` forces the NCCL all-gather variant (also: MMRS_NO_FUSED_GATHER=1).
     """
 
     def __init__(self, local, n_rows_global: int, group: Optional[dist.ProcessGroup] = None,
                  local_search: Optional[Callable] = None, merge: Optional[Callable] = None,
-                 fused: Optional[bool] = None):
+                 fused: Optional[bool] = None, local_range: Optional[Callable] = None,
+                 local_counts: Optional[Callable] = None):
+        if (local_range is None) != (local_counts is None):
+            raise ValueError("local_range and local_counts come together")
+        self._local_range, self._local_counts = local_range, local_counts
         self.local = local
         self.n_rows_global = int(n_rows_global)
         self.group = group
@@ -490,6 +499,65 @@ class ShardedGallery:
         if labels is not None:
             mi = torch.where(mv == float("-inf"), torch.full_like(mi, -1), mi)
         return (mv.cpu(), mi.cpu()) if on_host else (mv, mi)
+
+    def best_thresholds(self, queries, row_labels, query_labels, *, n_points: int = 200, scale: float = 100.0,
+                        normalize_queries: bool = False, row_filter=None, path: str = "auto",
+                        max_score_bytes: int = 4 << 30):
+        """`best_thresholds` over the sharded gallery, the same arrays on every rank.  `queries`, `query_labels`,
+        `row_labels` and `row_filter` are the same on every rank, the last two over the GLOBAL rows.  Per chunk
+        of queries each rank scores its shard and takes the range of its allowed rows; one all-reduce gives the
+        global (min, max) of every query, so every rank builds the same grid; each rank counts its rows against
+        it and one all-reduce sums the counts.  The chunk size comes from the longest shard of
+        `shard_bounds(n_rows_global, world)`, which every rank knows: all ranks run the same collectives."""
+        from .search import grid_f32
+        from .thresholds import (DeviceSweep, check_arguments, check_row_labels, chunk_queries, empty_result,
+                                 run_chunks)
+        if isinstance(queries, np.ndarray):
+            queries = torch.from_numpy(queries)
+        if queries.dim() == 1:
+            queries = queries.unsqueeze(0)
+        c = int(queries.shape[0])
+        dev = getattr(self.local, "device", None)
+        check_row_labels(row_labels, self.n_rows_global, dev)
+        ql = check_arguments(c, query_labels, n_points, dev)
+        local_filter = None
+        if row_filter is not None:
+            row_filter, local_filter = self._local_filter(row_filter)
+            if row_filter.n_allowed == 0:
+                raise ValueError("row_filter allows no row")
+        if c == 0:
+            return empty_result(int(n_points))
+        lo = self.local.row_offset
+        local_labels = row_labels.shard(lo, lo + len(self.local))
+        longest = max(hi - lo_ for lo_, hi in shard_bounds(self.n_rows_global, self.world))
+        qc = min(c, chunk_queries(longest, max_score_bytes))
+        n_points = int(n_points)
+        kw = dict(normalize_queries=normalize_queries, scale=scale, path=path)
+        if self._local_range is None:
+            sweep = DeviceSweep(self.local, qc, n_points, normalize_queries, scale, path, local_labels, local_filter,
+                                grid_f32())
+            range_step = sweep.range
+            count_step = lambda q, lab, rng: sweep.counts(lab, rng)
+        else:
+            range_step = lambda q: self._local_range(q, self.local, row_filter=local_filter, **kw)
+            count_step = lambda q, lab, rng: self._local_counts(q, self.local, rng, row_labels=local_labels,
+                                                                query_labels=lab, n_points=n_points,
+                                                                row_filter=local_filter, grid_f32=grid_f32(), **kw)
+        if self.world == 1:
+            return run_chunks(queries, ql, qc, n_points, range_step, count_step)
+
+        def reduce_range(rng):
+            # MIN of the min keys and MAX of the max keys in ONE exact int64 all-reduce: MIN of the negated max keys
+            t = torch.stack([rng[:, 0], -rng[:, 1]], 1).contiguous()
+            dist.all_reduce(t, op=dist.ReduceOp.MIN, group=self.group)
+            return torch.stack([t[:, 0], -t[:, 1]], 1)
+
+        def reduce_counts(counts, n_pos):
+            flat = torch.cat([counts.reshape(-1), n_pos.reshape(-1)])
+            dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=self.group)
+            return flat[:counts.numel()].view(counts.shape), flat[counts.numel():]
+
+        return run_chunks(queries, ql, qc, n_points, range_step, count_step, reduce_range, reduce_counts)
 
     def find_duplicate_pairs(self, emb_full: torch.Tensor, threshold: float, raw_join: Optional[Callable] = None):
         """Self-join with the gallery replicated (10M x 512 fp32 = 20 GB fits every GPU) and the
