@@ -22,6 +22,11 @@
  *   mmrs_score_range_batched + mmrs_threshold_sweep_batched
  *                         code/search_image.py:382-389 (the per-class loop of get_similarity :105-117 +
  *                         find_thresholds :58-79) for every class prototype of a batch at once
+ *   mmrs_range_search_window + mmrs_range_search_scatter
+ *                         code/merge_dataset.py:259-284 `preds = similarity >= threshold`,
+ *                         code/union_clip_llava2.py:153-162 (accept every image at or above a class's
+ *                         threshold), tool/delete repeated.py (every row within tau of a query) --
+ *                         the rows passing a per-query threshold, score matrix never stored
  *
  * Conventions
  *   - every function returns an int status: 0 = ok, negative = error (table below);
@@ -516,6 +521,40 @@ int mmrs_threshold_sweep_batched(const float* d_scores, int64_t ld_scores, int32
                                  int32_t n_thresholds, int32_t grid_f32, double* d_out_thresholds,
                                  int64_t* d_out_counts, int64_t* d_out_n_pos, void* d_workspace,
                                  size_t workspace_bytes, void* stream);
+
+/*
+ * Range search (code/merge_dataset.py:259-284 `preds = similarity >= threshold`): every row r of the gallery
+ * with score(q, r) >= d_thresholds[q] (fp32 [n_queries], compared in fp32), where score is the value
+ * mmrs_full_scores writes for the same queries, gallery and path.  The rows are processed in windows of
+ * `window_rows` rows (a positive multiple of 128, below 2^31) so that the candidate lists are bounded:
+ * the workspace holds window_rows 8-byte keys per query
+ * (mmrs_range_search_workspace_bytes(window_rows, dim, n_queries); n_queries in [1, 65535]).
+ *
+ * mmrs_range_search_window: prepares the queries and scans rows [row_begin, min(row_begin + window_rows,
+ * n_rows)) (row_begin a multiple of 128; a bf16x3 gallery is passed whole, as to mmrs_full_scores), appends
+ * every passing row, and sorts each query's rows by row index.  Blocks until done and writes h_counts
+ * [n_queries] int64 (HOST): the matches of each query in this window.  A NaN score never matches.
+ * d_row_filter (nullable) is the allow-list bitmap of the whole gallery (mmrs_pack_row_filter);
+ * d_row_labels (nullable) / d_query_labels / label_match restrict query q to rows with label ==
+ * d_query_labels[q] (MMRS_LABEL_SAME) or != (MMRS_LABEL_OTHER); a negative query label is unrestricted.
+ * Status MMRS_ERR_ZERO_NORM as mmrs_full_scores.
+ *
+ * mmrs_range_search_scatter: writes the window's matches of query q, in ascending row order, to
+ * d_out_values / d_out_indices [d_out_offsets[q], d_out_offsets[q] + h_counts[q]) (device int64
+ * offsets [n_queries]); an index is index_offset + the row's position inside the window, so pass
+ * index_offset = the gallery's global row offset + row_begin.  A -0.0 score is written as +0.0.  Asynchronous on
+ * `stream`; the workspace must still hold the preceding window call's state.
+ */
+size_t mmrs_range_search_workspace_bytes(int64_t window_rows, int32_t dim, int32_t n_queries);
+int mmrs_range_search_window(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                             int32_t gallery_dtype, const float* d_queries, int32_t n_queries, int64_t ld_queries,
+                             int32_t normalize_queries, float scale, int32_t path, const float* d_thresholds,
+                             int64_t row_begin, int64_t window_rows, const uint32_t* d_row_filter,
+                             const int32_t* d_row_labels, const int32_t* d_query_labels, int32_t label_match,
+                             int64_t* h_counts, void* d_workspace, size_t workspace_bytes, void* stream);
+int mmrs_range_search_scatter(int32_t n_queries, int64_t window_rows, int32_t dim, const int64_t* d_out_offsets,
+                              int64_t index_offset, float* d_out_values, int64_t* d_out_indices, void* d_workspace,
+                              size_t workspace_bytes, void* stream);
 
 /* ---- measurement hooks (bench.py; not needed by a product caller) --------------------------- */
 

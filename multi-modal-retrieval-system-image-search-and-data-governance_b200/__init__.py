@@ -22,7 +22,8 @@ functions for this path (same names, positional order and return tuples):
 plus the tensor-level entry points they sit on: search_topk, full_scores, find_duplicate_pairs,
 DeviceGallery, ShardedGallery, RowFilter (row-filtered search_topk: leave rows out per call) and
 RowLabels (label-conditioned search_topk: each query searches the rows of its own class, or of every other)
-and best_thresholds (the best-F1 threshold of every class prototype of a batch, find_thresholds per class).  Everything computes through the C-ABI CUDA library
+and best_thresholds (the best-F1 threshold of every class prototype of a batch, find_thresholds per class) and
+search_range (every row at or above a per-query threshold, in CSR form).  Everything computes through the C-ABI CUDA library
 (include/mmrs_b200.h); there is no CPU path -- without a B200 the calls raise.
 """
 from . import _cabi  # noqa: F401  (fails loudly when the CUDA library is missing)
@@ -37,6 +38,7 @@ from .search import (best_threshold_on_device, calc_combined_metrics, cls_acc, c
 from .dedup import (calculate_image_hash, detect_and_remove_cross_set_duplicates, find_and_remove_duplicate_images,
                     find_duplicate_pairs, find_and_remove_near_duplicate_images, get_all_images, greedy_first_keeper)
 from .sharded import ShardedGallery, shard_bounds
+from .range_search import search_range
 from .thresholds import best_thresholds
 
 __all__ = [
@@ -47,6 +49,6 @@ __all__ = [
     "find_and_remove_duplicate_images", "find_and_remove_near_duplicate_images",
     "find_duplicate_pairs", "full_scores", "get_all_images", "get_similarity", "get_similarity_from_matrix",
     "greedy_first_keeper", "load_feature_cache", "mix_image_text_query", "outlier_filter_features",
-    "score_classes", "search_topk", "shard_bounds",
+    "score_classes", "search_range", "search_topk", "shard_bounds",
     "threshold_sweep_counts",
 ]

@@ -122,6 +122,11 @@ SIGNATURES = {
     "mmrs_score_range_batched": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp]),
     "mmrs_threshold_sweep_batched": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp,
                                                _vp, _sz, _vp]),
+    # range search: the rows at or above a per-query threshold, one row window per call
+    "mmrs_range_search_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "mmrs_range_search_window": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _f32, _i32, _vp, _i64,
+                                           _i64, _vp, _vp, _vp, _i32, _vp, _vp, _sz, _vp]),
+    "mmrs_range_search_scatter": (C.c_int, [_i32, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
 }
 for _name, (_res, _args) in SIGNATURES.items():
     _fn = getattr(lib, _name)

@@ -53,10 +53,21 @@ cudaError_t launch_selfjoin_recheck(const int64_t* cand, int64_t n_cand, const f
                                     float threshold, int64_t* out_pairs, int64_t capacity,
                                     unsigned long long* out_count, cudaStream_t stream);
 // K2.  q_bf16 is the prepared [n_q_padded, ldq] bf16 query matrix; handles up to 256 queries.
+// g_plane_rows: rows between two planes of a bf16x3 gallery (the full gallery's n_rows).
 cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, int32_t n_q_padded,
-                            int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split);
+                            int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split,
+                            int64_t g_plane_rows);
 cudaError_t launch_split_bf16x3(const float* src, int64_t n_rows, int32_t dim, int64_t ld_src, __nv_bfloat16* dst,
                                 int64_t ld_dst, int sm_count, cudaStream_t stream);
+// range search finalize (range.cu)
+int64_t range_chunks(int64_t n_words);
+cudaError_t launch_range_mark_prefix(const uint64_t* cand, int64_t cap, const uint32_t* cnt, int32_t n_queries,
+                                     uint32_t* bitmap, uint32_t* word_base, uint32_t* chunk_sum, int64_t* total,
+                                     int sm_count, cudaStream_t stream);
+cudaError_t launch_range_scatter(const uint64_t* cand, int64_t cap, const uint32_t* cnt, int32_t n_queries,
+                                 const uint32_t* bitmap, const uint32_t* word_base, const int64_t* out_off,
+                                 int64_t index_offset, float* values, int64_t* indices, int sm_count,
+                                 cudaStream_t stream);
 int scan_mma_max_queries();
 int scan_mma_split_max_queries();
 bool scan_mma_available();
@@ -211,6 +222,43 @@ static Workspace carve(void* base, int64_t n_rows, int32_t dim, int32_t n_querie
   return w;
 }
 
+// Range search (mmrs_range_search_window / _scatter): the query matrices of carve() plus, per query, a
+// candidate list of one window (cap = window_rows keys), its counter, the window's row bitmap, the word
+// prefix sums, the chunk sums of the prefix and the total.
+// K2 stages its queries in UMMA columns padded up to 256 per launch; a padded column's threshold is +inf and
+// its query row zero, so only a NaN score (a NaN or infinite gallery value times 0) passes it, and K2 appends
+// that row to list q0 + column >= n_queries.  Those counters exist here and start at the list capacity, so
+// the kernel's `pos < cap` test drops the appends: no key memory is needed for the padded lists.
+constexpr int kRangePadLists = 256;
+
+struct RangeWorkspace {
+  Workspace base;          // flags, q_f32, q_bf16
+  uint32_t* cnt;           // [Q + kRangePadLists]
+  uint64_t* cand;          // [Q, window_rows]
+  uint32_t* bitmap;        // [Q, window_rows / 32]
+  uint32_t* word_base;     // [Q, window_rows / 32]
+  uint32_t* chunk_sum;     // [Q, range_chunks(window_rows / 32)]
+  int64_t* total;          // [Q]
+  size_t total_bytes;
+};
+
+static RangeWorkspace carve_range(void* base, int64_t window_rows, int32_t dim, int32_t n_queries) {
+  RangeWorkspace r{};
+  r.base = carve(base, window_rows, dim, n_queries, 1, false);
+  size_t off = r.base.total;
+  char* b = static_cast<char*>(base);
+  auto take = [&](size_t bytes) { char* p = b ? b + off : nullptr; off += align_up(bytes, 256); return p; };
+  const size_t q = static_cast<size_t>(n_queries), words = static_cast<size_t>(window_rows / 32);
+  r.cnt = reinterpret_cast<uint32_t*>(take((q + kRangePadLists) * sizeof(uint32_t)));
+  r.cand = reinterpret_cast<uint64_t*>(take(q * static_cast<size_t>(window_rows) * sizeof(uint64_t)));
+  r.bitmap = reinterpret_cast<uint32_t*>(take(q * words * sizeof(uint32_t)));
+  r.word_base = reinterpret_cast<uint32_t*>(take(q * words * sizeof(uint32_t)));
+  r.chunk_sum = reinterpret_cast<uint32_t*>(take(q * static_cast<size_t>(range_chunks(window_rows / 32)) * sizeof(uint32_t)));
+  r.total = reinterpret_cast<int64_t*>(take(q * sizeof(int64_t)));
+  r.total_bytes = off;
+  return r;
+}
+
 static int check_matrix(const void* p, int64_t n_rows, int32_t dim, int64_t ld, int32_t dtype,
                         const char* what) {
   if (!p) return fail(MMRS_ERR_ARG, "%s pointer is null", what);
@@ -277,9 +325,11 @@ static int profiled_scan(int32_t kind, int32_t dtype, const ScanParams& p, cudaS
 }
 
 // One scan over the tiles of `sched` for queries [q_lo, q_hi) of the prepared matrices.
+// plane_rows: rows between two bf16x3 planes when base.gallery is a row window (0: base.n_rows).
 static int run_scan(Path path, const DeviceInfo& dev, int32_t dtype, ScanParams base,
                     const Workspace& w, int32_t n_q_padded, int32_t q_lo, int32_t q_hi, int mode,
-                    cudaStream_t stream) {
+                    cudaStream_t stream, int64_t plane_rows = 0) {
+  if (plane_rows == 0) plane_rows = base.n_rows;
   if (path == Path::kMma) {
     // 256 queries per CTA (the UMMA N limit); when at least two full chunks remain, one launch takes
     // up to four of them and their CTAs share every gallery tile through L2 (scan_mma.cu, gridDim.y):
@@ -296,7 +346,7 @@ static int run_scan(Path path, const DeviceInfo& dev, int32_t dtype, ScanParams 
       p.nq = chunk;
       q += chunk;
       int rc = profiled_scan(MMRS_PATH_MMA, dtype, p, stream, [&]() {
-        return launch_scan_mma(p, w.q_bf16, n_q_padded, mode, w.flags, dev.sm_count, stream, split);
+        return launch_scan_mma(p, w.q_bf16, n_q_padded, mode, w.flags, dev.sm_count, stream, split, plane_rows);
       });
       if (rc != MMRS_OK) return rc;
     }
@@ -483,7 +533,8 @@ static int enqueue_exhaustive(const SearchArgs& a, const DeviceInfo& dev, const 
     p.cand = w.cand - static_cast<int64_t>(q) * all_rows;
     p.q0 = q; p.nq = 1;
     if (a.dtype == MMRS_DTYPE_BF16X3) {
-      MMRS_LAUNCH(launch_scan_mma(p, w.q_bf16, padded_queries(a.n_queries), kModeDense, w.flags, dev.sm_count, stream, 3));
+      MMRS_LAUNCH(launch_scan_mma(p, w.q_bf16, padded_queries(a.n_queries), kModeDense, w.flags, dev.sm_count, stream, 3,
+                                   a.n_rows));
     } else {
       MMRS_LAUNCH(launch_scan_gemv(p, a.dtype, kModeDense, dev.sm_count, stream));
     }
@@ -1596,6 +1647,103 @@ int mmrs_threshold_sweep_batched(const float* d_scores, int64_t ld_scores, int32
                                              d_row_filter, d_range, n_thresholds, grid_f32, d_out_thresholds,
                                              d_out_counts, d_out_n_pos, static_cast<unsigned long long*>(d_workspace),
                                              dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+size_t mmrs_range_search_workspace_bytes(int64_t window_rows, int32_t dim, int32_t n_queries) {
+  if (window_rows < kTileRows || window_rows % kTileRows != 0 || dim < 1 || n_queries < 1) return 0;
+  return carve_range(nullptr, window_rows, dim, n_queries).total_bytes;
+}
+
+static int check_range_window(int64_t window_rows, int32_t n_queries, const void* d_workspace, size_t workspace_bytes,
+                              int32_t dim) {
+  if (window_rows < kTileRows || window_rows % kTileRows != 0 || window_rows > 0x7fffffffll)
+    return fail(MMRS_ERR_ARG, "window_rows = %lld must be a positive multiple of %d below 2^31", (long long)window_rows,
+                kTileRows);
+  if (n_queries < 1 || n_queries > 65535) return fail(MMRS_ERR_ARG, "n_queries = %d must be in [1, 65535]", n_queries);
+  const size_t need = mmrs_range_search_workspace_bytes(window_rows, dim, n_queries);
+  if (!d_workspace || workspace_bytes < need || reinterpret_cast<uintptr_t>(d_workspace) % 256)
+    return fail(MMRS_ERR_WORKSPACE, "workspace %zu bytes, need %zu (256-byte aligned)", workspace_bytes, need);
+  return MMRS_OK;
+}
+
+int mmrs_range_search_window(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
+                             int32_t gallery_dtype, const float* d_queries, int32_t n_queries, int64_t ld_queries,
+                             int32_t normalize_queries, float scale, int32_t path, const float* d_thresholds,
+                             int64_t row_begin, int64_t window_rows, const uint32_t* d_row_filter,
+                             const int32_t* d_row_labels, const int32_t* d_query_labels, int32_t label_match,
+                             int64_t* h_counts, void* d_workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  rc = check_matrix(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, "gallery");
+  if (rc != MMRS_OK) return rc;
+  rc = check_range_window(window_rows, n_queries, d_workspace, workspace_bytes, dim);
+  if (rc != MMRS_OK) return rc;
+  if (row_begin < 0 || row_begin >= n_rows || row_begin % kTileRows != 0)
+    return fail(MMRS_ERR_ARG, "row_begin = %lld must be a multiple of %d inside the %lld rows", (long long)row_begin,
+                kTileRows, (long long)n_rows);
+  if (!d_queries || ld_queries < dim || !d_thresholds || !h_counts) return fail(MMRS_ERR_ARG, "bad query / output arguments");
+  rc = check_row_filter(d_row_filter);
+  if (rc != MMRS_OK) return rc;
+  rc = check_labels(d_row_labels, d_query_labels, label_match);
+  if (rc != MMRS_OK) return rc;
+  const Path p = choose_path(path, gallery_dtype, n_queries);
+  if (p == Path::kMma && gallery_dtype == MMRS_DTYPE_F32)
+    return fail(MMRS_ERR_ARG, "MMRS_PATH_MMA needs a bf16 (or bf16x3) gallery");
+  const RangeWorkspace w = carve_range(d_workspace, window_rows, dim, n_queries);
+  const int32_t ldq = padded_dim(dim), qp = padded_queries(n_queries);
+  const int64_t rows = n_rows - row_begin < window_rows ? n_rows - row_begin : window_rows;
+  const int64_t n_words = window_rows / 32;
+  MMRS_CUDA(cudaMemsetAsync(w.base.flags, 0, 8 * sizeof(int32_t), stream));
+  MMRS_CUDA(cudaMemsetAsync(w.cnt, 0, static_cast<size_t>(n_queries) * sizeof(uint32_t), stream));
+  MMRS_LAUNCH(launch_fill_u32(w.cnt + n_queries, static_cast<uint32_t>(window_rows), kRangePadLists, stream));
+  MMRS_CUDA(cudaMemsetAsync(w.bitmap, 0, static_cast<size_t>(n_queries) * n_words * sizeof(uint32_t), stream));
+  MMRS_LAUNCH(launch_prep_queries(d_queries, n_queries, ld_queries, dim, normalize_queries,
+                                gallery_dtype == MMRS_DTYPE_BF16 ? 1 : (gallery_dtype == MMRS_DTYPE_BF16X3 ? 2 : 0),
+                                w.base.q_f32, w.base.q_bf16, qp, ldq, w.base.flags, GatherPrologue{}, stream));
+  // the window is a view of the gallery, like a shard: rows [row_begin, row_begin + rows) as local rows 0..rows-1
+  // (row_begin is a multiple of 128, so the view's bitmap words and labels start on whole tiles)
+  const size_t elem = gallery_dtype == MMRS_DTYPE_F32 ? sizeof(float) : sizeof(__nv_bfloat16);
+  ScanParams base{};
+  base.gallery = static_cast<const char*>(d_gallery) + static_cast<size_t>(row_begin) * ld_gallery * elem;
+  base.n_rows = rows; base.ld = ld_gallery; base.dim = dim;
+  base.queries = w.base.q_f32; base.ldq = ldq; base.scale = scale;
+  const int32_t n_tiles = static_cast<int32_t>((rows + kTileRows - 1) / kTileRows);
+  base.sched = TileSchedule{n_tiles, 1, 0, n_tiles};
+  // cap = window_rows >= rows: a list holds at most one key per row, so it cannot overflow
+  base.cand = w.cand; base.cnt = w.cnt; base.thr = d_thresholds; base.cap = static_cast<int32_t>(window_rows);
+  base.row_filter = d_row_filter ? d_row_filter + row_begin / 32 : nullptr;
+  base.row_labels = d_row_labels ? d_row_labels + row_begin : nullptr;
+  base.query_labels = d_row_labels ? d_query_labels : nullptr;
+  base.label_match = d_row_labels ? label_match : 0;
+  rc = run_scan(p, dev, gallery_dtype, base, w.base, qp, 0, n_queries, kModeFilter, stream, n_rows);
+  if (rc != MMRS_OK) return rc;
+  MMRS_LAUNCH(launch_range_mark_prefix(w.cand, window_rows, w.cnt, n_queries, w.bitmap, w.word_base, w.chunk_sum,
+                                       w.total, dev.sm_count, stream));
+  int32_t* h = pinned_status();
+  if (!h) return fail(MMRS_ERR_CUDA, "cudaHostAlloc for the status word failed");
+  MMRS_CUDA(cudaMemcpyAsync(h, w.base.flags, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaMemcpyAsync(h_counts, w.total, static_cast<size_t>(n_queries) * sizeof(int64_t),
+                            cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  return flags_to_status(h[0]);
+}
+
+int mmrs_range_search_scatter(int32_t n_queries, int64_t window_rows, int32_t dim, const int64_t* d_out_offsets,
+                              int64_t index_offset, float* d_out_values, int64_t* d_out_indices, void* d_workspace,
+                              size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  rc = check_range_window(window_rows, n_queries, d_workspace, workspace_bytes, dim);
+  if (rc != MMRS_OK) return rc;
+  if (!d_out_offsets || !d_out_values || !d_out_indices) return fail(MMRS_ERR_ARG, "null output pointer");
+  const RangeWorkspace w = carve_range(d_workspace, window_rows, dim, n_queries);
+  MMRS_LAUNCH(launch_range_scatter(w.cand, window_rows, w.cnt, n_queries, w.bitmap, w.word_base, d_out_offsets,
+                                   index_offset, d_out_values, d_out_indices, dev.sm_count, stream));
   return MMRS_OK;
 }
 

@@ -556,8 +556,11 @@ int scan_mma_max_queries() {
 }
 bool scan_mma_available() { return true; }
 
+// g_plane_rows (split == 3): rows between two gallery planes -- the FULL gallery's row count, also when
+// p.gallery / p.n_rows are a row window of plane 0 (range search)
 cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, int32_t n_q_padded,
-                            int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split) {
+                            int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split,
+                            int64_t g_plane_rows) {
   const int n_qchunks = (p.nq + kMaxQ - 1) / kMaxQ;
   if (p.nq < 1 || n_qchunks > kMaxQChunks) return cudaErrorInvalidValue;
   if (split != 1 && split != 3) return cudaErrorInvalidValue;
@@ -568,7 +571,7 @@ cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, in
   cfg.n_umma = n_qchunks > 1 ? kMaxQ : (p.nq + 15) / 16 * 16;   // multi-chunk launches: full-width tiles (padded columns never pass)
   cfg.k_blocks = (p.dim + kBlockK - 1) / kBlockK;
   cfg.split = split;
-  cfg.g_plane_rows = p.n_rows;
+  cfg.g_plane_rows = g_plane_rows;
   cfg.q_plane_rows = n_q_padded;
   cfg.n_qchunks = n_qchunks;
   cfg.sticky = 0;
@@ -629,8 +632,9 @@ cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, in
   const size_t smem = 1024 + stage_bytes * stages + shared_struct + label_tail;
 
   CUtensorMap map_g, map_q;
-  if (static_cast<int64_t>(split) * p.n_rows > 0x7fffffffll - kBlockM) return cudaErrorInvalidValue;
-  if (!make_map(&map_g, p.gallery, static_cast<uint64_t>(split) * p.n_rows, static_cast<uint64_t>(p.dim),
+  const int64_t g_map_rows = static_cast<int64_t>(split - 1) * g_plane_rows + p.n_rows;   // = split * n_rows unwindowed
+  if (g_map_rows > 0x7fffffffll - kBlockM) return cudaErrorInvalidValue;
+  if (!make_map(&map_g, p.gallery, static_cast<uint64_t>(g_map_rows), static_cast<uint64_t>(p.dim),
                 static_cast<uint64_t>(p.ld), kBlockM))
     return cudaErrorNotSupported;
   if (!make_map(&map_q, q_bf16, static_cast<uint64_t>(split) * n_q_padded, static_cast<uint64_t>(p.ldq),

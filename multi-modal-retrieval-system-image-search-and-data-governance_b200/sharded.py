@@ -102,16 +102,19 @@ class ShardedGallery:
     score keys, and `local_counts(queries, shard, range, *, row_labels, query_labels, n_points, row_filter,
     normalize_queries, scale, path, grid_f32)` -> (thresholds [nq, T] float64, counts [nq, T, 2] int64, n_pos
     [nq] int64) of the shard; the product default is `thresholds.DeviceSweep`.
+    `local_range_search(queries, shard, thresholds, **kw)` -> CSR (offsets, values, indices) of the shard with
+    global indices is `search_range`'s local step (default: `range_search.search_range`).
     `fused=False` forces the NCCL all-gather variant (also: MMRS_NO_FUSED_GATHER=1).
     """
 
     def __init__(self, local, n_rows_global: int, group: Optional[dist.ProcessGroup] = None,
                  local_search: Optional[Callable] = None, merge: Optional[Callable] = None,
                  fused: Optional[bool] = None, local_range: Optional[Callable] = None,
-                 local_counts: Optional[Callable] = None):
+                 local_counts: Optional[Callable] = None, local_range_search: Optional[Callable] = None):
         if (local_range is None) != (local_counts is None):
             raise ValueError("local_range and local_counts come together")
         self._local_range, self._local_counts = local_range, local_counts
+        self._local_range_search = local_range_search
         self.local = local
         self.n_rows_global = int(n_rows_global)
         self.group = group
@@ -558,6 +561,52 @@ class ShardedGallery:
             return flat[:counts.numel()].view(counts.shape), flat[counts.numel():]
 
         return run_chunks(queries, ql, qc, n_points, range_step, count_step, reduce_range, reduce_counts)
+
+    def search_range(self, queries, thresholds, *, normalize_queries: bool = True, scale: float = 1.0,
+                     path: str = "auto", row_filter=None, row_labels=None, query_labels=None, label_match: str = "same",
+                     max_candidate_bytes: int = 4 << 30):
+        """`search_range` over the sharded gallery: the same CSR (offsets, values, indices) on every rank, equal
+        to the single-GPU call on the full gallery.  `queries`, `thresholds`, `query_labels`, `row_labels` and
+        `row_filter` are the same on every rank, the last two over the GLOBAL rows.  Each rank range-searches
+        its shard; one all-gather moves the per-query counts [world, Q], a second the values and indices
+        (padded to the largest total); the pieces are joined per query in rank order, which is row order
+        because shards are ascending row blocks."""
+        from .range_search import concat_per_query, search_range, thresholds_f32
+        if isinstance(queries, np.ndarray):
+            queries = torch.from_numpy(queries)
+        if queries.dim() == 1:
+            queries = queries.unsqueeze(0)
+        nq = int(queries.shape[0])
+        thr = thresholds_f32(thresholds, nq)      # a NaN threshold raises on every rank alike
+        labels = self._local_labels(row_labels, query_labels, label_match, queries)
+        kw = dict(normalize_queries=normalize_queries, scale=scale, path=path, max_candidate_bytes=max_candidate_bytes)
+        if row_filter is not None:
+            kw["row_filter"] = self._local_filter(row_filter)[1]
+        if labels is not None:
+            kw.update(row_labels=labels[0], query_labels=labels[1], label_match=label_match)
+        local = self._local_range_search or search_range
+        on_host = not queries.is_cuda
+        if self._local_range_search is None and self.world > 1 and on_host:
+            queries = queries.to(self.local.device)       # NCCL gathers device tensors: search there, copy back
+        off, v, i = local(queries, self.local, thr, **kw)
+        if self.world == 1:
+            return off, v, i
+        counts = _all_gather(off[1:] - off[:-1], self.world, self.group)          # [world, Q]
+        totals = counts.sum(1)
+        m = max(1, int(totals.max().item()))
+        bufs = []
+        for x in (v, i):
+            b = torch.zeros(m, dtype=x.dtype, device=x.device)
+            b[:x.numel()] = x
+            bufs.append(_all_gather(b, self.world, self.group))
+        pieces = []
+        for r in range(self.world):
+            o = torch.zeros(nq + 1, dtype=torch.int64, device=counts.device)
+            torch.cumsum(counts[r], 0, out=o[1:])
+            n_r = int(totals[r].item())
+            pieces.append((o, bufs[0][r, :n_r], bufs[1][r, :n_r]))
+        out = concat_per_query(pieces)
+        return tuple(x.cpu() for x in out) if on_host and self._local_range_search is None else out
 
     def find_duplicate_pairs(self, emb_full: torch.Tensor, threshold: float, raw_join: Optional[Callable] = None):
         """Self-join with the gallery replicated (10M x 512 fp32 = 20 GB fits every GPU) and the
