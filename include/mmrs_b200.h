@@ -27,6 +27,9 @@
  *                         code/union_clip_llava2.py:153-162 (accept every image at or above a class's
  *                         threshold), tool/delete repeated.py (every row within tau of a query) --
  *                         the rows passing a per-query threshold, score matrix never stored
+ *   mmrs_resolve_duplicates
+ *                         tool/find_repeated_in_same_folder.py:76-95 (the keep / delete walk over the
+ *                         similar pairs, in file-size order), on the device
  *
  * Conventions
  *   - every function returns an int status: 0 = ok, negative = error (table below);
@@ -555,6 +558,31 @@ int mmrs_range_search_window(const void* d_gallery, int64_t n_rows, int32_t dim,
 int mmrs_range_search_scatter(int32_t n_queries, int64_t window_rows, int32_t dim, const int64_t* d_out_offsets,
                               int64_t index_offset, float* d_out_values, int64_t* d_out_indices, void* d_workspace,
                               size_t workspace_bytes, void* stream);
+
+/* ---- duplicate resolve: the keep / delete decision on a pair list ------------------------------ */
+
+/*
+ * The greedy first-keeper walk of tool/find_repeated_in_same_folder.py:76-95 (for each image in file-size
+ * order, `for ref in reference_hashes: if similar: duplicate of ref; break`, else it becomes a reference) on
+ * the pairs of the self-join, on the device.  d_pairs is int64 [n_pairs, 2] with ids in [0, n_items), in any
+ * order and orientation; repeated pairs and self-pairs are allowed (a self-pair has no effect).  d_order is
+ * the walk order: n_order distinct int64 ids in [0, n_items), possibly a subset; null means 0..n_order-1
+ * (n_order <= n_items).  d_representative [n_items] int64 receives, for each row v:
+ *   v                                          v is kept;
+ *   the kept neighbour of v first in d_order   v is removed (a duplicate of that row);
+ *   -1                                         v is not in d_order.
+ * That is the host walk's result: its representatives are the kept rows in walk order, its duplicates the
+ * (row, representative) of the removed rows in walk order.  n_items < 2^31.  A repeated or out-of-range order
+ * id and an out-of-range pair id are found on the device and return MMRS_ERR_ARG.
+ * h_rounds (HOST int64[2], nullable) receives the rounds run over the worklist of undecided rows and the
+ * number of rows the single-warp tail decided (0: the rounds finished alone).
+ * Workspace: mmrs_resolve_duplicates_workspace_bytes(n_items, n_order, n_pairs), 256-byte aligned.
+ * Synchronises `stream`: it reads the status word and the worklist counts.
+ */
+size_t mmrs_resolve_duplicates_workspace_bytes(int64_t n_items, int64_t n_order, int64_t n_pairs);
+int mmrs_resolve_duplicates(const int64_t* d_pairs, int64_t n_pairs, const int64_t* d_order, int64_t n_order,
+                            int64_t n_items, int64_t* d_representative, int64_t* h_rounds, void* d_workspace,
+                            size_t workspace_bytes, void* stream);
 
 /* ---- measurement hooks (bench.py; not needed by a product caller) --------------------------- */
 

@@ -23,7 +23,8 @@ plus the tensor-level entry points they sit on: search_topk, full_scores, find_d
 DeviceGallery, ShardedGallery, RowFilter (row-filtered search_topk: leave rows out per call) and
 RowLabels (label-conditioned search_topk: each query searches the rows of its own class, or of every other)
 and best_thresholds (the best-F1 threshold of every class prototype of a batch, find_thresholds per class) and
-search_range (every row at or above a per-query threshold, in CSR form).  Everything computes through the C-ABI CUDA library
+search_range (every row at or above a per-query threshold, in CSR form) and resolve_duplicates / deduplicate
+(greedy_first_keeper's keep / delete decision on the device: the representative of every row).  Everything computes through the C-ABI CUDA library
 (include/mmrs_b200.h); there is no CPU path -- without a B200 the calls raise.
 """
 from . import _cabi  # noqa: F401  (fails loudly when the CUDA library is missing)
@@ -35,20 +36,21 @@ from .search import (best_threshold_on_device, calc_combined_metrics, cls_acc, c
                      get_cluster_features, get_image_text_features, get_similarity, get_similarity_from_matrix,
                      image_text_prototypes, mix_image_text_query, outlier_filter_features, score_classes, search_topk,
                      threshold_sweep_counts, topk_of_scores)
-from .dedup import (calculate_image_hash, detect_and_remove_cross_set_duplicates, find_and_remove_duplicate_images,
-                    find_duplicate_pairs, find_and_remove_near_duplicate_images, get_all_images, greedy_first_keeper)
+from .dedup import (calculate_image_hash, deduplicate, detect_and_remove_cross_set_duplicates,
+                    find_and_remove_duplicate_images, find_duplicate_pairs, find_and_remove_near_duplicate_images,
+                    get_all_images, greedy_first_keeper, resolve_duplicates)
 from .sharded import ShardedGallery, shard_bounds
 from .range_search import search_range
 from .thresholds import best_thresholds
 
 __all__ = [
     "DeviceGallery", "RowFilter", "RowLabels", "ShardedGallery", "best_threshold_on_device", "best_thresholds", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
-    "cluster_prototype", "construct_dataset", "cosine_similarity_scores", "get_cluster_features", "get_image_text_features",
+    "cluster_prototype", "construct_dataset", "cosine_similarity_scores", "deduplicate", "get_cluster_features", "get_image_text_features",
     "image_text_prototypes", "topk_of_scores",
     "detect_and_remove_cross_set_duplicates", "evaluate_thresholds", "eval_threshold", "find_thresholds",
     "find_and_remove_duplicate_images", "find_and_remove_near_duplicate_images",
     "find_duplicate_pairs", "full_scores", "get_all_images", "get_similarity", "get_similarity_from_matrix",
-    "greedy_first_keeper", "load_feature_cache", "mix_image_text_query", "outlier_filter_features",
+    "greedy_first_keeper", "load_feature_cache", "mix_image_text_query", "outlier_filter_features", "resolve_duplicates",
     "score_classes", "search_range", "search_topk", "shard_bounds",
     "threshold_sweep_counts",
 ]

@@ -127,6 +127,9 @@ SIGNATURES = {
     "mmrs_range_search_window": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _f32, _i32, _vp, _i64,
                                            _i64, _vp, _vp, _vp, _i32, _vp, _vp, _sz, _vp]),
     "mmrs_range_search_scatter": (C.c_int, [_i32, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
+    # duplicate resolve: the greedy first-keeper decision on a pair list
+    "mmrs_resolve_duplicates_workspace_bytes": (_sz, [_i64, _i64, _i64]),
+    "mmrs_resolve_duplicates": (C.c_int, [_vp, _i64, _vp, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
 }
 for _name, (_res, _args) in SIGNATURES.items():
     _fn = getattr(lib, _name)

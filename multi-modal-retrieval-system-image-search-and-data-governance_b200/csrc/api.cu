@@ -68,6 +68,21 @@ cudaError_t launch_range_scatter(const uint64_t* cand, int64_t cap, const uint32
                                  const uint32_t* bitmap, const uint32_t* word_base, const int64_t* out_off,
                                  int64_t index_offset, float* values, int64_t* indices, int sm_count,
                                  cudaStream_t stream);
+// greedy first-keeper resolve (dedup_resolve.cu)
+cudaError_t launch_resolve_rank(const int64_t* order, int64_t n_order, int64_t n_items, uint32_t* rank, int32_t* status,
+                                int sm_count, cudaStream_t stream);
+cudaError_t launch_resolve_orient(const int64_t* pairs, int64_t n_pairs, int64_t n_items, const uint32_t* rank,
+                                  int64_t* edges, int32_t* status, int sm_count, cudaStream_t stream);
+cudaError_t launch_resolve_offsets(const int64_t* edges, int64_t n_edges, int64_t n_order, int64_t* off, int64_t* cursor,
+                                   int sm_count, cudaStream_t stream);
+cudaError_t launch_resolve_round(const int32_t* wl_in, const uint32_t* cnt_in, int64_t n_first, int64_t n_bound,
+                                 int32_t* wl_out, uint32_t* cnt_out, const int64_t* off, const int64_t* edges,
+                                 int64_t* cursor, int32_t* res, int sm_count, cudaStream_t stream);
+cudaError_t launch_resolve_tail(const int32_t* wl, const uint32_t* cnt, int64_t n_bound, uint32_t* range,
+                                const int64_t* off, const int64_t* edges, const int64_t* cursor, int32_t* res,
+                                int sm_count, cudaStream_t stream);
+cudaError_t launch_resolve_map_back(const int64_t* order, int64_t n_order, int64_t n_items, const int32_t* res,
+                                    int64_t* rep, int sm_count, cudaStream_t stream);
 int scan_mma_max_queries();
 int scan_mma_split_max_queries();
 bool scan_mma_available();
@@ -258,6 +273,46 @@ static RangeWorkspace carve_range(void* base, int64_t window_rows, int32_t dim, 
   r.total_bytes = off;
   return r;
 }
+
+// Duplicate resolve (mmrs_resolve_duplicates): a 256-byte header, then the rank, edge, CSR, decision and
+// worklist arrays of dedup_resolve.cu.
+struct ResolveWorkspace {
+  int32_t* header;         // [0] status bits, [1] [2] worklist counters, [4] [5] worklist rank range
+  uint32_t* rank;          // [n_items] rank of each row, 0xffffffff = not in the order
+  int64_t* edges;          // [n_pairs, 2] oriented (high rank, low rank), sorted in place
+  uint64_t* sort;          // mmrs_sort_pairs_workspace_bytes(n_pairs)
+  int64_t* off;            // [n_order + 1] first edge of each rank
+  int64_t* cursor;         // [n_order] next edge each undecided rank looks at
+  int32_t* res;            // [n_order] -1 undecided, r kept, else the representative's rank
+  int32_t* wl[2];          // [n_order] each: worklists of undecided ranks, ping-pong
+  size_t total_bytes;
+};
+
+static ResolveWorkspace carve_resolve(void* base, int64_t n_items, int64_t n_order, int64_t n_pairs) {
+  ResolveWorkspace r{};
+  size_t off = 0;
+  char* b = static_cast<char*>(base);
+  auto take = [&](size_t bytes) { char* p = b ? b + off : nullptr; off += align_up(bytes, 256); return p; };
+  const size_t items = static_cast<size_t>(n_items), ord = static_cast<size_t>(n_order),
+               pairs = static_cast<size_t>(n_pairs);
+  r.header = reinterpret_cast<int32_t*>(take(256));
+  r.rank = reinterpret_cast<uint32_t*>(take(items * sizeof(uint32_t)));
+  r.edges = reinterpret_cast<int64_t*>(take(pairs * 2 * sizeof(int64_t)));
+  r.sort = reinterpret_cast<uint64_t*>(take(mmrs_sort_pairs_workspace_bytes(n_pairs)));
+  r.off = reinterpret_cast<int64_t*>(take((ord + 1) * sizeof(int64_t)));
+  r.cursor = reinterpret_cast<int64_t*>(take(ord * sizeof(int64_t)));
+  r.res = reinterpret_cast<int32_t*>(take(ord * sizeof(int32_t)));
+  r.wl[0] = reinterpret_cast<int32_t*>(take(ord * sizeof(int32_t)));
+  r.wl[1] = reinterpret_cast<int32_t*>(take(ord * sizeof(int32_t)));
+  r.total_bytes = off;
+  return r;
+}
+// The host reads the worklist count once per batch of rounds.  A batch that decides fewer than
+// kResolveTailBelow rows per round hands the rest to the one-warp tail: a round costs a launch and a pass
+// over the whole worklist, and that little progress means long dependent chains (a path in walk order
+// decides about one rank per round), which the tail walks in one ascending sweep.
+constexpr int kResolveBatch = 4;
+constexpr int64_t kResolveTailBelow = 2048;
 
 static int check_matrix(const void* p, int64_t n_rows, int32_t dim, int64_t ld, int32_t dtype,
                         const char* what) {
@@ -1744,6 +1799,74 @@ int mmrs_range_search_scatter(int32_t n_queries, int64_t window_rows, int32_t di
   const RangeWorkspace w = carve_range(d_workspace, window_rows, dim, n_queries);
   MMRS_LAUNCH(launch_range_scatter(w.cand, window_rows, w.cnt, n_queries, w.bitmap, w.word_base, d_out_offsets,
                                    index_offset, d_out_values, d_out_indices, dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+
+size_t mmrs_resolve_duplicates_workspace_bytes(int64_t n_items, int64_t n_order, int64_t n_pairs) {
+  if (n_items < 0 || n_order < 0 || n_pairs < 0) return 0;
+  return carve_resolve(nullptr, n_items, n_order, n_pairs).total_bytes;
+}
+
+int mmrs_resolve_duplicates(const int64_t* d_pairs, int64_t n_pairs, const int64_t* d_order, int64_t n_order,
+                            int64_t n_items, int64_t* d_representative, int64_t* h_rounds, void* d_workspace,
+                            size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_items < 0 || n_items > 0x7fffffffll)
+    return fail(MMRS_ERR_ARG, "n = %lld rows: the resolve takes 0 <= n < 2^31", (long long)n_items);
+  if (n_order < 0 || n_order > 0x7fffffffll)
+    return fail(MMRS_ERR_ARG, "order of %lld ids: at most 2^31 - 1", (long long)n_order);
+  if (!d_order && n_order > n_items) return fail(MMRS_ERR_ARG, "a null order stands for the ids 0..n_order-1 <= n");
+  if (n_pairs < 0 || (n_pairs > 0 && !d_pairs) || (n_items > 0 && !d_representative))
+    return fail(MMRS_ERR_ARG, "bad pair / output arguments");
+  const size_t need = mmrs_resolve_duplicates_workspace_bytes(n_items, n_order, n_pairs);
+  if (!d_workspace || workspace_bytes < need || reinterpret_cast<uintptr_t>(d_workspace) % 256)
+    return fail(MMRS_ERR_WORKSPACE, "workspace %zu bytes, need %zu (256-byte aligned)", workspace_bytes, need);
+  int32_t* h = pinned_status();
+  if (!h) return fail(MMRS_ERR_CUDA, "cudaHostAlloc for the status word failed");
+  const ResolveWorkspace w = carve_resolve(d_workspace, n_items, n_order, n_pairs);
+  uint32_t* cnt = reinterpret_cast<uint32_t*>(w.header + 1);
+  uint32_t* range = reinterpret_cast<uint32_t*>(w.header + 4);
+  MMRS_CUDA(cudaMemsetAsync(w.header, 0, 256, stream));
+  MMRS_CUDA(cudaMemsetAsync(w.rank, 0xff, static_cast<size_t>(n_items) * sizeof(uint32_t), stream));
+  MMRS_CUDA(cudaMemsetAsync(d_representative, 0xff, static_cast<size_t>(n_items) * sizeof(int64_t), stream));   // -1
+  MMRS_CUDA(cudaMemsetAsync(w.res, 0xff, static_cast<size_t>(n_order) * sizeof(int32_t), stream));             // undecided
+  MMRS_LAUNCH(launch_resolve_rank(d_order, n_order, n_items, w.rank, w.header, dev.sm_count, stream));
+  MMRS_LAUNCH(launch_resolve_orient(d_pairs, n_pairs, n_items, w.rank, w.edges, w.header, dev.sm_count, stream));
+  MMRS_LAUNCH(launch_sort_pairs(w.edges, n_pairs, w.sort, stream));
+  MMRS_LAUNCH(launch_resolve_offsets(w.edges, n_pairs, n_order, w.off, w.cursor, dev.sm_count, stream));
+  // round k reads worklist (k + 1) & 1 (round 0: every rank) and writes worklist k & 1
+  int64_t known = n_order, rounds = 0, tail = 0;
+  while (known > 0) {
+    for (int b = 0; b < kResolveBatch; ++b, ++rounds) {
+      const int o = static_cast<int>(rounds & 1), i = o ^ 1;
+      MMRS_LAUNCH(launch_resolve_round(rounds ? w.wl[i] : nullptr, cnt + i, n_order, known, w.wl[o], cnt + o, w.off,
+                                       w.edges, w.cursor, w.res, dev.sm_count, stream));
+    }
+    MMRS_CUDA(cudaMemcpyAsync(h, w.header, 8 * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    MMRS_CUDA(cudaStreamSynchronize(stream));
+    if (h[0]) break;
+    const int last = static_cast<int>((rounds - 1) & 1);
+    const int64_t left = static_cast<uint32_t>(h[1 + last]);
+    const int64_t decided = known - left;
+    known = left;
+    if (left > 0 && decided < kResolveBatch * kResolveTailBelow) {
+      MMRS_LAUNCH(launch_resolve_tail(w.wl[last], cnt + last, left, range, w.off, w.edges, w.cursor, w.res,
+                                      dev.sm_count, stream));
+      tail = left;
+      break;
+    }
+  }
+  MMRS_LAUNCH(launch_resolve_map_back(d_order, n_order, n_items, w.res, d_representative, dev.sm_count, stream));
+  MMRS_CUDA(cudaMemcpyAsync(h, w.header, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  if (h_rounds) { h_rounds[0] = rounds; h_rounds[1] = tail; }
+  if (h[0] & kResolvePairRange) return fail(MMRS_ERR_ARG, "a pair id is outside [0, %lld)", (long long)n_items);
+  if (h[0] & kResolveOrderRange) return fail(MMRS_ERR_ARG, "an order id is outside [0, %lld)", (long long)n_items);
+  if (h[0] & kResolveOrderRepeat) return fail(MMRS_ERR_ARG, "an id appears more than once in the order");
   return MMRS_OK;
 }
 

@@ -20,6 +20,11 @@ constexpr int kFlagShort = 4;         // fewer than k candidates reached a selec
 constexpr int kFlagWatchdog = 8;      // an mbarrier wait timed out (K2 debug guard)
 constexpr int kFlagGatherTimeout = 16;  // fused all-gather: a peer rank's flag did not arrive in time
 
+// Status bits of the duplicate resolve (dedup_resolve.cu), in its own status word.
+constexpr int kResolveOrderRange = 1;   // an order id outside [0, n_items)
+constexpr int kResolveOrderRepeat = 2;  // an id appears twice in the order
+constexpr int kResolvePairRange = 4;    // a pair id outside [0, n_items)
+
 // ---- order-preserving (score, row) -> u64 key ---------------------------------------------
 // Larger key == better match: higher score first, then LOWER row index.  Keys are unique
 // because row indices are, so "the k largest keys" is a deterministic set and order -- this is

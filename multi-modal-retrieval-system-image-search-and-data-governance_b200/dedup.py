@@ -9,6 +9,7 @@ BASELINE.json replaces the hash predicates by `cos(e_i, e_j) >= tau` on unit-nor
 """
 from __future__ import annotations
 
+import ctypes as C
 import os
 from typing import Callable, Optional, Sequence
 
@@ -145,12 +146,16 @@ def find_duplicate_pairs(emb, threshold: float, *, device=None, method: str = "a
     unit-norm for the margin to hold), ~20x the throughput.  "auto": "tc" from 2048 rows on."""
     on_host = not isinstance(emb, DeviceGallery) and not (isinstance(emb, torch.Tensor) and emb.is_cuda)
     x = _device_f32(emb, device)
+    pairs = sort_pairs(_join_raw(x, threshold, method), int(x.shape[0]))
+    return pairs.cpu() if on_host else pairs
+
+
+def _join_raw(x: torch.Tensor, threshold: float, method: str) -> torch.Tensor:
+    """The unsorted pair list of find_duplicate_pairs' `method` on a device fp32 matrix."""
     if method not in ("auto", "fp32", "tc"):
         raise ValueError("method must be 'auto', 'fp32' or 'tc'")
     use_tc = method == "tc" or (method == "auto" and x.shape[0] >= 2048)
-    raw = selfjoin_tc_raw(x, threshold) if use_tc else selfjoin_raw(x, threshold)
-    pairs = sort_pairs(raw, int(x.shape[0]))
-    return pairs.cpu() if on_host else pairs
+    return selfjoin_tc_raw(x, threshold) if use_tc else selfjoin_raw(x, threshold)
 
 
 def greedy_first_keeper(n: int, pairs, order: Sequence[int]):
@@ -178,6 +183,93 @@ def greedy_first_keeper(n: int, pairs, order: Sequence[int]):
             keep_rank[item] = len(reps)
             reps.append(int(item))
     return reps, dups
+
+
+MAX_RESOLVE_ROWS = 2 ** 31 - 1     # ranks and row ids are 32-bit on the device
+
+
+def _resolve_args(pairs, n, order):
+    """Host-side checks of resolve_duplicates -> (pairs, n, order or None, device or None); raises ValueError."""
+    if isinstance(n, bool) or not isinstance(n, (int, np.integer)):
+        raise ValueError(f"n must be an integer row count, got {n!r}")
+    n = int(n)
+    if not 0 <= n <= MAX_RESOLVE_ROWS:
+        raise ValueError(f"n = {n}: the resolve takes 0 <= n < 2^31 rows")
+    if isinstance(pairs, np.ndarray):
+        pairs = torch.from_numpy(np.ascontiguousarray(pairs))
+    if not isinstance(pairs, torch.Tensor):
+        raise ValueError(f"pairs must be an int64 [P, 2] tensor, got {type(pairs).__name__}")
+    if pairs.dtype != torch.int64:
+        raise ValueError(f"pairs must be int64, got {pairs.dtype}")
+    if pairs.dim() != 2 or pairs.shape[1] != 2:
+        raise ValueError(f"pairs must be [P, 2], got {tuple(pairs.shape)}")
+    if order is not None:
+        if isinstance(order, np.ndarray):
+            order = torch.from_numpy(np.ascontiguousarray(order))
+        elif not isinstance(order, torch.Tensor):
+            order = torch.as_tensor(list(order), dtype=torch.int64)
+        if order.dtype != torch.int64:
+            raise ValueError(f"order must be int64 row ids, got {order.dtype}")
+        if order.dim() != 1:
+            raise ValueError(f"order must be 1-D, got {tuple(order.shape)}")
+        if order.numel() > MAX_RESOLVE_ROWS:
+            raise ValueError(f"order has {order.numel()} ids: at most 2^31 - 1")
+    dev = pairs.device if pairs.is_cuda else (order.device if order is not None and order.is_cuda else None)
+    return pairs, n, order, dev
+
+
+def _resolve(pairs, n: int, order=None):
+    """resolve_duplicates plus the schedule it took: (representative, rounds, rows decided by the tail)."""
+    pairs, n, order, dev = _resolve_args(pairs, n, order)
+    on_host = dev is None
+    if on_host:
+        dev = torch.device("cuda", torch.cuda.current_device() if torch.cuda.is_available() else 0)
+    _cabi.require_b200(dev.index or 0)
+    with torch.cuda.device(dev):
+        p = pairs.to(dev).contiguous()
+        o = order.to(dev).contiguous() if order is not None else None
+        n_order = n if o is None else int(o.numel())
+        rep = torch.empty(n, dtype=torch.int64, device=dev)
+        lib = _cabi.lib
+        ws_bytes = int(lib.mmrs_resolve_duplicates_workspace_bytes(n, n_order, int(p.shape[0])))
+        ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
+        stats = (C.c_int64 * 2)()
+        st = lib.mmrs_resolve_duplicates(p.data_ptr() if p.numel() else None, int(p.shape[0]),
+                                         o.data_ptr() if o is not None and o.numel() else None,   # null: 0..n_order-1
+                                         n_order, n, rep.data_ptr() if n else None, stats,
+                                         DeviceGallery.aligned_ptr(ws), ws_bytes, _stream_handle(dev))
+        if st == _cabi.ERR_ARG:
+            raise ValueError(_cabi.last_error())
+        _cabi.check(st)
+    return (rep.cpu() if on_host else rep), int(stats[0]), int(stats[1])
+
+
+def resolve_duplicates(pairs, n: int, *, order=None) -> torch.Tensor:
+    """The decision of `greedy_first_keeper` on the device: int64 [n] with representative[v] =
+        v                                        if v is kept,
+        the kept neighbour of v first in order   if v is removed (v duplicates it),
+        -1                                       if v is not in `order`.
+    `pairs` is int64 [P, 2] with ids in [0, n), in any order and orientation (repeated and self-pairs
+    allowed; a self-pair has no effect); `order` the walk order, distinct ids in [0, n) (default
+    0..n-1; a subset is allowed -- the reference walks by file size, pass that permutation).  For such
+    inputs `[v for v in order if rep[v] == v]` is greedy_first_keeper's representatives and
+    `[(v, rep[v]) for v in order if rep[v] not in (v, -1)]` its duplicates.  A repeated or out-of-range
+    order id, an out-of-range pair id and n >= 2^31 raise ValueError.  Device input gives a device
+    result; host input runs on the current device and returns a host tensor.
+    `rep == torch.arange(n, device=rep.device)` is the keep mask (RowFilter of the deduplicated gallery)."""
+    return _resolve(pairs, n, order)[0]
+
+
+def deduplicate(emb, threshold: float, *, order=None, method: str = "auto", device=None) -> torch.Tensor:
+    """find_duplicate_pairs followed by resolve_duplicates, with the pair list kept on the device and
+    unsorted (the resolve does not need the lexicographic order).  Same inputs and `method` as
+    find_duplicate_pairs; returns the [n] representative tensor (host input gives a host result)."""
+    on_host = not isinstance(emb, DeviceGallery) and not (isinstance(emb, torch.Tensor) and emb.is_cuda)
+    if method not in ("auto", "fp32", "tc"):
+        raise ValueError("method must be 'auto', 'fp32' or 'tc'")     # before the embeddings are uploaded
+    x = _device_f32(emb, device)
+    rep = resolve_duplicates(_join_raw(x, threshold, method), int(x.shape[0]), order=order)
+    return rep.cpu() if on_host else rep
 
 
 # ---- file level -------------------------------------------------------------------------------

@@ -632,3 +632,12 @@ class ShardedGallery:
         allbuf = _all_gather(buf, self.world, self.group)
         parts = [allbuf[r, :int(cnts[r].item())] for r in range(self.world)]
         return sort_pairs(torch.cat(parts, dim=0), n)
+
+    def deduplicate(self, emb_full: torch.Tensor, threshold: float, *, order=None,
+                    raw_join: Optional[Callable] = None) -> torch.Tensor:
+        """`deduplicate` over the ranks: the pairs of `find_duplicate_pairs` (every rank holds the whole
+        gathered list), then `resolve_duplicates` on each rank.  The resolve is deterministic, so every rank
+        returns the same [n] representative tensor without another collective."""
+        from .dedup import resolve_duplicates
+        pairs = self.find_duplicate_pairs(emb_full, threshold, raw_join=raw_join)
+        return resolve_duplicates(pairs, int(emb_full.shape[0]), order=order)
