@@ -411,7 +411,8 @@ size_t mmrs_selfjoin_workspace_bytes(int64_t n_rows, int32_t dim, int32_t dtype)
  * in UNSPECIFIED order (the Python tier sorts them lexicographically); *d_out_count (device
  * int64) receives the number found even when it exceeds `capacity`
  * (then MMRS_ERR_CAPACITY is returned and only `capacity` pairs are valid).
- * [row_begin, row_end) is this rank's slice of the upper-triangular schedule.
+ * [row_begin, row_end) is this rank's slice of the upper-triangular schedule; any
+ * 0 <= row_begin <= row_end <= n_rows is allowed, so consecutive ranges partition the join.
  * The call synchronises `stream`.
  */
 int mmrs_selfjoin_pairs(const void* d_emb, int64_t n_rows, int32_t dim, int64_t ld_emb,
@@ -423,8 +424,9 @@ int mmrs_selfjoin_pairs(const void* d_emb, int64_t n_rows, int32_t dim, int64_t 
  * Tensor-core form of the same join: a bf16 tcgen05 pass over d_emb_bf16 (the same rows rounded to
  * bf16) keeps pairs with <e_i, e_j> >= threshold - margin, and every survivor is re-scored in fp32
  * from d_emb_f32 with the arithmetic of mmrs_selfjoin_pairs, so the emitted set is identical to
- * the exact mode's provided margin covers the bf16 rounding (unit-norm rows: margin >= 0.004, see
- * csrc/selfjoin_mma.cu).  The upper triangle is split into panels of 2048 columns dealt round-robin
+ * the exact mode's provided margin covers the bf16 rounding and both fp32 accumulations: for rows of
+ * norm at most r, margin >= (2^-7 + 2^-16 + dim * 2^-22) * max(1, r^2) (derived in
+ * csrc/selfjoin_mma.cu; the Python tier passes exactly this).  The upper triangle is split into panels of 2048 columns dealt round-robin
  * to `world` ranks; this call does rank `rank`'s share.  d_out_count is device int64[2]:
  * [0] pairs found, [1] candidates that passed the prefilter; MMRS_ERR_CAPACITY when either exceeds
  * its capacity (the counts are still reported so the caller can size a retry).

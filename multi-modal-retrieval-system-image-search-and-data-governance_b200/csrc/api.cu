@@ -1435,9 +1435,8 @@ int mmrs_selfjoin_pairs(const void* d_emb, int64_t n_rows, int32_t dim, int64_t 
   if (rc != MMRS_OK) return rc;
   if (dtype != MMRS_DTYPE_F32) return fail(MMRS_ERR_ARG, "self-join exact mode takes fp32 embeddings");
   if (dim % 8 != 0) return fail(MMRS_ERR_ARG, "self-join dim must be a multiple of 8 (pad with zeros)");
-  if (row_begin < 0 || row_end > n_rows || row_begin > row_end || row_begin % 128 != 0)
-    return fail(MMRS_ERR_ARG, "row range [%lld, %lld) invalid (begin must be a multiple of 128)",
-                (long long)row_begin, (long long)row_end);
+  if (row_begin < 0 || row_end > n_rows || row_begin > row_end)
+    return fail(MMRS_ERR_ARG, "row range [%lld, %lld) invalid", (long long)row_begin, (long long)row_end);
   if (capacity < 0 || (capacity > 0 && !d_out_pairs) || !d_out_count)
     return fail(MMRS_ERR_ARG, "bad output arguments");
   MMRS_CUDA(cudaMemsetAsync(d_out_count, 0, sizeof(int64_t), stream));

@@ -25,7 +25,8 @@ struct SelfJoinParams {
   int64_t ld;
   int32_t dim;
   float threshold;
-  int64_t bi_begin, bi_end;   // row-block range of the "i" side owned by this call
+  int64_t row_begin, row_end; // rows of the "i" side owned by this call
+  int64_t bi_begin, bi_end;   // the row blocks that hold them
   int64_t nb;                 // number of row blocks
   int64_t total_tiles;
   int64_t* out_pairs;
@@ -100,7 +101,7 @@ __global__ void __launch_bounds__(kSjThreads) selfjoin_f32_kernel(const SelfJoin
 #pragma unroll
       for (int y = 0; y < 8; ++y) {
         const int64_t i = i0 + ty * 8 + x, j = j0 + tx * 8 + y;
-        if (i < j && j < p.n_rows && acc[x][y] >= p.threshold) {
+        if (i >= p.row_begin && i < p.row_end && i < j && j < p.n_rows && acc[x][y] >= p.threshold) {
           const unsigned long long pos = atomicAdd(p.out_count, 1ull);
           if (pos < static_cast<unsigned long long>(p.capacity)) {
             p.out_pairs[2 * pos] = i;
@@ -118,6 +119,7 @@ cudaError_t launch_selfjoin_f32(const float* emb, int64_t n_rows, int32_t dim, i
   SelfJoinParams p{};
   p.emb = emb; p.n_rows = n_rows; p.ld = ld; p.dim = dim; p.threshold = threshold;
   p.nb = (n_rows + kSjTile - 1) / kSjTile;
+  p.row_begin = row_begin; p.row_end = row_end;   // the blocks at either end may hold rows outside the range
   p.bi_begin = row_begin / kSjTile;
   p.bi_end = (row_end + kSjTile - 1) / kSjTile;
   if (p.bi_end > p.nb) p.bi_end = p.nb;

@@ -6,12 +6,17 @@
 // by a PAIR of CTAs (one TPC): each CTA stages its own 128-row i-block and half of the j-block,
 // CTA 0's MMA warp issues for both, each CTA's 128 x 256 accumulator lands in its own TMEM (less
 // operand traffic per SM, see scan_mma.cu); long joins use single CTAs (M=128) instead, see
-// sjm_pair_mode.  The epilogue keeps pairs (i < j) with S >= tau - margin.  Rounding unit rows to bf16 moves a
-// dot product by at most ||a|| ||b - b^|| + ||a - a^|| ||b^|| <= 2 * 2^-9 (1 + 2^-9) < 0.004
-// (Cauchy-Schwarz; round-to-nearest is within 2^-9 relative per element), so with margin >= 0.004
-// every true pair survives; the few survivors are then re-scored in fp32 with exactly the
-// arithmetic of the exact kernel (selfjoin.cu: one fmaf chain, k ascending), which makes the
-// emitted pair set identical to the exact mode's.
+// sjm_pair_mode.  The epilogue keeps pairs (i < j) with S >= tau - margin.  bf16 keeps 8 significant
+// bits, so round-to-nearest moves each element by at most u = 2^-8 of its value, and rounding both rows
+// moves their dot product by at most ||a|| ||b - b^|| + ||a - a^|| ||b^|| <= (2u + u^2) ||a|| ||b||
+// (Cauchy-Schwarz).  Rows whose elements all sit just above a power of two, 2^e (1 + 0.99 * 2^-8), reach
+// 99 % of that bound: 0.0077 for unit rows.  Each fp32 dot product adds at most
+// dim * 2^-24 / (1 - dim * 2^-24) ||a|| ||b|| when rounded to nearest: the exact mode's sum that decides
+// the pair, and S, whose accumulation order and rounding on the tensor cores are not documented; the
+// margin allows dim * 2^-22 for the two.  So with margin >= (2^-7 + 2^-16 + dim * 2^-22) max(1, max ||a||^2)
+// (dedup.tc_margin) every pair the exact mode emits survives; the few survivors are then re-scored in
+// fp32 with exactly the arithmetic of the exact kernel (selfjoin.cu: one fmaf chain, k ascending),
+// which makes the emitted pair set identical to the exact mode's.
 //
 // Schedule: the upper triangle is cut into panels of 8 j-blocks (2048 rows: 2 MB of bf16 at
 // D = 512, L2 resident); inside a panel tiles are numbered j-fastest, so CTAs that run together

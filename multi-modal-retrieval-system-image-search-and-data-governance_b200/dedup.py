@@ -45,7 +45,9 @@ def _device_f32(emb, device=None) -> torch.Tensor:
 def selfjoin_raw(x: torch.Tensor, threshold: float, row_begin: int = 0, row_end: Optional[int] = None,
                  capacity: Optional[int] = None) -> torch.Tensor:
     """Unsorted int64 [P, 2] pairs (i < j, row_begin <= i < row_end) from the CUDA kernel;
-    grows the pair buffer and retries when the kernel reports more pairs than `capacity`."""
+    grows the pair buffer and retries when the kernel reports more pairs than `capacity`.
+    A NaN or infinite row raises ValueError, as on the tensor-core path."""
+    _max_row_norm(x)
     n = int(x.shape[0])
     row_end = n if row_end is None else int(row_end)
     lib = _cabi.lib
@@ -65,7 +67,19 @@ def selfjoin_raw(x: torch.Tensor, threshold: float, row_begin: int = 0, row_end:
             return pairs[:found]
 
 
-BF16_MARGIN = 0.0045   # > 2 * 2^-9 * (1 + 2^-9): bound on the bf16 rounding of a unit-norm dot product
+# bf16 keeps 8 significant bits, so rounding an element moves it by at most u = 2^-8 of its value, and
+# rounding both operands moves a dot product by at most (2u + u^2) |a| |b| (Cauchy-Schwarz).
+BF16_MARGIN = 2.0 ** -7 + 2.0 ** -16
+
+
+def tc_margin(dim: int, max_norm: float, unit_margin: float = BF16_MARGIN) -> float:
+    """The prefilter margin of the tensor-core join on rows of at most `max_norm`: a pair the exact
+    fp32 mode emits scores at least threshold - margin in the bf16 pass.  `unit_margin` bounds the bf16
+    operand rounding for unit rows; `dim * 2^-22` covers the two fp32 dot products (the tensor cores'
+    and the recheck's fmaf chain, each within dim * 2^-24 |a||b| when rounded to nearest), twice over
+    because the tensor cores' accumulation order and rounding are not documented.  Both terms scale
+    with |a||b| <= max_norm^2 (1.0001 absorbs the rounding of the measured norm)."""
+    return (float(unit_margin) + dim * 2.0 ** -22) * max(1.0, max_norm * max_norm * 1.0001)
 
 
 def row_norm_range(x32: torch.Tensor) -> "tuple[float, float]":
@@ -78,21 +92,28 @@ def row_norm_range(x32: torch.Tensor) -> "tuple[float, float]":
     return float(lo), float(hi)
 
 
+def _max_row_norm(x32: torch.Tensor) -> float:
+    """The largest row norm; ValueError when a row holds a NaN or an infinity (both joins refuse them:
+    the deletions that follow would depend on how each kernel treats a NaN score)."""
+    _, max_norm = row_norm_range(x32)
+    if not (max_norm < float("inf")):
+        raise ValueError("embeddings contain non-finite rows")
+    return max_norm
+
+
 def selfjoin_tc_raw(x32: torch.Tensor, threshold: float, rank: int = 0, world: int = 1,
                     x16: Optional[torch.Tensor] = None, margin: float = BF16_MARGIN,
                     capacity: Optional[int] = None) -> torch.Tensor:
     """Unsorted int64 [P, 2] pairs of rank `rank`'s panels: tcgen05 bf16 prefilter at
-    threshold - margin, exact fp32 recheck (mmrs_selfjoin_pairs_tc); buffers grow on demand.
-    `margin` bounds the bf16 rounding error of a dot product of UNIT rows; it is scaled by the
-    largest squared row norm found on the device (|<a,b> - <a16,b16>| <= ~2^-8 |a||b|), so rows that
-    are not unit-norm (raw CLIP features) cannot lose true pairs before the exact recheck."""
+    threshold - tc_margin(dim, max_norm, margin), exact fp32 recheck (mmrs_selfjoin_pairs_tc); buffers
+    grow on demand.  `margin` bounds the bf16 rounding error of a dot product of UNIT rows; the kernel
+    gets it widened by the fp32 accumulation bound and scaled by the largest squared row norm found on
+    the device, so rows that are not unit-norm (raw CLIP features) cannot lose true pairs before the
+    exact recheck.  A NaN or infinite row raises ValueError."""
     n, d = int(x32.shape[0]), int(x32.shape[1])
     lib = _cabi.lib
     dev = x32.device
-    _, max_norm = row_norm_range(x32)
-    if not (max_norm < float("inf")):
-        raise ValueError("embeddings contain non-finite rows")
-    margin = float(margin) * max(1.0, max_norm * max_norm * 1.0001)
+    margin = tc_margin(d, _max_row_norm(x32), margin)
     if x16 is None:
         x16 = x32.to(torch.bfloat16)
     cap = int(capacity) if capacity is not None else max(4096, n // 4)
@@ -142,8 +163,9 @@ def find_duplicate_pairs(emb, threshold: float, *, device=None, method: str = "a
     sorted lexicographically.  Host input gives a host result.
 
     method "fp32": every pair in fp32 on the CUDA cores.  "tc": bf16 tensor-core prefilter with a
-    safety margin + exact fp32 recheck of the survivors -- the same pair set (rows must be
-    unit-norm for the margin to hold), ~20x the throughput.  "auto": "tc" from 2048 rows on."""
+    safety margin (tc_margin) + exact fp32 recheck of the survivors -- the same pair set, ~20x the
+    throughput.  "auto": "tc" from 2048 rows on.  Every method raises ValueError on a NaN or
+    infinite row."""
     on_host = not isinstance(emb, DeviceGallery) and not (isinstance(emb, torch.Tensor) and emb.is_cuda)
     x = _device_f32(emb, device)
     pairs = sort_pairs(_join_raw(x, threshold, method), int(x.shape[0]))

@@ -349,3 +349,104 @@ def synthetic_dedup(n: int, d: int, dup_frac: float = 0.01, noise: float = 0.1, 
     x = l2_normalize(x)
     planted = sorted((min(int(a), int(b)), max(int(a), int(b))) for a, b in zip(src, dst))
     return x, planted
+
+
+# --------------------------------------------------------------------------------------------
+# self-join data at the edges of bf16 and fp32 rounding (the tensor-core join's prefilter margin)
+# --------------------------------------------------------------------------------------------
+def to_bf16_f64(x) -> np.ndarray:
+    """The values the bf16 tensor-core pass multiplies (round to nearest even), as float64."""
+    return torch.as_tensor(np.asarray(x, dtype=np.float32)).to(torch.bfloat16).to(torch.float64).numpy()
+
+
+def _fill_bf16_edge(x: np.ndarray, coords, target: float, rng, round_up: bool) -> float:
+    """Give coordinates of `x`, in the order given, entries +-2^e (1 + c 2^-8): c in (0.9, 1) rounds to bf16
+    as 2^e, c in (1, 1.1) as 2^e (1 + 2^-7), so every entry moves by 0.9-1 x 2^-8 of its value towards zero
+    (or away from it) and the rounding errors of a dot product add up instead of cancelling.  Each entry
+    takes the largest exponent that keeps the sum of squares within `target`; returns that sum (float64)."""
+    ss = float(np.square(x.astype(np.float64)).sum())
+    for k in coords:
+        rem = target - ss
+        if rem <= 2.0 ** -40:
+            break
+        e = int(np.floor(0.5 * np.log2(rem)))
+        while True:
+            c = rng.uniform(1.0, 1.1) if round_up else rng.uniform(0.9, 1.0)
+            v = np.float32(2.0 ** e * (1.0 + c * 2.0 ** -8))
+            if float(v) ** 2 <= rem:
+                break
+            e -= 1
+        x[k] = v if rng.random() < 0.5 else -v
+        ss += float(v) ** 2
+    return ss
+
+
+def bf16_edge_pairs(n_pairs: int, d: int, lo: float, hi: float, round_up: bool, seed: int = 0):
+    """Pairs of fp32 rows whose exact dot product lies in [lo, hi) (0 < lo < hi <= 1) and whose bf16
+    rounding moves that dot product by nearly the most it can: all entries of both rows round towards
+    zero (round_up=False: the bf16 dot product is ~2^-7 |<a, b>| SMALLER) or away from zero (LARGER).
+    Row b equals row a on a random half of the coordinates (all of them when d <= 8), a and b fill the
+    rest with disjoint tails; both rows have norm <= 1.  Returns (rows [2 * n_pairs, d] float32 with
+    pair t in rows 2t, 2t + 1, exact dot products float64 [n_pairs])."""
+    rng = np.random.default_rng(seed)
+    rows = np.zeros((2 * n_pairs, d), dtype=np.float32)
+    dots = np.zeros(n_pairs)
+    for t in range(n_pairs):
+        for _ in range(1000):
+            a = np.zeros(d, dtype=np.float32)
+            perm = rng.permutation(d)
+            n_shared = d if d <= 8 else d // 2
+            dot = _fill_bf16_edge(a, perm[:n_shared], rng.uniform(lo, hi), rng, round_up)
+            if dot >= lo:
+                break
+        else:
+            raise RuntimeError(f"no pair with a dot product in [{lo}, {hi}) at d = {d}")
+        b = a.copy()
+        tail = perm[n_shared:]
+        _fill_bf16_edge(a, tail[: len(tail) // 2], 1.0, rng, round_up)
+        _fill_bf16_edge(b, tail[len(tail) // 2:], 1.0, rng, round_up)
+        rows[2 * t], rows[2 * t + 1] = a, b
+        dots[t] = dot
+    return rows, dots
+
+
+def threshold_pairs(n_pairs: int, d: int, threshold: float, seed: int = 0):
+    """Pairs whose exact dot product lies within a few fp32 ulps of `threshold`: a random unit row a and
+    b = fp32(a * s), s = threshold (1 + k 2^-23) / |a|^2 with k in -4..4.  Returns rows as bf16_edge_pairs."""
+    g = torch.Generator().manual_seed(seed)
+    a = l2_normalize(torch.randn(n_pairs, d, generator=g, dtype=torch.float64)).to(torch.float32)
+    k = torch.randint(-4, 5, (n_pairs, 1), generator=g).to(torch.float64)
+    a64 = a.to(torch.float64)
+    s = threshold * (1.0 + k * 2.0 ** -23) / (a64 * a64).sum(1, keepdim=True)
+    b = (a64 * s).to(torch.float32)
+    return torch.stack([a, b], 1).reshape(2 * n_pairs, d).numpy()
+
+
+def dedup_pairs_fp32_band(emb, threshold: float, block: int = 4096):
+    """The self-join's pair set as far as fp32 arithmetic decides it, from float64 scores S of the fp32
+    rows: (must, may), int64 [P, 2] sorted, with i < j.  `must` holds the pairs with S >= t + delta,
+    `may` those with S >= t - delta, t = float32(threshold) and delta = d 2^-24 / (1 - d 2^-24) |a| |b|,
+    the error bound of a d-term fp32 dot product rounded to nearest.  Any fp32 kernel's pair set lies
+    between the two."""
+    g = torch.as_tensor(np.asarray(emb, dtype=np.float32)).to(torch.float64)
+    n, d = g.shape
+    t = float(np.float32(threshold))
+    gamma = d * 2.0 ** -24 / (1.0 - d * 2.0 ** -24)
+    norms = g.norm(dim=1)
+    out = {"must": [], "may": []}
+    for i0 in range(0, n, block):
+        gi = g[i0:i0 + block]
+        for j0 in range(i0, n, block):
+            s = gi @ g[j0:j0 + block].t()
+            delta = gamma * norms[i0:i0 + block, None] * norms[None, j0:j0 + block]
+            ii = torch.arange(i0, i0 + gi.shape[0])[:, None]
+            jj = torch.arange(j0, min(n, j0 + block))[None, :]
+            upper = ii < jj
+            for key, hit in (("must", s >= t + delta), ("may", s >= t - delta)):
+                a, b = (hit & upper).nonzero(as_tuple=True)
+                out[key].append(torch.stack([a + i0, b + j0], 1))
+    res = []
+    for key in ("must", "may"):
+        p = torch.cat(out[key]) if out[key] else torch.empty((0, 2), dtype=torch.int64)
+        res.append(p[torch.argsort(p[:, 0] * n + p[:, 1])].contiguous())
+    return tuple(res)
