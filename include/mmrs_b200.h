@@ -65,7 +65,7 @@ extern "C" {
 #pragma GCC visibility push(default) /* the library itself is built with -fvisibility=hidden */
 #endif
 
-#define MMRS_ABI_VERSION 2
+#define MMRS_ABI_VERSION 3
 
 /* status codes */
 #define MMRS_OK 0
@@ -169,20 +169,25 @@ int mmrs_search_topk_host(const void* d_gallery, int64_t n_rows, int32_t dim, in
  * stream (or an event recorded behind the call) has completed, mmrs_search_status(h_status) returns
  * the outcome of that batch -- MMRS_OK, an error, or MMRS_ERR_RETRY.  Results are valid only when
  * it returns MMRS_OK.  One workspace may be shared by consecutive calls on the same stream.
+ * d_row_filter, d_row_labels, d_query_labels, label_match restrict the rows a query may return (see
+ * "row constraints" below); NULL, NULL, NULL, 0 searches every row.  The same four arguments end the
+ * exhaustive, keys and fused-gather searches below.
  */
 int mmrs_search_topk_async(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
                            int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
                            int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                            int64_t index_offset, int32_t path, float* d_out_values,
                            int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-                           int32_t* h_status, void* stream);
+                           int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                           const int32_t* d_query_labels, int32_t label_match, void* stream);
 int mmrs_search_topk_host_async(const void* d_gallery, int64_t n_rows, int32_t dim,
                                 int64_t ld_gallery, int32_t gallery_dtype, const float* h_queries,
                                 int32_t n_queries, int64_t ld_queries, int32_t k,
                                 int32_t normalize_queries, float scale, int64_t index_offset,
                                 int32_t path, float* h_out_values, int64_t* h_out_indices,
                                 void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-                                void* stream);
+                                const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                const int32_t* d_query_labels, int32_t label_match, void* stream);
 int mmrs_search_status(const int32_t* h_status);
 
 /*
@@ -197,7 +202,9 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
                                 int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
                                 int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                                 int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                void* d_workspace, size_t workspace_bytes, void* stream);
+                                void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
+                                const int32_t* d_row_labels, const int32_t* d_query_labels,
+                                int32_t label_match, void* stream);
 
 /*
  * Sharded search without a host round trip: each rank writes its local top-k as packed 64-bit keys
@@ -208,18 +215,22 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
  * d_out_keys must hold n_queries * k + 1 elements: the LAST one receives the shard's device status
  * word (0 = ok, 1 = candidate-list overflow, ...), so it is gathered along with the keys and every
  * rank can see whether any rank has to repeat the batch.  d_status is one device int32 of scratch,
- * h_status as above.
+ * h_status as above.  pad_short == 0: every query must have at least k_out non-zero keys over all lists.
+ * pad_short != 0: it may have fewer (the gathered keys of a label-conditioned search), and the missing
+ * positions get value -inf, index -1.
  */
 int mmrs_search_topk_keys_async(const void* d_gallery, int64_t n_rows, int32_t dim,
                                 int64_t ld_gallery, int32_t gallery_dtype, const float* d_queries,
                                 int32_t n_queries, int64_t ld_queries, int32_t k,
                                 int32_t normalize_queries, float scale, int64_t index_offset,
                                 int32_t path, uint64_t* d_out_keys, void* d_workspace,
-                                size_t workspace_bytes, int32_t* h_status, void* stream);
+                                size_t workspace_bytes, int32_t* h_status,
+                                const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                const int32_t* d_query_labels, int32_t label_match, void* stream);
 int mmrs_topk_merge_keys_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries,
                                int32_t k_in, int64_t list_stride, int32_t k_out,
                                float* d_out_values, int64_t* d_out_indices, int32_t* d_status,
-                               int32_t* h_status, void* stream);
+                               int32_t* h_status, int32_t pad_short, void* stream);
 
 /*
  * Search fused with its all-gather (one process per GPU, NVLink peer memory instead of NCCL):
@@ -242,134 +253,10 @@ int mmrs_topk_merge_keys_async(const uint64_t* d_keys_in, int32_t n_lists, int32
  * rank overflowed; MMRS_ERR_TIMEOUT when a peer never arrived).  n_queries <= 1024, world <= 64,
  * k_local must be the same on every rank and every shard must hold at least k_local rows -- a rank that
  * contributes fewer keys than min(k_out, its rows) can drop rows of the global top-k; callers with shorter
- * shards use the keys variant below and pad.
+ * shards use the keys variant above and pad.  With a row constraint the merge select pads: fewer than k_out
+ * eligible rows over all ranks give -inf / -1.
  */
 int mmrs_search_topk_fused_gather_async(
-    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
-    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
-    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path,
-    uint64_t* const* d_peer_bufs, uint32_t* const* d_peer_flags, uint64_t* d_local_buf,
-    uint32_t* d_local_flags, int32_t rank, int32_t world, int64_t list_stride, float* d_out_values,
-    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status, void* stream);
-int mmrs_gather_status(const int32_t* h_status, int32_t world);
-
-/* ---- row-filtered search ---------------------------------------------------------------- */
-
-/*
- * A row filter is an allow-list bitmap over the rows of one gallery (shard): uint32 words, bit
- * (r & 31) of word (r >> 5) set when local row r may be returned.  PADDING CONTRACT: the array holds
- * at least 4 * ceil(n_rows / 128) words (whole 128-row tiles); bits at or past n_rows are ignored, but
- * those words must be readable.  A shard of a global filter whose first row is a multiple of 128 is the
- * pointer d_words + first_row / 32 (its tail bits belong to the next shard and are ignored).
- *
- * mmrs_pack_row_filter builds one from a device byte mask d_allowed [n_rows] (non-zero = allowed):
- * n_words >= 4 * ceil(n_rows / 128), words past the last row are zeroed; *d_count (device int64)
- * receives the number of allowed rows.  Asynchronous on `stream`.
- */
-int mmrs_pack_row_filter(const uint8_t* d_allowed, int64_t n_rows, uint32_t* d_words, int64_t n_words,
-                         int64_t* d_count, void* stream);
-
-/*
- * The _filtered forms of the searches above: the same arguments plus d_row_filter (before `stream`),
- * and the same top-k as an unfiltered search over the allowed rows only, indices still those of the
- * full gallery (+ index_offset).  NULL = every row (exactly the unfiltered call).  k may exceed the
- * number of allowed rows: the missing positions get value -inf, index -1 (key 0 in the key outputs,
- * which every merge ignores), so a shard with few or no allowed rows still contributes k entries.
- * A captured graph is keyed on the filter pointer; the words are read when the search runs.
- */
-int mmrs_search_topk_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                    int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                    int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                    int64_t index_offset, int32_t path, float* d_out_values,
-                                    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-                                    int32_t* h_status, const uint32_t* d_row_filter, void* stream);
-int mmrs_search_topk_host_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim,
-                                         int64_t ld_gallery, int32_t gallery_dtype, const float* h_queries,
-                                         int32_t n_queries, int64_t ld_queries, int32_t k,
-                                         int32_t normalize_queries, float scale, int64_t index_offset,
-                                         int32_t path, float* h_out_values, int64_t* h_out_indices,
-                                         void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-                                         const uint32_t* d_row_filter, void* stream);
-int mmrs_search_topk_exhaustive_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                         int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                         void* d_workspace, size_t workspace_bytes,
-                                         const uint32_t* d_row_filter, void* stream);
-int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim,
-                                         int64_t ld_gallery, int32_t gallery_dtype, const float* d_queries,
-                                         int32_t n_queries, int64_t ld_queries, int32_t k,
-                                         int32_t normalize_queries, float scale, int64_t index_offset,
-                                         int32_t path, uint64_t* d_out_keys, void* d_workspace,
-                                         size_t workspace_bytes, int32_t* h_status,
-                                         const uint32_t* d_row_filter, void* stream);
-/* k_out must not exceed the allowed rows over all ranks (the merge pads with -inf / -1 otherwise). */
-int mmrs_search_topk_fused_gather_async_filtered(
-    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
-    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
-    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path,
-    uint64_t* const* d_peer_bufs, uint32_t* const* d_peer_flags, uint64_t* d_local_buf,
-    uint32_t* d_local_flags, int32_t rank, int32_t world, int64_t list_stride, float* d_out_values,
-    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-    const uint32_t* d_row_filter, void* stream);
-
-/* ---- label-conditioned search ----------------------------------------------------------- */
-
-/* label_match of the _labeled searches */
-#define MMRS_LABEL_SAME 0    /* only rows whose label equals the query's label             */
-#define MMRS_LABEL_OTHER 1   /* only rows whose label differs from it (hard negatives)      */
-
-/*
- * Row labels are one int32 class id per row of the gallery (shard), each in [0, 2^31 - 1).
- * PADDING CONTRACT (the bitmap's): the array holds at least 128 * ceil(n_rows / 128) elements (whole
- * 128-row tiles); labels at or past n_rows are never compared, but must be readable.  A shard of a
- * global label array whose first row is a multiple of 128 is the pointer d_row_labels + first_row.
- *
- * The _labeled forms of the five _filtered searches take the _filtered arguments plus d_row_labels,
- * d_query_labels and label_match (before `stream`).  d_query_labels is a DEVICE int32 [n_queries] in
- * every form, the host-I/O one included.  For query q with c = d_query_labels[q]:
- *   c < 0               no label restriction: exactly the unlabeled search of that query;
- *   MMRS_LABEL_SAME     only rows r with d_row_labels[r] == c;
- *   MMRS_LABEL_OTHER    only rows r with d_row_labels[r] != c;
- * and with d_row_filter as well, a row must pass both.  Values, order and tie rule are those of the
- * unlabeled search over the eligible rows.  A query with fewer than k eligible rows (a small class, a
- * label absent from the gallery) is NOT an error: positions n_eligible .. k-1 get value -inf, index -1
- * (key 0 in the key outputs).  d_row_labels == NULL is exactly the _filtered call.  A captured graph is
- * keyed on both label pointers and label_match; the labels are read when the search runs, so a caller
- * that rewrites the query labels in place between calls keeps replaying one graph.
- */
-int mmrs_search_topk_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                   int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                   int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                   int64_t index_offset, int32_t path, float* d_out_values,
-                                   int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-                                   int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                   const int32_t* d_query_labels, int32_t label_match, void* stream);
-int mmrs_search_topk_host_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim,
-                                        int64_t ld_gallery, int32_t gallery_dtype, const float* h_queries,
-                                        int32_t n_queries, int64_t ld_queries, int32_t k,
-                                        int32_t normalize_queries, float scale, int64_t index_offset,
-                                        int32_t path, float* h_out_values, int64_t* h_out_indices,
-                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                        const int32_t* d_query_labels, int32_t label_match, void* stream);
-int mmrs_search_topk_exhaustive_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                        int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                        void* d_workspace, size_t workspace_bytes,
-                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                        const int32_t* d_query_labels, int32_t label_match, void* stream);
-int mmrs_search_topk_keys_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim,
-                                        int64_t ld_gallery, int32_t gallery_dtype, const float* d_queries,
-                                        int32_t n_queries, int64_t ld_queries, int32_t k,
-                                        int32_t normalize_queries, float scale, int64_t index_offset,
-                                        int32_t path, uint64_t* d_out_keys, void* d_workspace,
-                                        size_t workspace_bytes, int32_t* h_status,
-                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                        const int32_t* d_query_labels, int32_t label_match, void* stream);
-/* The merge select pads: fewer than k_out eligible rows over all ranks give -inf / -1. */
-int mmrs_search_topk_fused_gather_async_labeled(
     const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
     const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
     int32_t normalize_queries, float scale, int64_t index_offset, int32_t path,
@@ -378,14 +265,49 @@ int mmrs_search_topk_fused_gather_async_labeled(
     int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes, int32_t* h_status,
     const uint32_t* d_row_filter, const int32_t* d_row_labels, const int32_t* d_query_labels,
     int32_t label_match, void* stream);
+int mmrs_gather_status(const int32_t* h_status, int32_t world);
+
+/* ---- row constraints ------------------------------------------------------------------- */
+
 /*
- * mmrs_topk_merge_keys_async for lists that may hold fewer than k_out non-zero keys per query over all
- * lists (the gathered keys of a labeled search): the missing positions get value -inf, index -1.
+ * d_row_filter (NULL = every row) is an allow-list bitmap over the rows of one gallery (shard): uint32
+ * words, bit (r & 31) of word (r >> 5) set when local row r may be returned.  PADDING CONTRACT: the array
+ * holds at least 4 * ceil(n_rows / 128) words (whole 128-row tiles); bits at or past n_rows are ignored,
+ * but those words must be readable.  A shard of a global filter whose first row is a multiple of 128 is
+ * the pointer d_words + first_row / 32 (its tail bits belong to the next shard and are ignored).
+ *
+ * mmrs_pack_row_filter builds one from a device byte mask d_allowed [n_rows] (non-zero = allowed):
+ * n_words >= 4 * ceil(n_rows / 128), words past the last row are zeroed; *d_count (device int64)
+ * receives the number of allowed rows.  Asynchronous on `stream`.
  */
-int mmrs_topk_merge_keys_padded_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries,
-                                      int32_t k_in, int64_t list_stride, int32_t k_out,
-                                      float* d_out_values, int64_t* d_out_indices, int32_t* d_status,
-                                      int32_t* h_status, void* stream);
+int mmrs_pack_row_filter(const uint8_t* d_allowed, int64_t n_rows, uint32_t* d_words, int64_t n_words,
+                         int64_t* d_count, void* stream);
+
+/* label_match */
+#define MMRS_LABEL_SAME 0    /* only rows whose label equals the query's label             */
+#define MMRS_LABEL_OTHER 1   /* only rows whose label differs from it (hard negatives)      */
+
+/*
+ * d_row_labels (NULL = no label restriction; d_query_labels and label_match are then ignored) is one
+ * int32 class id per row of the gallery (shard), each in [0, 2^31 - 1).  PADDING CONTRACT (the
+ * bitmap's): the array holds at least 128 * ceil(n_rows / 128) elements (whole 128-row tiles); labels
+ * at or past n_rows are never compared, but must be readable.  A shard of a global label array whose
+ * first row is a multiple of 128 is the pointer d_row_labels + first_row.  d_query_labels is a DEVICE
+ * int32 [n_queries] in every form, the host-I/O one included.  For query q with c = d_query_labels[q]:
+ *   c < 0               no label restriction: exactly the unlabeled search of that query;
+ *   MMRS_LABEL_SAME     only rows r with d_row_labels[r] == c;
+ *   MMRS_LABEL_OTHER    only rows r with d_row_labels[r] != c;
+ * and with d_row_filter as well, a row must pass both.
+ *
+ * A constrained search returns the top-k of an unconstrained one over the eligible rows only (same
+ * values, order and tie rule), indices still those of the full gallery (+ index_offset).  k may exceed
+ * the eligible rows of a query (a small class, a label absent from the gallery, a shard with few or no
+ * allowed rows): that is NOT an error, positions n_eligible .. k-1 get value -inf, index -1 (key 0 in
+ * the key outputs, which every merge ignores), so every shard still contributes k entries.
+ * A captured graph is keyed on the filter pointer, both label pointers and label_match; the words and
+ * labels are read when the search runs, so a caller that rewrites them in place between calls keeps
+ * replaying one graph.  NULL, NULL, NULL, 0 gives exactly the graph of the unconstrained search.
+ */
 
 /* ---- multi-GPU merge -------------------------------------------------------------------- */
 

@@ -10,7 +10,7 @@ LIB_PATH = _PKG_DIR / "lib" / "libmmrs_b200.so"
 
 OK = 0
 ERR_ARG, ERR_CUDA, ERR_ARCH, ERR_WORKSPACE, ERR_ZERO_NORM, ERR_CAPACITY, ERR_INTERNAL, ERR_RETRY, ERR_TIMEOUT = -1, -2, -3, -4, -5, -6, -7, -8, -9
-ABI_VERSION = 2
+ABI_VERSION = 3
 DTYPE_F32, DTYPE_BF16, DTYPE_BF16X3 = 0, 1, 2
 PATH_AUTO, PATH_GEMV, PATH_MMA = 0, 1, 2
 PATHS = {"auto": PATH_AUTO, "gemv": PATH_GEMV, "mma": PATH_MMA}
@@ -24,6 +24,19 @@ class MmrsError(RuntimeError):
         self.code = code
 
 
+def open_library(path: Path) -> C.CDLL:
+    """Load the library at `path`, refusing one built from another version of include/mmrs_b200.h:
+    ctypes cannot see argument lists, so a stale library would read this binding's arguments wrongly."""
+    lib = C.CDLL(str(path))
+    lib.mmrs_abi_version.restype = C.c_int
+    lib.mmrs_abi_version.argtypes = []
+    found = lib.mmrs_abi_version()
+    if found != ABI_VERSION:
+        raise ImportError(f"{path} has C ABI version {found}, this package needs {ABI_VERSION}: rebuild it with "
+                          f"`python {_PKG_DIR / 'build.py'} --force`")
+    return lib
+
+
 def _load() -> C.CDLL:
     if not LIB_PATH.exists():
         # build in-tree on first use (needs nvcc); never fall back to anything else
@@ -32,7 +45,7 @@ def _load() -> C.CDLL:
     if not LIB_PATH.exists():
         raise ImportError(f"{LIB_PATH} is missing and could not be built: the mmrs_b200 CUDA "
                           "library is required (there is no CPU fallback)")
-    return C.CDLL(str(LIB_PATH))
+    return open_library(LIB_PATH)
 
 
 lib = _load()
@@ -55,21 +68,23 @@ SIGNATURES = {
     "mmrs_search_host_staging_bytes": (_sz, [_i32, _i32, _i32]),
     "mmrs_search_topk_host": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
                                         _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp]),
+    # the async, exhaustive, keys and fused forms end in: row filter, row labels, query labels, label_match, stream
     "mmrs_search_topk_async": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                         _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp]),
+                                         _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
     "mmrs_search_topk_host_async": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
-                                              _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp]),
+                                              _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32,
+                                              _vp]),
     "mmrs_search_status": (C.c_int, [_vp]),
     "mmrs_search_exhaustive_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "mmrs_search_topk_exhaustive": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                              _i64, _vp, _vp, _vp, _sz, _vp]),
+                                              _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _i32, _vp]),
     "mmrs_search_topk_fused_gather_async": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _i32,
                                                       _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i64,
-                                                      _vp, _vp, _vp, _sz, _vp, _vp]),
+                                                      _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
     "mmrs_gather_status": (C.c_int, [_vp, _i32]),
     "mmrs_search_topk_keys_async": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                              _i64, _i32, _vp, _vp, _sz, _vp, _vp]),
-    "mmrs_topk_merge_keys_async": (C.c_int, [_vp, _i32, _i32, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
+                                              _i64, _i32, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "mmrs_topk_merge_keys_async": (C.c_int, [_vp, _i32, _i32, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
     "mmrs_topk_merge_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "mmrs_topk_merge": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "mmrs_selfjoin_workspace_bytes": (_sz, [_i64, _i32, _i32]),
@@ -89,34 +104,7 @@ SIGNATURES = {
     "mmrs_profile_read": (C.c_int, [_vp, _vp, _vp, _vp, _i32]),
     "mmrs_threshold_sweep_labeled": (C.c_int, [_vp, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "mmrs_threshold_sweep": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _sz, _vp]),
-    # row-filtered search: the unfiltered signature + the bitmap pointer before the stream
     "mmrs_pack_row_filter": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp]),
-    "mmrs_search_topk_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                                  _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
-    "mmrs_search_topk_host_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
-                                                       _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
-    "mmrs_search_topk_exhaustive_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                                       _i64, _vp, _vp, _vp, _sz, _vp, _vp]),
-    "mmrs_search_topk_keys_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                                       _i64, _i32, _vp, _vp, _sz, _vp, _vp, _vp]),
-    "mmrs_search_topk_fused_gather_async_filtered": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
-                                                               _i32, _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32,
-                                                               _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
-    # label-conditioned search: the _filtered signature + row labels, query labels, label_match before the stream
-    "mmrs_search_topk_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                                 _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
-    "mmrs_search_topk_host_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
-                                                      _f32, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32,
-                                                      _vp]),
-    "mmrs_search_topk_exhaustive_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                                      _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _i32, _vp]),
-    "mmrs_search_topk_keys_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
-                                                      _i64, _i32, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),
-    "mmrs_search_topk_fused_gather_async_labeled": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32,
-                                                              _i32, _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32,
-                                                              _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _i32,
-                                                              _vp]),
-    "mmrs_topk_merge_keys_padded_async": (C.c_int, [_vp, _i32, _i32, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
     # per-class threshold tuning of a batch of prototypes (best_thresholds)
     "mmrs_threshold_sweep_batched_workspace_bytes": (_sz, [_i32, _i32]),
     "mmrs_score_range_batched": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp]),

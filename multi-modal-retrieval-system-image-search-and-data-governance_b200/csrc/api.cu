@@ -841,17 +841,14 @@ static int validate_search(const SearchArgs& a, const void* ws, size_t ws_bytes,
     return fail(MMRS_ERR_WORKSPACE, "workspace %zu bytes, need %zu", ws_bytes, need);
   if (reinterpret_cast<uintptr_t>(ws) % 256 != 0)
     return fail(MMRS_ERR_WORKSPACE, "workspace must be 256-byte aligned");
-  return MMRS_OK;
+  rc = check_row_filter(a.row_filter);
+  if (rc != MMRS_OK) return rc;
+  return check_labels(a.row_labels, a.query_labels, a.label_match);
 }
 
 }  // namespace mmrs
 
 using namespace mmrs;
-
-// the key merge of mmrs_topk_merge_keys_async / _padded_async (defined below)
-static int merge_keys(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
-                      int64_t list_stride, int32_t k_out, float* d_out_values, int64_t* d_out_indices,
-                      int32_t* d_status, int32_t* h_status, bool pad_short, void* stream_);
 
 extern "C" {
 
@@ -1011,31 +1008,9 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
                                 int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
                                 int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                                 int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                void* d_workspace, size_t workspace_bytes, void* stream) {
-  return mmrs_search_topk_exhaustive_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
-                                              ld_queries, k, normalize_queries, scale, index_offset, d_out_values,
-                                              d_out_indices, d_workspace, workspace_bytes, nullptr, stream);
-}
-
-int mmrs_search_topk_exhaustive_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                         int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                         void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
-                                         void* stream) {
-  return mmrs_search_topk_exhaustive_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
-                                             ld_queries, k, normalize_queries, scale, index_offset, d_out_values,
-                                             d_out_indices, d_workspace, workspace_bytes, d_row_filter, nullptr,
-                                             nullptr, 0, stream);
-}
-
-int mmrs_search_topk_exhaustive_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                        int64_t index_offset, float* d_out_values, int64_t* d_out_indices,
-                                        void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
-                                        const int32_t* d_row_labels, const int32_t* d_query_labels,
-                                        int32_t label_match, void* stream_) {
+                                void* d_workspace, size_t workspace_bytes, const uint32_t* d_row_filter,
+                                const int32_t* d_row_labels, const int32_t* d_query_labels,
+                                int32_t label_match, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceInfo dev;
   int rc = current_device(&dev);
@@ -1101,39 +1076,12 @@ int mmrs_search_topk_async(const void* d_gallery, int64_t n_rows, int32_t dim, i
                            int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                            int64_t index_offset, int32_t path, float* d_out_values,
                            int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-                           int32_t* h_status, void* stream) {
-  return mmrs_search_topk_async_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
-                                         ld_queries, k, normalize_queries, scale, index_offset, path, d_out_values,
-                                         d_out_indices, d_workspace, workspace_bytes, h_status, nullptr, stream);
-}
-
-int mmrs_search_topk_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                    int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                    int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                    int64_t index_offset, int32_t path, float* d_out_values,
-                                    int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-                                    int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
-  return mmrs_search_topk_async_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
-                                        ld_queries, k, normalize_queries, scale, index_offset, path, d_out_values,
-                                        d_out_indices, d_workspace, workspace_bytes, h_status, d_row_filter, nullptr,
-                                        nullptr, 0, stream);
-}
-
-int mmrs_search_topk_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                   int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                   int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                   int64_t index_offset, int32_t path, float* d_out_values,
-                                   int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-                                   int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                   const int32_t* d_query_labels, int32_t label_match, void* stream) {
+                           int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                           const int32_t* d_query_labels, int32_t label_match, void* stream) {
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, d_out_values, d_out_indices};
   a.row_filter = d_row_filter;
   a.row_labels = d_row_labels; a.query_labels = d_query_labels; a.label_match = label_match;
-  int rc = check_row_filter(d_row_filter);
-  if (rc != MMRS_OK) return rc;
-  rc = check_labels(d_row_labels, d_query_labels, label_match);
-  if (rc != MMRS_OK) return rc;
   return search_enqueue(a, nullptr, nullptr, nullptr, d_workspace, workspace_bytes, h_status,
                         static_cast<cudaStream_t>(stream), nullptr, nullptr);
 }
@@ -1143,36 +1091,9 @@ int mmrs_search_topk_host_async(const void* d_gallery, int64_t n_rows, int32_t d
                                 int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                                 int64_t index_offset, int32_t path, float* h_out_values,
                                 int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
-                                int32_t* h_status, void* stream) {
-  return mmrs_search_topk_host_async_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, h_queries, n_queries,
-                                              ld_queries, k, normalize_queries, scale, index_offset, path, h_out_values,
-                                              h_out_indices, d_workspace, workspace_bytes, h_status, nullptr, stream);
-}
-
-int mmrs_search_topk_host_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                         int32_t gallery_dtype, const float* h_queries, int32_t n_queries,
-                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                         int64_t index_offset, int32_t path, float* h_out_values,
-                                         int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
-                                         int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
-  return mmrs_search_topk_host_async_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, h_queries, n_queries,
-                                             ld_queries, k, normalize_queries, scale, index_offset, path, h_out_values,
-                                             h_out_indices, d_workspace, workspace_bytes, h_status, d_row_filter,
-                                             nullptr, nullptr, 0, stream);
-}
-
-int mmrs_search_topk_host_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                        int32_t gallery_dtype, const float* h_queries, int32_t n_queries,
-                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                        int64_t index_offset, int32_t path, float* h_out_values,
-                                        int64_t* h_out_indices, void* d_workspace, size_t workspace_bytes,
-                                        int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                        const int32_t* d_query_labels, int32_t label_match, void* stream) {
+                                int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                const int32_t* d_query_labels, int32_t label_match, void* stream) {
   if (n_queries > 0 && !h_queries) return fail(MMRS_ERR_ARG, "null host query pointer");
-  int rc = check_row_filter(d_row_filter);
-  if (rc != MMRS_OK) return rc;
-  rc = check_labels(d_row_labels, d_query_labels, label_match);
-  if (rc != MMRS_OK) return rc;
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, nullptr, n_queries, ld_queries,
                k, normalize_queries, scale, index_offset, path, nullptr, nullptr};
   a.row_filter = d_row_filter;
@@ -1188,37 +1109,8 @@ int mmrs_search_topk_keys_async(const void* d_gallery, int64_t n_rows, int32_t d
                                 int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
                                 int64_t index_offset, int32_t path, uint64_t* d_out_keys,
                                 void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-                                void* stream) {
-  return mmrs_search_topk_keys_async_filtered(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
-                                              ld_queries, k, normalize_queries, scale, index_offset, path, d_out_keys,
-                                              d_workspace, workspace_bytes, h_status, nullptr, stream);
-}
-
-int mmrs_search_topk_keys_async_filtered(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                         int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                         int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                         int64_t index_offset, int32_t path, uint64_t* d_out_keys,
-                                         void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-                                         const uint32_t* d_row_filter, void* stream) {
-  return mmrs_search_topk_keys_async_labeled(d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries,
-                                             ld_queries, k, normalize_queries, scale, index_offset, path, d_out_keys,
-                                             d_workspace, workspace_bytes, h_status, d_row_filter, nullptr, nullptr, 0,
-                                             stream);
-}
-
-int mmrs_search_topk_keys_async_labeled(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                        int64_t ld_queries, int32_t k, int32_t normalize_queries, float scale,
-                                        int64_t index_offset, int32_t path, uint64_t* d_out_keys,
-                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status,
-                                        const uint32_t* d_row_filter, const int32_t* d_row_labels,
-                                        const int32_t* d_query_labels, int32_t label_match, void* stream) {
-  {
-    int rc = check_row_filter(d_row_filter);
-    if (rc != MMRS_OK) return rc;
-    rc = check_labels(d_row_labels, d_query_labels, label_match);
-    if (rc != MMRS_OK) return rc;
-  }
+                                const uint32_t* d_row_filter, const int32_t* d_row_labels,
+                                const int32_t* d_query_labels, int32_t label_match, void* stream) {
   if (index_offset < 0 || index_offset + n_rows > 0x100000000ll)
     return fail(MMRS_ERR_ARG, "global row ids must fit 32 bits");
   SearchArgs a{d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries,
@@ -1242,24 +1134,7 @@ int mmrs_search_topk_keys_async_labeled(const void* d_gallery, int64_t n_rows, i
 int mmrs_topk_merge_keys_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
                                int64_t list_stride, int32_t k_out, float* d_out_values,
                                int64_t* d_out_indices, int32_t* d_status, int32_t* h_status,
-                               void* stream) {
-  return merge_keys(d_keys_in, n_lists, n_queries, k_in, list_stride, k_out, d_out_values, d_out_indices, d_status,
-                    h_status, false, stream);
-}
-
-int mmrs_topk_merge_keys_padded_async(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
-                                      int64_t list_stride, int32_t k_out, float* d_out_values,
-                                      int64_t* d_out_indices, int32_t* d_status, int32_t* h_status,
-                                      void* stream) {
-  return merge_keys(d_keys_in, n_lists, n_queries, k_in, list_stride, k_out, d_out_values, d_out_indices, d_status,
-                    h_status, true, stream);
-}
-
-}  // extern "C"
-
-static int merge_keys(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_queries, int32_t k_in,
-                      int64_t list_stride, int32_t k_out, float* d_out_values, int64_t* d_out_indices,
-                      int32_t* d_status, int32_t* h_status, bool pad_short, void* stream_) {
+                               int32_t pad_short, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceInfo dev;
   int rc = current_device(&dev);
@@ -1278,43 +1153,13 @@ static int merge_keys(const uint64_t* d_keys_in, int32_t n_lists, int32_t n_quer
   sp.out_values = d_out_values; sp.out_indices = d_out_indices; sp.index_offset = 0; sp.flags = d_status;
   if (list_stride < static_cast<int64_t>(n_queries) * k_in) return fail(MMRS_ERR_ARG, "list_stride too small");
   sp.seg_len = k_in; sp.seg_stride = list_stride;
-  sp.pad_short = pad_short;
+  sp.pad_short = pad_short != 0;
   MMRS_LAUNCH(launch_select(sp, n_queries, stream));
   MMRS_CUDA(cudaMemcpyAsync(h_status, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
   return MMRS_OK;
 }
 
-extern "C" {
-
-int mmrs_search_topk_fused_gather_async(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,
-                                        int32_t gallery_dtype, const float* d_queries, int32_t n_queries,
-                                        int64_t ld_queries, int32_t k_local, int32_t k_out,
-                                        int32_t normalize_queries, float scale, int64_t index_offset, int32_t path,
-                                        uint64_t* const* d_peer_bufs, uint32_t* const* d_peer_flags,
-                                        uint64_t* d_local_buf, uint32_t* d_local_flags, int32_t rank, int32_t world,
-                                        int64_t list_stride, float* d_out_values, int64_t* d_out_indices,
-                                        void* d_workspace, size_t workspace_bytes, int32_t* h_status, void* stream) {
-  return mmrs_search_topk_fused_gather_async_filtered(
-      d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries, k_local, k_out,
-      normalize_queries, scale, index_offset, path, d_peer_bufs, d_peer_flags, d_local_buf, d_local_flags, rank, world,
-      list_stride, d_out_values, d_out_indices, d_workspace, workspace_bytes, h_status, nullptr, stream);
-}
-
-int mmrs_search_topk_fused_gather_async_filtered(
-    const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
-    const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
-    int32_t normalize_queries, float scale, int64_t index_offset, int32_t path, uint64_t* const* d_peer_bufs,
-    uint32_t* const* d_peer_flags, uint64_t* d_local_buf, uint32_t* d_local_flags, int32_t rank, int32_t world,
-    int64_t list_stride, float* d_out_values, int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
-    int32_t* h_status, const uint32_t* d_row_filter, void* stream) {
-  return mmrs_search_topk_fused_gather_async_labeled(
-      d_gallery, n_rows, dim, ld_gallery, gallery_dtype, d_queries, n_queries, ld_queries, k_local, k_out,
-      normalize_queries, scale, index_offset, path, d_peer_bufs, d_peer_flags, d_local_buf, d_local_flags, rank, world,
-      list_stride, d_out_values, d_out_indices, d_workspace, workspace_bytes, h_status, d_row_filter, nullptr, nullptr,
-      0, stream);
-}
-
-int mmrs_search_topk_fused_gather_async_labeled(
+int mmrs_search_topk_fused_gather_async(
     const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery, int32_t gallery_dtype,
     const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t k_local, int32_t k_out,
     int32_t normalize_queries, float scale, int64_t index_offset, int32_t path, uint64_t* const* d_peer_bufs,
@@ -1323,12 +1168,6 @@ int mmrs_search_topk_fused_gather_async_labeled(
     int32_t* h_status, const uint32_t* d_row_filter, const int32_t* d_row_labels, const int32_t* d_query_labels,
     int32_t label_match, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  {
-    int rc = check_row_filter(d_row_filter);
-    if (rc != MMRS_OK) return rc;
-    rc = check_labels(d_row_labels, d_query_labels, label_match);
-    if (rc != MMRS_OK) return rc;
-  }
   if (world < 1 || world > kMaxWorld || rank < 0 || rank >= world || !d_peer_bufs || !d_peer_flags || !d_local_buf ||
       !d_local_flags)
     return fail(MMRS_ERR_ARG, "bad rank / world / peer pointers");

@@ -116,14 +116,8 @@ def _search_exhaustive(gal: DeviceGallery, q: torch.Tensor, k: int, normalize_qu
         args = (g_ptr, gal.n_rows, gal.padded_dim, g_ld, g_dtype, qd.data_ptr(), nq, qd.stride(0), k,
                 int(bool(normalize_queries)), float(scale), gal.row_offset, dv.data_ptr(), di.data_ptr(),
                 DeviceGallery.aligned_ptr(ws), ws_bytes)
-        if labels is not None:
-            row_labels, ql, match = labels
-            _cabi.check(lib.mmrs_search_topk_exhaustive_labeled(*args, row_filter_ptr, row_labels.labels.data_ptr(),
-                                                                ql.data_ptr(), match, _stream_handle(dev)))
-        elif row_filter_ptr:
-            _cabi.check(lib.mmrs_search_topk_exhaustive_filtered(*args, row_filter_ptr, _stream_handle(dev)))
-        else:
-            _cabi.check(lib.mmrs_search_topk_exhaustive(*args, _stream_handle(dev)))
+        lab = (0, 0, 0) if labels is None else (labels[0].labels.data_ptr(), labels[1].data_ptr(), labels[2])
+        _cabi.check(lib.mmrs_search_topk_exhaustive(*args, row_filter_ptr, *lab, _stream_handle(dev)))
         if dv is not values:
             values.copy_(dv)
             indices.copy_(di)
@@ -279,23 +273,7 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
             f = filt if isinstance(filt, RowFilter) else RowFilter(filt)
             _search_exhaustive(gal, q, k, normalize_queries, scale, path, v, i, f.words.data_ptr(), lab)
 
-    if filt is not None or labels is not None:
-        ticket, status, event = slot.acquire()
-        if labels is None:
-            fn = lib.mmrs_search_topk_host_async_filtered if on_host else lib.mmrs_search_topk_async_filtered
-            st = fn(*args, status.data_ptr(), filt_ptr, stream.cuda_stream)
-        else:
-            fn = lib.mmrs_search_topk_host_async_labeled if on_host else lib.mmrs_search_topk_async_labeled
-            st = fn(*args, status.data_ptr(), filt_ptr, labels[0].labels.data_ptr(), labels[1].data_ptr(), labels[2],
-                    stream.cuda_stream)
-        if st != _cabi.OK:
-            slot.release(ticket)
-            _cabi.check(st)
-        event.record(stream)
-        pend = PendingSearch(values, indices, slot, ticket, status, event, redo)
-        pend._keepalive = (q, filt, labels)
-        return pend.wait() if sync else pend
-    if sync:
+    if sync and filt is None and labels is None:
         fn = lib.mmrs_search_topk_host if on_host else lib.mmrs_search_topk
         st = fn(*args, stream.cuda_stream)
         if st == _cabi.ERR_RETRY:
@@ -305,14 +283,15 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
         return values, indices
     ticket, status, event = slot.acquire()
     fn = lib.mmrs_search_topk_host_async if on_host else lib.mmrs_search_topk_async
-    st = fn(*args, status.data_ptr(), stream.cuda_stream)
+    lab = (0, 0, 0) if labels is None else (labels[0].labels.data_ptr(), labels[1].data_ptr(), labels[2])
+    st = fn(*args, status.data_ptr(), filt_ptr, *lab, stream.cuda_stream)
     if st != _cabi.OK:
         slot.release(ticket)
         _cabi.check(st)
     event.record(stream)
     pend = PendingSearch(values, indices, slot, ticket, status, event, redo)
-    pend._keepalive = q        # the enqueued copies / kernels read it
-    return pend
+    pend._keepalive = (q, filt, labels)        # the enqueued copies / kernels read them
+    return pend.wait() if sync else pend
 
 
 def full_scores(queries, gallery: GalleryLike, *, normalize_queries: bool = True, scale: float = 1.0,

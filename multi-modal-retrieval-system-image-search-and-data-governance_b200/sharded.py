@@ -228,14 +228,10 @@ class ShardedGallery:
             args = (gal.data.data_ptr(), gal.n_rows, gal.padded_dim, gal.data.stride(0), gal.dtype_code,
                     q.data_ptr(), nq, q.stride(0), k_local, int(bool(normalize_queries)), float(scale),
                     gal.row_offset, _cabi.PATHS[path], dst.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr())
+            # a shard with fewer than k eligible rows for a query pads its list with key 0
             filt_ptr = local_filter.words.data_ptr() if local_filter is not None else 0
-            if labels is not None:   # a query with fewer than k eligible rows here: its list is padded with key 0
-                st = lib.mmrs_search_topk_keys_async_labeled(*args, filt_ptr, labels[0].labels.data_ptr(),
-                                                             staged[0].data_ptr(), labels[2], stream.cuda_stream)
-            elif local_filter is None:
-                st = lib.mmrs_search_topk_keys_async(*args, stream.cuda_stream)
-            else:
-                st = lib.mmrs_search_topk_keys_async_filtered(*args, local_filter.words.data_ptr(), stream.cuda_stream)
+            lab = (0, 0, 0) if labels is None else (labels[0].labels.data_ptr(), staged[0].data_ptr(), labels[2])
+            st = lib.mmrs_search_topk_keys_async(*args, filt_ptr, *lab, stream.cuda_stream)
             if st != _cabi.OK:
                 slot.release(ticket)
                 _cabi.check(st)
@@ -245,9 +241,10 @@ class ShardedGallery:
         dist.all_gather_into_tensor(gathered.view(-1), buf, group=self.group)      # [world, nq*k + 1]
         if nq:
             # labeled: fewer than k eligible rows over all ranks is legitimate -> -inf / -1
-            merge = lib.mmrs_topk_merge_keys_padded_async if labels is not None else lib.mmrs_topk_merge_keys_async
-            _cabi.check(merge(gathered.data_ptr(), self.world, nq, k, n_keys + 1, k, dv.data_ptr(), di.data_ptr(),
-                              d_status.data_ptr(), status[1:].data_ptr(), stream.cuda_stream))
+            _cabi.check(lib.mmrs_topk_merge_keys_async(gathered.data_ptr(), self.world, nq, k, n_keys + 1, k,
+                                                       dv.data_ptr(), di.data_ptr(), d_status.data_ptr(),
+                                                       status[1:].data_ptr(), int(labels is not None),
+                                                       stream.cuda_stream))
             table = slot.extra.get("shard_status")          # one pinned row per status ticket of the slot
             if table is None or table.shape[0] <= ticket:
                 table = slot.extra["shard_status"] = torch.zeros((max(ticket + 1, slot.N_STATUS), self.world),
@@ -332,14 +329,11 @@ class ShardedGallery:
                 gal.row_offset, _cabi.PATHS[path], st["bufs"].data_ptr(), st["flags"].data_ptr(),
                 st["t"].data_ptr(), st["local_flags"], self.rank, self.world, st["stride"],
                 dv.data_ptr(), di.data_ptr(), slot.ptr, slot.nbytes, status.data_ptr())
-        if labels is not None:   # the merge select pads queries with fewer than k eligible rows with -inf / -1
-            rc = lib.mmrs_search_topk_fused_gather_async_labeled(
-                *args, local_filter.words.data_ptr() if local_filter is not None else 0, labels[0].labels.data_ptr(),
-                staged[0].data_ptr(), labels[2], stream.cuda_stream)
-        elif local_filter is None:
-            rc = lib.mmrs_search_topk_fused_gather_async(*args, stream.cuda_stream)
-        else:   # a shard with fewer than k allowed rows still stores k keys (padded with key 0)
-            rc = lib.mmrs_search_topk_fused_gather_async_filtered(*args, local_filter.words.data_ptr(), stream.cuda_stream)
+        # a shard with fewer than k eligible rows still stores k keys (padded with key 0), and the merge select
+        # pads queries with fewer than k eligible rows over all ranks with -inf / -1
+        filt_ptr = local_filter.words.data_ptr() if local_filter is not None else 0
+        lab = (0, 0, 0) if labels is None else (labels[0].labels.data_ptr(), staged[0].data_ptr(), labels[2])
+        rc = lib.mmrs_search_topk_fused_gather_async(*args, filt_ptr, *lab, stream.cuda_stream)
         if rc != _cabi.OK:
             slot.release(ticket)
             _cabi.check(rc)

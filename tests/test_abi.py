@@ -33,15 +33,27 @@ def test_python_binding_covers_the_header(mm):
     assert sorted(mm._cabi.SIGNATURES) == declared_symbols()
 
 
-def test_version_and_pure_host_queries(mm):
+def test_abi_version_3_and_pure_host_queries(mm):
     lib = mm._cabi.lib
-    assert lib.mmrs_abi_version() == mm._cabi.ABI_VERSION == 2
+    assert lib.mmrs_abi_version() == mm._cabi.ABI_VERSION == 3
     # workspace queries are pure host arithmetic: usable without a device
     small = lib.mmrs_search_workspace_bytes(10_000, 512, 0, 100, 10)
     big = lib.mmrs_search_workspace_bytes(1_000_000, 512, 1, 256, 100)
     assert 0 < small < big
     assert lib.mmrs_search_host_staging_bytes(512, 16, 100) >= 16 * 512 * 4 + 16 * 100 * 12
     assert lib.mmrs_topk_merge_workspace_bytes(8, 256, 100) >= 8 * 256 * 100 * 8
+
+
+def test_stale_library_is_refused(mm, tmp_path):
+    """A library left over from ABI version 2 loads, but its entry points take other arguments: the
+    loader must refuse it and name the rebuild."""
+    src = tmp_path / "stale.cpp"
+    src.write_text('extern "C" int mmrs_abi_version(void) { return 2; }\n')
+    so = tmp_path / "libstale.so"
+    subprocess.run(["g++", "-O1", "-shared", "-fPIC", str(src), "-o", str(so)], check=True)
+    with pytest.raises(ImportError, match=r"version 2, this package needs 3.*build\.py --force"):
+        mm._cabi.open_library(so)
+    assert mm._cabi.open_library(mm._cabi.LIB_PATH).mmrs_abi_version() == 3
 
 
 def test_no_cpu_fallback(mm):
