@@ -84,6 +84,7 @@ extern "C" {
                                     repeat it through mmrs_search_topk_exhaustive              */
 #define MMRS_ERR_TIMEOUT (-9)    /* fused all-gather: a peer rank did not arrive within
                                     MMRS_GATHER_TIMEOUT_MS (default 20 000)                   */
+#define MMRS_ERR_NONFINITE (-10) /* int8 quantisation: a gallery or query row holds a NaN or an infinity */
 
 /* element types of the gallery / embedding matrix */
 #define MMRS_DTYPE_F32 0
@@ -92,11 +93,31 @@ extern "C" {
                                plane stride n_rows * ld elements; mmrs_split_bf16x3 builds it): searched
                                on the tensor cores with six bf16 MMAs per tile and UNROUNDED queries --
                                fp32-mode results (scores within 1e-6) at tensor-core speed */
+#define MMRS_DTYPE_I8 3     /* per-row-scaled int8 rows (mmrs_quantize_rows_i8 builds them), see "int8 galleries" */
+
+/*
+ * int8 galleries.  Row r is ld bytes: the codes int8[dim] (dim a multiple of 16: zero codes pad the
+ * embedding width D up to round_up(D, 16)), then the row's fp32 scale s_r at byte `dim`, then padding;
+ * ld >= dim + 16 and ld % 16 == 0 (mmrs_quantize_rows_i8 writes ld = dim + 16).  A row view
+ * (gallery + r0 * ld) carries its own scales, so shards and row windows need no second pointer.
+ * For ld_gallery, dim and every `ld_*` of an int8 gallery, an element is one byte.
+ *
+ * Quantisation of a row x (gallery rows on ingest, queries in every search after their optional
+ * normalisation): m = max_j |x_j| (fp32), s = fl(m / 127), c_j = clamp(rint(x_j / s), -127, 127) with IEEE
+ * division and round half to even; a zero row has s = 0 and zero codes.  A row holding a NaN or an infinity
+ * is refused: MMRS_ERR_NONFINITE.
+ *
+ * Score, on every path (K1, K2, the exhaustive path, full scores, range search):
+ *   score(q, r) = fl(fl(float(dot) * a_q) * s_r),   a_q = fl(s_q * scale)
+ * where dot = sum_j c_qj * c_rj is the EXACT int32 code dot product; -0.0 is returned as +0.0.  float(dot)
+ * is exact for dim <= 1040 (127^2 * 1040 < 2^24) and rounds to nearest above.  The score is a deterministic
+ * function of the codes: it does not depend on the path, the tile schedule or the shard count.
+ */
 
 /* kernel selection for mmrs_search_topk / mmrs_full_scores */
 #define MMRS_PATH_AUTO 0   /* K1 for small batches, K2 (tcgen05) otherwise               */
 #define MMRS_PATH_GEMV 1   /* K1: 128-bit streaming + warp-shuffle dot products            */
-#define MMRS_PATH_MMA 2    /* K2: TMA + tcgen05.mma, bf16 gallery only                      */
+#define MMRS_PATH_MMA 2    /* K2: TMA + tcgen05.mma, bf16 / bf16x3 / int8 gallery              */
 
 int mmrs_abi_version(void);
 const char* mmrs_last_error(void);
@@ -124,6 +145,16 @@ int mmrs_full_scores(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t
 /* fp32 [n_rows, ld_src] -> bf16 planes [3, n_rows, ld_dst] (ld_dst % 8 == 0, >= dim; padding zeroed). */
 int mmrs_split_bf16x3(const float* d_src, int64_t n_rows, int32_t dim, int64_t ld_src, void* d_dst,
                       int64_t ld_dst, void* stream);
+
+/*
+ * Quantise d_src [n_rows, ld_src] (src_dtype MMRS_DTYPE_F32 or MMRS_DTYPE_BF16, `dim` real columns) into int8
+ * gallery rows d_dst [n_rows, ld_dst] bytes (see "int8 galleries"): codes [round_up(dim, 16)], zero past dim,
+ * the scale at byte round_up(dim, 16), zero up to ld_dst >= round_up(dim, 16) + 16 (ld_dst % 16 == 0).
+ * MMRS_ERR_NONFINITE when a row holds a NaN or an infinity (the other rows are still written).
+ * Synchronises `stream`.
+ */
+int mmrs_quantize_rows_i8(const void* d_src, int32_t src_dtype, int64_t n_rows, int32_t dim, int64_t ld_src,
+                          void* d_dst, int64_t ld_dst, void* stream);
 
 /* ---- search: fused top-k ------------------------------------------------------------- */
 
@@ -522,7 +553,8 @@ int mmrs_graph_stats(int64_t* h_out4);
  * bracketed by CUDA events on the caller's stream.  mmrs_profile_read() synchronises those events,
  * returns up to `cap` records (oldest first) and clears the log: duration in ms, kind
  * (MMRS_PATH_GEMV or MMRS_PATH_MMA), and the algorithmic gallery bytes the launch streamed
- * (rows visited * dim * element size).  Returns the number of records written.
+ * (rows visited * dim * element size; int8: rows visited * (dim + 16), the codes and the scale's tail).
+ * Returns the number of records written.
  */
 int mmrs_profile_enable(int on);
 int mmrs_profile_read(float* h_ms, int32_t* h_kind, int64_t* h_bytes, int64_t* h_flops, int32_t cap);

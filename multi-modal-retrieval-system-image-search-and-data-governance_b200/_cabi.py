@@ -10,8 +10,9 @@ LIB_PATH = _PKG_DIR / "lib" / "libmmrs_b200.so"
 
 OK = 0
 ERR_ARG, ERR_CUDA, ERR_ARCH, ERR_WORKSPACE, ERR_ZERO_NORM, ERR_CAPACITY, ERR_INTERNAL, ERR_RETRY, ERR_TIMEOUT = -1, -2, -3, -4, -5, -6, -7, -8, -9
+ERR_NONFINITE = -10
 ABI_VERSION = 3
-DTYPE_F32, DTYPE_BF16, DTYPE_BF16X3 = 0, 1, 2
+DTYPE_F32, DTYPE_BF16, DTYPE_BF16X3, DTYPE_I8 = 0, 1, 2, 3
 PATH_AUTO, PATH_GEMV, PATH_MMA = 0, 1, 2
 PATHS = {"auto": PATH_AUTO, "gemv": PATH_GEMV, "mma": PATH_MMA}
 LABEL_SAME, LABEL_OTHER = 0, 1
@@ -22,6 +23,10 @@ class MmrsError(RuntimeError):
     def __init__(self, code: int, message: str):
         super().__init__(f"mmrs_b200 error {code}: {message}")
         self.code = code
+
+
+class NonFiniteError(MmrsError, ValueError):
+    """int8 quantisation met a row (gallery or query) holding a NaN or an infinity."""
 
 
 def open_library(path: Path) -> C.CDLL:
@@ -62,6 +67,7 @@ SIGNATURES = {
     "mmrs_full_scores": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _f32, _i32,
                                    _vp, _i64, _vp, _sz, _vp]),
     "mmrs_split_bf16x3": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _i64, _vp]),
+    "mmrs_quantize_rows_i8": (C.c_int, [_vp, _i32, _i64, _i32, _i64, _vp, _i64, _vp]),
     "mmrs_search_workspace_bytes": (_sz, [_i64, _i32, _i32, _i32, _i32]),
     "mmrs_search_topk": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
                                    _i64, _i32, _vp, _vp, _vp, _sz, _vp]),
@@ -130,6 +136,8 @@ def last_error() -> str:
 
 
 def check(status: int) -> None:
+    if status == ERR_NONFINITE:
+        raise NonFiniteError(status, last_error())
     if status != OK:
         raise MmrsError(status, last_error())
 

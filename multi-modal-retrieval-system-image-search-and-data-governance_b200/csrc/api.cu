@@ -54,9 +54,10 @@ cudaError_t launch_selfjoin_recheck(const int64_t* cand, int64_t n_cand, const f
                                     unsigned long long* out_count, cudaStream_t stream);
 // K2.  q_bf16 is the prepared [n_q_padded, ldq] bf16 query matrix; handles up to 256 queries.
 // g_plane_rows: rows between two planes of a bf16x3 gallery (the full gallery's n_rows).
+// i8: an int8 gallery with the prepared int8 query rows in q_bf16.
 cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, int32_t n_q_padded,
                             int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split,
-                            int64_t g_plane_rows);
+                            int64_t g_plane_rows, bool i8 = false);
 cudaError_t launch_split_bf16x3(const float* src, int64_t n_rows, int32_t dim, int64_t ld_src, __nv_bfloat16* dst,
                                 int64_t ld_dst, int sm_count, cudaStream_t stream);
 // range search finalize (range.cu)
@@ -196,7 +197,7 @@ static int32_t padded_queries(int32_t nq) { return (nq + 15) / 16 * 16; }
 struct Workspace {
   int32_t* flags;          // [8]
   float* q_f32;            // [Qp, ldq]
-  __nv_bfloat16* q_bf16;   // [Qp, ldq]
+  __nv_bfloat16* q_bf16;   // [Qp, ldq]; int8 gallery: the int8 query rows [Qp, ldq + 16] bytes (fit: ldq >= 16)
   float* thr;              // [Qs]
   uint32_t* cnt;           // [Qs]
   uint64_t* cand;          // [Qs, cap] (>= n_tiles * kTileRows keys for the exhaustive path)
@@ -319,8 +320,18 @@ static int check_matrix(const void* p, int64_t n_rows, int32_t dim, int64_t ld, 
   if (!p) return fail(MMRS_ERR_ARG, "%s pointer is null", what);
   if (n_rows < 1) return fail(MMRS_ERR_ARG, "%s has %lld rows", what, (long long)n_rows);
   if (n_rows > 0xffffffffll) return fail(MMRS_ERR_ARG, "%s: more than 2^32 rows per shard", what);
-  if (dtype != MMRS_DTYPE_F32 && dtype != MMRS_DTYPE_BF16 && dtype != MMRS_DTYPE_BF16X3)
+  if (dtype != MMRS_DTYPE_F32 && dtype != MMRS_DTYPE_BF16 && dtype != MMRS_DTYPE_BF16X3 && dtype != MMRS_DTYPE_I8)
     return fail(MMRS_ERR_ARG, "%s dtype %d unknown", what, dtype);
+  if (dtype == MMRS_DTYPE_I8) {   // codes [dim], the row's scale at byte dim (include/mmrs_b200.h, "int8 galleries")
+    if (dim < 1 || dim % 16 != 0)
+      return fail(MMRS_ERR_ARG, "%s: int8 dim %d must be a positive multiple of 16 (zero codes pad it)", what, dim);
+    if (ld < dim + 16 || ld % 16 != 0)
+      return fail(MMRS_ERR_ARG, "%s: int8 row stride %lld must be >= dim + 16 and a multiple of 16 bytes", what,
+                  (long long)ld);
+    if (reinterpret_cast<uintptr_t>(p) % 16 != 0)
+      return fail(MMRS_ERR_ARG, "%s pointer must be 16-byte aligned", what);
+    return MMRS_OK;
+  }
   const int elems16 = dtype == MMRS_DTYPE_F32 ? 4 : 8;
   if (dim < 1 || dim % elems16 != 0)
     return fail(MMRS_ERR_ARG, "%s dim %d must be a positive multiple of %d (pad with zeros)", what,
@@ -349,7 +360,7 @@ static Path choose_path(int32_t requested, int32_t dtype, int32_t n_queries) {
   if (requested == MMRS_PATH_GEMV) return Path::kGemv;
   if (requested == MMRS_PATH_MMA) return Path::kMma;
   // measured on B200 (profiles/r01_tune3.log): K1 wins for 1-2 queries, K2 from 3 on
-  if (dtype == MMRS_DTYPE_BF16 && n_queries > 2 && scan_mma_available()) return Path::kMma;
+  if ((dtype == MMRS_DTYPE_BF16 || dtype == MMRS_DTYPE_I8) && n_queries > 2 && scan_mma_available()) return Path::kMma;
   return Path::kGemv;
 }
 
@@ -375,8 +386,26 @@ static int profiled_launch(int32_t kind, int64_t bytes, int64_t flops, cudaStrea
 template <typename F>
 static int profiled_scan(int32_t kind, int32_t dtype, const ScanParams& p, cudaStream_t stream, F launch) {
   const int64_t rows = g_prof_on.load(std::memory_order_relaxed) ? rows_in_schedule(p.sched, p.n_rows) : 0;
-  return profiled_launch(kind, rows * p.dim * (dtype == MMRS_DTYPE_BF16 ? 2 : (dtype == MMRS_DTYPE_BF16X3 ? 6 : 4)), 2 * rows * p.dim * p.nq,
-                         stream, launch);
+  // int8: the codes and the 16-byte tail that holds the row's scale
+  const int64_t row_bytes = dtype == MMRS_DTYPE_I8 ? p.dim + 16 : p.dim * (dtype == MMRS_DTYPE_BF16 ? 2 : (dtype == MMRS_DTYPE_BF16X3 ? 6 : 4));
+  return profiled_launch(kind, rows * row_bytes, 2 * rows * p.dim * p.nq, stream, launch);
+}
+
+// The mode of the prep kernel for a gallery dtype: 1 bf16 rounding, 2 bf16x3 planes, 3 int8 rows, 0 fp32.
+static int32_t prep_mode(int32_t dtype) {
+  return dtype == MMRS_DTYPE_BF16 ? 1 : (dtype == MMRS_DTYPE_BF16X3 ? 2 : (dtype == MMRS_DTYPE_I8 ? 3 : 0));
+}
+
+// The prepared queries the scan kernels read: fp32 rows [Qp, ldq], or for an int8 gallery the int8 query rows
+// the prep kernel wrote into q_bf16 in the gallery's row format (ldq + 16 bytes apart, s_q at byte ldq).
+static void set_queries(ScanParams& p, int32_t dtype, const Workspace& w, int32_t ldq) {
+  if (dtype == MMRS_DTYPE_I8) {
+    p.queries = reinterpret_cast<const float*>(w.q_bf16);
+    p.ldq = ldq + 16;
+  } else {
+    p.queries = w.q_f32;
+    p.ldq = ldq;
+  }
 }
 
 // One scan over the tiles of `sched` for queries [q_lo, q_hi) of the prepared matrices.
@@ -401,7 +430,8 @@ static int run_scan(Path path, const DeviceInfo& dev, int32_t dtype, ScanParams 
       p.nq = chunk;
       q += chunk;
       int rc = profiled_scan(MMRS_PATH_MMA, dtype, p, stream, [&]() {
-        return launch_scan_mma(p, w.q_bf16, n_q_padded, mode, w.flags, dev.sm_count, stream, split, plane_rows);
+        return launch_scan_mma(p, w.q_bf16, n_q_padded, mode, w.flags, dev.sm_count, stream, split, plane_rows,
+                               dtype == MMRS_DTYPE_I8);
       });
       if (rc != MMRS_OK) return rc;
     }
@@ -475,9 +505,8 @@ static int enqueue_prep(const SearchArgs& a, const Workspace& w, cudaStream_t st
     gp.timeout_ns = a.g_timeout_ns;
   }
   return profiled_launch(4, 0, 0, stream, [&]() {
-    return launch_prep_queries(a.d_queries, a.n_queries, a.ldq_in, a.dim, a.normalize,
-                               a.dtype == MMRS_DTYPE_BF16 ? 1 : (a.dtype == MMRS_DTYPE_BF16X3 ? 2 : 0), w.q_f32, w.q_bf16, qp, ldq,
-                               w.flags, gp, stream);
+    return launch_prep_queries(a.d_queries, a.n_queries, a.ldq_in, a.dim, a.normalize, prep_mode(a.dtype), w.q_f32,
+                               w.q_bf16, qp, ldq, w.flags, gp, stream);
   });
 }
 
@@ -500,7 +529,7 @@ static int enqueue_search(const SearchArgs& a, const DeviceInfo& dev, const Work
   }
   ScanParams base{};
   base.gallery = a.gallery; base.n_rows = a.n_rows; base.ld = a.ld; base.dim = a.dim;
-  base.queries = w.q_f32; base.ldq = ldq; base.scale = a.scale;
+  set_queries(base, a.dtype, w, ldq); base.scale = a.scale;
   base.cap = pl.cap;
   base.row_filter = a.row_filter;
   set_labels(base, a);
@@ -573,7 +602,7 @@ static int enqueue_exhaustive(const SearchArgs& a, const DeviceInfo& dev, const 
   const int32_t all_rows = pl.n_tiles * kTileRows;
   ScanParams base{};
   base.gallery = a.gallery; base.n_rows = a.n_rows; base.ld = a.ld; base.dim = a.dim;
-  base.queries = w.q_f32; base.ldq = ldq; base.scale = a.scale;
+  set_queries(base, a.dtype, w, ldq); base.scale = a.scale;
   base.cap = all_rows;
   base.sched = TileSchedule{pl.n_tiles, 1, 0, pl.n_tiles};
   base.row_filter = a.row_filter;
@@ -800,6 +829,8 @@ static int launch_search_graph(const SearchArgs& a, const DeviceInfo& dev, const
 static int flags_to_status(int32_t f) {
   if (f & kFlagZeroNorm)
     return fail(MMRS_ERR_ZERO_NORM, "a query row has zero L2 norm and normalize_queries is set");
+  if (f & kFlagNonFinite)
+    return fail(MMRS_ERR_NONFINITE, "a query row holds a NaN or an infinity: int8 quantisation refuses it");
   if (f & kFlagGatherTimeout)
     return fail(MMRS_ERR_TIMEOUT, "fused all-gather: a peer rank did not deliver / acknowledge its top-k lists within "
                 "MMRS_GATHER_TIMEOUT_MS (a dead or diverged rank; results of this batch are invalid)");
@@ -898,12 +929,11 @@ int mmrs_full_scores(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t
   if (p == Path::kMma && gallery_dtype == MMRS_DTYPE_F32)
     return fail(MMRS_ERR_ARG, "MMRS_PATH_MMA needs a bf16 (or bf16x3) gallery");
   MMRS_CUDA(cudaMemsetAsync(w.flags, 0, 8 * sizeof(int32_t), stream));
-  MMRS_LAUNCH(launch_prep_queries(d_queries, n_queries, ld_queries, dim, normalize_queries,
-                                gallery_dtype == MMRS_DTYPE_BF16 ? 1 : (gallery_dtype == MMRS_DTYPE_BF16X3 ? 2 : 0),
+  MMRS_LAUNCH(launch_prep_queries(d_queries, n_queries, ld_queries, dim, normalize_queries, prep_mode(gallery_dtype),
                                 w.q_f32, w.q_bf16, qp, ldq, w.flags, GatherPrologue{}, stream));
   ScanParams base{};
   base.gallery = d_gallery; base.n_rows = n_rows; base.ld = ld_gallery; base.dim = dim;
-  base.queries = w.q_f32; base.ldq = ldq; base.scale = scale;
+  set_queries(base, gallery_dtype, w, ldq); base.scale = scale;
   base.out_scores = d_out_scores; base.ld_out = ld_out;
   const int32_t n_tiles = static_cast<int32_t>((n_rows + kTileRows - 1) / kTileRows);
   base.sched = TileSchedule{n_tiles, 1, 0, n_tiles};
@@ -925,6 +955,35 @@ int mmrs_split_bf16x3(const float* d_src, int64_t n_rows, int32_t dim, int64_t l
     return fail(MMRS_ERR_ARG, "bad arguments (ld_dst must be a multiple of 8 and >= dim)");
   MMRS_LAUNCH(launch_split_bf16x3(d_src, n_rows, dim, ld_src, static_cast<__nv_bfloat16*>(d_dst), ld_dst,
                                   dev.sm_count, static_cast<cudaStream_t>(stream)));
+  return MMRS_OK;
+}
+
+int mmrs_quantize_rows_i8(const void* d_src, int32_t src_dtype, int64_t n_rows, int32_t dim, int64_t ld_src,
+                          void* d_dst, int64_t ld_dst, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (src_dtype != MMRS_DTYPE_F32 && src_dtype != MMRS_DTYPE_BF16)
+    return fail(MMRS_ERR_ARG, "quantise: source dtype %d must be MMRS_DTYPE_F32 or MMRS_DTYPE_BF16", src_dtype);
+  const int64_t dp = (static_cast<int64_t>(dim) + 15) / 16 * 16;
+  if (!d_src || !d_dst || n_rows < 0 || dim < 1 || ld_src < dim || ld_dst < dp + 16 || ld_dst % 16 != 0 ||
+      reinterpret_cast<uintptr_t>(d_dst) % 16 != 0)
+    return fail(MMRS_ERR_ARG, "quantise: bad arguments (ld_dst must be >= round_up(dim, 16) + 16, a multiple of 16, "
+                "and d_dst 16-byte aligned)");
+  if (n_rows == 0) return MMRS_OK;
+  int32_t* h = pinned_status();
+  if (!h) return fail(MMRS_ERR_CUDA, "cudaHostAlloc for the status word failed");
+  // a transient device status word: the call owns no workspace and keeps no device memory
+  int32_t* d_status = nullptr;
+  MMRS_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d_status), sizeof(int32_t), stream));
+  MMRS_CUDA(cudaMemsetAsync(d_status, 0, sizeof(int32_t), stream));
+  MMRS_LAUNCH(launch_quantize_rows_i8(d_src, src_dtype, n_rows, dim, ld_src, static_cast<int8_t*>(d_dst), ld_dst,
+                                      d_status, dev.sm_count, stream));
+  MMRS_CUDA(cudaMemcpyAsync(h, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaFreeAsync(d_status, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  if (h[0]) return fail(MMRS_ERR_NONFINITE, "a row holds a NaN or an infinity: int8 quantisation refuses it");
   return MMRS_OK;
 }
 
@@ -1593,16 +1652,15 @@ int mmrs_range_search_window(const void* d_gallery, int64_t n_rows, int32_t dim,
   MMRS_CUDA(cudaMemsetAsync(w.cnt, 0, static_cast<size_t>(n_queries) * sizeof(uint32_t), stream));
   MMRS_LAUNCH(launch_fill_u32(w.cnt + n_queries, static_cast<uint32_t>(window_rows), kRangePadLists, stream));
   MMRS_CUDA(cudaMemsetAsync(w.bitmap, 0, static_cast<size_t>(n_queries) * n_words * sizeof(uint32_t), stream));
-  MMRS_LAUNCH(launch_prep_queries(d_queries, n_queries, ld_queries, dim, normalize_queries,
-                                gallery_dtype == MMRS_DTYPE_BF16 ? 1 : (gallery_dtype == MMRS_DTYPE_BF16X3 ? 2 : 0),
+  MMRS_LAUNCH(launch_prep_queries(d_queries, n_queries, ld_queries, dim, normalize_queries, prep_mode(gallery_dtype),
                                 w.base.q_f32, w.base.q_bf16, qp, ldq, w.base.flags, GatherPrologue{}, stream));
   // the window is a view of the gallery, like a shard: rows [row_begin, row_begin + rows) as local rows 0..rows-1
   // (row_begin is a multiple of 128, so the view's bitmap words and labels start on whole tiles)
-  const size_t elem = gallery_dtype == MMRS_DTYPE_F32 ? sizeof(float) : sizeof(__nv_bfloat16);
+  const size_t elem = gallery_dtype == MMRS_DTYPE_F32 ? sizeof(float) : (gallery_dtype == MMRS_DTYPE_I8 ? 1 : sizeof(__nv_bfloat16));
   ScanParams base{};
   base.gallery = static_cast<const char*>(d_gallery) + static_cast<size_t>(row_begin) * ld_gallery * elem;
   base.n_rows = rows; base.ld = ld_gallery; base.dim = dim;
-  base.queries = w.base.q_f32; base.ldq = ldq; base.scale = scale;
+  set_queries(base, gallery_dtype, w.base, ldq); base.scale = scale;
   const int32_t n_tiles = static_cast<int32_t>((rows + kTileRows - 1) / kTileRows);
   base.sched = TileSchedule{n_tiles, 1, 0, n_tiles};
   // cap = window_rows >= rows: a list holds at most one key per row, so it cannot overflow

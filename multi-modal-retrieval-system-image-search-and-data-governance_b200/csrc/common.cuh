@@ -19,6 +19,7 @@ constexpr int kFlagZeroNorm = 2;      // normalize_queries and ||q|| == 0
 constexpr int kFlagShort = 4;         // fewer than k candidates reached a select (bug guard)
 constexpr int kFlagWatchdog = 8;      // an mbarrier wait timed out (K2 debug guard)
 constexpr int kFlagGatherTimeout = 16;  // fused all-gather: a peer rank's flag did not arrive in time
+constexpr int kFlagNonFinite = 32;      // int8 mode: a query row holds a NaN or an infinity
 
 // Status bits of the duplicate resolve (dedup_resolve.cu), in its own status word.
 constexpr int kResolveOrderRange = 1;   // an order id outside [0, n_items)
@@ -54,6 +55,17 @@ __host__ __device__ __forceinline__ float key_score(uint64_t key) {
 }
 __host__ __device__ __forceinline__ uint32_t key_row(uint64_t key) {
   return ~static_cast<uint32_t>(key);
+}
+
+// ---- int8 galleries (include/mmrs_b200.h, "int8 galleries") ----------------------------------------
+// The one score formula of every int8 path: fl(fl(float(dot) * a_q) * s_r), -0.0 returned as +0.0.
+// dot is the exact int32 code product; a_q = fl(s_q * scale) is taken once per query.
+__device__ __forceinline__ float i8_score(int32_t dot, float a_q, float s_r) {
+  return __fmul_rn(__fmul_rn(__int2float_rn(dot), a_q), s_r) + 0.0f;
+}
+// the row's fp32 scale sits at byte `dim` of the row (dim = the padded code count)
+__device__ __forceinline__ float i8_row_scale(const void* row, int32_t dim) {
+  return __ldg(reinterpret_cast<const float*>(static_cast<const int8_t*>(row) + dim));
 }
 
 // ---- streaming loads -------------------------------------------------------------------------
@@ -161,7 +173,8 @@ struct ScanParams {
   int64_t ld;             // elements
   int32_t dim;
   int32_t label_match;    // label-conditioned search: MMRS_LABEL_SAME / MMRS_LABEL_OTHER (see row_labels)
-  const float* queries;   // prepared fp32 queries [*, ldq] (normalised, bf16-rounded in bf16 mode)
+  const float* queries;   // prepared fp32 queries [*, ldq] (normalised, bf16-rounded in bf16 mode); int8 mode:
+                          // the prepared int8 query rows in the gallery's row format (s_q at byte dim), ldq bytes
   int32_t ldq;
   int32_t q0;             // first query of this pass
   int32_t nq;             // queries in this pass (<= template QN)
@@ -249,6 +262,8 @@ cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t dim, i
                                   int sm_count, cudaStream_t stream);
 cudaError_t launch_scan_gemv(const ScanParams& p, int32_t dtype, int mode, int sm_count,
                              cudaStream_t stream);
+cudaError_t launch_quantize_rows_i8(const void* src, int32_t src_dtype, int64_t n_rows, int32_t dim, int64_t ld_src,
+                                    int8_t* dst, int64_t ld_dst, int32_t* status, int sm_count, cudaStream_t stream);
 cudaError_t launch_select(const SelectParams& p, int32_t n_queries, cudaStream_t stream);
 cudaError_t launch_fill_u32(uint32_t* p, uint32_t v, int64_t n, cudaStream_t stream);
 cudaError_t launch_pack_row_filter(const uint8_t* allowed, int64_t n_rows, uint32_t* words, int64_t n_words,

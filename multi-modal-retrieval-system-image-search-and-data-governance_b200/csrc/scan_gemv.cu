@@ -11,6 +11,8 @@
 // HBM roofline: N*D*sizeof(T) bytes per pass (SURVEY.md section 8d).  The FP32 pipe allows about
 // 11.5 bf16 elements/clk/SM at 6.5 TB/s, i.e. QN <= 4 keeps the kernel memory-bound; larger
 // batches belong to K2 (scan_mma.cu).
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace mmrs {
@@ -32,19 +34,24 @@ template <> struct Chunk<float> {
     f[2] = __uint_as_float(g.z); f[3] = __uint_as_float(g.w);
   }
 };
+// int8 rows: 16 codes per load, multiplied four at a time with __dp4a into exact int32 sums
+template <> struct Chunk<int8_t> {
+  static constexpr int CH = 16;
+};
 
 // Sum V per-lane partials across the warp.  While more than one value is live each stage
 // halves the set (lanes with bit `O` keep the upper half), afterwards it is a plain butterfly.
 // On return lane l holds the total of value index l / (32 / V).
 template <int N, int O>
 struct TransposeReduce {
-  static __device__ __forceinline__ void run(float* v, int lane) {
+  template <typename X>
+  static __device__ __forceinline__ void run(X* v, int lane) {
     if constexpr (N > 1) {
       const bool up = (lane & O) != 0;
 #pragma unroll
       for (int i = 0; i < N / 2; ++i) {
-        const float send = up ? v[i] : v[i + N / 2];
-        const float keep = up ? v[i + N / 2] : v[i];
+        const X send = up ? v[i] : v[i + N / 2];
+        const X keep = up ? v[i + N / 2] : v[i];
         v[i] = keep + __shfl_xor_sync(0xffffffffu, send, O);
       }
       if constexpr (O > 1) TransposeReduce<N / 2, O / 2>::run(v, lane);
@@ -60,8 +67,12 @@ constexpr int kGemvWarps = kGemvThreads / 32;
 
 // LABELED: label-conditioned search (p.row_labels != nullptr, dense / filter modes only).  A separate
 // instantiation, so that the unlabeled kernels keep their code and registers.
+// T = int8_t: int8 gallery rows and int8 query rows (the gallery's row format, p.ldq bytes apart), exact
+// int32 sums, the score of i8_score with the row's scale read from its tail.
 template <typename T, int QN, int R, int MODE, bool LABELED = false>
 __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanParams p) {
+  constexpr bool I8 = std::is_same<T, int8_t>::value;
+  using Acc = typename std::conditional<I8, int32_t, float>::type;
   constexpr int CH = Chunk<T>::CH;
   constexpr int H = CH / 4;  // float4 pieces of a query chunk
   constexpr int V = QN * R;
@@ -69,11 +80,20 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
   static_assert(kTileRows % (kGemvWarps * R) == 0, "tile must split evenly over the warps");
 
   // Query chunks, laid out [QN][H][n_chunks] in float4 so that consecutive lanes read
-  // consecutive 16-byte words (conflict-free LDS.128).
+  // consecutive 16-byte words (conflict-free LDS.128).  int8: [QN][n_chunks] 16-code words.
   extern __shared__ float4 q_smem[];
   const int n_chunks = p.dim / CH;
   pdl_launch_dependents();
   pdl_wait();   // queries (prep kernel) and thresholds (previous select) come from predecessors
+  const int8_t* q_i8 = reinterpret_cast<const int8_t*>(p.queries);
+  if constexpr (I8) {
+    for (int i = threadIdx.x; i < QN * n_chunks; i += kGemvThreads) {
+      const int c = i % n_chunks, qi = i / n_chunks;
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      if (qi < p.nq) v = *reinterpret_cast<const uint4*>(q_i8 + static_cast<size_t>(p.q0 + qi) * p.ldq + c * CH);
+      q_smem[i] = *reinterpret_cast<const float4*>(&v);
+    }
+  } else
   for (int i = threadIdx.x; i < QN * H * n_chunks; i += kGemvThreads) {
     const int c = i % n_chunks;
     const int h = (i / n_chunks) % H;
@@ -95,6 +115,10 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
   float my_thr = 0.f;
   if constexpr (MODE == kModeFilter) {
     if (owner) my_thr = p.thr[p.q0 + my_q];
+  }
+  float my_aq = 0.f;       // int8: a_q = fl(s_q * scale) of the owned query
+  if constexpr (I8) {
+    if (owner) my_aq = __fmul_rn(i8_row_scale(q_i8 + static_cast<size_t>(p.q0 + my_q) * p.ldq, p.dim), p.scale);
   }
   int32_t my_label = -1;   // label-conditioned search: the owned query's label (< 0: no restriction)
   if constexpr (LABELED) {
@@ -121,12 +145,31 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
         const int64_t row = row0 + r;
         rp[r] = gal + (row <= last_row ? row : last_row) * p.ld;  // clamp: tail rows re-read the last row
       }
-      float acc[R][QN];
+      Acc acc[R][QN];
 #pragma unroll
       for (int r = 0; r < R; ++r)
 #pragma unroll
-        for (int qi = 0; qi < QN; ++qi) acc[r][qi] = 0.f;
+        for (int qi = 0; qi < QN; ++qi) acc[r][qi] = 0;
 
+      if constexpr (I8) {
+        for (int c = lane; c < n_chunks; c += 32) {
+          uint4 g[R];
+#pragma unroll
+          for (int r = 0; r < R; ++r) g[r] = ldg_stream_16B(rp[r] + c * CH);
+#pragma unroll
+          for (int qi = 0; qi < QN; ++qi) {
+            const float4 x = q_smem[qi * n_chunks + c];
+            const int qw[4] = {__float_as_int(x.x), __float_as_int(x.y), __float_as_int(x.z), __float_as_int(x.w)};
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+              acc[r][qi] = __dp4a(static_cast<int>(g[r].x), qw[0], acc[r][qi]);
+              acc[r][qi] = __dp4a(static_cast<int>(g[r].y), qw[1], acc[r][qi]);
+              acc[r][qi] = __dp4a(static_cast<int>(g[r].z), qw[2], acc[r][qi]);
+              acc[r][qi] = __dp4a(static_cast<int>(g[r].w), qw[3], acc[r][qi]);
+            }
+          }
+        }
+      } else
       for (int c = lane; c < n_chunks; c += 32) {
         uint4 g[R];
 #pragma unroll
@@ -151,7 +194,7 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
         }
       }
 
-      float v[V];
+      Acc v[V];
 #pragma unroll
       for (int r = 0; r < R; ++r)
 #pragma unroll
@@ -160,7 +203,11 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
 
       if (owner) {
         const int64_t row = row0 + my_r;
-        const float s = v[0] * p.scale;
+        float s;
+        if constexpr (I8)
+          s = i8_score(v[0], my_aq, i8_row_scale(gal + (row <= last_row ? row : last_row) * p.ld, p.dim));
+        else
+          s = v[0] * p.scale;
         const int q = p.q0 + my_q;
         // the bitmap covers whole tiles, so the word of a tail row past last_row is readable (and zero)
         bool row_ok = row <= last_row;
@@ -192,7 +239,7 @@ __global__ void __launch_bounds__(kGemvThreads, 2) scan_gemv_kernel(const ScanPa
 template <typename T, int QN, int R>
 static cudaError_t launch_gemv_mode(const ScanParams& p, int mode, int sm_count,
                                     cudaStream_t stream) {
-  const size_t smem = static_cast<size_t>(QN) * p.dim * sizeof(float);
+  const size_t smem = static_cast<size_t>(QN) * p.dim * (std::is_same<T, int8_t>::value ? 1 : sizeof(float));
   auto go = [&](auto kernel) -> cudaError_t {
     cudaError_t e = cudaSuccess;
     if (smem > 48 * 1024) {
@@ -231,13 +278,29 @@ cudaError_t launch_scan_gemv(const ScanParams& p, int32_t dtype, int mode, int s
                              cudaStream_t stream) {
   if (p.nq < 1 || p.nq > 8) return cudaErrorInvalidValue;
   if (dtype == MMRS_DTYPE_BF16) return launch_gemv_q<__nv_bfloat16>(p, mode, sm_count, stream);
+  if (dtype == MMRS_DTYPE_I8) return launch_gemv_q<int8_t>(p, mode, sm_count, stream);
   return launch_gemv_q<float>(p, mode, sm_count, stream);
+}
+
+// ---- int8 quantisation (include/mmrs_b200.h, "int8 galleries") -------------------------------------
+// s = fl(m / 127) for the row's max |x|; c = clamp(rint(x / s), -127, 127), IEEE division, half to even
+__device__ __forceinline__ float i8_scale_of(float max_abs) { return __fdiv_rn(max_abs, 127.f); }
+__device__ __forceinline__ int32_t i8_code(float x, float s) {
+  if (!(s > 0.f)) return 0;
+  return static_cast<int32_t>(fminf(fmaxf(rintf(__fdiv_rn(x, s)), -127.f), 127.f));
+}
+__device__ __forceinline__ float warp_max(float m) {
+#pragma unroll
+  for (int o = 16; o >= 1; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  return m;
 }
 
 // ---- query preparation ------------------------------------------------------------------------
 // One warp per query row: optional L2 normalisation `x / x.norm()` (the reference idiom,
 // code/search_image.py:157 -- sqrt of the fp32 sum of squares, true division, no epsilon),
 // optional rounding to bf16 (tensor-core mode), zero padding to [n_rows_padded, ld_out].
+// round_bf16 == 3 (int8 gallery): the normalised row is quantised like a gallery row into out_bf16 viewed as
+// int8 rows of ld_out + 16 bytes -- codes [ld_out], s_q at byte ld_out -- the operand of K1 and K2.
 __global__ void __launch_bounds__(256) prep_queries_kernel(
     const float* __restrict__ q, int32_t n_queries, int64_t ldq, int32_t dim, int32_t normalize,
     int32_t round_bf16, float* __restrict__ out_f32, __nv_bfloat16* __restrict__ out_bf16,
@@ -265,6 +328,23 @@ __global__ void __launch_bounds__(256) prep_queries_kernel(
     for (int o = 16; o >= 1; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
     inv_den = sqrtf(ss);
     if (!(inv_den > 0.f) && lane == 0) atomicOr(flags, kFlagZeroNorm);
+  }
+  if (round_bf16 == 3) {
+    auto val = [&](int d) -> float { return (real && d < dim) ? (normalize ? src[d] / inv_den : src[d]) : 0.f; };
+    float m = 0.f;
+    bool bad = false;
+    for (int d = lane; d < dim; d += 32) {
+      const float v = val(d);
+      bad |= !isfinite(v);
+      m = fmaxf(m, fabsf(v));
+    }
+    m = warp_max(m);
+    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(flags, kFlagNonFinite);
+    const float sq = i8_scale_of(m);
+    int8_t* out = reinterpret_cast<int8_t*>(out_bf16) + static_cast<int64_t>(row) * (ld_out + 16);
+    for (int d = lane; d < ld_out; d += 32) out[d] = static_cast<int8_t>(i8_code(val(d), sq));
+    if (lane == 0) *reinterpret_cast<float4*>(out + ld_out) = make_float4(sq, 0.f, 0.f, 0.f);
+    return;
   }
   for (int d = lane; d < ld_out; d += 32) {
     float v = 0.f;
@@ -322,6 +402,57 @@ cudaError_t launch_split_bf16x3(const float* src, int64_t n_rows, int32_t dim, i
   int64_t grid = (n_rows * ld_dst + 255) / 256;
   if (grid > static_cast<int64_t>(sm_count) * 16) grid = static_cast<int64_t>(sm_count) * 16;
   split_bf16x3_kernel<<<static_cast<int>(grid), 256, 0, stream>>>(src, n_rows, dim, ld_src, dst, ld_dst);
+  return cudaGetLastError();
+}
+
+// ---- gallery ingest: fp32 / bf16 rows -> int8 rows with their scale (mmrs_quantize_rows_i8) -------------
+// One warp per row; each lane handles 4 consecutive columns per step and stores them as one word.
+template <typename S>
+__global__ void __launch_bounds__(256) quantize_rows_i8_kernel(const S* __restrict__ src, int64_t n_rows, int32_t dim,
+                                                               int64_t ld_src, int8_t* __restrict__ dst, int64_t ld_dst,
+                                                               int32_t* status) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+  const int32_t dp = (dim + 15) / 16 * 16;
+  for (int64_t r = (blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5; r < n_rows; r += n_warps) {
+    const S* x = src + r * ld_src;
+    auto val = [&](int d) -> float {
+      if (d >= dim) return 0.f;
+      if constexpr (std::is_same<S, float>::value) return x[d];
+      else return __bfloat162float(x[d]);
+    };
+    float m = 0.f;
+    bool bad = false;
+    for (int d = lane; d < dim; d += 32) {
+      const float v = val(d);
+      bad |= !isfinite(v);
+      m = fmaxf(m, fabsf(v));
+    }
+    m = warp_max(m);
+    if (__any_sync(0xffffffffu, bad) && lane == 0) *status = 1;
+    const float s = i8_scale_of(m);
+    int8_t* o = dst + r * ld_dst;
+    for (int d0 = lane * 4; d0 < dp; d0 += 128) {
+      uint32_t w = 0;
+#pragma unroll
+      for (int e = 0; e < 4; ++e) w |= (static_cast<uint32_t>(i8_code(val(d0 + e), s)) & 0xffu) << (8 * e);
+      *reinterpret_cast<uint32_t*>(o + d0) = w;
+    }
+    for (int64_t b = dp + lane * 4; b < ld_dst; b += 128)   // the scale, then zeros
+      *reinterpret_cast<uint32_t*>(o + b) = b == dp ? __float_as_uint(s) : 0u;
+  }
+}
+cudaError_t launch_quantize_rows_i8(const void* src, int32_t src_dtype, int64_t n_rows, int32_t dim, int64_t ld_src,
+                                    int8_t* dst, int64_t ld_dst, int32_t* status, int sm_count, cudaStream_t stream) {
+  if (n_rows <= 0) return cudaSuccess;
+  int64_t grid = (n_rows * 32 + 255) / 256;
+  if (grid > static_cast<int64_t>(sm_count) * 16) grid = static_cast<int64_t>(sm_count) * 16;
+  if (src_dtype == MMRS_DTYPE_BF16)
+    quantize_rows_i8_kernel<__nv_bfloat16><<<static_cast<int>(grid), 256, 0, stream>>>(
+        static_cast<const __nv_bfloat16*>(src), n_rows, dim, ld_src, dst, ld_dst, status);
+  else
+    quantize_rows_i8_kernel<float><<<static_cast<int>(grid), 256, 0, stream>>>(static_cast<const float*>(src), n_rows,
+                                                                                dim, ld_src, dst, ld_dst, status);
   return cudaGetLastError();
 }
 

@@ -1,4 +1,4 @@
-// scan_mma.cu -- K2: tcgen05 tensor-core scan for batched queries over a bf16 gallery.
+// scan_mma.cu -- K2: tcgen05 tensor-core scan for batched queries over a bf16 (or int8, kind::i8) gallery.
 //
 // "Batched queries really are a dense contraction" (BASELINE.json): scores[128 rows, Q] =
 // G_tile[128, D] * Qmat[Q, D]^T, both operands K-major bf16.  One persistent CTA per SM walks its
@@ -90,7 +90,12 @@ struct MmaCfg {
 // (profiles/r02_prefetch_ab.log against r02_sticky_ab.log) -- that loop is issue-bound, every instruction counts.
 // LABELED: label-conditioned search (p.row_labels != nullptr, dense / filter modes only), a separate
 // instantiation so that the unlabeled kernels keep their code and registers.
-template <int MODE, int EPI_WARPS, bool PAIR, int SPLIT, bool LABELED = false>
+// I8: int8 gallery and query rows (include/mmrs_b200.h, "int8 galleries").  The TMA boxes move the same
+// 128-byte rows (128 codes per k-block), tcgen05.mma.kind::i8 takes K = 32 per instruction -- four per
+// k-block, the same +32-byte descriptor step -- into an s32 accumulator, and the epilogue turns each exact
+// int32 sum into i8_score with a_q from shared memory (the thr_raw slots, unused by int8) and the row's scale
+// s_r from the row's tail.  Every pair's exact score is compared with thr: no raw-accumulator prefilter.
+template <int MODE, int EPI_WARPS, bool PAIR, int SPLIT, bool LABELED = false, bool I8 = false>
 __global__ void __launch_bounds__((kCtrlWarps + EPI_WARPS) * 32, EPI_WARPS == 8 ? 2 : 1)
 scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant__ CUtensorMap map_q,
                 const ScanParams p, const MmaCfg cfg, int32_t* flags) {
@@ -198,6 +203,10 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
         tr = t / p.scale;
         tr = tr - fabsf(tr) * 4.8e-7f - 1e-37f;
       }
+      if constexpr (I8)   // a_q = fl(s_q * scale); padded columns 0
+        tr = c < n_q ? __fmul_rn(i8_row_scale(reinterpret_cast<const int8_t*>(p.queries) +
+                                                  static_cast<size_t>(first_q + c) * p.ldq, p.dim), p.scale)
+                     : 0.f;
       sh->thr_raw[c] = tr;
     }
     if constexpr (labeled) {
@@ -277,7 +286,8 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
     // four MMAs keep the tensor pipe busy (ncu: ring always full, pipe 66 % active,
     // profiles/r01_k2_c5like_summary.txt).  Warp-uniform code keeps them in uniform registers.
     if (rank == 0) {
-      const uint32_t idesc = make_idesc(static_cast<uint32_t>(cfg.n_umma), PAIR ? 256u : 128u);
+      const uint32_t idesc = I8 ? make_idesc_i8(static_cast<uint32_t>(cfg.n_umma), PAIR ? 256u : 128u)
+                                : make_idesc(static_cast<uint32_t>(cfg.n_umma), PAIR ? 256u : 128u);
       const uint32_t ring_addr = smem_u32(ring);
       uint32_t stage = 0, phase = 0, it = 0;
       bool ok = true;
@@ -292,7 +302,19 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
           tcgen05_fence_after();
           const uint32_t a_addr = ring_addr + stage * stage_bytes;
           if (elect_one()) {
-            if constexpr (SPLIT == 1) {
+            if constexpr (I8) {
+              const uint64_t adesc = make_sw128_desc(a_addr);
+              const uint64_t bdesc = make_sw128_desc(a_addr + kABytes);
+#pragma unroll
+              for (int k = 0; k < kBlockK / kUmmaK; ++k) {   // 32 codes = 32 bytes per instruction
+                if constexpr (PAIR)
+                  umma_i8_pair(d_tmem, adesc + static_cast<uint64_t>(k * 2), bdesc + static_cast<uint64_t>(k * 2), idesc,
+                               (kb | k) != 0 ? 1u : 0u);
+                else
+                  umma_i8(d_tmem, adesc + static_cast<uint64_t>(k * 2), bdesc + static_cast<uint64_t>(k * 2), idesc,
+                          (kb | k) != 0 ? 1u : 0u);
+              }
+            } else if constexpr (SPLIT == 1) {
               const uint64_t adesc = make_sw128_desc(a_addr);
               const uint64_t bdesc = make_sw128_desc(a_addr + kABytes);
 #pragma unroll
@@ -380,6 +402,9 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
       // reason -- one coalesced 128-byte load per warp
       int32_t row_label = 0;
       if constexpr (labeled) row_label = __ldg(p.row_labels + row);
+      float s_r = 0.f;   // int8: the row's scale (a tail row past the end reads the last row's)
+      if constexpr (I8)
+        s_r = i8_row_scale(static_cast<const int8_t*>(p.gallery) + (row <= last_row ? row : last_row) * p.ld, p.dim);
       const int32_t* lab_u = lab_s + (PAIR ? un.chunk * kMaxQ : 0);
       if (!mbar_wait(&sh->tmem_full[as], aphase, &sh->abort, flags)) break;
       tcgen05_fence_after();
@@ -427,9 +452,23 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
         auto process16 = [&](const uint32_t (&acc)[16], int c0, uint32_t eligible) {
           // branch-free pass mask for the 16 columns (every taken branch would expose its full
           // latency), then a short loop over the set bits
+          uint32_t bits = 0;
+          if constexpr (I8) {
+            const float4* thr4 = reinterpret_cast<const float4*>(thr_s + c0);
+            const float4* aq4 = reinterpret_cast<const float4*>(thr_raw_s + c0);
+#pragma unroll
+            for (int c4 = 0; c4 < 4; ++c4) {
+              const float4 tq = thr4[c4], aq = aq4[c4];
+              const float tv[4] = {tq.x, tq.y, tq.z, tq.w}, av[4] = {aq.x, aq.y, aq.z, aq.w};
+#pragma unroll
+              for (int u4 = 0; u4 < 4; ++u4) {
+                const float sc = i8_score(static_cast<int32_t>(acc[c4 * 4 + u4]), av[u4], s_r);
+                bits |= (sc < tv[u4]) ? 0u : (1u << (c4 * 4 + u4));
+              }
+            }
+          } else {
           const float4* thr4 = reinterpret_cast<const float4*>((raw_ok ? thr_raw_s : thr_s) + c0);
           const float mul = raw_ok ? 1.0f : p.scale;
-          uint32_t bits = 0;
 #pragma unroll
           for (int c4 = 0; c4 < 4; ++c4) {
             const float4 tq = thr4[c4];
@@ -440,6 +479,7 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
               bits |= ((raw_ok ? a : a * mul) < tv[u4]) ? 0u : (1u << (c4 * 4 + u4));
             }
           }
+          }
           if (!row_ok) bits = 0;
           if constexpr (labeled) bits &= eligible;
           while (bits) {
@@ -448,7 +488,7 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
             uint32_t a = acc[0];
 #pragma unroll
             for (int u4 = 1; u4 < 16; ++u4) a = (c == u4) ? acc[u4] : a;
-            const float sc = __uint_as_float(a) * p.scale;
+            const float sc = I8 ? i8_score(static_cast<int32_t>(a), thr_raw_s[c0 + c], s_r) : __uint_as_float(a) * p.scale;
             if (sc < thr_s[c0 + c]) continue;        // the exact test
             if (n_st == kStash) flush();
             my_stash[n_st * 32] = make_uint2(static_cast<uint32_t>(c0 + c), __float_as_uint(sc));
@@ -470,8 +510,8 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
           return m;
         };
         // the labeled small-pair variant (off by default) reads one 16-column load at a time: with two in
-        // flight it spilled
-        constexpr int kColStep = (labeled && EPI_WARPS == 8 && PAIR) ? 16 : 32;
+        // flight it spilled; so did the int8 variants of 8 epilogue warps (80 registers), which keep 16 scores live
+        constexpr int kColStep = ((labeled && EPI_WARPS == 8 && PAIR) || (I8 && EPI_WARPS == 8)) ? 16 : 32;
         for (int c0 = c_begin; c0 < c_end; c0 += kColStep) {
           uint32_t acc0[16], acc1[16];
           const bool two = kColStep == 32 && c0 + 16 < c_end;     // warp-uniform
@@ -505,7 +545,8 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
 #pragma unroll
           for (int c = 0; c < 16; ++c) {
             if (c0 + c < nq) {
-              const float s = __uint_as_float(acc[c]) * p.scale;
+              const float s = I8 ? i8_score(static_cast<int32_t>(acc[c]), thr_raw_s[c0 + c], s_r)
+                                 : __uint_as_float(acc[c]) * p.scale;
               const bool ok = row_ok && (!labeled || label_ok(row_label, lab_u[c0 + c], p.label_match));
               p.cand[static_cast<int64_t>(q0 + c0 + c) * p.cap + slot] =
                   ok ? make_key(s, static_cast<uint32_t>(row)) : 0ull;
@@ -517,7 +558,8 @@ scan_mma_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_constant
             for (int c = 0; c < 16; ++c) {
               if (c0 + c < nq)
                 p.out_scores[static_cast<int64_t>(q0 + c0 + c) * p.ld_out + row] =
-                    __uint_as_float(acc[c]) * p.scale;
+                    I8 ? i8_score(static_cast<int32_t>(acc[c]), thr_raw_s[c0 + c], s_r)
+                       : __uint_as_float(acc[c]) * p.scale;
             }
           }
         }
@@ -556,20 +598,36 @@ int scan_mma_max_queries() {
 }
 bool scan_mma_available() { return true; }
 
+// The int8 launches pick among the same variants as the bf16 ones.
+template <int EPI, bool PAIR, typename Go>
+static cudaError_t go_i8(int mode, bool labeled, Go&& go) {
+  switch (mode) {
+    case kModeScores: return go(scan_mma_kernel<kModeScores, EPI, PAIR, 1, false, true>);
+    case kModeDense:
+      return labeled ? go(scan_mma_kernel<kModeDense, EPI, PAIR, 1, true, true>) : go(scan_mma_kernel<kModeDense, EPI, PAIR, 1, false, true>);
+    default:
+      return labeled ? go(scan_mma_kernel<kModeFilter, EPI, PAIR, 1, true, true>) : go(scan_mma_kernel<kModeFilter, EPI, PAIR, 1, false, true>);
+  }
+}
+
 // g_plane_rows (split == 3): rows between two gallery planes -- the FULL gallery's row count, also when
 // p.gallery / p.n_rows are a row window of plane 0 (range search)
+// i8: int8 gallery rows and prepared int8 query rows (q_bf16 holds them, p.ldq bytes apart); p.dim and p.ld
+// count bytes.  The tensor maps see each 128-byte k-block as 64 bf16 columns: TMA only moves bytes.
 cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, int32_t n_q_padded,
                             int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split,
-                            int64_t g_plane_rows) {
+                            int64_t g_plane_rows, bool i8) {
   const int n_qchunks = (p.nq + kMaxQ - 1) / kMaxQ;
   if (p.nq < 1 || n_qchunks > kMaxQChunks) return cudaErrorInvalidValue;
   if (split != 1 && split != 3) return cudaErrorInvalidValue;
+  if (i8 && (split != 1 || p.dim % 16 != 0 || p.ld % 16 != 0 || p.ldq % 16 != 0)) return cudaErrorInvalidValue;
   if (split == 3 && p.nq > scan_mma_split_max_queries()) return cudaErrorInvalidValue;
   if (p.n_rows > 0x7fffffffll - kBlockM) return cudaErrorInvalidValue;   // TMA coordinates are int32
   if (p.sched.tile_exc != 0 && p.sched.tile_exc % p.sched.tile_inc != 0) return cudaErrorInvalidValue;
   MmaCfg cfg;
   cfg.n_umma = n_qchunks > 1 ? kMaxQ : (p.nq + 15) / 16 * 16;   // multi-chunk launches: full-width tiles (padded columns never pass)
-  cfg.k_blocks = (p.dim + kBlockK - 1) / kBlockK;
+  const int32_t map_cols = i8 ? p.dim / 2 : p.dim;   // in bf16 columns of 2 bytes
+  cfg.k_blocks = (map_cols + kBlockK - 1) / kBlockK;
   cfg.split = split;
   cfg.g_plane_rows = g_plane_rows;
   cfg.q_plane_rows = n_q_padded;
@@ -634,11 +692,13 @@ cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, in
   CUtensorMap map_g, map_q;
   const int64_t g_map_rows = static_cast<int64_t>(split - 1) * g_plane_rows + p.n_rows;   // = split * n_rows unwindowed
   if (g_map_rows > 0x7fffffffll - kBlockM) return cudaErrorInvalidValue;
-  if (!make_map(&map_g, p.gallery, static_cast<uint64_t>(g_map_rows), static_cast<uint64_t>(p.dim),
-                static_cast<uint64_t>(p.ld), kBlockM))
+  // int8: the inner extent is the codes only, so the scale bytes are never loaded as codes and K2 gets zero
+  // fill past dim
+  if (!make_map(&map_g, p.gallery, static_cast<uint64_t>(g_map_rows), static_cast<uint64_t>(map_cols),
+                static_cast<uint64_t>(i8 ? p.ld / 2 : p.ld), kBlockM))
     return cudaErrorNotSupported;
-  if (!make_map(&map_q, q_bf16, static_cast<uint64_t>(split) * n_q_padded, static_cast<uint64_t>(p.ldq),
-                static_cast<uint64_t>(p.ldq), static_cast<uint32_t>(b_rows)))
+  if (!make_map(&map_q, q_bf16, static_cast<uint64_t>(split) * n_q_padded, static_cast<uint64_t>(i8 ? map_cols : p.ldq),
+                static_cast<uint64_t>(i8 ? p.ldq / 2 : p.ldq), static_cast<uint32_t>(b_rows)))
     return cudaErrorNotSupported;
 
   const int R = plan_exclusion_ratio(p.sched.tile_inc, p.sched.tile_exc);
@@ -677,6 +737,12 @@ cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, in
     return launch_pdl_cluster(kernel, grid, dim3((kCtrlWarps + (half_sm ? 8 : 16)) * 32), smem, stream, pair ? 2u : 1u,
                               map_g, map_q, p, cfg, flags);
   };
+  if (i8) {
+    if (small) return go_i8<8, false>(mode, labeled, go);
+    if (small_pair) return go_i8<8, true>(mode, labeled, go);
+    if (pair) return go_i8<16, true>(mode, labeled, go);
+    return go_i8<16, false>(mode, labeled, go);
+  }
   if (small) {
     switch (mode) {
       case kModeScores: return go(scan_mma_kernel<kModeScores, 8, false, 1>);

@@ -85,6 +85,16 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// kind::i8: signed int8 A / B, s32 accumulator, K = 32 per instruction
+__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                        uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // 32 lanes x 16 consecutive fp32 columns: thread i of the warp gets TMEM lane (base + i)
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
   asm volatile(
@@ -143,6 +153,15 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, 
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                             uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // arrives (once the MMAs issued so far retire) on the barrier at this offset in BOTH CTAs of the pair
 __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
   asm volatile(
@@ -165,6 +184,10 @@ __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
 // kind::f16 instruction descriptor: D fp32, A/B bf16, both K-major, M=128, N=n.
 __host__ __device__ constexpr uint32_t make_idesc(uint32_t n, uint32_t m = 128u) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// kind::i8 instruction descriptor: D s32 (c_format 2), A/B signed int8 (format 1), both K-major, M=128, N=n.
+__host__ __device__ constexpr uint32_t make_idesc_i8(uint32_t n, uint32_t m = 128u) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
 }
 
 constexpr uint64_t kEvictFirst = 0x12F0000000000000ull;   // gallery: streamed once

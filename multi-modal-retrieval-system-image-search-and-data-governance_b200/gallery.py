@@ -4,7 +4,8 @@ The reference keeps its gallery as a pickle `{relpath: float[D]}` (code/search_i
 rebuilds an `np.array` -> `torch.tensor [N, D]` per class (`construct_dataset`, :167-182) and
 uploads the WHOLE matrix on every score call (`features.cuda()`, :107).  Here the matrix is
 uploaded once into HBM, row-major, rows 16-byte aligned (D padded with zeros to a multiple of 8),
-in fp32 (exact mode) or bf16 (tensor-core mode), and stays resident across calls.
+in fp32 (exact mode), bf16 (tensor-core mode) or per-row-scaled int8 (compact mode), and stays resident
+across calls.
 """
 from __future__ import annotations
 
@@ -21,11 +22,19 @@ def _pad_dim(d: int) -> int:
     return (d + 7) // 8 * 8
 
 
+def _pad_dim_i8(d: int) -> int:
+    return (d + 15) // 16 * 16
+
+
 class DeviceGallery:
     """[N, D] embedding matrix resident on one B200.
 
     mode "fp32": values kept as given (exact mode: scores within 1e-5 of the torch CPU path).
     mode "bf16": values rounded to bf16 -- that bf16 tensor IS the gallery (BASELINE.md section 5).
+    mode "int8": each row quantised on the device to int8 codes with one fp32 scale (include/mmrs_b200.h,
+    "int8 galleries"): `data` is int8 [N, padded_dim + 16], codes [padded_dim] (padded_dim = D rounded up to
+    16) then the scale's 16-byte tail -- 784 bytes per row at D = 768 instead of 1536.  Scores are an exact
+    function of the codes; a row holding a NaN or an infinity raises ValueError.  Never chosen by default.
     `row_offset` is the global index of row 0 when this is one shard of a larger gallery.
     """
 
@@ -37,8 +46,8 @@ class DeviceGallery:
             raise TypeError("features must be a 2-D torch.Tensor / numpy array [N, D]")
         if mode is None:
             mode = "bf16" if features.dtype == torch.bfloat16 else "fp32"
-        if mode not in ("fp32", "bf16"):
-            raise ValueError("mode must be 'fp32' or 'bf16'")
+        if mode not in ("fp32", "bf16", "int8"):
+            raise ValueError("mode must be 'fp32', 'bf16' or 'int8'")
         if device is None:
             device = features.device if features.is_cuda else torch.device("cuda", torch.cuda.current_device() if torch.cuda.is_available() else 0)
         device = torch.device(device)
@@ -50,6 +59,12 @@ class DeviceGallery:
             raise ValueError("gallery must have at least one row and one column")
         self.row_offset = int(row_offset)
         self.paths = list(paths) if paths is not None else None
+        self._workspaces: dict = {}
+        self._split = None
+        if mode == "int8":
+            self.padded_dim = _pad_dim_i8(self.dim)
+            self.data = self._quantize(features.detach(), device)
+            return
         dt = torch.bfloat16 if mode == "bf16" else torch.float32
         dp = _pad_dim(self.dim)
         src = features.detach()
@@ -67,10 +82,36 @@ class DeviceGallery:
         self._workspaces: dict = {}
         self._split = None
 
+    def _quantize(self, src: torch.Tensor, device: torch.device) -> torch.Tensor:
+        """int8 rows [N, padded_dim + 16] quantised on the device (mmrs_quantize_rows_i8); host input goes up
+        in fp32 (bf16 input as bf16) chunks of at most 256 MB."""
+        data = torch.empty((self.n_rows, self.padded_dim + 16), dtype=torch.int8, device=device)
+        sdt = torch.bfloat16 if src.dtype == torch.bfloat16 else torch.float32
+        code = _cabi.DTYPE_BF16 if sdt == torch.bfloat16 else _cabi.DTYPE_F32
+        step = max(1, (256 << 20) // max(1, self.dim * 4))
+        with torch.cuda.device(device):
+            stream = int(torch.cuda.current_stream(device).cuda_stream)
+            for lo in range(0, self.n_rows, step):
+                blk = src[lo:lo + step].to(device=device, dtype=sdt)
+                if blk.stride(1) != 1:
+                    blk = blk.contiguous()
+                _cabi.check(_cabi.lib.mmrs_quantize_rows_i8(blk.data_ptr(), code, blk.shape[0], self.dim, blk.stride(0),
+                                                            data[lo].data_ptr(), data.stride(0), stream))
+        return data
+
     # -- C-ABI views ---------------------------------------------------------------------------
     @property
     def dtype_code(self) -> int:
+        if self.mode == "int8":
+            return _cabi.DTYPE_I8
         return _cabi.DTYPE_BF16 if self.mode == "bf16" else _cabi.DTYPE_F32
+
+    def int8_codes_scales(self):
+        """int8 mode: (codes int8 [N, D], scales fp32 [N]) -- views of the resident rows."""
+        if self.mode != "int8":
+            raise ValueError("codes and scales exist for int8 galleries only")
+        scales = self.data[:, self.padded_dim:self.padded_dim + 4].contiguous().view(torch.float32).reshape(-1)
+        return self.data[:, :self.dim], scales
 
     @property
     def nbytes(self) -> int:
