@@ -18,7 +18,7 @@ LIB_DIR = PKG_DIR / "lib"
 LIB_PATH = LIB_DIR / "libmmrs_b200.so"
 SOURCES = ["api.cu", "scan_gemv.cu", "scan_mma.cu", "select.cu", "selfjoin.cu", "selfjoin_mma.cu", "range.cu",
            "dedup_resolve.cu"]
-HEADERS = ["common.cuh", "plan.h", "tcgen05_utils.cuh"]
+HEADERS = ["common.cuh", "host.h", "plan.h", "tcgen05_utils.cuh"]
 ARCH_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

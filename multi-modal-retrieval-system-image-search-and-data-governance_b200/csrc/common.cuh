@@ -10,7 +10,7 @@
 namespace mmrs {
 
 // Every scan kernel walks the gallery in row tiles of this many rows; the phase
-// schedule (api.cu) is expressed in tiles.
+// schedule (plan.h) is expressed in tiles.
 constexpr int kTileRows = 128;
 
 // Status bits a kernel can raise in the device-side flag word.
@@ -240,7 +240,7 @@ struct SelectParams {
   int32_t pad_short;
 };
 
-// launchers (defined in the .cu files, called from api.cu)
+// launchers called from another file than the one that defines them
 // Fused all-gather bookkeeping done by block 0 of the prep kernel (the first kernel of a call):
 // bump the slot's epoch and wait until every rank has acknowledged the previous one.
 struct GatherPrologue {
@@ -258,8 +258,6 @@ constexpr int kPrepKernelParams = 12;
 const void* select_kernel_handle();
 cudaError_t launch_gather_wait(const uint32_t* my_flags, int32_t world, const uint32_t* epoch, int32_t* status,
                                uint64_t timeout_ns, cudaStream_t stream);
-cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t dim, int64_t ld, float* out_min_max,
-                                  int sm_count, cudaStream_t stream);
 cudaError_t launch_scan_gemv(const ScanParams& p, int32_t dtype, int mode, int sm_count,
                              cudaStream_t stream);
 cudaError_t launch_quantize_rows_i8(const void* src, int32_t src_dtype, int64_t n_rows, int32_t dim, int64_t ld_src,
@@ -271,5 +269,26 @@ cudaError_t launch_pack_row_filter(const uint8_t* allowed, int64_t n_rows, uint3
 cudaError_t launch_pack_keys(const float* values, const int64_t* indices, int32_t n_lists,
                              int32_t n_queries, int32_t k_in, uint64_t* cand, int32_t cap,
                              cudaStream_t stream);
+// K2.  q_bf16 is the prepared [n_q_padded, ldq] bf16 query matrix; handles up to 256 queries.
+// g_plane_rows: rows between two planes of a bf16x3 gallery (the full gallery's n_rows).
+// i8: an int8 gallery with the prepared int8 query rows in q_bf16.
+cudaError_t launch_scan_mma(const ScanParams& p, const __nv_bfloat16* q_bf16, int32_t n_q_padded,
+                            int mode, int32_t* flags, int sm_count, cudaStream_t stream, int split,
+                            int64_t g_plane_rows, bool i8 = false);
+int scan_mma_max_queries();
+int scan_mma_split_max_queries();
+cudaError_t launch_split_bf16x3(const float* src, int64_t n_rows, int32_t dim, int64_t ld_src, __nv_bfloat16* dst,
+                                int64_t ld_dst, int sm_count, cudaStream_t stream);
+// range search finalize (range.cu)
+int64_t range_chunks(int64_t n_words);
+cudaError_t launch_range_mark_prefix(const uint64_t* cand, int64_t cap, const uint32_t* cnt, int32_t n_queries,
+                                     uint32_t* bitmap, uint32_t* word_base, uint32_t* chunk_sum, int64_t* total,
+                                     int sm_count, cudaStream_t stream);
+cudaError_t launch_range_scatter(const uint64_t* cand, int64_t cap, const uint32_t* cnt, int32_t n_queries,
+                                 const uint32_t* bitmap, const uint32_t* word_base, const int64_t* out_off,
+                                 int64_t index_offset, float* values, int64_t* indices, int sm_count,
+                                 cudaStream_t stream);
+// lexicographic sort of [n_pairs, 2] row pairs (selfjoin.cu); scratch: mmrs_sort_pairs_workspace_bytes(n_pairs)
+cudaError_t launch_sort_pairs(int64_t* pairs, int64_t n_pairs, uint64_t* scratch, cudaStream_t stream);
 
 }  // namespace mmrs

@@ -1,5 +1,5 @@
 // dedup_resolve.cu -- the greedy first-keeper decision of tool/find_repeated_in_same_folder.py:76-95 on
-// the device (mmrs_resolve_duplicates in api.cu).
+// the device (mmrs_resolve_duplicates).
 //
 // The host walk visits the rows in `order`; a row with an already kept neighbour is a duplicate of the
 // earliest kept one, any other row is kept.  In rank space (rank[order[t]] = t) that is: a rank is KEPT iff
@@ -22,7 +22,7 @@
 // the turn early.  The lowest undecided rank has only decided lower neighbours, so every round decides at
 // least one rank or moves a cursor.  No thread ever waits for another: kernel boundaries and the warp's own
 // program order are the only ordering used.
-#include "common.cuh"
+#include "host.h"
 
 namespace mmrs {
 
@@ -220,32 +220,32 @@ __global__ void __launch_bounds__(kResolveThreads) resolve_map_back_kernel(const
   }
 }
 
-cudaError_t launch_resolve_rank(const int64_t* order, int64_t n_order, int64_t n_items, uint32_t* rank, int32_t* status,
-                                int sm_count, cudaStream_t stream) {
+static cudaError_t launch_resolve_rank(const int64_t* order, int64_t n_order, int64_t n_items, uint32_t* rank, int32_t* status,
+                                       int sm_count, cudaStream_t stream) {
   if (n_order < 1) return cudaSuccess;
   resolve_rank_kernel<<<resolve_grid(n_order, sm_count), kResolveThreads, 0, stream>>>(order, n_order, n_items, rank,
                                                                                           status);
   return cudaGetLastError();
 }
 
-cudaError_t launch_resolve_orient(const int64_t* pairs, int64_t n_pairs, int64_t n_items, const uint32_t* rank,
-                                  int64_t* edges, int32_t* status, int sm_count, cudaStream_t stream) {
+static cudaError_t launch_resolve_orient(const int64_t* pairs, int64_t n_pairs, int64_t n_items, const uint32_t* rank,
+                                         int64_t* edges, int32_t* status, int sm_count, cudaStream_t stream) {
   if (n_pairs < 1) return cudaSuccess;
   resolve_orient_kernel<<<resolve_grid(n_pairs, sm_count), kResolveThreads, 0, stream>>>(pairs, n_pairs, n_items, rank,
                                                                                             edges, status);
   return cudaGetLastError();
 }
 
-cudaError_t launch_resolve_offsets(const int64_t* edges, int64_t n_edges, int64_t n_order, int64_t* off, int64_t* cursor,
-                                   int sm_count, cudaStream_t stream) {
+static cudaError_t launch_resolve_offsets(const int64_t* edges, int64_t n_edges, int64_t n_order, int64_t* off, int64_t* cursor,
+                                          int sm_count, cudaStream_t stream) {
   resolve_offsets_kernel<<<resolve_grid(n_order + 1, sm_count), kResolveThreads, 0, stream>>>(edges, n_edges, n_order,
                                                                                                  off, cursor);
   return cudaGetLastError();
 }
 
-cudaError_t launch_resolve_round(const int32_t* wl_in, const uint32_t* cnt_in, int64_t n_first, int64_t n_bound,
-                                 int32_t* wl_out, uint32_t* cnt_out, const int64_t* off, const int64_t* edges,
-                                 int64_t* cursor, int32_t* res, int sm_count, cudaStream_t stream) {
+static cudaError_t launch_resolve_round(const int32_t* wl_in, const uint32_t* cnt_in, int64_t n_first, int64_t n_bound,
+                                        int32_t* wl_out, uint32_t* cnt_out, const int64_t* off, const int64_t* edges,
+                                        int64_t* cursor, int32_t* res, int sm_count, cudaStream_t stream) {
   cudaError_t e = cudaMemsetAsync(cnt_out, 0, sizeof(uint32_t), stream);
   if (e != cudaSuccess || n_bound < 1) return e;
   resolve_round_kernel<<<resolve_grid(n_bound, sm_count), kResolveThreads, 0, stream>>>(wl_in, cnt_in, n_first, wl_out,
@@ -254,9 +254,9 @@ cudaError_t launch_resolve_round(const int32_t* wl_in, const uint32_t* cnt_in, i
   return cudaGetLastError();
 }
 
-cudaError_t launch_resolve_tail(const int32_t* wl, const uint32_t* cnt, int64_t n_bound, uint32_t* range,
-                                const int64_t* off, const int64_t* edges, const int64_t* cursor, int32_t* res,
-                                int sm_count, cudaStream_t stream) {
+static cudaError_t launch_resolve_tail(const int32_t* wl, const uint32_t* cnt, int64_t n_bound, uint32_t* range,
+                                       const int64_t* off, const int64_t* edges, const int64_t* cursor, int32_t* res,
+                                       int sm_count, cudaStream_t stream) {
   cudaError_t e = cudaMemsetAsync(range, 0, 2 * sizeof(uint32_t), stream);
   if (e != cudaSuccess || n_bound < 1) return e;
   resolve_worklist_range_kernel<<<resolve_grid(n_bound, sm_count), kResolveThreads, 0, stream>>>(wl, cnt, range);
@@ -264,12 +264,123 @@ cudaError_t launch_resolve_tail(const int32_t* wl, const uint32_t* cnt, int64_t 
   return cudaGetLastError();
 }
 
-cudaError_t launch_resolve_map_back(const int64_t* order, int64_t n_order, int64_t n_items, const int32_t* res,
-                                    int64_t* rep, int sm_count, cudaStream_t stream) {
+static cudaError_t launch_resolve_map_back(const int64_t* order, int64_t n_order, int64_t n_items, const int32_t* res,
+                                           int64_t* rep, int sm_count, cudaStream_t stream) {
   if (n_order < 1) return cudaSuccess;
   resolve_map_back_kernel<<<resolve_grid(n_order, sm_count), kResolveThreads, 0, stream>>>(order, n_order, n_items, res,
                                                                                               rep);
   return cudaGetLastError();
 }
 
+// ---- host side -------------------------------------------------------------------------------------
+// The workspace: a 256-byte header, then the rank, edge, CSR, decision and worklist arrays of the kernels above.
+struct ResolveWorkspace {
+  int32_t* header;         // [0] status bits, [1] [2] worklist counters, [4] [5] worklist rank range
+  uint32_t* rank;          // [n_items] rank of each row, 0xffffffff = not in the order
+  int64_t* edges;          // [n_pairs, 2] oriented (high rank, low rank), sorted in place
+  uint64_t* sort;          // mmrs_sort_pairs_workspace_bytes(n_pairs)
+  int64_t* off;            // [n_order + 1] first edge of each rank
+  int64_t* cursor;         // [n_order] next edge each undecided rank looks at
+  int32_t* res;            // [n_order] -1 undecided, r kept, else the representative's rank
+  int32_t* wl[2];          // [n_order] each: worklists of undecided ranks, ping-pong
+};
+
+static ResolveWorkspace carve_resolve(Carver& c, int64_t n_items, int64_t n_order, int64_t n_pairs) {
+  ResolveWorkspace r{};
+  const size_t items = static_cast<size_t>(n_items), ord = static_cast<size_t>(n_order),
+               pairs = static_cast<size_t>(n_pairs);
+  r.header = c.take<int32_t>(256);
+  r.rank = c.take<uint32_t>(items * sizeof(uint32_t));
+  r.edges = c.take<int64_t>(pairs * 2 * sizeof(int64_t));
+  r.sort = c.take<uint64_t>(mmrs_sort_pairs_workspace_bytes(n_pairs));
+  r.off = c.take<int64_t>((ord + 1) * sizeof(int64_t));
+  r.cursor = c.take<int64_t>(ord * sizeof(int64_t));
+  r.res = c.take<int32_t>(ord * sizeof(int32_t));
+  r.wl[0] = c.take<int32_t>(ord * sizeof(int32_t));
+  r.wl[1] = c.take<int32_t>(ord * sizeof(int32_t));
+  return r;
+}
+
+// The host reads the worklist count once per batch of rounds.  A batch that decides fewer than
+// kResolveTailBelow rows per round hands the rest to the one-warp tail: a round costs a launch and a pass
+// over the whole worklist, and that little progress means long dependent chains (a path in walk order
+// decides about one rank per round), which the tail walks in one ascending sweep.
+constexpr int kResolveBatch = 4;
+constexpr int64_t kResolveTailBelow = 2048;
+
 }  // namespace mmrs
+
+using namespace mmrs;
+
+extern "C" {
+
+size_t mmrs_resolve_duplicates_workspace_bytes(int64_t n_items, int64_t n_order, int64_t n_pairs) {
+  if (n_items < 0 || n_order < 0 || n_pairs < 0) return 0;
+  Carver c(nullptr);
+  carve_resolve(c, n_items, n_order, n_pairs);
+  return c.off;
+}
+
+int mmrs_resolve_duplicates(const int64_t* d_pairs, int64_t n_pairs, const int64_t* d_order, int64_t n_order,
+                            int64_t n_items, int64_t* d_representative, int64_t* h_rounds, void* d_workspace,
+                            size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_items < 0 || n_items > 0x7fffffffll)
+    return fail(MMRS_ERR_ARG, "n = %lld rows: the resolve takes 0 <= n < 2^31", (long long)n_items);
+  if (n_order < 0 || n_order > 0x7fffffffll)
+    return fail(MMRS_ERR_ARG, "order of %lld ids: at most 2^31 - 1", (long long)n_order);
+  if (!d_order && n_order > n_items) return fail(MMRS_ERR_ARG, "a null order stands for the ids 0..n_order-1 <= n");
+  if (n_pairs < 0 || (n_pairs > 0 && !d_pairs) || (n_items > 0 && !d_representative))
+    return fail(MMRS_ERR_ARG, "bad pair / output arguments");
+  rc = check_workspace(d_workspace, workspace_bytes, mmrs_resolve_duplicates_workspace_bytes(n_items, n_order, n_pairs));
+  if (rc != MMRS_OK) return rc;
+  int32_t* h = pinned_status();
+  if (!h) return fail(MMRS_ERR_CUDA, "cudaHostAlloc for the status word failed");
+  Carver c(d_workspace);
+  const ResolveWorkspace w = carve_resolve(c, n_items, n_order, n_pairs);
+  uint32_t* cnt = reinterpret_cast<uint32_t*>(w.header + 1);
+  uint32_t* range = reinterpret_cast<uint32_t*>(w.header + 4);
+  MMRS_CUDA(cudaMemsetAsync(w.header, 0, 256, stream));
+  MMRS_CUDA(cudaMemsetAsync(w.rank, 0xff, static_cast<size_t>(n_items) * sizeof(uint32_t), stream));
+  MMRS_CUDA(cudaMemsetAsync(d_representative, 0xff, static_cast<size_t>(n_items) * sizeof(int64_t), stream));   // -1
+  MMRS_CUDA(cudaMemsetAsync(w.res, 0xff, static_cast<size_t>(n_order) * sizeof(int32_t), stream));             // undecided
+  MMRS_LAUNCH(launch_resolve_rank(d_order, n_order, n_items, w.rank, w.header, dev.sm_count, stream));
+  MMRS_LAUNCH(launch_resolve_orient(d_pairs, n_pairs, n_items, w.rank, w.edges, w.header, dev.sm_count, stream));
+  MMRS_LAUNCH(launch_sort_pairs(w.edges, n_pairs, w.sort, stream));
+  MMRS_LAUNCH(launch_resolve_offsets(w.edges, n_pairs, n_order, w.off, w.cursor, dev.sm_count, stream));
+  // round k reads worklist (k + 1) & 1 (round 0: every rank) and writes worklist k & 1
+  int64_t known = n_order, rounds = 0, tail = 0;
+  while (known > 0) {
+    for (int b = 0; b < kResolveBatch; ++b, ++rounds) {
+      const int o = static_cast<int>(rounds & 1), i = o ^ 1;
+      MMRS_LAUNCH(launch_resolve_round(rounds ? w.wl[i] : nullptr, cnt + i, n_order, known, w.wl[o], cnt + o, w.off,
+                                       w.edges, w.cursor, w.res, dev.sm_count, stream));
+    }
+    MMRS_CUDA(cudaMemcpyAsync(h, w.header, 8 * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    MMRS_CUDA(cudaStreamSynchronize(stream));
+    if (h[0]) break;
+    const int last = static_cast<int>((rounds - 1) & 1);
+    const int64_t left = static_cast<uint32_t>(h[1 + last]);
+    const int64_t decided = known - left;
+    known = left;
+    if (left > 0 && decided < kResolveBatch * kResolveTailBelow) {
+      MMRS_LAUNCH(launch_resolve_tail(w.wl[last], cnt + last, left, range, w.off, w.edges, w.cursor, w.res,
+                                      dev.sm_count, stream));
+      tail = left;
+      break;
+    }
+  }
+  MMRS_LAUNCH(launch_resolve_map_back(d_order, n_order, n_items, w.res, d_representative, dev.sm_count, stream));
+  MMRS_CUDA(cudaMemcpyAsync(h, w.header, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  if (h_rounds) { h_rounds[0] = rounds; h_rounds[1] = tail; }
+  if (h[0] & kResolvePairRange) return fail(MMRS_ERR_ARG, "a pair id is outside [0, %lld)", (long long)n_items);
+  if (h[0] & kResolveOrderRange) return fail(MMRS_ERR_ARG, "an order id is outside [0, %lld)", (long long)n_items);
+  if (h[0] & kResolveOrderRepeat) return fail(MMRS_ERR_ARG, "an id appears more than once in the order");
+  return MMRS_OK;
+}
+
+}  // extern "C"

@@ -596,7 +596,6 @@ int scan_mma_max_queries() {
   const int c = e ? atoi(e) : kMaxQChunks;
   return kMaxQ * (c >= 1 && c <= kMaxQChunks ? c : kMaxQChunks);
 }
-bool scan_mma_available() { return true; }
 
 // The int8 launches pick among the same variants as the bf16 ones.
 template <int EPI, bool PAIR, typename Go>

@@ -9,9 +9,12 @@
 // Exact mode: fp32 FFMA, k ascending, one accumulator per pair -- the pair set does not depend
 // on tile shape or launch geometry.  selfjoin_mma.cu is the tensor-core prefilter whose survivors are
 // re-scored with exactly this arithmetic; this kernel serves small inputs and as its cross-check.
+//
+// The file ends with the extern "C" entry points of its kernels: the exact self-join, the pair sort, the
+// row-norm range and the threshold sweeps.
 #include <type_traits>
 
-#include "common.cuh"
+#include "host.h"
 
 namespace mmrs {
 
@@ -112,10 +115,10 @@ __global__ void __launch_bounds__(kSjThreads) selfjoin_f32_kernel(const SelfJoin
   }
 }
 
-cudaError_t launch_selfjoin_f32(const float* emb, int64_t n_rows, int32_t dim, int64_t ld,
-                                float threshold, int64_t row_begin, int64_t row_end,
-                                int64_t* out_pairs, int64_t capacity, int64_t* out_count,
-                                int sm_count, cudaStream_t stream) {
+static cudaError_t launch_selfjoin_f32(const float* emb, int64_t n_rows, int32_t dim, int64_t ld,
+                                       float threshold, int64_t row_begin, int64_t row_end,
+                                       int64_t* out_pairs, int64_t capacity, int64_t* out_count,
+                                       int sm_count, cudaStream_t stream) {
   SelfJoinParams p{};
   p.emb = emb; p.n_rows = n_rows; p.ld = ld; p.dim = dim; p.threshold = threshold;
   p.nb = (n_rows + kSjTile - 1) / kSjTile;
@@ -384,16 +387,6 @@ static cudaError_t launch_threshold_sweep_t(const S* pos, int64_t n_pos, const S
   sweep_suffix_kernel<<<1, 32, 0, stream>>>(hist_ws, 1, n_thr, out_counts, nullptr);
   return cudaGetLastError();
 }
-cudaError_t launch_threshold_sweep(const float* pos, int64_t n_pos, const float* neg, int64_t n_neg,
-                                   const double* thr, int32_t n_thr, int64_t* out_counts,
-                                   unsigned long long* hist_ws, int sm_count, cudaStream_t stream) {
-  return launch_threshold_sweep_t<float>(pos, n_pos, neg, n_neg, thr, n_thr, out_counts, hist_ws, sm_count, stream);
-}
-cudaError_t launch_threshold_sweep_f64(const double* pos, int64_t n_pos, const double* neg, int64_t n_neg,
-                                       const double* thr, int32_t n_thr, int64_t* out_counts,
-                                       unsigned long long* hist_ws, int sm_count, cudaStream_t stream) {
-  return launch_threshold_sweep_t<double>(pos, n_pos, neg, n_neg, thr, n_thr, out_counts, hist_ws, sm_count, stream);
-}
 
 // Shared memory of the labeled histogram: per query its grid, 1 / step, two histograms, its label and bin mode.
 static size_t sweep_hist_query_bytes(int32_t n_thr) {
@@ -442,10 +435,10 @@ static cudaError_t launch_sweep_labeled(const float* scores, int64_t ld, int32_t
   return cudaGetLastError();
 }
 
-cudaError_t launch_threshold_sweep_labeled(const float* scores, const int64_t* targets, int64_t label, int64_t n,
-                                           int32_t n_thr, int32_t grid_f32, double* thr_out, int64_t* out_counts,
-                                           unsigned long long* hist_ws, uint32_t* mm_ws, int sm_count,
-                                           cudaStream_t stream) {
+static cudaError_t launch_threshold_sweep_labeled(const float* scores, const int64_t* targets, int64_t label, int64_t n,
+                                                  int32_t n_thr, int32_t grid_f32, double* thr_out, int64_t* out_counts,
+                                                  unsigned long long* hist_ws, uint32_t* mm_ws, int sm_count,
+                                                  cudaStream_t stream) {
   if (n_thr < 1 || n_thr > kSweepMaxT || n < 1) return cudaErrorInvalidValue;
   cudaError_t e = cudaMemsetAsync(mm_ws, 0xff, sizeof(uint32_t), stream);           // min <- 0xffffffff
   if (e != cudaSuccess) return e;
@@ -457,16 +450,11 @@ cudaError_t launch_threshold_sweep_labeled(const float* scores, const int64_t* t
                               out_counts, nullptr, hist_ws, sm_count, stream);
 }
 
-cudaError_t launch_score_range_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n, const uint32_t* filt,
-                                       uint32_t* range, int sm_count, cudaStream_t stream) {
-  return launch_score_range(scores, ld, n_q, n, filt, range, sm_count, stream);
-}
-
-cudaError_t launch_threshold_sweep_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n,
-                                           const int32_t* row_labels, const int32_t* query_labels, const uint32_t* filt,
-                                           const uint32_t* range, int32_t n_thr, int32_t grid_f32, double* thr_out,
-                                           int64_t* out_counts, int64_t* out_n_pos, unsigned long long* hist_ws,
-                                           int sm_count, cudaStream_t stream) {
+static cudaError_t launch_threshold_sweep_batched(const float* scores, int64_t ld, int32_t n_q, int64_t n,
+                                                  const int32_t* row_labels, const int32_t* query_labels, const uint32_t* filt,
+                                                  const uint32_t* range, int32_t n_thr, int32_t grid_f32, double* thr_out,
+                                                  int64_t* out_counts, int64_t* out_n_pos, unsigned long long* hist_ws,
+                                                  int sm_count, cudaStream_t stream) {
   if (n_thr < 1 || n_thr > kSweepMaxT || n < 1 || n_q < 1) return cudaErrorInvalidValue;
   return launch_sweep_labeled(scores, ld, n_q, n, RowLabelsSource{row_labels, query_labels}, filt, range, n_thr, grid_f32,
                               thr_out, out_counts, out_n_pos, hist_ws, sm_count, stream);
@@ -572,8 +560,8 @@ __global__ void __launch_bounds__(256) row_norm_range_kernel(const float* __rest
   }
   if (lane == 0 && lo != 0xffffffffu) { atomicMin(mm, lo); atomicMax(mm + 1, hi); }
 }
-cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t dim, int64_t ld, float* out_min_max,
-                                  int sm_count, cudaStream_t stream) {
+static cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t dim, int64_t ld, float* out_min_max,
+                                         int sm_count, cudaStream_t stream) {
   uint32_t* mm = reinterpret_cast<uint32_t*>(out_min_max);
   cudaError_t e = cudaMemsetAsync(mm, 0xff, sizeof(uint32_t), stream);
   if (e != cudaSuccess) return e;
@@ -585,4 +573,201 @@ cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t dim, i
   return cudaGetLastError();
 }
 
+
+// ---- host side: the entry points --------------------------------------------------------------------------------
+// The sweeps' histograms: two [n_thresholds + 1] counter arrays per query.  The labeled sweep keeps the bits of the
+// score range it bins in front of them.
+struct SweepWorkspace {
+  uint32_t* range;             // [2] min, max score (order-preserving bits); labeled sweep only
+  unsigned long long* hist;    // [n_queries, 2, n_thresholds + 1]
+};
+
+static SweepWorkspace carve_sweep(Carver& c, int32_t n_queries, int32_t n_thresholds, bool with_range) {
+  SweepWorkspace w{};
+  if (with_range) w.range = c.take<uint32_t>(2 * sizeof(uint32_t));
+  w.hist = c.take<unsigned long long>(sizeof(unsigned long long) * 2 * (static_cast<size_t>(n_thresholds) + 1) *
+                                      n_queries);
+  return w;
+}
+
+// mmrs_threshold_sweep (fp32 scores) and mmrs_threshold_sweep_f64
+template <typename S>
+static int threshold_sweep(const S* d_pos, int64_t n_pos, const S* d_neg, int64_t n_neg, const double* d_thresholds,
+                           int32_t n_thresholds, int64_t* d_out_counts, void* d_workspace, size_t workspace_bytes,
+                           void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_thresholds < 1 || n_thresholds > 4096) return fail(MMRS_ERR_ARG, "n_thresholds must be in [1, 4096]");
+  if (n_pos < 0 || n_neg < 0 || (n_pos > 0 && !d_pos) || (n_neg > 0 && !d_neg) || !d_thresholds || !d_out_counts)
+    return fail(MMRS_ERR_ARG, "bad arguments");
+  rc = check_workspace(d_workspace, workspace_bytes, mmrs_threshold_sweep_workspace_bytes(n_thresholds),
+                       /*aligned=*/false);
+  if (rc != MMRS_OK) return rc;
+  Carver c(d_workspace);
+  const SweepWorkspace w = carve_sweep(c, 1, n_thresholds, false);
+  MMRS_LAUNCH(launch_threshold_sweep_t<S>(d_pos, n_pos, d_neg, n_neg, d_thresholds, n_thresholds, d_out_counts, w.hist,
+                                          dev.sm_count, stream));
+  return MMRS_OK;
+}
+
 }  // namespace mmrs
+
+using namespace mmrs;
+
+extern "C" {
+
+size_t mmrs_selfjoin_workspace_bytes(int64_t n_rows, int32_t dim, int32_t dtype) {
+  (void)n_rows; (void)dim; (void)dtype;
+  return 0;   // the exact-mode join keeps everything in registers / shared memory: d_workspace may be NULL
+}
+
+int mmrs_selfjoin_pairs(const void* d_emb, int64_t n_rows, int32_t dim, int64_t ld_emb,
+                        int32_t dtype, float threshold, int64_t row_begin, int64_t row_end,
+                        int64_t* d_out_pairs, int64_t capacity, int64_t* d_out_count,
+                        void* d_workspace, size_t workspace_bytes, void* stream_) {
+  (void)d_workspace; (void)workspace_bytes;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  rc = check_matrix(d_emb, n_rows, dim, ld_emb, dtype, "embeddings");
+  if (rc != MMRS_OK) return rc;
+  if (dtype != MMRS_DTYPE_F32) return fail(MMRS_ERR_ARG, "self-join exact mode takes fp32 embeddings");
+  if (dim % 8 != 0) return fail(MMRS_ERR_ARG, "self-join dim must be a multiple of 8 (pad with zeros)");
+  if (row_begin < 0 || row_end > n_rows || row_begin > row_end)
+    return fail(MMRS_ERR_ARG, "row range [%lld, %lld) invalid", (long long)row_begin, (long long)row_end);
+  if (capacity < 0 || (capacity > 0 && !d_out_pairs) || !d_out_count)
+    return fail(MMRS_ERR_ARG, "bad output arguments");
+  MMRS_CUDA(cudaMemsetAsync(d_out_count, 0, sizeof(int64_t), stream));
+  MMRS_LAUNCH(launch_selfjoin_f32(static_cast<const float*>(d_emb), n_rows, dim, ld_emb, threshold,
+                                row_begin, row_end, d_out_pairs, capacity, d_out_count,
+                                dev.sm_count, stream));
+  int32_t* h = pinned_status();
+  if (!h) return fail(MMRS_ERR_CUDA, "cudaHostAlloc for the status word failed");
+  int64_t* h64 = reinterpret_cast<int64_t*>(h);
+  MMRS_CUDA(cudaMemcpyAsync(h64, d_out_count, sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  if (h64[0] > capacity)
+    return fail(MMRS_ERR_CAPACITY, "%lld pairs found, capacity %lld", (long long)h64[0], (long long)capacity);
+  return MMRS_OK;
+}
+
+size_t mmrs_sort_pairs_workspace_bytes(int64_t n_pairs) {
+  if (n_pairs < 1) n_pairs = 1;
+  int64_t m = 1;
+  while (m < n_pairs) m <<= 1;
+  return static_cast<size_t>(m) * sizeof(uint64_t);
+}
+
+int mmrs_sort_pairs(int64_t* d_pairs, int64_t n_pairs, void* d_workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_pairs < 0 || (n_pairs > 0 && !d_pairs)) return fail(MMRS_ERR_ARG, "bad arguments");
+  if (n_pairs < 2) return MMRS_OK;
+  rc = check_workspace(d_workspace, workspace_bytes, mmrs_sort_pairs_workspace_bytes(n_pairs), /*aligned=*/false);
+  if (rc != MMRS_OK) return rc;
+  MMRS_LAUNCH(launch_sort_pairs(d_pairs, n_pairs, static_cast<uint64_t*>(d_workspace), stream));
+  return MMRS_OK;
+}
+
+int mmrs_row_norm_range(const float* d_emb, int64_t n_rows, int32_t dim, int64_t ld, float* d_out_min_max, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (!d_emb || !d_out_min_max || n_rows < 1 || dim < 1 || ld < dim) return fail(MMRS_ERR_ARG, "bad arguments");
+  MMRS_LAUNCH(launch_row_norm_range(d_emb, n_rows, dim, ld, d_out_min_max, dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+size_t mmrs_threshold_sweep_workspace_bytes(int32_t n_thresholds) {
+  if (n_thresholds < 1) n_thresholds = 1;
+  Carver c(nullptr);
+  carve_sweep(c, 1, n_thresholds, false);
+  return c.off;
+}
+
+int mmrs_threshold_sweep(const float* d_pos, int64_t n_pos, const float* d_neg, int64_t n_neg,
+                         const double* d_thresholds, int32_t n_thresholds, int64_t* d_out_counts,
+                         void* d_workspace, size_t workspace_bytes, void* stream) {
+  return threshold_sweep(d_pos, n_pos, d_neg, n_neg, d_thresholds, n_thresholds, d_out_counts, d_workspace,
+                         workspace_bytes, stream);
+}
+
+int mmrs_threshold_sweep_f64(const double* d_pos, int64_t n_pos, const double* d_neg, int64_t n_neg,
+                             const double* d_thresholds, int32_t n_thresholds, int64_t* d_out_counts,
+                             void* d_workspace, size_t workspace_bytes, void* stream) {
+  return threshold_sweep(d_pos, n_pos, d_neg, n_neg, d_thresholds, n_thresholds, d_out_counts, d_workspace,
+                         workspace_bytes, stream);
+}
+
+int mmrs_threshold_sweep_labeled(const float* d_scores, const int64_t* d_targets, int64_t label, int64_t n,
+                                 int32_t n_thresholds, int32_t grid_f32, double* d_out_thresholds, int64_t* d_out_counts,
+                                 void* d_workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_thresholds < 1 || n_thresholds > 4096) return fail(MMRS_ERR_ARG, "n_thresholds must be in [1, 4096]");
+  if (n < 1 || !d_scores || !d_targets || !d_out_thresholds || !d_out_counts) return fail(MMRS_ERR_ARG, "bad arguments");
+  Carver sizing(nullptr);
+  carve_sweep(sizing, 1, n_thresholds, true);   // mmrs_threshold_sweep_workspace_bytes + 256
+  rc = check_workspace(d_workspace, workspace_bytes, sizing.off, /*aligned=*/false);
+  if (rc != MMRS_OK) return rc;
+  Carver c(d_workspace);
+  const SweepWorkspace w = carve_sweep(c, 1, n_thresholds, true);
+  MMRS_LAUNCH(launch_threshold_sweep_labeled(d_scores, d_targets, label, n, n_thresholds, grid_f32, d_out_thresholds,
+                                             d_out_counts, w.hist, w.range, dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+size_t mmrs_threshold_sweep_batched_workspace_bytes(int32_t n_queries, int32_t n_thresholds) {
+  if (n_queries < 1) n_queries = 1;
+  if (n_thresholds < 1) n_thresholds = 1;
+  Carver c(nullptr);
+  carve_sweep(c, n_queries, n_thresholds, false);
+  return c.off;
+}
+
+int mmrs_score_range_batched(const float* d_scores, int64_t ld_scores, int32_t n_queries, int64_t n_rows,
+                             const uint32_t* d_row_filter, uint32_t* d_range, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_queries == 0 || n_rows == 0) return MMRS_OK;
+  if (n_queries < 0 || n_rows < 0 || ld_scores < n_rows || !d_scores || !d_range) return fail(MMRS_ERR_ARG, "bad arguments");
+  MMRS_LAUNCH(launch_score_range(d_scores, ld_scores, n_queries, n_rows, d_row_filter, d_range, dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+int mmrs_threshold_sweep_batched(const float* d_scores, int64_t ld_scores, int32_t n_queries, int64_t n_rows,
+                                 const int32_t* d_row_labels, const int32_t* d_query_labels,
+                                 const uint32_t* d_row_filter, const uint32_t* d_range, int32_t n_thresholds,
+                                 int32_t grid_f32, double* d_out_thresholds, int64_t* d_out_counts,
+                                 int64_t* d_out_n_pos, void* d_workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (n_thresholds < 1 || n_thresholds > 4096) return fail(MMRS_ERR_ARG, "n_thresholds must be in [1, 4096]");
+  if (n_queries == 0) return MMRS_OK;
+  if (n_queries < 0 || n_rows < 1 || ld_scores < n_rows || !d_scores || !d_row_labels || !d_query_labels || !d_range ||
+      !d_out_thresholds || !d_out_counts || !d_out_n_pos)
+    return fail(MMRS_ERR_ARG, "bad arguments");
+  rc = check_workspace(d_workspace, workspace_bytes, mmrs_threshold_sweep_batched_workspace_bytes(n_queries, n_thresholds),
+                       /*aligned=*/false);
+  if (rc != MMRS_OK) return rc;
+  Carver c(d_workspace);
+  const SweepWorkspace w = carve_sweep(c, n_queries, n_thresholds, false);
+  MMRS_LAUNCH(launch_threshold_sweep_batched(d_scores, ld_scores, n_queries, n_rows, d_row_labels, d_query_labels,
+                                             d_row_filter, d_range, n_thresholds, grid_f32, d_out_thresholds,
+                                             d_out_counts, d_out_n_pos, w.hist, dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+}  // extern "C"

@@ -24,6 +24,7 @@
 // multi-GPU run (work per panel grows linearly with its index, so cyclic dealing balances).
 #include <stdlib.h>
 
+#include "host.h"
 #include "tcgen05_utils.cuh"
 
 namespace mmrs {
@@ -296,15 +297,15 @@ __global__ void __launch_bounds__(256) selfjoin_recheck_kernel(const int64_t* __
 // ~0.1 s), but a long join runs against the board's power cap, where what counts is energy per
 // flop and the single-CTA kernel came out 5 % ahead (same-box A/B on one rank's share of C3:
 // 5.91 s vs 6.20-6.31 s, profiles/r01_selfjoin_ab.log).  So: pairs below ~0.12 s of estimated work.
-bool sjm_pair_mode(int64_t n_rows, int32_t dim, int32_t world) {
+static bool sjm_pair_mode(int64_t n_rows, int32_t dim, int32_t world) {
   if (const char* e = getenv("MMRS_SJ_PAIR")) return atoi(e) != 0;
   const double flops = static_cast<double>(dim) * static_cast<double>(n_rows) * static_cast<double>(n_rows) /
                        static_cast<double>(world > 0 ? world : 1);
   return flops < 1.44e14;
 }
 
-int64_t sjm_plan(int64_t n_rows, int32_t rank, int32_t world, bool pair, int64_t* h_panel_start, int32_t max_panels,
-                 int32_t* n_my_panels) {
+static int64_t sjm_plan(int64_t n_rows, int32_t rank, int32_t world, bool pair, int64_t* h_panel_start, int32_t max_panels,
+                        int32_t* n_my_panels) {
   const int64_t nbi = (n_rows + kSjmBM - 1) / kSjmBM, nbj = (n_rows + kSjmBN - 1) / kSjmBN;
   const int64_t n_panels = (nbj + kSjmPanel - 1) / kSjmPanel;
   int32_t m = 0;
@@ -322,16 +323,16 @@ int64_t sjm_plan(int64_t n_rows, int32_t rank, int32_t world, bool pair, int64_t
   return tiles;
 }
 
-int64_t sjm_max_panels(int64_t n_rows) {
+static int64_t sjm_max_panels(int64_t n_rows) {
   const int64_t nbj = (n_rows + kSjmBN - 1) / kSjmBN;
   return (nbj + kSjmPanel - 1) / kSjmPanel;
 }
 
-cudaError_t launch_selfjoin_mma(const __nv_bfloat16* emb16, int64_t n_rows, int32_t dim, int64_t ld16,
-                                float thr_lo, int32_t rank, int32_t world, bool pair, const int64_t* d_panel_start,
-                                int32_t n_my_panels, int64_t total_tiles, int64_t* cand, int64_t cand_cap,
-                                unsigned long long* cand_count, int32_t* flags, int sm_count,
-                                cudaStream_t stream) {
+static cudaError_t launch_selfjoin_mma(const __nv_bfloat16* emb16, int64_t n_rows, int32_t dim, int64_t ld16,
+                                       float thr_lo, int32_t rank, int32_t world, bool pair, const int64_t* d_panel_start,
+                                       int32_t n_my_panels, int64_t total_tiles, int64_t* cand, int64_t cand_cap,
+                                       unsigned long long* cand_count, int32_t* flags, int sm_count,
+                                       cudaStream_t stream) {
   if (total_tiles <= 0) return cudaSuccess;
   if (n_rows > 0x7fffffffll - kSjmBN) return cudaErrorInvalidValue;
   SjmParams p{};
@@ -370,13 +371,102 @@ cudaError_t launch_selfjoin_mma(const __nv_bfloat16* emb16, int64_t n_rows, int3
   return cudaLaunchKernelEx(&cfg, kernel, map_a, map_b, p, flags);
 }
 
-cudaError_t launch_selfjoin_recheck(const int64_t* cand, int64_t n_cand, const float* emb, int64_t ld, int32_t dim,
-                                    float threshold, int64_t* out_pairs, int64_t capacity,
-                                    unsigned long long* out_count, cudaStream_t stream) {
+static cudaError_t launch_selfjoin_recheck(const int64_t* cand, int64_t n_cand, const float* emb, int64_t ld, int32_t dim,
+                                           float threshold, int64_t* out_pairs, int64_t capacity,
+                                           unsigned long long* out_count, cudaStream_t stream) {
   if (n_cand <= 0) return cudaSuccess;
   selfjoin_recheck_kernel<<<static_cast<int>((n_cand + 255) / 256), 256, 0, stream>>>(
       cand, n_cand, emb, ld, dim, threshold, out_pairs, capacity, out_count);
   return cudaGetLastError();
 }
 
+
+// The workspace of mmrs_selfjoin_pairs_tc: the flag word, the two counts, the panel starts, the candidate pairs.
+struct SjmWorkspace {
+  int32_t* flags;
+  unsigned long long* counts;   // [0] pairs, [1] candidates
+  int64_t* panel_start;         // [max_panels + 1]
+  int64_t* cand;                // [cand_capacity, 2]
+};
+
+static SjmWorkspace carve_sjm(Carver& c, int64_t n_rows, int64_t cand_capacity) {
+  SjmWorkspace w;
+  w.flags = c.take<int32_t>(sizeof(int32_t));
+  w.counts = c.take<unsigned long long>(2 * sizeof(unsigned long long));
+  w.panel_start = c.take<int64_t>(static_cast<size_t>(sjm_max_panels(n_rows) + 1) * sizeof(int64_t));
+  w.cand = c.take<int64_t>(static_cast<size_t>(cand_capacity) * 2 * sizeof(int64_t));
+  return w;
+}
+
 }  // namespace mmrs
+
+using namespace mmrs;
+
+extern "C" {
+
+size_t mmrs_selfjoin_tc_workspace_bytes(int64_t n_rows, int64_t cand_capacity) {
+  if (n_rows < 1) n_rows = 1;
+  if (cand_capacity < 1) cand_capacity = 1;
+  Carver c(nullptr);
+  carve_sjm(c, n_rows, cand_capacity);
+  return c.off;
+}
+
+int mmrs_selfjoin_pairs_tc(const float* d_emb_f32, int64_t ld_f32, const void* d_emb_bf16, int64_t ld_bf16,
+                           int64_t n_rows, int32_t dim, float threshold, float margin, int32_t rank,
+                           int32_t world, int64_t* d_out_pairs, int64_t capacity, int64_t* d_out_count,
+                           int64_t cand_capacity, void* d_workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  rc = check_matrix(d_emb_f32, n_rows, dim, ld_f32, MMRS_DTYPE_F32, "fp32 embeddings");
+  if (rc != MMRS_OK) return rc;
+  rc = check_matrix(d_emb_bf16, n_rows, dim, ld_bf16, MMRS_DTYPE_BF16, "bf16 embeddings");
+  if (rc != MMRS_OK) return rc;
+  if (!(margin >= 0.f) || world < 1 || rank < 0 || rank >= world)
+    return fail(MMRS_ERR_ARG, "bad margin / rank / world");
+  if (capacity < 0 || cand_capacity < 1 || (capacity > 0 && !d_out_pairs) || !d_out_count)
+    return fail(MMRS_ERR_ARG, "bad output arguments");
+  rc = check_workspace(d_workspace, workspace_bytes, mmrs_selfjoin_tc_workspace_bytes(n_rows, cand_capacity));
+  if (rc != MMRS_OK) return rc;
+  Carver c(d_workspace);
+  const SjmWorkspace w = carve_sjm(c, n_rows, cand_capacity);
+  const int64_t max_panels = sjm_max_panels(n_rows);
+
+  std::vector<int64_t> h_panel(static_cast<size_t>(max_panels) + 1);
+  int32_t n_my = 0;
+  const bool pair = sjm_pair_mode(n_rows, dim, world);
+  const int64_t tiles = sjm_plan(n_rows, rank, world, pair, h_panel.data(), static_cast<int32_t>(max_panels), &n_my);
+  MMRS_CUDA(cudaMemsetAsync(w.flags, 0, 512, stream));   // the flag word and the counts: the first two 256-byte pieces
+  MMRS_CUDA(cudaMemcpyAsync(w.panel_start, h_panel.data(), static_cast<size_t>(n_my + 1) * sizeof(int64_t),
+                            cudaMemcpyHostToDevice, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));   // h_panel is pageable and goes out of scope
+  MMRS_LAUNCH(launch_selfjoin_mma(static_cast<const __nv_bfloat16*>(d_emb_bf16), n_rows, dim, ld_bf16,
+                                  threshold - margin, rank, world, pair, w.panel_start, n_my, tiles, w.cand,
+                                  cand_capacity, w.counts + 1, w.flags, dev.sm_count, stream));
+  int32_t* h = pinned_status();
+  if (!h) return fail(MMRS_ERR_CUDA, "cudaHostAlloc for the status word failed");
+  int64_t* h64 = reinterpret_cast<int64_t*>(h);      // 32 bytes: [0] pairs, [1] candidates, [2] flags
+  MMRS_CUDA(cudaMemcpyAsync(h64 + 1, w.counts + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaMemcpyAsync(h64 + 2, w.flags, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  if (h[4] & kFlagWatchdog) return fail(MMRS_ERR_INTERNAL, "self-join pipeline watchdog fired");
+  const int64_t n_cand = h64[1];
+  h64[0] = 0;
+  if (n_cand <= cand_capacity) {
+    MMRS_LAUNCH(launch_selfjoin_recheck(w.cand, n_cand, d_emb_f32, ld_f32, dim, threshold, d_out_pairs, capacity,
+                                        w.counts, stream));
+    MMRS_CUDA(cudaMemcpyAsync(h64, w.counts, sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+  }
+  MMRS_CUDA(cudaMemcpyAsync(d_out_count, w.counts, 2 * sizeof(int64_t), cudaMemcpyDeviceToDevice, stream));
+  MMRS_CUDA(cudaStreamSynchronize(stream));
+  if (n_cand > cand_capacity)
+    return fail(MMRS_ERR_CAPACITY, "%lld candidate pairs, candidate capacity %lld", (long long)n_cand,
+                (long long)cand_capacity);
+  if (h64[0] > capacity)
+    return fail(MMRS_ERR_CAPACITY, "%lld pairs found, capacity %lld", (long long)h64[0], (long long)capacity);
+  return MMRS_OK;
+}
+
+}  // extern "C"
