@@ -15,7 +15,7 @@
  *   mmrs_search_topk      code/search_image.py:107 + code/utils.py:17
  *                         `output.topk(k, 1, True, True)` fused, score matrix never stored
  *   mmrs_topk_merge       (new) merge of per-shard top-k after the all-gather
- *   mmrs_selfjoin_pairs(_tc)  tool/find_repeated_in_same_folder.py:76-95 /
+ *   mmrs_selfjoin_pairs(_tc, _stored)  tool/find_repeated_in_same_folder.py:76-95 /
  *                         tool/delete repeated.py:127-135 (pairwise join loop), with the
  *                         predicate cos(e_i, e_j) >= tau named by BASELINE.json
  *   mmrs_threshold_sweep  code/search_image.py:39-79 (eval_threshold / find_thresholds)
@@ -393,6 +393,29 @@ int mmrs_selfjoin_pairs_tc(const float* d_emb_f32, int64_t ld_f32, const void* d
                            void* d_workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * The same join on a gallery in its stored format (d_rows as resident: ld_rows in elements for bf16, in bytes
+ * for int8), for galleries too large to keep in fp32 next to a copy.  Rank panels, d_out_count [0] pairs /
+ * [1] candidates, the capacity protocol and the synchronisation are those of mmrs_selfjoin_pairs_tc.
+ *   MMRS_DTYPE_BF16: the tcgen05 pass multiplies the stored values exactly, so the margin only has to cover the
+ *     two fp32 accumulations: margin >= dim * 2^-22 * max(1, r^2) for rows of norm at most r
+ *     (mmrs_row_norm_range_bf16).  Survivors are re-scored from the same bf16 rows, each element widened to fp32,
+ *     with the fmaf chain of mmrs_selfjoin_pairs: the pair set is that join's on the widened rows.
+ *   MMRS_DTYPE_I8 (rows as in "int8 galleries", dim <= 131072): tcgen05.mma.kind::i8 gives the exact code product
+ *     dot, and the epilogue keeps i < j with fl(fl(float(dot) * s_i) * s_j) >= threshold -- the int8 score with
+ *     the lower row as the query at scale 1.  margin must be 0; there is no recheck, candidates are the pairs
+ *     (d_out_count[1] == [0]) and cand_capacity is ignored.
+ * Any other dtype: MMRS_ERR_ARG.  Replaces tool/find_repeated_in_same_folder.py:76-95's pairwise hash
+ * comparison like mmrs_selfjoin_pairs; workspace: mmrs_selfjoin_stored_workspace_bytes(n_rows, dtype,
+ * cand_capacity).
+ */
+size_t mmrs_selfjoin_stored_workspace_bytes(int64_t n_rows, int32_t dtype, int64_t cand_capacity);
+int mmrs_selfjoin_pairs_stored(const void* d_rows, int32_t dtype, int64_t ld_rows, int64_t n_rows,
+                               int32_t dim, float threshold, float margin, int32_t rank, int32_t world,
+                               int64_t* d_out_pairs, int64_t capacity, int64_t* d_out_count,
+                               int64_t cand_capacity, void* d_workspace, size_t workspace_bytes,
+                               void* stream);
+
+/*
  * Lexicographic (i, j) sort of an int64 [n_pairs, 2] pair list in place -- the order of
  * `triu(S >= tau, 1).nonzero()`.  Row ids must fit 32 bits.  Workspace:
  * mmrs_sort_pairs_workspace_bytes(n_pairs).  Asynchronous on `stream`.
@@ -408,6 +431,10 @@ int mmrs_sort_pairs(int64_t* d_pairs, int64_t n_pairs, void* d_workspace, size_t
  */
 int mmrs_row_norm_range(const float* d_emb, int64_t n_rows, int32_t dim, int64_t ld,
                         float* d_out_min_max, void* stream);
+/* The same over bf16 rows (d_emb [n_rows, ld] bf16), each element widened to fp32: the margin of the bf16
+ * stored-format join.  A row holding a NaN or an infinity makes the max non-finite. */
+int mmrs_row_norm_range_bf16(const void* d_emb, int64_t n_rows, int32_t dim, int64_t ld,
+                             float* d_out_min_max, void* stream);
 
 /* ---- threshold / F1 sweep (the reference's consumer of the scores) ------------------ */
 

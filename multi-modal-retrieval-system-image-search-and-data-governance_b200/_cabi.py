@@ -99,9 +99,13 @@ SIGNATURES = {
     "mmrs_selfjoin_tc_workspace_bytes": (_sz, [_i64, _i64]),
     "mmrs_selfjoin_pairs_tc": (C.c_int, [_vp, _i64, _vp, _i64, _i64, _i32, _f32, _f32, _i32, _i32, _vp, _i64,
                                          _vp, _i64, _vp, _sz, _vp]),
+    "mmrs_selfjoin_stored_workspace_bytes": (_sz, [_i64, _i32, _i64]),
+    "mmrs_selfjoin_pairs_stored": (C.c_int, [_vp, _i32, _i64, _i64, _i32, _f32, _f32, _i32, _i32, _vp, _i64, _vp, _i64,
+                                             _vp, _sz, _vp]),
     "mmrs_sort_pairs_workspace_bytes": (_sz, [_i64]),
     "mmrs_sort_pairs": (C.c_int, [_vp, _i64, _vp, _sz, _vp]),
     "mmrs_row_norm_range": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp]),
+    "mmrs_row_norm_range_bf16": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _vp]),
     "mmrs_graph_stats": (C.c_int, [_vp]),
     "mmrs_threshold_sweep_f64": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _sz, _vp]),
     "mmrs_threshold_sweep_workspace_bytes": (_sz, [_i32]),

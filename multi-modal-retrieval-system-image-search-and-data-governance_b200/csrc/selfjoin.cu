@@ -543,15 +543,21 @@ cudaError_t launch_sort_pairs(int64_t* pairs, int64_t n_pairs, uint64_t* scratch
 }
 
 // ---- range of the row norms (guard of the bf16 prefilter margin, which assumes unit rows) -------------------
-__global__ void __launch_bounds__(256) row_norm_range_kernel(const float* __restrict__ x, int64_t n_rows, int32_t dim,
+// T = __nv_bfloat16: the rows of a bf16 gallery, each element widened to fp32 (exactly).  A row holding a NaN or an
+// infinity has a NaN or infinite norm, whose bits order above every finite one: the max reports it.
+template <typename T>
+__global__ void __launch_bounds__(256) row_norm_range_kernel(const T* __restrict__ x, int64_t n_rows, int32_t dim,
                                                              int64_t ld, uint32_t* __restrict__ mm) {
   const int lane = threadIdx.x & 31;
   const int64_t warps = static_cast<int64_t>(gridDim.x) * (blockDim.x >> 5);
   uint32_t lo = 0xffffffffu, hi = 0u;
   for (int64_t r = blockIdx.x * static_cast<int64_t>(blockDim.x >> 5) + (threadIdx.x >> 5); r < n_rows; r += warps) {
-    const float* row = x + r * ld;
+    const T* row = x + r * ld;
     float ss = 0.f;
-    for (int d = lane; d < dim; d += 32) ss = fmaf(row[d], row[d], ss);
+    for (int d = lane; d < dim; d += 32) {
+      const float v = static_cast<float>(row[d]);
+      ss = fmaf(v, v, ss);
+    }
 #pragma unroll
     for (int o = 16; o >= 1; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
     const uint32_t bits = __float_as_uint(sqrtf(ss));     // norms are >= 0: bit order == value order
@@ -560,7 +566,8 @@ __global__ void __launch_bounds__(256) row_norm_range_kernel(const float* __rest
   }
   if (lane == 0 && lo != 0xffffffffu) { atomicMin(mm, lo); atomicMax(mm + 1, hi); }
 }
-static cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t dim, int64_t ld, float* out_min_max,
+template <typename T>
+static cudaError_t launch_row_norm_range(const T* x, int64_t n_rows, int32_t dim, int64_t ld, float* out_min_max,
                                          int sm_count, cudaStream_t stream) {
   uint32_t* mm = reinterpret_cast<uint32_t*>(out_min_max);
   cudaError_t e = cudaMemsetAsync(mm, 0xff, sizeof(uint32_t), stream);
@@ -569,7 +576,7 @@ static cudaError_t launch_row_norm_range(const float* x, int64_t n_rows, int32_t
   if (e != cudaSuccess) return e;
   int64_t grid = (n_rows + 7) / 8;
   if (grid > static_cast<int64_t>(sm_count) * 8) grid = static_cast<int64_t>(sm_count) * 8;
-  row_norm_range_kernel<<<static_cast<int>(grid), 256, 0, stream>>>(x, n_rows, dim, ld, mm);
+  row_norm_range_kernel<T><<<static_cast<int>(grid), 256, 0, stream>>>(x, n_rows, dim, ld, mm);
   return cudaGetLastError();
 }
 
@@ -681,6 +688,18 @@ int mmrs_row_norm_range(const float* d_emb, int64_t n_rows, int32_t dim, int64_t
   if (rc != MMRS_OK) return rc;
   if (!d_emb || !d_out_min_max || n_rows < 1 || dim < 1 || ld < dim) return fail(MMRS_ERR_ARG, "bad arguments");
   MMRS_LAUNCH(launch_row_norm_range(d_emb, n_rows, dim, ld, d_out_min_max, dev.sm_count, stream));
+  return MMRS_OK;
+}
+
+int mmrs_row_norm_range_bf16(const void* d_emb, int64_t n_rows, int32_t dim, int64_t ld, float* d_out_min_max,
+                             void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (!d_emb || !d_out_min_max || n_rows < 1 || dim < 1 || ld < dim) return fail(MMRS_ERR_ARG, "bad arguments");
+  MMRS_LAUNCH(launch_row_norm_range(static_cast<const __nv_bfloat16*>(d_emb), n_rows, dim, ld, d_out_min_max,
+                                    dev.sm_count, stream));
   return MMRS_OK;
 }
 

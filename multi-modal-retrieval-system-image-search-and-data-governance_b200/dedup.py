@@ -78,24 +78,28 @@ def tc_margin(dim: int, max_norm: float, unit_margin: float = BF16_MARGIN) -> fl
     operand rounding for unit rows; `dim * 2^-22` covers the two fp32 dot products (the tensor cores'
     and the recheck's fmaf chain, each within dim * 2^-24 |a||b| when rounded to nearest), twice over
     because the tensor cores' accumulation order and rounding are not documented.  Both terms scale
-    with |a||b| <= max_norm^2 (1.0001 absorbs the rounding of the measured norm)."""
+    with |a||b| <= max_norm^2 (1.0001 absorbs the rounding of the measured norm).
+    The stored-format join of a bf16 gallery passes unit_margin=0: its tensor-core pass multiplies the
+    very values the recheck widens to fp32, bf16 products are exact in fp32, and no operand is rounded,
+    so only the two accumulations separate the prefilter's score from the recheck's."""
     return (float(unit_margin) + dim * 2.0 ** -22) * max(1.0, max_norm * max_norm * 1.0001)
 
 
-def row_norm_range(x32: torch.Tensor) -> "tuple[float, float]":
-    """(min, max) L2 norm over the rows of a device fp32 matrix (mmrs_row_norm_range)."""
-    with torch.cuda.device(x32.device):
-        mm = torch.empty(2, dtype=torch.float32, device=x32.device)
-        _cabi.check(_cabi.lib.mmrs_row_norm_range(x32.data_ptr(), int(x32.shape[0]), int(x32.shape[1]), x32.stride(0),
-                                                  mm.data_ptr(), _stream_handle(x32.device)))
+def row_norm_range(x: torch.Tensor) -> "tuple[float, float]":
+    """(min, max) L2 norm over the rows of a device fp32 or bf16 matrix (mmrs_row_norm_range / _bf16)."""
+    fn = _cabi.lib.mmrs_row_norm_range_bf16 if x.dtype == torch.bfloat16 else _cabi.lib.mmrs_row_norm_range
+    with torch.cuda.device(x.device):
+        mm = torch.empty(2, dtype=torch.float32, device=x.device)
+        _cabi.check(fn(x.data_ptr(), int(x.shape[0]), int(x.shape[1]), x.stride(0), mm.data_ptr(),
+                       _stream_handle(x.device)))
         lo, hi = mm.tolist()
     return float(lo), float(hi)
 
 
-def _max_row_norm(x32: torch.Tensor) -> float:
-    """The largest row norm; ValueError when a row holds a NaN or an infinity (both joins refuse them:
+def _max_row_norm(x: torch.Tensor) -> float:
+    """The largest row norm; ValueError when a row holds a NaN or an infinity (every join refuses them:
     the deletions that follow would depend on how each kernel treats a NaN score)."""
-    _, max_norm = row_norm_range(x32)
+    _, max_norm = row_norm_range(x)
     if not (max_norm < float("inf")):
         raise ValueError("embeddings contain non-finite rows")
     return max_norm
@@ -138,6 +142,41 @@ def selfjoin_tc_raw(x32: torch.Tensor, threshold: float, rank: int = 0, world: i
             return pairs[:found]
 
 
+def selfjoin_stored_raw(gal: DeviceGallery, threshold: float, rank: int = 0, world: int = 1,
+                        capacity: Optional[int] = None) -> torch.Tensor:
+    """Unsorted int64 [P, 2] pairs of rank `rank`'s panels, joined on a bf16 or int8 gallery as stored
+    (mmrs_selfjoin_pairs_stored); buffers grow on demand.
+    bf16: tensor-core prefilter at threshold - tc_margin(dim, max_norm, 0) and a recheck of the survivors
+    with the exact join's fmaf chain on the widened rows -- the pair set of the fp32 join of gal.data.float().
+    A NaN or infinite row raises ValueError.
+    int8: every pair decided exactly on the tensor cores, fl(fl(float(dot) s_i) s_j) >= threshold with the
+    lower row as the query -- the int8 score of the stored codes and scales, no margin and no recheck."""
+    i8 = gal.mode == "int8"
+    dev, n, d = gal.device, gal.n_rows, gal.padded_dim
+    lib = _cabi.lib
+    margin = 0.0 if i8 else tc_margin(d, _max_row_norm(gal.data))
+    cap = int(capacity) if capacity is not None else max(4096, n // 4)
+    cand_cap = 1 if i8 else 2 * cap
+    with torch.cuda.device(dev):
+        counts = torch.zeros(2, dtype=torch.int64, device=dev)
+        while True:
+            pairs = torch.empty((cap, 2), dtype=torch.int64, device=dev)
+            ws_bytes = lib.mmrs_selfjoin_stored_workspace_bytes(n, gal.dtype_code, cand_cap)
+            ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
+            st = lib.mmrs_selfjoin_pairs_stored(gal.data.data_ptr(), gal.dtype_code, gal.data.stride(0), n, d,
+                                                float(threshold), float(margin), int(rank), int(world),
+                                                pairs.data_ptr(), cap, counts.data_ptr(), cand_cap,
+                                                DeviceGallery.aligned_ptr(ws), ws_bytes, _stream_handle(dev))
+            found, n_cand = (int(v) for v in counts.tolist())
+            if st == _cabi.ERR_CAPACITY:
+                if not i8:
+                    cand_cap = max(cand_cap, n_cand)
+                cap = max(cap, found, n_cand)
+                continue
+            _cabi.check(st)
+            return pairs[:found]
+
+
 def sort_pairs(pairs: torch.Tensor, n: int) -> torch.Tensor:
     """Lexicographic (i, j) order -- what `triu(S >= tau, 1).nonzero()` yields row-major.
     Device pair lists are sorted by the library's own bitonic sort on packed (i << 32 | j) keys
@@ -165,19 +204,46 @@ def find_duplicate_pairs(emb, threshold: float, *, device=None, method: str = "a
     method "fp32": every pair in fp32 on the CUDA cores.  "tc": bf16 tensor-core prefilter with a
     safety margin (tc_margin) + exact fp32 recheck of the survivors -- the same pair set, ~20x the
     throughput.  "auto": "tc" from 2048 rows on.  Every method raises ValueError on a NaN or
-    infinite row."""
+    infinite row.
+    "stored" joins a bf16 or int8 DeviceGallery in its stored format, for galleries too large to keep
+    in fp32 (selfjoin_stored_raw): on bf16 rows the pair set of "fp32" on gal.data.float(); on int8 rows
+    the pairs whose int8 score (the lower row as the query) reaches threshold -- a property of the
+    quantised rows that differs from the fp32 predicate near the threshold, so it is never chosen by
+    default.  Pair ids are the gallery's own rows (row_offset is not added)."""
     on_host = not isinstance(emb, DeviceGallery) and not (isinstance(emb, torch.Tensor) and emb.is_cuda)
-    x = _device_f32(emb, device)
-    pairs = sort_pairs(_join_raw(x, threshold, method), int(x.shape[0]))
+    x = _join_input(emb, method, device)
+    pairs = sort_pairs(_join_raw(x, threshold, method), len(x))
     return pairs.cpu() if on_host else pairs
 
 
-def _join_raw(x: torch.Tensor, threshold: float, method: str) -> torch.Tensor:
-    """The unsorted pair list of find_duplicate_pairs' `method` on a device fp32 matrix."""
-    if method not in ("auto", "fp32", "tc"):
-        raise ValueError("method must be 'auto', 'fp32' or 'tc'")
+METHODS = ("auto", "fp32", "tc", "stored")
+
+
+def _check_method(method: str) -> None:
+    if method not in METHODS:
+        raise ValueError("method must be 'auto', 'fp32', 'tc' or 'stored'")
+
+
+def _join_input(emb, method: str, device=None):
+    """What _join_raw joins: the gallery itself for "stored" (bf16 or int8 only), else the device fp32 matrix.
+    The method is checked before anything is uploaded."""
+    _check_method(method)
+    if method != "stored":
+        return _device_f32(emb, device)
+    if not isinstance(emb, DeviceGallery) or emb.mode not in ("bf16", "int8"):
+        raise ValueError('method="stored" joins a bf16 or int8 DeviceGallery in its stored format; '
+                         'fp32 rows take method "fp32" or "tc"')
+    return emb
+
+
+def _join_raw(x, threshold: float, method: str, rank: int = 0, world: int = 1) -> torch.Tensor:
+    """The unsorted pair list of find_duplicate_pairs' `method` on _join_input's result (rank panels for
+    "stored" and "tc"; the exact join takes none)."""
+    _check_method(method)
+    if method == "stored":
+        return selfjoin_stored_raw(x, threshold, rank, world)
     use_tc = method == "tc" or (method == "auto" and x.shape[0] >= 2048)
-    return selfjoin_tc_raw(x, threshold) if use_tc else selfjoin_raw(x, threshold)
+    return selfjoin_tc_raw(x, threshold, rank, world) if use_tc else selfjoin_raw(x, threshold)
 
 
 def greedy_first_keeper(n: int, pairs, order: Sequence[int]):
@@ -287,10 +353,8 @@ def deduplicate(emb, threshold: float, *, order=None, method: str = "auto", devi
     unsorted (the resolve does not need the lexicographic order).  Same inputs and `method` as
     find_duplicate_pairs; returns the [n] representative tensor (host input gives a host result)."""
     on_host = not isinstance(emb, DeviceGallery) and not (isinstance(emb, torch.Tensor) and emb.is_cuda)
-    if method not in ("auto", "fp32", "tc"):
-        raise ValueError("method must be 'auto', 'fp32' or 'tc'")     # before the embeddings are uploaded
-    x = _device_f32(emb, device)
-    rep = resolve_duplicates(_join_raw(x, threshold, method), int(x.shape[0]), order=order)
+    x = _join_input(emb, method, device)
+    rep = resolve_duplicates(_join_raw(x, threshold, method), len(x), order=order)
     return rep.cpu() if on_host else rep
 
 

@@ -602,20 +602,31 @@ class ShardedGallery:
         out = concat_per_query(pieces)
         return tuple(x.cpu() for x in out) if on_host and self._local_range_search is None else out
 
-    def find_duplicate_pairs(self, emb_full: torch.Tensor, threshold: float, raw_join: Optional[Callable] = None):
+    def find_duplicate_pairs(self, emb_full, threshold: float, raw_join: Optional[Callable] = None,
+                             method: str = "auto"):
         """Self-join with the gallery replicated (10M x 512 fp32 = 20 GB fits every GPU) and the
         upper-triangular tile grid split by equal pair count; variable-length pair lists are
-        gathered (counts first, then padded buffers) and sorted lexicographically."""
-        from .dedup import selfjoin_tc_raw, sort_pairs
-        n = int(emb_full.shape[0])
-        if raw_join is None and emb_full.is_cuda and n >= 2048:
-            # tensor-core path: column panels dealt round-robin to the ranks
-            pairs = selfjoin_tc_raw(emb_full, threshold, self.rank, self.world)
+        gathered (counts first, then padded buffers) and sorted lexicographically.
+        `method` as in dedup.find_duplicate_pairs.  With "stored", `emb_full` is a bf16 or int8 DeviceGallery
+        holding every row on every rank (2x / 3.9x smaller than fp32), and the tensor-core panels are dealt by
+        rank as for "tc"."""
+        from .dedup import _check_method, _join_input, _join_raw, sort_pairs
+        _check_method(method)
+        if method == "stored":
+            gal = _join_input(emb_full, method)
+            n = len(gal)
+            pairs = _join_raw(gal, threshold, method, self.rank, self.world)
         else:
-            from .dedup import selfjoin_raw
-            raw_join = raw_join or selfjoin_raw
-            lo, hi = triangle_bounds(n, self.world)[self.rank]
-            pairs = raw_join(emb_full, threshold, lo, hi) if hi > lo else emb_full.new_empty((0, 2), dtype=torch.int64)
+            n = int(emb_full.shape[0])
+            use_tc = raw_join is None and emb_full.is_cuda and (method == "tc" or (method == "auto" and n >= 2048))
+            if use_tc:
+                # tensor-core path: column panels dealt round-robin to the ranks
+                pairs = _join_raw(emb_full, threshold, "tc", self.rank, self.world)
+            else:
+                from .dedup import selfjoin_raw
+                raw_join = raw_join or selfjoin_raw
+                lo, hi = triangle_bounds(n, self.world)[self.rank]
+                pairs = raw_join(emb_full, threshold, lo, hi) if hi > lo else emb_full.new_empty((0, 2), dtype=torch.int64)
         if self.world == 1:
             return sort_pairs(pairs, n)
         cnt = torch.tensor([pairs.shape[0]], dtype=torch.int64, device=pairs.device)
@@ -627,11 +638,11 @@ class ShardedGallery:
         parts = [allbuf[r, :int(cnts[r].item())] for r in range(self.world)]
         return sort_pairs(torch.cat(parts, dim=0), n)
 
-    def deduplicate(self, emb_full: torch.Tensor, threshold: float, *, order=None,
-                    raw_join: Optional[Callable] = None) -> torch.Tensor:
+    def deduplicate(self, emb_full, threshold: float, *, order=None,
+                    raw_join: Optional[Callable] = None, method: str = "auto") -> torch.Tensor:
         """`deduplicate` over the ranks: the pairs of `find_duplicate_pairs` (every rank holds the whole
         gathered list), then `resolve_duplicates` on each rank.  The resolve is deterministic, so every rank
         returns the same [n] representative tensor without another collective."""
         from .dedup import resolve_duplicates
-        pairs = self.find_duplicate_pairs(emb_full, threshold, raw_join=raw_join)
-        return resolve_duplicates(pairs, int(emb_full.shape[0]), order=order)
+        pairs = self.find_duplicate_pairs(emb_full, threshold, raw_join=raw_join, method=method)
+        return resolve_duplicates(pairs, len(emb_full), order=order)
