@@ -238,6 +238,39 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
                                 int32_t label_match, void* stream);
 
 /*
+ * Refined top-k: rescore candidate rows against a full-precision copy of the gallery and keep the k best.
+ * d_store [n_rows, ld_store] is that copy (store_dtype MMRS_DTYPE_F32 or MMRS_DTYPE_BF16, dim and ld_store as
+ * for a gallery of that dtype); it may live in device memory or in host memory registered with
+ * mmrs_host_register (pass the device pointer it returns).  d_queries [n_queries, ld_queries] fp32 (device),
+ * d_candidates [n_queries, k_cand] int64 LOCAL rows, -1 = no candidate; the rows of one query must be distinct.
+ * The call runs, in stream order: the search's query preparation in the store's dtype (normalisation, bf16
+ * rounding for a bf16 store); one score per candidate; the select of the k largest (score, row) keys.
+ * Scores: the score of row r for query q is bit for bit mmrs_full_scores(store, path = MMRS_PATH_GEMV)[q, r]
+ * (K1's chunk order, fmaf chain and warp reduction; -0.0 returned as +0.0).  Output as mmrs_search_topk:
+ * values [n_queries, k] descending, indices + index_offset, equal scores by ascending row; a query with fewer
+ * than k candidates is padded with value -inf, index -1.  1 <= k <= min(1024, k_cand).
+ * A candidate outside [-1, n_rows) is found on the device and reported as MMRS_ERR_ARG (it is never read).
+ * Workspace: mmrs_refine_workspace_bytes(dim, n_queries, k_cand), 256-byte aligned.
+ * h_status NULL: the call synchronises `stream` and returns the outcome.  Otherwise h_status is one int32 of
+ * pinned host memory: the call returns after enqueueing, and mmrs_search_status(h_status) gives the outcome
+ * once the stream has passed the call.
+ */
+size_t mmrs_refine_workspace_bytes(int32_t dim, int32_t n_queries, int32_t k_cand);
+int mmrs_refine_topk(const void* d_store, int32_t store_dtype, int64_t n_rows, int32_t dim, int64_t ld_store,
+                     const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t normalize_queries,
+                     float scale, const int64_t* d_candidates, int32_t k_cand, int64_t index_offset, int32_t k,
+                     float* d_out_values, int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+                     int32_t* h_status, void* stream);
+
+/*
+ * Page-lock `bytes` of ordinary host memory at h_ptr (cudaHostRegister, portable and mapped) and return in
+ * *d_ptr_out the address kernels read it through: a refine store kept in host memory.  Undo with
+ * mmrs_host_unregister(h_ptr) before the memory is freed.
+ */
+int mmrs_host_register(void* h_ptr, size_t bytes, void** d_ptr_out);
+int mmrs_host_unregister(void* h_ptr);
+
+/*
  * Sharded search without a host round trip: each rank writes its local top-k as packed 64-bit keys
  * (order-preserving fp32 score in the high word, ~global_row in the low word; a larger key is a
  * better match and keys are unique), ONE all-gather moves n_queries * k * 8 bytes per rank, and

@@ -24,11 +24,13 @@ DeviceGallery, ShardedGallery, RowFilter (row-filtered search_topk: leave rows o
 RowLabels (label-conditioned search_topk: each query searches the rows of its own class, or of every other)
 and best_thresholds (the best-F1 threshold of every class prototype of a batch, find_thresholds per class) and
 search_range (every row at or above a per-query threshold, in CSR form) and resolve_duplicates / deduplicate
-(greedy_first_keeper's keep / delete decision on the device: the representative of every row).  Everything computes through the C-ABI CUDA library
+(greedy_first_keeper's keep / delete decision on the device: the representative of every row) and RefineStore
+(refined search_topk: a compact gallery's candidates rescored against full-precision rows in host or device memory).  Everything computes through the C-ABI CUDA library
 (include/mmrs_b200.h); there is no CPU path -- without a B200 the calls raise.
 """
 from . import _cabi  # noqa: F401  (fails loudly when the CUDA library is missing)
 from .gallery import DeviceGallery, load_feature_cache
+from .refine import RefineStore
 from .row_filter import RowFilter
 from .row_labels import RowLabels
 from .search import (best_threshold_on_device, calc_combined_metrics, cls_acc, cluster_prototype, construct_dataset,
@@ -44,7 +46,7 @@ from .range_search import search_range
 from .thresholds import best_thresholds
 
 __all__ = [
-    "DeviceGallery", "RowFilter", "RowLabels", "ShardedGallery", "best_threshold_on_device", "best_thresholds", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
+    "DeviceGallery", "RefineStore", "RowFilter", "RowLabels", "ShardedGallery", "best_threshold_on_device", "best_thresholds", "calc_combined_metrics", "calculate_image_hash", "cls_acc",
     "cluster_prototype", "construct_dataset", "cosine_similarity_scores", "deduplicate", "get_cluster_features", "get_image_text_features",
     "image_text_prototypes", "topk_of_scores",
     "detect_and_remove_cross_set_duplicates", "evaluate_thresholds", "eval_threshold", "find_thresholds",

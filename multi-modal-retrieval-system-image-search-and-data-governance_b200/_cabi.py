@@ -84,6 +84,12 @@ SIGNATURES = {
     "mmrs_search_exhaustive_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "mmrs_search_topk_exhaustive": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _f32,
                                               _i64, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _i32, _vp]),
+    # refined top-k: rescore candidate rows against a full-precision store (device or registered host memory)
+    "mmrs_refine_workspace_bytes": (_sz, [_i32, _i32, _i32]),
+    "mmrs_refine_topk": (C.c_int, [_vp, _i32, _i64, _i32, _i64, _vp, _i32, _i64, _i32, _f32, _vp, _i32, _i64, _i32,
+                                   _vp, _vp, _vp, _sz, _vp, _vp]),
+    "mmrs_host_register": (C.c_int, [_vp, _sz, _vp]),
+    "mmrs_host_unregister": (C.c_int, [_vp]),
     "mmrs_search_topk_fused_gather_async": (C.c_int, [_vp, _i64, _i32, _i64, _i32, _vp, _i32, _i64, _i32, _i32, _i32,
                                                       _f32, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i64,
                                                       _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp, _i32, _vp]),

@@ -151,6 +151,19 @@ static RangeWorkspace carve_range(Carver& c, int64_t window_rows, int32_t dim, i
   return r;
 }
 
+// mmrs_refine_topk: the prepared queries of carve(), then one key per (query, candidate)
+struct RefineWorkspace {
+  Workspace base;   // flags, q_f32, q_bf16
+  uint64_t* keys;   // [n_queries, k_cand]
+};
+
+static RefineWorkspace carve_refine(Carver& c, int32_t dim, int32_t n_queries, int32_t k_cand) {
+  RefineWorkspace r{};
+  r.base = carve(c, 1, dim, n_queries, 1, false);
+  r.keys = c.take<uint64_t>(static_cast<size_t>(n_queries) * k_cand * sizeof(uint64_t));
+  return r;
+}
+
 enum class Path { kGemv, kMma };
 
 static int choose_path(int32_t requested, int32_t dtype, int32_t n_queries, Path* path) {
@@ -611,6 +624,7 @@ static int launch_search_graph(const SearchArgs& a, const DeviceInfo& dev, const
 }
 
 static int flags_to_status(int32_t f) {
+  if (f & kFlagBadCandidate) return fail(MMRS_ERR_ARG, "refine: a candidate row is outside [-1, n_rows)");
   if (f & kFlagZeroNorm)
     return fail(MMRS_ERR_ZERO_NORM, "a query row has zero L2 norm and normalize_queries is set");
   if (f & kFlagNonFinite)
@@ -877,6 +891,82 @@ int mmrs_search_topk_exhaustive(const void* d_gallery, int64_t n_rows, int32_t d
   rc = enqueue_exhaustive(a, dev, w, stream);
   if (rc != MMRS_OK) return rc;
   return read_status(w.flags, stream);
+}
+
+size_t mmrs_refine_workspace_bytes(int32_t dim, int32_t n_queries, int32_t k_cand) {
+  if (dim < 1 || n_queries < 1 || k_cand < 1) return 0;
+  Carver c(nullptr);
+  carve_refine(c, dim, n_queries, k_cand);
+  return c.off;
+}
+
+int mmrs_refine_topk(const void* d_store, int32_t store_dtype, int64_t n_rows, int32_t dim, int64_t ld_store,
+                     const float* d_queries, int32_t n_queries, int64_t ld_queries, int32_t normalize_queries,
+                     float scale, const int64_t* d_candidates, int32_t k_cand, int64_t index_offset, int32_t k,
+                     float* d_out_values, int64_t* d_out_indices, void* d_workspace, size_t workspace_bytes,
+                     int32_t* h_status, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceInfo dev;
+  int rc = current_device(&dev);
+  if (rc != MMRS_OK) return rc;
+  if (store_dtype != MMRS_DTYPE_F32 && store_dtype != MMRS_DTYPE_BF16)
+    return fail(MMRS_ERR_ARG, "refine: store dtype %d must be MMRS_DTYPE_F32 or MMRS_DTYPE_BF16", store_dtype);
+  rc = check_matrix(d_store, n_rows, dim, ld_store, store_dtype, "refine store");
+  if (rc != MMRS_OK) return rc;
+  if (h_status) h_status[0] = 0;
+  if (n_queries == 0) return MMRS_OK;
+  if (n_queries < 0 || !d_queries || !d_candidates || !d_out_values || !d_out_indices || ld_queries < dim)
+    return fail(MMRS_ERR_ARG, "bad query / candidate / output arguments");
+  if (k_cand < 1 || k < 1 || k > 1024 || k > k_cand)
+    return fail(MMRS_ERR_ARG, "refine: k = %d must be in [1, min(1024, k_cand = %d)]", k, k_cand);
+  rc = check_workspace(d_workspace, workspace_bytes, mmrs_refine_workspace_bytes(dim, n_queries, k_cand));
+  if (rc != MMRS_OK) return rc;
+  Carver c(d_workspace);
+  const RefineWorkspace w = carve_refine(c, dim, n_queries, k_cand);
+  MMRS_CUDA(cudaMemsetAsync(w.base.flags, 0, 8 * sizeof(int32_t), stream));
+  rc = enqueue_prep(d_queries, n_queries, ld_queries, dim, normalize_queries, store_dtype, w.base, stream);
+  if (rc != MMRS_OK) return rc;
+  MMRS_LAUNCH(launch_refine_scores(d_store, store_dtype, n_rows, ld_store, dim, w.base.q_f32, padded_dim(dim), scale,
+                                   d_candidates, n_queries, k_cand, w.keys, w.base.flags, stream));
+  // the k best keys of each list; a list with fewer than k candidates (-1 entries) is padded with -inf / -1
+  SelectParams sp{};
+  sp.cand = w.keys; sp.cap = k_cand; sp.fixed_n = k_cand; sp.k = k; sp.final_pass = 1;
+  sp.out_values = d_out_values; sp.out_indices = d_out_indices; sp.index_offset = index_offset;
+  sp.flags = w.base.flags; sp.pad_short = 1;
+  MMRS_LAUNCH(launch_select(sp, n_queries, stream));
+  if (h_status) {
+    MMRS_CUDA(cudaMemcpyAsync(h_status, w.base.flags, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    return MMRS_OK;
+  }
+  return read_status(w.base.flags, stream);
+}
+
+int mmrs_host_register(void* h_ptr, size_t bytes, void** d_ptr_out) {
+  if (!h_ptr || bytes == 0 || !d_ptr_out) return fail(MMRS_ERR_ARG, "host register: null pointer or zero bytes");
+  // a refused registration (e.g. pages already registered) is not sticky: clear it, or the next launcher's
+  // cudaGetLastError() would report it
+  cudaError_t e = cudaHostRegister(h_ptr, bytes, cudaHostRegisterPortable | cudaHostRegisterMapped);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(MMRS_ERR_CUDA, "cudaHostRegister of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+  }
+  e = cudaHostGetDevicePointer(d_ptr_out, h_ptr, 0);
+  if (e != cudaSuccess) {
+    cudaHostUnregister(h_ptr);
+    cudaGetLastError();
+    return fail(MMRS_ERR_CUDA, "cudaHostGetDevicePointer failed: %s", cudaGetErrorString(e));
+  }
+  return MMRS_OK;
+}
+
+int mmrs_host_unregister(void* h_ptr) {
+  if (!h_ptr) return fail(MMRS_ERR_ARG, "host unregister: null pointer");
+  const cudaError_t e = cudaHostUnregister(h_ptr);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(MMRS_ERR_CUDA, "cudaHostUnregister failed: %s", cudaGetErrorString(e));
+  }
+  return MMRS_OK;
 }
 
 int mmrs_search_topk(const void* d_gallery, int64_t n_rows, int32_t dim, int64_t ld_gallery,

@@ -20,6 +20,7 @@ constexpr int kFlagShort = 4;         // fewer than k candidates reached a selec
 constexpr int kFlagWatchdog = 8;      // an mbarrier wait timed out (K2 debug guard)
 constexpr int kFlagGatherTimeout = 16;  // fused all-gather: a peer rank's flag did not arrive in time
 constexpr int kFlagNonFinite = 32;      // int8 mode: a query row holds a NaN or an infinity
+constexpr int kFlagBadCandidate = 64;   // refine: a candidate row outside [-1, n_rows)
 
 // Status bits of the duplicate resolve (dedup_resolve.cu), in its own status word.
 constexpr int kResolveOrderRange = 1;   // an order id outside [0, n_items)
@@ -260,6 +261,11 @@ cudaError_t launch_gather_wait(const uint32_t* my_flags, int32_t world, const ui
                                uint64_t timeout_ns, cudaStream_t stream);
 cudaError_t launch_scan_gemv(const ScanParams& p, int32_t dtype, int mode, int sm_count,
                              cudaStream_t stream);
+// refine (scan_gemv.cu): one key per (query, candidate) into keys [n_queries, k_cand]
+cudaError_t launch_refine_scores(const void* store, int32_t dtype, int64_t n_rows, int64_t ld, int32_t dim,
+                                 const float* queries, int32_t ldq, float scale, const int64_t* cand,
+                                 int32_t n_queries, int32_t k_cand, uint64_t* keys, int32_t* flags,
+                                 cudaStream_t stream);
 cudaError_t launch_quantize_rows_i8(const void* src, int32_t src_dtype, int64_t n_rows, int32_t dim, int64_t ld_src,
                                     int8_t* dst, int64_t ld_dst, int32_t* status, int sm_count, cudaStream_t stream);
 cudaError_t launch_select(const SelectParams& p, int32_t n_queries, cudaStream_t stream);

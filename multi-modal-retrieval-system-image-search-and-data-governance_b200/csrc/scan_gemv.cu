@@ -282,6 +282,81 @@ cudaError_t launch_scan_gemv(const ScanParams& p, int32_t dtype, int mode, int s
   return launch_gemv_q<float>(p, mode, sm_count, stream);
 }
 
+// ---- refine: rescore a list of candidate rows (mmrs_refine_topk) ---------------------------------------
+// One warp per (query, candidate): the same 16-byte row loads, lane chunk order (c = lane, lane + 32, ...,
+// ascending), fmaf chain and xor butterfly as K1, so a row's score is bit for bit K1's whatever QN / R K1 ran
+// with: K1's TransposeReduce<V, 16> adds the partials of lanes l and l ^ O at O = 16, 8, 4, 2, 1 for every V,
+// and a float sum of two terms does not depend on their order.  The store may be registered host memory: a
+// grid over every pair keeps enough warps (and loads) in flight to cover a PCIe read.  A -1 candidate is key
+// 0 (no entry); a candidate outside [-1, n_rows) is key 0 and raises kFlagBadCandidate.
+constexpr int kRefineThreads = 256;
+constexpr int kRefineUnroll = 4;   // row chunks each lane loads before it multiplies them
+
+template <typename T>
+__global__ void __launch_bounds__(kRefineThreads) refine_scores_kernel(
+    const T* __restrict__ store, int64_t n_rows, int64_t ld, int32_t dim, const float* __restrict__ queries,
+    int32_t ldq, float scale, const int64_t* __restrict__ cand, int64_t n_pairs, int32_t k_cand,
+    uint64_t* __restrict__ keys, int32_t* flags) {
+  constexpr int CH = Chunk<T>::CH;
+  const int64_t pair = (blockIdx.x * static_cast<int64_t>(kRefineThreads) + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  pdl_launch_dependents();
+  pdl_wait();   // the prepared queries come from the prep kernel
+  if (pair >= n_pairs) return;
+  const int64_t row = __ldg(cand + pair);
+  if (row < 0 || row >= n_rows) {
+    if (lane == 0) {
+      keys[pair] = 0ull;
+      if (row != -1) atomicOr(flags, kFlagBadCandidate);
+    }
+    return;
+  }
+  const T* rp = store + row * ld;
+  const float* qp = queries + (pair / k_cand) * static_cast<int64_t>(ldq);
+  const int n_chunks = dim / CH;
+  float acc = 0.f;
+  for (int c0 = lane; c0 < n_chunks; c0 += 32 * kRefineUnroll) {
+    uint4 g[kRefineUnroll];
+#pragma unroll
+    for (int u = 0; u < kRefineUnroll; ++u)
+      if (c0 + 32 * u < n_chunks) g[u] = ldg_stream_16B(rp + (c0 + 32 * u) * CH);
+#pragma unroll
+    for (int u = 0; u < kRefineUnroll; ++u) {
+      const int c = c0 + 32 * u;
+      if (c < n_chunks) {
+        float f[CH], qv[CH];
+        Chunk<T>::unpack(g[u], f);
+#pragma unroll
+        for (int h = 0; h < CH / 4; ++h) {
+          const float4 x = __ldg(reinterpret_cast<const float4*>(qp + c * CH) + h);
+          qv[h * 4 + 0] = x.x; qv[h * 4 + 1] = x.y; qv[h * 4 + 2] = x.z; qv[h * 4 + 3] = x.w;
+        }
+#pragma unroll
+        for (int e = 0; e < CH; ++e) acc = fmaf(f[e], qv[e], acc);
+      }
+    }
+  }
+  float v[1] = {acc};
+  TransposeReduce<1, 16>::run(v, lane);
+  if (lane == 0) keys[pair] = make_key(v[0] * scale, static_cast<uint32_t>(row));
+}
+
+cudaError_t launch_refine_scores(const void* store, int32_t dtype, int64_t n_rows, int64_t ld, int32_t dim,
+                                 const float* queries, int32_t ldq, float scale, const int64_t* cand,
+                                 int32_t n_queries, int32_t k_cand, uint64_t* keys, int32_t* flags,
+                                 cudaStream_t stream) {
+  const int64_t n_pairs = static_cast<int64_t>(n_queries) * k_cand;
+  if (n_pairs <= 0) return cudaSuccess;
+  const dim3 grid(static_cast<unsigned>((n_pairs + kRefineThreads / 32 - 1) / (kRefineThreads / 32)));
+  if (dtype == MMRS_DTYPE_BF16)
+    return launch_pdl(refine_scores_kernel<__nv_bfloat16>, grid, dim3(kRefineThreads), 0, stream,
+                      static_cast<const __nv_bfloat16*>(store), n_rows, ld, dim, queries, ldq, scale, cand, n_pairs,
+                      k_cand, keys, flags);
+  return launch_pdl(refine_scores_kernel<float>, grid, dim3(kRefineThreads), 0, stream,
+                    static_cast<const float*>(store), n_rows, ld, dim, queries, ldq, scale, cand, n_pairs, k_cand,
+                    keys, flags);
+}
+
 // ---- int8 quantisation (include/mmrs_b200.h, "int8 galleries") -------------------------------------
 // s = fl(m / 127) for the row's max |x|; c = clamp(rint(x / s), -127, 127), IEEE division, half to even
 __device__ __forceinline__ float i8_scale_of(float max_abs) { return __fdiv_rn(max_abs, 127.f); }

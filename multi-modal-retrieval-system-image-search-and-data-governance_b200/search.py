@@ -82,6 +82,7 @@ class PendingSearch:
         self.values, self.indices = values, indices
         self._slot, self._ticket, self._status, self._event, self._redo = slot, ticket, status, event, redo
         self._done = slot is None
+        self.retried = False       # True once wait() has repeated the batch on the exhaustive path
 
     def wait(self):
         if not self._done:
@@ -90,6 +91,7 @@ class PendingSearch:
             self._slot.release(self._ticket)      # only now may the status word serve another batch
             self._done = True
             if st == _cabi.ERR_RETRY:
+                self.retried = True
                 self._redo(self.values, self.indices)
             else:
                 _cabi.check(st)
@@ -176,9 +178,27 @@ def _stage_query_labels(slot, ql: torch.Tensor, dev: torch.device):
     return buf, src
 
 
+def _result_tensors(out, nq: int, k: int, on_host: bool, dev: torch.device):
+    """(values, indices) a search writes: `out` checked, or new tensors (pinned host tensors for host queries)."""
+    if out is not None:
+        values, indices = out
+        if (tuple(values.shape) != (nq, k) or tuple(indices.shape) != (nq, k) or values.dtype != torch.float32
+                or indices.dtype != torch.int64 or values.is_cuda == on_host or indices.is_cuda == on_host
+                or not values.is_contiguous() or not indices.is_contiguous()):
+            raise ValueError(f"out must be contiguous (float32 [{nq}, {k}], int64 [{nq}, {k}]) tensors on the "
+                             f"{'host' if on_host else 'device'}")
+        return values, indices
+    if on_host:
+        return (torch.empty((nq, k), dtype=torch.float32, pin_memory=True),
+                torch.empty((nq, k), dtype=torch.int64, pin_memory=True))
+    return (torch.empty((nq, k), dtype=torch.float32, device=dev),
+            torch.empty((nq, k), dtype=torch.int64, device=dev))
+
+
 def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: bool = True,
                 scale: float = 1.0, mode: Optional[str] = None, path: str = "auto", sync: bool = True,
-                out=None, row_filter=None, row_labels=None, query_labels=None, label_match: str = "same"):
+                out=None, row_filter=None, row_labels=None, query_labels=None, label_match: str = "same",
+                refine=None, refine_k: Optional[int] = None):
     """Per-query top-k of `scale * q @ G.T` without materialising the score matrix.
 
     Returns `(values [Q, k] fp32 descending, indices [Q, k] int64)` exactly like
@@ -201,8 +221,19 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
     Unlike `row_filter`'s `k > allowed` error, a query with fewer than k eligible rows (a small class, a
     label absent from the gallery) is padded: positions n_eligible .. k-1 hold value -inf, index -1.
     The labels are copied into a buffer of the slot on every call (no host sync, one graph per slot).
+    `refine` (a RefineStore holding the gallery's rows in fp32 or bf16) makes the search two-stage: the search
+    above with k_c = min(refine_k, N, rows a row_filter allows) candidates and every other argument as given
+    (its exhaustive retry included), then each candidate rescored against the store and the k best kept.  A
+    refined score is bit for bit `full_scores(queries, DeviceGallery(features, store.mode), path="gemv")` at
+    that row; whenever the candidates contain the store's exact top-k under the same constraints the result is
+    that gallery's `search_topk(..., path="gemv")`.  `refine_k` (default 2 k, at most 1024) must be >= k; the
+    store must match the gallery's rows, width and (for a device store) device.  DESIGN.md section 4.
     """
     gal = _as_gallery(gallery, mode)
+    if refine is not None or refine_k is not None:
+        return _search_refined(queries, gal, k, refine, refine_k, normalize_queries, scale, path, sync, out,
+                               row_filter, dict(row_labels=row_labels, query_labels=query_labels,
+                                                label_match=label_match))
     q, on_host = _prep_queries(queries, gal)
     nq = int(q.shape[0])
     k = int(k)
@@ -219,19 +250,7 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
     if torch.cuda.current_device() != dev.index:
         torch.cuda.set_device(dev)
     stream = torch.cuda.current_stream(dev)
-    if out is not None:
-        values, indices = out
-        if (tuple(values.shape) != (nq, k) or tuple(indices.shape) != (nq, k) or values.dtype != torch.float32
-                or indices.dtype != torch.int64 or values.is_cuda == on_host or indices.is_cuda == on_host
-                or not values.is_contiguous() or not indices.is_contiguous()):
-            raise ValueError(f"out must be contiguous (float32 [{nq}, {k}], int64 [{nq}, {k}]) tensors on the "
-                             f"{'host' if on_host else 'device'}")
-    elif on_host:
-        values = torch.empty((nq, k), dtype=torch.float32, pin_memory=True)
-        indices = torch.empty((nq, k), dtype=torch.int64, pin_memory=True)
-    else:
-        values = torch.empty((nq, k), dtype=torch.float32, device=dev)
-        indices = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    values, indices = _result_tensors(out, nq, k, on_host, dev)
     if nq == 0:
         if filt is not None and not isinstance(filt, RowFilter) and k > int(filt.sum()):
             raise RuntimeError("selected index k out of range")
@@ -292,6 +311,100 @@ def search_topk(queries, gallery: GalleryLike, k: int, *, normalize_queries: boo
     pend = PendingSearch(values, indices, slot, ticket, status, event, redo)
     pend._keepalive = (q, filt, labels)        # the enqueued copies / kernels read them
     return pend.wait() if sync else pend
+
+
+class _PendingRefined:
+    """Handle of an asynchronous refined search: `wait()` finishes the candidate stage first; when that batch
+    was repeated on the exhaustive path, its candidates are refined again before the result is returned."""
+
+    def __init__(self, values, indices, cand, refine_again, status, event):
+        self.values, self.indices = values, indices
+        self._cand, self._again, self._status, self._event = cand, refine_again, status, event
+        self._done = False
+
+    def wait(self):
+        if not self._done:
+            self._event.synchronize()
+            self._cand.wait()
+            self._done = True
+            if self._cand.retried:
+                self._again()                    # the enqueued refine read the overflowed lists
+            else:
+                _cabi.check(_cabi.lib.mmrs_search_status(self._status.data_ptr()))
+        return self.values, self.indices
+
+
+def _search_refined(queries, gal: DeviceGallery, k, store, refine_k, normalize_queries, scale, path, sync, out,
+                    row_filter, label_kw):
+    """search_topk with a RefineStore: candidate stage, then mmrs_refine_topk on the same stream."""
+    from .refine import RefineStore, candidate_k
+    if not isinstance(store, RefineStore):
+        raise ValueError(f"refine must be a RefineStore, got {type(store).__name__}")
+    store.check_matches(gal)
+    q, on_host = _prep_queries(queries, gal)
+    nq = int(q.shape[0])
+    k = int(k)
+    if k < 1:
+        raise ValueError("k must be >= 1")
+    if k > gal.n_rows:
+        raise RuntimeError("selected index k out of range")
+    filt = _filter_arg(row_filter, gal)
+    allowed = None
+    if isinstance(filt, RowFilter):
+        allowed = filt.n_allowed
+    elif filt is not None:
+        allowed = int(filt.sum())
+    if allowed is not None and k > allowed:
+        raise RuntimeError("selected index k out of range")
+    k_c = candidate_k(k, refine_k, gal.n_rows, allowed)
+    dev = gal.device
+    if torch.cuda.current_device() != dev.index:
+        torch.cuda.set_device(dev)
+    stream = torch.cuda.current_stream(dev)
+    values, indices = _result_tensors(out, nq, k, on_host, dev)
+    if nq == 0:
+        return (values, indices) if sync else PendingSearch(values, indices, None, None, None, None, None)
+    qd = q.pin_memory().to(dev, non_blocking=True) if on_host else q      # [nq, gal.padded_dim] fp32
+    cand = search_topk(qd[:, :gal.dim], gal, k_c, normalize_queries=normalize_queries, scale=scale, path=path,
+                       sync=sync, row_filter=filt, **label_kw)
+    cand_idx = cand[1] if sync else cand.indices
+    dv, di = (torch.empty((nq, k), dtype=torch.float32, device=dev),
+              torch.empty((nq, k), dtype=torch.int64, device=dev)) if on_host else (values, indices)
+    lib = _cabi.lib
+    ws_bytes = lib.mmrs_refine_workspace_bytes(store.padded_dim, nq, k_c)
+    ws = gal.workspace(("refine", nq, k_c, stream.cuda_stream), ws_bytes)
+
+    def run(status_ptr: int):
+        local = cand_idx
+        if gal.row_offset:                       # a shard's candidates carry global rows: the store is local
+            local = torch.where(cand_idx >= 0, cand_idx - gal.row_offset, cand_idx)
+        _cabi.check(lib.mmrs_refine_topk(store.ptr, store.dtype_code, store.n_rows, store.padded_dim, store.ld,
+                                         qd.data_ptr(), nq, qd.stride(0), int(bool(normalize_queries)), float(scale),
+                                         local.data_ptr(), k_c, gal.row_offset, k, dv.data_ptr(), di.data_ptr(),
+                                         DeviceGallery.aligned_ptr(ws), ws_bytes, status_ptr, stream.cuda_stream))
+        if on_host:
+            values.copy_(dv, non_blocking=True)
+            indices.copy_(di, non_blocking=True)
+        return local
+
+    if sync:
+        run(0)
+        if on_host:
+            stream.synchronize()
+        return values, indices
+    status = torch.zeros(1, dtype=torch.int32).pin_memory()
+    local = run(status.data_ptr())
+    event = torch.cuda.Event()
+    event.record(stream)
+
+    def again():
+        with torch.cuda.stream(stream):
+            run(0)
+        stream.synchronize()
+
+    pend = _PendingRefined(values, indices, cand, again, status, event)
+    pend._keepalive = (qd, local, ws)            # the enqueued kernels read them
+    return pend
 
 
 def full_scores(queries, gallery: GalleryLike, *, normalize_queries: bool = True, scale: float = 1.0,

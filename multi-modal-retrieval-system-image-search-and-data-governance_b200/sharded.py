@@ -391,7 +391,8 @@ class ShardedGallery:
 
     def search_topk(self, queries: torch.Tensor, k: int, *, normalize_queries: bool = True,
                     scale: float = 1.0, path: str = "auto", sync: bool = True, out=None, row_filter=None,
-                    row_labels=None, query_labels=None, label_match: str = "same"):
+                    row_labels=None, query_labels=None, label_match: str = "same", refine=None,
+                    refine_k: Optional[int] = None):
         """Global top-k, identical on every rank.  `queries` must be the same on all ranks.
         `sync=False` returns an object whose `.wait()` yields `(values, indices)`, so that several
         batches (and their all-gathers) can be in flight.  `out=(values, indices)`: caller-owned result
@@ -399,9 +400,22 @@ class ShardedGallery:
         GLOBAL rows, the same on every rank like the queries; each rank searches its slice of it.
         `row_labels` (a RowLabels over the GLOBAL rows) / `query_labels` / `label_match`: label-conditioned
         search as in `search_topk`, the same on every rank (query labels replicated like the queries); a
-        query with fewer than k eligible rows over all shards is padded with -inf / -1."""
+        query with fewer than k eligible rows over all shards is padded with -inf / -1.
+        `refine` (this rank's RefineStore, over the rows of its shard) / `refine_k`: refined search as in
+        `search_topk` -- each rank takes min(refine_k, its rows, its allowed rows) candidates from its shard,
+        refines them to its local top-k, and the merge keeps the global top-k of those lists.  Refined calls
+        always take `search_topk_general` (the fused NVLink gather and the NCCL keys variant are not used)."""
         if k > self.n_rows_global:
             raise RuntimeError("selected index k out of range")
+        if refine is not None or refine_k is not None:
+            from .refine import default_refine_k
+            refine_k = default_refine_k(k) if refine_k is None else int(refine_k)
+            if refine_k < k:                  # every rank decides alike, before any collective
+                raise ValueError(f"refine_k = {refine_k} must be >= k = {k}")
+            out_t = self.search_topk_general(queries, k, normalize_queries=normalize_queries, scale=scale, path=path,
+                                             row_filter=row_filter, row_labels=row_labels, query_labels=query_labels,
+                                             label_match=label_match, refine=refine, refine_k=refine_k)
+            return out_t if sync else _PendingSharded(lambda: out_t, None)
         if isinstance(queries, np.ndarray):
             queries = torch.from_numpy(queries)
         labels = self._local_labels(row_labels, query_labels, label_match, queries)
@@ -443,12 +457,14 @@ class ShardedGallery:
 
     def search_topk_general(self, queries: torch.Tensor, k: int, *, normalize_queries: bool = True,
                             scale: float = 1.0, path: str = "auto", row_filter=None, row_labels=None,
-                            query_labels=None, label_match: str = "same"):
+                            query_labels=None, label_match: str = "same", refine=None,
+                            refine_k: Optional[int] = None):
         """(values, indices) lists, two all-gathers, merge -- also the path every rank takes together
         when some rank's candidate list overflowed (None from the fast path on EVERY rank alike: the
         shard statuses were gathered with the keys).  With a `row_filter` a rank searches for
         min(k, its allowed rows) and one without allowed rows skips its local search.  Labeled: positions
-        that no rank could fill hold -inf / -1, as on one GPU."""
+        that no rank could fill hold -inf / -1, as on one GPU.  `refine` / `refine_k` are handed to the local
+        search (see `search_topk`)."""
         if isinstance(queries, np.ndarray):
             queries = torch.from_numpy(queries)
         labels = self._local_labels(row_labels, query_labels, label_match, queries)
@@ -467,6 +483,8 @@ class ShardedGallery:
         kw = {} if local_filter is None else {"row_filter": local_filter}
         if labels is not None:
             kw.update(row_labels=labels[0], query_labels=labels[1], label_match=label_match)
+        if refine is not None or refine_k is not None:
+            kw.update(refine=refine, refine_k=refine_k)
         if local_filter is None or k_local > 0:
             v, i = self._search(queries, self.local, k_local, normalize_queries=normalize_queries,
                                 scale=scale, path=path, **kw)
